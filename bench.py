@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - aligned frames/s of the frame-alignment hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  The
 default workload ("align") is the north_star's "DFPN+CPN alignment of 5-frame
@@ -780,11 +780,16 @@ def run_gpu(args):
             ms = float(t.item())
         return ms
 
-    # the timed region is repeated until >= --min-ms of device time have been integrated (a 20-step run of a
-    # 100 us step is 2 ms: too short for the clock sampler and at the mercy of one stray interrupt); every
-    # repetition times exactly K steps, the reported one is the median
+    # by default the timed region is run once; with --min-ms it is repeated until that much device time has been
+    # integrated (a 20-step run of a 100 us step is 2 ms: too short for the clock sampler and at the mercy of one
+    # stray interrupt); every repetition times exactly K steps, the reported one is the median
     sampler = ClockSampler(local)
     sampler.start()
+    # one untimed pass over the same K steps first (counted in the line's "warmup"): after the --warmup steps, the
+    # first back-to-back pass still ran ~25 us slower in all, with or without the clock sampler (align, 20 steps on
+    # one B200 at 1000 W, two runs: 90.4 / 90.3 against medians of 89.0 / 89.1 us per step; after this pass the
+    # first timed pass ran at 89.1 / 89.0)
+    timed_round()
     first = timed_round()
     n_rounds = int(min(args.max_rounds, max(1, -(-args.min_ms // max(first, 1e-3)))))
     if world > 1:                 # every rank must run the same number of rounds (they contain barriers)
@@ -794,6 +799,14 @@ def run_gpu(args):
     rounds = [first] + [timed_round() for _ in range(n_rounds - 1)]
     ms = sorted(rounds)[len(rounds) // 2]
     value = wl.frames_per_step * world * K / (ms * 1e-3)
+    # the results of the last timed step (step K - 1 used input set (K - 1) % nsets), copied on the device before
+    # anything else runs; written out at the end so that the host work stays outside every timed region
+    last = None
+    if args.dump_outputs and rank == 0:
+        last, skipped = result_tensors(outs[nsets + (K - 1) % nsets] if graphs else outs[(K - 1) % nsets])
+        last = {k: t.detach().clone() for k, t in last.items()}
+        if skipped:
+            log("--dump-outputs: not tensors, not written:", ", ".join(skipped))
 
     # one more repetition of the same K steps, instrumented: one event after every C-ABI call (individual
     # launches instead of the graph replay, so each interval also carries the launch gap that back-to-back
@@ -878,7 +891,7 @@ def run_gpu(args):
 
     line = {
         "metric": "aligned_frames_per_sec", "value": value, "unit": "frames/s", "n_gpus": world,
-        "steps": K, "warmup": max(args.warmup, 3), "ms_per_step": ms / K, "higher_is_better": True,
+        "steps": K, "warmup": max(args.warmup, 3) + K, "ms_per_step": ms / K, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": wl.describe, "frames_per_step_per_gpu": wl.frames_per_step,
                    "l2": "inputs rotate over %d buffer sets; %.0f MB algorithmic traffic per step, "
@@ -887,8 +900,9 @@ def run_gpu(args):
                    "sharding": "shard.batch_shard: contiguous blocks of %d of the job's %d samples per rank, %d ranks, "
                                "no data-path collective" % (wl.b, wl.b * world, world),
                    "launch": "CUDA graph replay per step" if graphs else "one C-ABI call per kernel group",
-                   "timed_region": "%d repetitions of exactly %d steps (barrier + sync around each); value = "
-                                   "the median repetition" % (len(rounds), K)},
+                   "timed_region": "%d repetitions of exactly %d steps (barrier + sync around each) after %d warm-up "
+                                   "steps and one untimed pass of the %d steps (\"warmup\" counts both); value = the "
+                                   "median repetition" % (len(rounds), K, max(args.warmup, 3), K)},
         "rounds_ms": {"n": len(rounds), "min": min(rounds), "median": ms, "max": max(rounds),
                       "integrated_ms": sum(rounds), "instrumented": ms_instr},
         "clocks": clocks, "e2e": e2e, "host_affinity": affinity, "gpu_launches": launches_per_step * K,
@@ -936,11 +950,58 @@ def run_gpu(args):
             "value": v, "unit": "frames/s", "cores": cores, "kind": "port",
             "sample": "%s at batch_size=%d: %d reps of %.3f s (torch %s CPU port of the reference "
                       "call sequence)" % (wl.name, sample.b, reps, mean, torch.__version__)}
+    if last is not None:
+        line["dumped_outputs"] = dump_outputs(last, args.dump_outputs)
     if rank == 0:
         OUT.emit(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_BYTES = 60_000_000      # all .npy files of --dump-outputs together (the limit is 64 MB; headroom for headers)
+
+
+def result_tensors(step_out):
+    """The tensors of a step's result dict by name: a tuple or list entry (cfg5's "keep", the intermediates its step
+    also returns) becomes <name>_<i>.  Returns (tensors, names of the entries that are not tensors)."""
+    import torch
+    tensors, skipped = {}, []
+    for k, v in step_out.items():
+        for name, t in ([("%s_%d" % (k, i), e) for i, e in enumerate(v)] if isinstance(v, (tuple, list))
+                        else [(k, v)]):
+            if isinstance(t, torch.Tensor):
+                tensors[name] = t
+            else:
+                skipped.append(name)
+    return tensors, skipped
+
+
+def dump_outputs(tensors, directory):
+    """Writes every tensor as <directory>/<name>.npy: float64 for 64-bit floats and for integers (exact), float32
+    otherwise.  The byte budget is shared out from the smallest array up; an array larger than its share is
+    replaced by a fixed sample of its elements: the flattened array at the sorted indices that
+    numpy.random.default_rng(0) draws without replacement, so two runs on the same shapes sample the same
+    elements.  Returns {name: [shape, number of elements written]}."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    written, left = {}, DUMP_BYTES
+    items = sorted(tensors.items(), key=lambda kv: (kv[1].numel(), kv[0]))
+    for i, (name, t) in enumerate(items):
+        wide = t.dtype == torch.float64 or not (t.is_floating_point() or t.dtype == torch.bool)
+        dtype = torch.float64 if wide else torch.float32
+        share = left // (len(items) - i) // (8 if wide else 4)
+        if t.numel() > share:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), share, replace=False))
+            t_out = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        else:
+            t_out = t
+        a = t_out.to(dtype).cpu().numpy()
+        np.save(os.path.join(directory, name + ".npy"), a)
+        left -= a.nbytes
+        written[name] = [list(t.shape), int(a.size)]
+    return written
 
 
 def run_e2e(args, wl, mtb, ops, host, dev, world):
@@ -1058,8 +1119,9 @@ def main():
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="align", choices=sorted(WORKLOADS))
-    ap.add_argument("--min-ms", type=float, default=60.0,
-                    help="repeat the timed region of exactly --steps steps until this much device time is integrated")
+    ap.add_argument("--min-ms", type=float, default=0.0,
+                    help="repeat the timed region of exactly --steps steps until this much device time is integrated "
+                         "and report the median repetition (default: one timed region)")
     ap.add_argument("--max-rounds", type=int, default=400)
     ap.add_argument("--ddp-mb", type=float, default=-1.0,
                     help="N > 1: all-reduce a gradient-sized fp32 buffer of this many MB next to every step (NCCL); "
@@ -1072,7 +1134,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", dest="graph", action="store_false",
                     help="issue every step as individual C-ABI calls instead of a CUDA graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (rank 0; at most 64 MB in all, "
+                         "larger results as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; --impl reference runs a smaller batch on the CPU")
     if args.gpus > 1 and "RANK" not in os.environ and args.impl != "reference":
         # convenience: re-launch under torchrun (the driver launches torchrun itself)
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1",
