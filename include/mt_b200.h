@@ -346,6 +346,36 @@ MT_API int mt_flow_pack(const float *x_refs, int64_t xr_sb, int64_t xr_sc, int64
                  const float *flow, int64_t fl_sb, int64_t fl_sf, int64_t fl_sy, int64_t fl_sx, int64_t fl_sc,
                  float *nn_in, int B, int F, int H, int W, mt_stream_t stream);
 
+/* ---- F5  resampling of DFPN's training step -----------------------------------
+ * Bit-identical to torch's CPU F.interpolate (align_corners=False; legacy 'nearest').
+ * mt_resize_set       replaces TransformsUtils.resize_set utils.py:522-560, called at
+ *                     model_dfpn.py:350-351 (sizes 16 and 64)
+ *   x, y (B,C,F,H,W), v (B,1,F,H,W) strided with contiguous planes -> x_s, y_s (bilinear) and
+ *   v_s (nearest), each written frame-major: contiguous (B,F,C|1,size,size) memory, which is the
+ *   memory of the reference's `.reshape(b, f, ch, s, s).transpose(1, 2)` result.  No transpose copy.
+ * mt_resize_flow      replaces FlowsUtils.resize_flow utils.py:107-126, called at
+ *                     model_dfpn.py:86,93 (bilinear) and :354-355 (nearest)
+ *   flow (B,F,h,w,2) with ALL five strides -> out (B,F,H,W,2) through its five strides (the reference
+ *   returns planar (B,F,2,H,W) memory for a planar input and interleaved memory for an interleaved one).
+ *   mode: MT_RESIZE_NEAREST or MT_RESIZE_BILINEAR.
+ * mt_resize_flow_bwd  gradient of the bilinear mode w.r.t. the input flow (autograd of utils.py:121)
+ *   g_out (B,F,H,W,2) strided -> g_flow (B,F,2,h,w) contiguous.  A gather without atomics: every input
+ *   pixel sums its output pixels in a fixed order, so two runs are bitwise equal.
+ */
+#define MT_RESIZE_NEAREST 0
+#define MT_RESIZE_BILINEAR 1
+MT_API int mt_resize_set(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                  const float *v, int64_t v_sb, int64_t v_sf,
+                  const float *y, int64_t y_sb, int64_t y_sc, int64_t y_sf,
+                  float *x_s, float *v_s, float *y_s,
+                  int B, int C, int F, int H, int W, int size, mt_stream_t stream);
+MT_API int mt_resize_flow(const float *flow, int64_t sb, int64_t sf, int64_t sy, int64_t sx, int64_t sc,
+                   float *out, int64_t o_sb, int64_t o_sf, int64_t o_sy, int64_t o_sx, int64_t o_sc,
+                   int B, int F, int h, int w, int H, int W, int mode, mt_stream_t stream);
+MT_API int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
+                       int64_t g_sc, float *g_flow, int B, int F, int h, int w, int H, int W,
+                       mt_stream_t stream);
+
 /* ---- host-buffer entry points (end-to-end: H2D + kernels + D2H inside) ----
  * The reference-facing calls with HOST memory, used for the e2e metric.
  * All pointers are host pointers (pinned memory recommended); tensors are

@@ -846,3 +846,94 @@ def flow_pack(x_target, m_target, x_refs, m_refs, flow_pre):
     if torch.is_grad_enabled() and flow_pre.requires_grad:
         return FlowPackFn.apply(flow_pre, x_target, m_target, x_refs, m_refs)
     return flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre)
+
+
+# --------------------------------------------------------------------------
+# F5 resampling of DFPN's training step
+# --------------------------------------------------------------------------
+RESIZE_MODES = {"nearest": 0, "bilinear": 1}
+
+
+def resize_set(x, v, y, size):
+    """TransformsUtils.resize_set (utils.py:522-560): x, y (B,C,F,H,W) bilinear and v (B,1,F,H,W) nearest to
+    (size, size), in one launch.  Returns (x_s, v_s, y_s), (B,C|1,F,size,size) views of frame-major memory: the
+    shapes and strides of the reference's ``.reshape(b, f, ch, s, s).transpose(1, 2)``.  No backward (the
+    reference resizes data)."""
+    _need_cuda(x, v, y)
+    _no_grad_inputs("resize_set", x, v, y)
+    b, c, f, h, w = x.shape
+    if tuple(y.shape) != (b, c, f, h, w) or tuple(v.shape) != (b, 1, f, h, w):
+        raise ValueError("resize_set: x, y (B,C,F,H,W) and v (B,1,F,H,W) expected, got %s, %s, %s"
+                         % (tuple(x.shape), tuple(v.shape), tuple(y.shape)))
+    size = int(size)
+    x, x_sb, x_sc, x_sf = _s5(x)
+    v, v_sb, _, v_sf = _s5(v)
+    y, y_sb, y_sc, y_sf = _s5(y)
+    xs_mem, xs = _frame_major(b, c, f, size, size, x)
+    vs_mem, vs = _frame_major(b, 1, f, size, size, x)
+    ys_mem, ys = _frame_major(b, c, f, size, size, x)
+    _call("mt_resize_set", _ptr(x), x_sb, x_sc, x_sf, _ptr(v), v_sb, v_sf, _ptr(y), y_sb, y_sc, y_sf,
+          _ptr(xs_mem), _ptr(vs_mem), _ptr(ys_mem), b, c, f, h, w, size, _stream(x))
+    return xs, vs, ys
+
+
+def _flow_size(size):
+    return (int(size), int(size)) if isinstance(size, int) else (int(size[0]), int(size[1]))
+
+
+def resize_flow_raw(flow, size, mode):
+    """mt_resize_flow without autograd: flow (B,F,h,w,2), read through its five strides, -> (B,F,H,W,2) in the
+    memory layout the reference returns: its ``flow.reshape(b * f, h, w, 2).permute(0, 3, 1, 2)`` is channels-last
+    for an interleaved flow and after the copy ``reshape`` makes when (B, F) do not merge, and F.interpolate keeps
+    that layout (interleaved (B,F,H,W,2) memory); otherwise the result is planar (B,F,2,H,W) memory."""
+    _need_cuda(flow)
+    if flow.dim() != 5 or flow.shape[4] != 2:
+        raise ValueError("resize_flow: flow (B,F,h,w,2) expected, got %s" % (tuple(flow.shape),))
+    b, f, h, w, _ = flow.shape
+    H, W = _flow_size(size)
+    fs = flow.stride()
+    merges = b == 1 or f == 1 or fs[0] == f * fs[1]
+    if not merges or fs[4] < fs[3]:
+        out = _empty((b, f, H, W, 2), dtype=torch.float32, device=flow.device)
+    else:
+        out = _empty((b, f, 2, H, W), dtype=torch.float32, device=flow.device).permute(0, 1, 3, 4, 2)
+    _call("mt_resize_flow", _ptr(_lib.keep(flow)), *fs, _ptr(out), *out.stride(), b, f, h, w, H, W,
+          RESIZE_MODES[mode], _stream(flow))
+    return out
+
+
+def resize_flow_bwd_raw(g_out, h, w):
+    """mt_resize_flow_bwd: d loss / d flow (B,F,h,w,2) of the bilinear resize, as a view of planar memory."""
+    _need_cuda(g_out)
+    b, f, H, W, _ = g_out.shape
+    g_flow = _empty((b, f, 2, h, w), dtype=torch.float32, device=g_out.device)
+    _call("mt_resize_flow_bwd", _ptr(_lib.keep(g_out)), *g_out.stride(), _ptr(g_flow), b, f, h, w, H, W,
+          _stream(g_out))
+    return g_flow.permute(0, 1, 3, 4, 2)
+
+
+class ResizeFlowFn(torch.autograd.Function):
+    """FlowsUtils.resize_flow(flow, size, 'bilinear') with autograd w.r.t. ``flow`` (deterministic gather)."""
+
+    @staticmethod
+    def forward(ctx, flow, size):
+        ctx.hw = flow.shape[2:4]
+        return resize_flow_raw(flow.detach(), size, "bilinear")
+
+    @staticmethod
+    def backward(ctx, g):
+        if not ctx.needs_input_grad[0]:
+            return None, None
+        return resize_flow_bwd_raw(g.to(torch.float32), *ctx.hw), None
+
+
+def resize_flow(flow, size, mode="nearest"):
+    """FlowsUtils.resize_flow (utils.py:107-126): (B,F,h,w,2) -> (B,F,H,W,2), mode 'nearest' or 'bilinear'
+    (align_corners=False); differentiable w.r.t. ``flow`` in the bilinear mode."""
+    if mode not in RESIZE_MODES:
+        raise ValueError("resize_flow: mode must be one of %s, got %r" % (sorted(RESIZE_MODES), mode))
+    if torch.is_grad_enabled() and flow.requires_grad:
+        if mode != "bilinear":
+            _no_grad_inputs("resize_flow(mode='nearest')", flow)
+        return ResizeFlowFn.apply(flow, size)
+    return resize_flow_raw(flow, size, mode)

@@ -17,6 +17,21 @@ import torch.nn as nn
 from . import ops
 
 
+def _cuda_fp32(*ts):
+    return all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 for t in ts)
+
+
+def _reference_original(cls, attr):
+    """The reference's own ``cls.attr``, saved by ``patch()``: the resampling mirrors hand it every call their
+    kernels do not serve (the reference's dataset code calls the same helpers on host tensors)."""
+    import master_thesis as mt
+    fn = getattr(getattr(mt, cls), "_mt_b200_orig_" + attr, _ABSENT)
+    if fn is _ABSENT:
+        raise RuntimeError("master_thesis_b200: %s.%s got a call its kernel does not serve (host or non-fp32 "
+                           "tensors, another mode, or a gradient) and no original was saved by patch()" % (cls, attr))
+    return fn
+
+
 class FlowsUtils:
     """Mirror of master_thesis.utils.FlowsUtils (hot-path members only)."""
 
@@ -25,6 +40,31 @@ class FlowsUtils:
         """utils.py:78-104.  x (B,C,F,H,W), v (B,1,F,H,W), flow (B,F,H,W,2) ->
         (x_aligned (B,C,F,H,W), v_aligned (B,1,F,H,W)); differentiable w.r.t. flow."""
         return ops.align_set(x, v, flow)
+
+    @staticmethod
+    def resize_flow(flow, size, mode='nearest'):
+        """utils.py:107-126.  flow (B,F,h,w,2) -> (B,F,H,W,2), F.interpolate 'nearest' or 'bilinear'
+        (align_corners=False), bit-identical; differentiable w.r.t. flow in the bilinear mode.  CUDA fp32 flows in
+        those two modes (and nearest without a gradient) run on the kernel, anything else on the reference's own
+        function."""
+        grad = torch.is_grad_enabled() and isinstance(flow, torch.Tensor) and flow.requires_grad
+        if _cuda_fp32(flow) and (mode == 'bilinear' or (mode == 'nearest' and not grad)):
+            return ops.resize_flow(flow, size, mode)
+        return _reference_original("FlowsUtils", "resize_flow")(flow, size, mode)
+
+
+class TransformsUtils:
+    """Mirror of master_thesis.utils.TransformsUtils (the member DFPN's training step calls)."""
+
+    @staticmethod
+    def resize_set(x, v, y, size):
+        """utils.py:522-560.  x, y (B,C,F,H,W) bilinear and v (B,1,F,H,W) nearest to (size, size), bit-identical,
+        one launch, no transpose copies.  CUDA fp32 inputs without a gradient run on the kernel, anything else on
+        the reference's own function."""
+        grad = torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (x, v, y))
+        if _cuda_fp32(x, v, y) and not grad:
+            return ops.resize_set(x, v, y, size)
+        return _reference_original("TransformsUtils", "resize_set")(x, v, y, size)
 
 
 class LossesUtils:
@@ -419,6 +459,8 @@ _ABSENT = object()      # marker: the attribute did not exist before patch() (he
 _PATCHES = (
     # (module path, class, attribute, replacement, static?)
     ("utils", "FlowsUtils", "align_set", FlowsUtils.align_set, True),
+    ("utils", "FlowsUtils", "resize_flow", FlowsUtils.resize_flow, True),
+    ("utils", "TransformsUtils", "resize_set", TransformsUtils.resize_set, True),
     ("utils", "LossesUtils", "masked_l1", LossesUtils.masked_l1, True),
     ("model_dfpn", "CorrelationVGG", "correlation_masked_4d",
      CorrelationVGG.correlation_masked_4d, True),
