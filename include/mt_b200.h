@@ -235,6 +235,33 @@ MT_API int mt_chn_fill_step_gated(const float *nn_out, const float *x_t, int64_t
                            float *y_comp0, float *m_new, float *x_new,
                            float *inp_per, void *workspace, int B, int64_t P, mt_stream_t stream);
 
+/* mt_chn_fill_lanes: the composite + hole update of mt_chn_fill_step for L independent target frames of a clip
+ * ("lanes") in one launch, each with its own hole percentage: the batched form of the inference loops of
+ * CHN.inpaint_ff (model_chn.py:111-131) and CHN.inpaint_cp (model_chn.py:225-248), where every target of a round
+ * (ff) or of a pass's parity group (cp) reads only frames no other target of the round writes.
+ *   nn_out (L,3,P) contiguous; x_t (L,3,P) strided (xt_sl, xt_sc); m_t, v_map0 (L,1,P) strided (mt_sl, vm_sl);
+ *   v_t = 1 - m_t is formed on load.  All planes contiguous.
+ *   slots (L) int32 on the device: lane i writes state slot slots[i]; the slots must be unique (lanes write in
+ *   place).  Outputs through the slot table, strided: y_out[slot] (yo_ss, yo_sc) = y_comp (:83-84),
+ *   m_state[slot] (ms_ss) = m_new = m_t - v_map0 (:128), x_state[slot] (xs_ss, xs_sc) = x_new (:129-130),
+ *   per_out[slot] = (float)sum(m_new of the lane) * 100 / P (:131) - for every lane bit-identical to
+ *   mt_chn_fill_step at B = 1 on that lane's slice ({0,1} masks: the fold order cannot change the sum).
+ *   In place: x_t / m_t may alias x_state[slot] / m_state[slot]; no output may alias nn_out.
+ *   finalize != 0 (CHN.inpaint_cp, model_chn.py:246-248): a lane with (double)per_out[slot] < e, or every lane
+ *   when force != 0 (the last two passes, i >= N - 2), ends with m_state[slot] = 0 and x_state[slot] = y_comp.
+ *   The comparison is made on the device after the lane's reduction (a second launch, chained with PDL, rewrites
+ *   only the flagged lanes); force is applied by the first launch itself.  No host synchronisation.
+ *   workspace: at least mt_chn_fill_lanes_workspace_bytes(L) bytes on the current device, zero-initialised once.
+ *   The lane tickets sit at a fixed offset sized for the largest L (65535), so one buffer serves calls with any
+ *   lane count in any order; every call re-arms the tickets it used.  1 <= L <= 65535. */
+MT_API int mt_chn_fill_lanes(const float *nn_out, const float *x_t, int64_t xt_sl, int64_t xt_sc,
+                      const float *m_t, int64_t mt_sl, const float *v_map0, int64_t vm_sl,
+                      const int *slots, float *y_out, int64_t yo_ss, int64_t yo_sc,
+                      float *m_state, int64_t ms_ss, float *x_state, int64_t xs_ss, int64_t xs_sc,
+                      float *per_out, void *workspace, int L, int64_t P,
+                      int finalize, double e, int force, mt_stream_t stream);
+MT_API int64_t mt_chn_fill_lanes_workspace_bytes(int L);
+
 /* ---- K2  masked cosine correlation on tcgen05 ----------------------------
  * replaces CorrelationVGG.correlation_masked_4d  model_dfpn.py:534-565  (a7)
  * feats_t (B,C,P) contiguous, v_t (B,P) or NULL, feats_r (B,C,F,P) contiguous,

@@ -19,12 +19,14 @@ _CTYPES = {
     "int": ctypes.c_int,
     "int64_t": ctypes.c_int64,
     "float": ctypes.c_float,
+    "double": ctypes.c_double,
     "mt_stream_t": ctypes.c_void_p,
     "void *": ctypes.c_void_p,
     "const void *": ctypes.c_void_p,
     "float *": ctypes.c_void_p,
     "const float *": ctypes.c_void_p,
     "const uint8_t *": ctypes.c_void_p,
+    "const int *": ctypes.c_void_p,
     "int *": ctypes.POINTER(ctypes.c_int),
     "const char *": ctypes.c_char_p,
 }

@@ -791,6 +791,69 @@ def chn_fill(nn_out, x_t, v_t, m_t, v_map0, gate=None):
     return yc, m_new, x_new, per[0]
 
 
+def index_tensor(values, device, dtype=torch.int64):
+    """A host list of integers on the device, copied from pinned memory without synchronising the host (a plain
+    ``torch.tensor(values, device=...)`` waits for the stream to drain)."""
+    return torch.tensor(values, dtype=dtype).pin_memory().to(device, non_blocking=True)
+
+
+def _lane_slots(slots, lanes, n_slots):
+    """The host-side slot table of chn_fill_lanes, checked before anything is launched: one slot per lane, each in
+    range, none repeated (two lanes on one slot would race on the in-place state writes)."""
+    slots = [int(s) for s in slots]
+    if len(slots) != lanes:
+        raise ValueError("chn_fill_lanes: %d slots for %d lanes" % (len(slots), lanes))
+    bad = [s for s in slots if not 0 <= s < n_slots]
+    if bad:
+        raise ValueError("chn_fill_lanes: slots %s out of range [0, %d)" % (bad, n_slots))
+    if len(set(slots)) != len(slots):
+        raise ValueError("chn_fill_lanes: duplicate slots %s (lanes write their state in place)" % sorted(slots))
+    return slots
+
+
+def _out_planes(t, who):
+    """Outputs are written where they are: a plane that is not contiguous is an error, not a copy."""
+    h, w = t.shape[-2:]
+    if (w > 1 and t.stride(-1) != 1) or (h > 1 and t.stride(-2) != w):
+        raise RuntimeError("chn_fill_lanes: %s needs contiguous (H, W) planes" % who)
+    return t
+
+
+def chn_fill_lanes(nn_out, x_t, m_t, v_map0, slots, x_state, m_state, y_out, per_out, finalize=None):
+    """mt_chn_fill_lanes: composite (model_chn.py:83-84) + hole update (:128-131) of L independent F = 1 steps, one
+    target frame per lane, with a hole percentage per lane.  nn_out (L,3,H,W); x_t (L,3,H,W), m_t and v_map0
+    (L,1,H,W), strided with contiguous planes (v_t = 1 - m_t is formed in the kernel).  ``slots``: a host list,
+    lane i writes state slot slots[i] of x_state (S,3,H,W) (x_new), m_state (S,1,H,W) (m_new), y_out (S,3,H,W)
+    (y_comp) and per_out (S,) (inp_per), all in place and strided.  x_t / m_t may be views of the state slots
+    they update.  ``finalize = (e, force)``: CHN.inpaint_cp's `if float(per) < e or force: m = 0, y = y_comp`
+    (model_chn.py:246-248) per lane, decided on the device.  Nothing is returned; nothing synchronises."""
+    lanes, n_slots = nn_out.shape[0], x_state.shape[0]
+    slots = _lane_slots(slots, lanes, n_slots)
+    _need_cuda(nn_out, x_t, m_t, v_map0, x_state, m_state, y_out, per_out)
+    _no_grad_inputs("chn_fill_lanes", nn_out, x_t, m_t, v_map0)
+    h, w = x_t.shape[-2:]
+    want = {"nn_out": (nn_out, (lanes, 3, h, w)), "x_t": (x_t, (lanes, 3, h, w)), "m_t": (m_t, (lanes, 1, h, w)),
+            "v_map0": (v_map0, (lanes, 1, h, w)), "x_state": (x_state, (n_slots, 3, h, w)),
+            "m_state": (m_state, (n_slots, 1, h, w)), "y_out": (y_out, (n_slots, 3, h, w)),
+            "per_out": (per_out, (n_slots,))}
+    for name, (t, shape) in want.items():
+        if tuple(t.shape) != shape:
+            raise ValueError("chn_fill_lanes: %s must be %s, got %s" % (name, shape, tuple(t.shape)))
+    if not per_out.is_contiguous():
+        raise RuntimeError("chn_fill_lanes: per_out must be contiguous")
+    no, xt, mt, vm = _contig(nn_out), _planes(x_t), _planes(m_t), _planes(v_map0)
+    xs, ms, yo = _out_planes(x_state, "x_state"), _out_planes(m_state, "m_state"), _out_planes(y_out, "y_out")
+    sl = _lib.keep(index_tensor(slots, no.device, torch.int32))
+    e, force = (1.0, False) if finalize is None else (float(finalize[0]), bool(finalize[1]))
+    with torch.cuda.device(no.device):      # the size depends on the SM count of the launching device
+        nbytes = int(_lib.load().mt_chn_fill_lanes_workspace_bytes(lanes))
+    ws = zeroed_scratch(no, "lanes", nbytes)
+    _call("mt_chn_fill_lanes", _ptr(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(mt), mt.stride(0), _ptr(vm),
+          vm.stride(0), _ptr(sl), _ptr(yo), yo.stride(0), yo.stride(1), _ptr(ms), ms.stride(0), _ptr(xs),
+          xs.stride(0), xs.stride(1), _ptr(per_out), _ptr(ws), lanes, h * w, int(finalize is not None), e,
+          int(force), _stream(no))
+
+
 def trivial_copy(x_t, x_al, v_map):
     """model_dfpn.py:427-429."""
     _need_cuda(x_t, x_al, v_map)

@@ -396,9 +396,69 @@ def _fill_loop(chn, cands, x_t, m_t, ref_of, e):
     return y_comp, m_t, x_t
 
 
-def chn_inpaint_ff(self, x, m, s=1, D=20, e=1):
-    """Replaces CHN.inpaint_ff (model_chn.py:87-133).  x (C,F,H,W), m (1,F,H,W)."""
+def _batch_frames(chn):
+    """Target frames in flight in the patched inpaint_ff / inpaint_cp: attribute ``mt_b200_batch_frames`` of the CHN
+    module, else $MT_INPAINT_BATCH_FRAMES, else 1 (one target frame and one reference per fill step, the reference's
+    loops).  With L > 1 up to L independent target frames share every fill step (``_lanes_step``); this bounds the
+    batch of the CNNs and their activation memory.  Opt-in because the reference's CNNs (the DFPN / CPN forward and
+    the RRDBNet) then see L frames per call, and cuDNN does not promise results that are independent of the batch."""
+    import os
+    return max(1, int(getattr(chn, "mt_b200_batch_frames", os.environ.get("MT_INPAINT_BATCH_FRAMES", "1"))))
+
+
+def _lanes_grid(chn, n):
+    """The aligner's grid function if the batched loops apply: batch size above 1, a patched DFPN / CPN aligner (the
+    two-kernel step) and a clip of n >= 2 frames; else None (the one-frame-at-a-time loops)."""
+    if n < 2 or _batch_frames(chn) < 2:
+        return None
+    fn = getattr(type(chn.model_aligner), "align", None)
+    return _dfpn_grid if fn is dfpn_align else (_cpn_grid if fn is cpn_align else None)
+
+
+def _lanes_step(chn, grid_fn, x_t, m_t, x_ref, m_ref, slots, x_state, m_state, y_out, per, finalize=None):
+    """_fill_step's two-kernel route for L independent target frames (lanes) at once: one aligner call, one warp +
+    CNN-input pack and one RRDBNet call on L rows, then ops.chn_fill_lanes, which writes y_comp, the new state and
+    the hole percentage of lane i into slot ``slots[i]`` of y_out / x_state / m_state / per, in place."""
+    grid, flags = grid_fn(chn.model_aligner, x_t, m_t, x_ref, m_ref)
+    nn_in, v_map, _, _ = ops.warp_pack_fwd(x_ref, m_ref, grid, m_t, x_t, 1 - m_t, flags)
+    ops.chn_fill_lanes(chn.nn(nn_in), x_t, m_t, v_map[:, :, 0], slots, x_state, m_state, y_out, per, finalize)
+
+
+def _inpaint_ff_lanes(chn, grid_fn, x, m, s, D, e, lanes):
+    """CHN.inpaint_ff (model_chn.py:87-133) with up to ``lanes`` target frames per fill step.  Every target reads
+    only the original clip, so the targets are independent: each round, every active target takes its next
+    candidate (its first step is unconditional, as in _fill_loop), and after ONE host read of the round's
+    percentages the targets whose `inp_per > e` failed or whose candidates ran out retire and pending targets
+    take their lanes.  Frame by frame the steps are those of the sequential loop."""
     n = x.size(1)
+    xs, ms = x.clone(), m.clone()
+    x_state, m_state = xs.transpose(0, 1), ms.transpose(0, 1)          # (n,3,H,W), (n,1,H,W): slot = target frame
+    y_inpainted = torch.zeros_like(x)
+    per = torch.empty(n, dtype=torch.float32, device=x.device)
+    pending, active = list(range(n)), []
+    while pending or active:
+        while pending and len(active) < lanes:
+            t = pending.pop(0)
+            active.append((t, type(chn).get_indexes_ff(t, n, s=s, D=D)))
+        tgt = [t for t, _ in active]
+        idx = ops.index_tensor(tgt + [cands.pop(0) for _, cands in active], x.device)
+        ti, ri = idx[:len(tgt)], idx[len(tgt):]
+        x_ref = x.index_select(1, ri).transpose(0, 1).unsqueeze(2)     # (L,3,1,H,W)
+        m_ref = m.index_select(1, ri).transpose(0, 1).unsqueeze(2)
+        _lanes_step(chn, grid_fn, x_state.index_select(0, ti), m_state.index_select(0, ti), x_ref, m_ref, tgt,
+                    x_state, m_state, y_inpainted.transpose(0, 1), per)
+        go = per.index_select(0, ti).tolist()       # the only device->host synchronisation of a round
+        active = [(t, cands) for (t, cands), p in zip(active, go) if len(cands) > 0 and p > e]
+    return y_inpainted
+
+
+def chn_inpaint_ff(self, x, m, s=1, D=20, e=1):
+    """Replaces CHN.inpaint_ff (model_chn.py:87-133).  x (C,F,H,W), m (1,F,H,W).  See _batch_frames for the
+    batched form."""
+    n = x.size(1)
+    grid_fn = _lanes_grid(self, n)
+    if grid_fn is not None:
+        return _inpaint_ff_lanes(self, grid_fn, x, m, s, D, e, _batch_frames(self))
     y_inpainted = torch.zeros_like(x)
     for t in range(n):
         cands = type(self).get_indexes_ff(t, n, s=s, D=D)
@@ -424,8 +484,41 @@ def chn_inpaint_ip(self, x, m, s=1, D=20, e=1):
     return y_inp[0]
 
 
+def _inpaint_cp_lanes(chn, grid_fn, x, m, N, s, e, lanes):
+    """CHN.inpaint_cp (model_chn.py:191-254) with up to ``lanes`` target frames per fill step.  The targets of a pass
+    form one parity group and their references t +- s lie in another group, so no target reads a frame another
+    target of the pass writes.  Per pass: ONE host read of which targets still have a hole (for {0,1} masks the
+    batched sum == 0 is the reference's per-frame check), then chunks of up to ``lanes`` targets, each the `dt = -s`
+    step on the lanes with a reference before them and the `+s` step on those with one after; the finalisation
+    (`per < e` or the last two passes) is decided on the device.  The clip is updated in place, as in the reference."""
+    n = x.size(1)
+    x_state, m_state = x.transpose(0, 1), m.transpose(0, 1)            # views of the clip: (n,3,H,W), (n,1,H,W)
+    y_comp = torch.empty_like(x_state)
+    per = torch.empty(n, dtype=torch.float32, device=x.device)
+    for i in range(N):
+        group = [k for k in range(n) if (k // s) % (s if s > 1 else 2) == i % 2]
+        if not group:
+            continue
+        holes = m_state.index_select(0, ops.index_tensor(group, x.device)).sum((1, 2, 3)) != 0
+        targets = [t for t, hole in zip(group, holes.tolist()) if hole]   # the only host sync of a pass
+        for c0 in range(0, len(targets), lanes):
+            for dt in (-s, s):
+                tgt = [t for t in targets[c0:c0 + lanes] if 0 <= t + dt < n]
+                if not tgt:
+                    continue
+                idx = ops.index_tensor(tgt + [t + dt for t in tgt], x.device)
+                ti, ri = idx[:len(tgt)], idx[len(tgt):]
+                _lanes_step(chn, grid_fn, x_state.index_select(0, ti), m_state.index_select(0, ti),
+                            x_state.index_select(0, ri).unsqueeze(2), m_state.index_select(0, ri).unsqueeze(2),
+                            tgt, x_state, m_state, y_comp, per, (e, i >= N - 2))
+    return x
+
+
 def chn_inpaint_cp(self, x, m, N=20, s=1, e=1):
-    """Replaces CHN.inpaint_cp (model_chn.py:191-254)."""
+    """Replaces CHN.inpaint_cp (model_chn.py:191-254).  See _batch_frames for the batched form."""
+    grid_fn = _lanes_grid(self, x.size(1))
+    if grid_fn is not None:
+        return _inpaint_cp_lanes(self, grid_fn, x, m, N, s, e, _batch_frames(self))
     y_inp, m_inp = x.unsqueeze(0), m.unsqueeze(0)
     n = y_inp.size(2)
     for i in range(N):
