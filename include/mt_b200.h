@@ -55,6 +55,15 @@ typedef void *mt_stream_t; /* cudaStream_t */
 #define MT_REDUCE_MEAN 0
 #define MT_REDUCE_SUM 1
 
+/* element type of a network operand in the *_dt entry points (the CNN output of CHN.forward, the inputs of
+ * LossesUtils.masked_l1): under autocast (`--precision 16|bf16`, __main__.py:69) the RRDBNet and the Sobel convs of
+ * LossesUtils.grad hand over fp16 / bf16 tensors.  The kernels widen them to fp32 on load (exact) and compute in
+ * fp32 exactly as the fp32 entry points do; a gradient w.r.t. such an operand is stored in its dtype, rounded to
+ * nearest even (what autograd returns for a half input whose fp32 use produced an fp32 gradient). */
+#define MT_DT_F32 0
+#define MT_DT_F16 1
+#define MT_DT_BF16 2
+
 MT_API int mt_version(void);
 MT_API const char *mt_last_error(void);
 /* developer knob (tests, sweeps): overrides one of the MT_* tuning variables the library
@@ -189,6 +198,25 @@ MT_API int mt_masked_l1_bwd(const float *y_hat, int64_t a_sb, int64_t a_sc, int6
                      int B, int C, int F, int64_t P, int mask_c, int reduction, float weight,
                      mt_stream_t stream);
 
+/* mt_masked_l1_fwd / _bwd with a dtype code (MT_DT_*) per operand           utils.py:139-169, 166 under autocast
+ * (l1_loss is on autocast's fp32 list; LossesUtils.grad, utils.py:194-224, passes its Sobel-conv outputs at :221).
+ * y_hat and y may each be fp32, fp16 or bf16; the mask (m_dtype) is fp32 or a {0,1} mask in the dtype of y_hat.
+ * Arithmetic, reductions and out3 are those of mt_masked_l1_fwd on the widened operands; grad_y_hat / grad_y are
+ * written in the dtypes of y_hat / y.  The fp32 entry points are these with MT_DT_F32 everywhere. */
+MT_API int mt_masked_l1_fwd_dt(int a_dtype, const void *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
+                        int b_dtype, const void *y, int64_t b_sb, int64_t b_sc, int64_t b_sf,
+                        int m_dtype, const void *mask, int64_t m_sb, int64_t m_sc, int64_t m_sf,
+                        const uint8_t *batch_mask, float *out3, void *workspace,
+                        int B, int C, int F, int64_t P, int mask_c, int64_t mask_repeat, int reduction,
+                        float weight, mt_stream_t stream);
+MT_API int mt_masked_l1_bwd_dt(int a_dtype, const void *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
+                        int b_dtype, const void *y, int64_t b_sb, int64_t b_sc, int64_t b_sf,
+                        int m_dtype, const void *mask, int64_t m_sb, int64_t m_sc, int64_t m_sf,
+                        const uint8_t *batch_mask, const float *out3, const float *grad_out,
+                        void *grad_y_hat, void *grad_y,
+                        int B, int C, int F, int64_t P, int mask_c, int reduction, float weight,
+                        mt_stream_t stream);
+
 /* The three masked-L1 terms of CHN.compute_loss in one pass          model_chn.py:347-362  (a5)
  *   loss_nh  = masked_l1(y_hat,      target, v_target repeated over F, 'sum', w_nh)
  *   loss_vh  = masked_l1(y_hat,      target, v_map,                    'sum', w_vh)
@@ -222,6 +250,14 @@ MT_API int mt_chn_fill_step(const float *nn_out, const float *x_t, int64_t xt_sb
                      const float *v_map0, int64_t vm_sb, float *y_comp0, float *m_new, float *x_new,
                      float *inp_per, void *workspace, int B, int64_t P, mt_stream_t stream);
 
+/* mt_chn_fill_step with nn_out in the dtype nn_dtype (MT_DT_*): the RRDBNet output under autocast, model_chn.py:83
+ * (`nn_out * self.std` with fp32 buffers promotes it to fp32).  Widened on load; every other operand and every
+ * output stays fp32 and is what mt_chn_fill_step writes for the widened nn_out. */
+MT_API int mt_chn_fill_step_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
+                        const float *v_t, int64_t vt_sb, const float *m_t, int64_t mt_sb,
+                        const float *v_map0, int64_t vm_sb, float *y_comp0, float *m_new, float *x_new,
+                        float *inp_per, void *workspace, int B, int64_t P, mt_stream_t stream);
+
 /* mt_chn_fill_step under device-side loop control (SURVEY 8f-4).  The reference's inpainting loops run
  * `while ... and inp_per > e` (model_chn.py:112, 163) and therefore read inp_per back to the host after
  * every step.  Here the step takes the PREVIOUS step's inp_per as a device scalar: while *gate_per > gate_e it
@@ -234,6 +270,14 @@ MT_API int mt_chn_fill_step_gated(const float *nn_out, const float *x_t, int64_t
                            const float *gate_per, float gate_e,
                            float *y_comp0, float *m_new, float *x_new,
                            float *inp_per, void *workspace, int B, int64_t P, mt_stream_t stream);
+
+/* mt_chn_fill_step_gated with nn_out in the dtype nn_dtype, as mt_chn_fill_step_dt   model_chn.py:83, 112 */
+MT_API int mt_chn_fill_step_gated_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
+                              int64_t xt_sc, const float *v_t, int64_t vt_sb, const float *m_t, int64_t mt_sb,
+                              const float *v_map0, int64_t vm_sb, const float *y_prev,
+                              const float *gate_per, float gate_e,
+                              float *y_comp0, float *m_new, float *x_new,
+                              float *inp_per, void *workspace, int B, int64_t P, mt_stream_t stream);
 
 /* mt_chn_fill_lanes: the composite + hole update of mt_chn_fill_step for L independent target frames of a clip
  * ("lanes") in one launch, each with its own hole percentage: the batched form of the inference loops of
@@ -260,6 +304,13 @@ MT_API int mt_chn_fill_lanes(const float *nn_out, const float *x_t, int64_t xt_s
                       float *m_state, int64_t ms_ss, float *x_state, int64_t xs_ss, int64_t xs_sc,
                       float *per_out, void *workspace, int L, int64_t P,
                       int finalize, double e, int force, mt_stream_t stream);
+/* mt_chn_fill_lanes with nn_out in the dtype nn_dtype (MT_DT_*), as mt_chn_fill_step_dt   model_chn.py:83, 128-131 */
+MT_API int mt_chn_fill_lanes_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sl, int64_t xt_sc,
+                         const float *m_t, int64_t mt_sl, const float *v_map0, int64_t vm_sl,
+                         const int *slots, float *y_out, int64_t yo_ss, int64_t yo_sc,
+                         float *m_state, int64_t ms_ss, float *x_state, int64_t xs_ss, int64_t xs_sc,
+                         float *per_out, void *workspace, int L, int64_t P,
+                         int finalize, double e, int force, mt_stream_t stream);
 MT_API int64_t mt_chn_fill_lanes_workspace_bytes(int L);
 
 /* ---- K2  masked cosine correlation on tcgen05 ----------------------------
@@ -349,6 +400,16 @@ MT_API int mt_chn_composite_bwd(const float *nn_out, const float *v_t, int64_t v
                          const float *g_yhat, int64_t gy_sb, int64_t gy_sc, int64_t gy_sf,
                          const float *g_comp, int64_t gc_sb, int64_t gc_sc, int64_t gc_sf,
                          float *g_nn, int B, int F, int64_t P, mt_stream_t stream);
+/* mt_chn_composite_fwd / _bwd with nn_out in the dtype nn_dtype (MT_DT_*)          model_chn.py:80-85 under autocast
+ * (`nn_out * self.std` promotes the half RRDBNet output to fp32, :83).  y_hat / y_comp and the upstream gradients
+ * stay fp32; g_nn is written in nn_dtype: the fp32 gradient rounded to nearest even (inf where it overflows fp16). */
+MT_API int mt_chn_composite_fwd_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
+                            int64_t xt_sc, const float *v_t, int64_t vt_sb, float *y_hat, float *y_comp,
+                            int B, int F, int64_t P, mt_stream_t stream);
+MT_API int mt_chn_composite_bwd_dt(int nn_dtype, const void *nn_out, const float *v_t, int64_t vt_sb,
+                            const float *g_yhat, int64_t gy_sb, int64_t gy_sc, int64_t gy_sf,
+                            const float *g_comp, int64_t gc_sb, int64_t gc_sc, int64_t gc_sf,
+                            void *g_nn, int B, int F, int64_t P, mt_stream_t stream);
 MT_API int mt_hole_update(const float *m_t, int64_t mt_sb, const float *v_map0, int64_t vm_sb,
                    const float *y_comp0, int64_t yc_sb, int64_t yc_sc,
                    float *m_new, float *x_new, float *inp_per, void *workspace,

@@ -63,19 +63,20 @@ __global__ void __launch_bounds__(256, 4) chn_pack_kernel(const PackArgs a) {
 }
 
 // ---- a10 composite ------------------------------------------------------------
+template <typename T>  // element type of nn_out and g_nn (float, __half, __nv_bfloat16)
 struct CompArgs {
-    const float *nn_out;
+    const T *nn_out;
     const float *x_t; int64_t xt_sb, xt_sc;
     const float *v_t; int64_t vt_sb;
     float *y_hat, *y_comp;  // frame-major (B,F,3,P)
     const float *g_yhat; int64_t gy_sb, gy_sc, gy_sf;
     const float *g_comp; int64_t gc_sb, gc_sc, gc_sf;
-    float *g_nn;
+    T *g_nn;
     int F; int64_t P;
 };
 
-template <int VEC>
-__global__ void __launch_bounds__(256, 4) chn_composite_fwd_kernel(const CompArgs a) {
+template <typename T, int VEC>
+__global__ void __launch_bounds__(256, 4) chn_composite_fwd_kernel(const CompArgs<T> a) {
     pdl_sync();
     const int64_t p0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
     if (p0 >= a.P) return;
@@ -106,8 +107,8 @@ __global__ void __launch_bounds__(256, 4) chn_composite_fwd_kernel(const CompArg
     }
 }
 
-template <int VEC>
-__global__ void __launch_bounds__(256, 4) chn_composite_bwd_kernel(const CompArgs a) {
+template <typename T, int VEC>
+__global__ void __launch_bounds__(256, 4) chn_composite_bwd_kernel(const CompArgs<T> a) {
     pdl_sync();
     const int64_t p0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
     if (p0 >= a.P) return;
@@ -185,8 +186,9 @@ __global__ void __launch_bounds__(256) hole_update_kernel(const HoleArgs a) {
 }
 
 // ---- a10 + a11: composite and hole update of one inference step (F = 1) in one pass ------------
+template <typename T>  // element type of nn_out
 struct FillArgs {
-    const float *nn_out;
+    const T *nn_out;
     const float *x_t; int64_t xt_sb, xt_sc;
     const float *v_t; int64_t vt_sb;
     const float *m_t; int64_t mt_sb;
@@ -199,8 +201,8 @@ struct FillArgs {
     const float *gate_per, *y_prev; float gate_e;
 };
 
-template <int VEC>
-__global__ void __launch_bounds__(256) chn_fill_kernel(const FillArgs a) {
+template <typename T, int VEC>
+__global__ void __launch_bounds__(256) chn_fill_kernel(const FillArgs<T> a) {
     pdl_sync();
     __shared__ float red[32];
     float acc[1] = {0.0f};
@@ -295,13 +297,14 @@ __global__ void __launch_bounds__(256) trivial_copy_kernel(const TrivArgs a) {
 }
 
 // ---- a5 masked L1 -------------------------------------------------------------
+template <typename TA, typename TB, typename TM>  // element types of y_hat (and ga), y (and gb), mask
 struct L1Args {
-    const float *a; int64_t a_sb, a_sc, a_sf;
-    const float *b; int64_t b_sb, b_sc, b_sf;
-    const float *m; int64_t m_sb, m_sc, m_sf;
+    const TA *a; int64_t a_sb, a_sc, a_sf;
+    const TB *b; int64_t b_sb, b_sc, b_sf;
+    const TM *m; int64_t m_sb, m_sc, m_sf;
     const uint8_t *bm;
     float *out3; void *ws;
-    const float *out3_in; const float *grad_out; float *ga, *gb;
+    const float *out3_in; const float *grad_out; TA *ga; TB *gb;
     int B, C, F; int64_t P; int mask_c, reduction; float weight;
     int chunks; int64_t total_chunks;  // over (B, F, chunk)
     double mask_repeat;                // times every mask element is visited through stride-0 broadcasting
@@ -314,8 +317,8 @@ constexpr int kL1Unroll = 4;
 
 constexpr int kL1CtasPerSm = 2;   // resident CTAs the register budget is stated for; the grid is one such wave
 
-template <int VEC>
-__global__ void __launch_bounds__(256, kL1CtasPerSm) masked_l1_fwd_kernel(const L1Args a) {
+template <typename TA, typename TB, typename TM, int VEC>
+__global__ void __launch_bounds__(256, kL1CtasPerSm) masked_l1_fwd_kernel(const L1Args<TA, TB, TM> a) {
     pdl_sync();
     __shared__ float red[3 * 32];
     float acc[3] = {0.0f, 0.0f, 0.0f};  // sum |.|, sum(mask), selected element count / P-chunks
@@ -393,8 +396,8 @@ __global__ void __launch_bounds__(256, kL1CtasPerSm) masked_l1_fwd_kernel(const 
     });
 }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) masked_l1_bwd_kernel(const L1Args a) {
+template <typename TA, typename TB, typename TM, int VEC>
+__global__ void __launch_bounds__(256) masked_l1_bwd_kernel(const L1Args<TA, TB, TM> a) {
     pdl_sync();
     const int64_t p0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
     if (p0 >= a.P) return;
@@ -577,41 +580,61 @@ extern "C" int mt_chn_pack(const float *x_t, int64_t xt_sb, int64_t xt_sc, const
     return launch_status("mt_chn_pack");
 }
 
+extern "C" int mt_chn_composite_fwd_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
+                                       int64_t xt_sc, const float *v_t, int64_t vt_sb, float *y_hat,
+                                       float *y_comp, int B, int F, int64_t P, mt_stream_t stream) {
+    MT_REQUIRE(nn_out && x_t && v_t && y_hat && y_comp, "mt_chn_composite_fwd: NULL argument");
+    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_fwd: bad shape");
+    return with_dtype(nn_dtype, "mt_chn_composite_fwd", [&](auto tag) {
+        using T = decltype(tag);
+        CompArgs<T> a{};
+        a.nn_out = static_cast<const T *>(nn_out); a.x_t = x_t; a.xt_sb = xt_sb; a.xt_sc = xt_sc; a.v_t = v_t;
+        a.vt_sb = vt_sb; a.y_hat = y_hat; a.y_comp = y_comp; a.F = F; a.P = P;
+        bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(y_hat) &&
+                  aligned16(y_comp) && mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb);
+        const int vec = v4 ? 4 : 1;
+        dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
+        if (v4) launch(chn_composite_fwd_kernel<T, 4>, grid, 256, 0, (cudaStream_t)stream, a);
+        else launch(chn_composite_fwd_kernel<T, 1>, grid, 256, 0, (cudaStream_t)stream, a);
+        return launch_status("mt_chn_composite_fwd");
+    });
+}
+
 extern "C" int mt_chn_composite_fwd(const float *nn_out, const float *x_t, int64_t xt_sb,
                                     int64_t xt_sc, const float *v_t, int64_t vt_sb, float *y_hat,
                                     float *y_comp, int B, int F, int64_t P, mt_stream_t stream) {
-    MT_REQUIRE(nn_out && x_t && v_t && y_hat && y_comp, "mt_chn_composite_fwd: NULL argument");
-    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_fwd: bad shape");
-    CompArgs a{};
-    a.nn_out = nn_out; a.x_t = x_t; a.xt_sb = xt_sb; a.xt_sc = xt_sc; a.v_t = v_t; a.vt_sb = vt_sb;
-    a.y_hat = y_hat; a.y_comp = y_comp; a.F = F; a.P = P;
-    bool v4 = mult4(P) && aligned16(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(y_hat) &&
-              aligned16(y_comp) && mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb);
-    const int vec = v4 ? 4 : 1;
-    dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
-    if (v4) launch(chn_composite_fwd_kernel<4>, grid, 256, 0, (cudaStream_t)stream, a);
-    else launch(chn_composite_fwd_kernel<1>, grid, 256, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_chn_composite_fwd");
+    return mt_chn_composite_fwd_dt(MT_DT_F32, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, y_hat, y_comp, B, F, P, stream);
+}
+
+extern "C" int mt_chn_composite_bwd_dt(int nn_dtype, const void *nn_out, const float *v_t, int64_t vt_sb,
+                                       const float *g_yhat, int64_t gy_sb, int64_t gy_sc, int64_t gy_sf,
+                                       const float *g_comp, int64_t gc_sb, int64_t gc_sc, int64_t gc_sf,
+                                       void *g_nn, int B, int F, int64_t P, mt_stream_t stream) {
+    MT_REQUIRE(nn_out && v_t && g_nn, "mt_chn_composite_bwd: NULL argument");
+    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_bwd: bad shape");
+    return with_dtype(nn_dtype, "mt_chn_composite_bwd", [&](auto tag) {
+        using T = decltype(tag);
+        CompArgs<T> a{};
+        a.nn_out = static_cast<const T *>(nn_out); a.v_t = v_t; a.vt_sb = vt_sb; a.g_yhat = g_yhat; a.gy_sb = gy_sb;
+        a.gy_sc = gy_sc; a.gy_sf = gy_sf; a.g_comp = g_comp; a.gc_sb = gc_sb; a.gc_sc = gc_sc;
+        a.gc_sf = gc_sf; a.g_nn = static_cast<T *>(g_nn); a.F = F; a.P = P;
+        bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(v_t) && aligned16(g_yhat) && aligned16(g_comp) &&
+                  aligned_vec4<T>(g_nn) && mult4(vt_sb) && mult4(gy_sb) && mult4(gy_sc) && mult4(gy_sf) &&
+                  mult4(gc_sb) && mult4(gc_sc) && mult4(gc_sf);
+        const int vec = v4 ? 4 : 1;
+        dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
+        if (v4) launch(chn_composite_bwd_kernel<T, 4>, grid, 256, 0, (cudaStream_t)stream, a);
+        else launch(chn_composite_bwd_kernel<T, 1>, grid, 256, 0, (cudaStream_t)stream, a);
+        return launch_status("mt_chn_composite_bwd");
+    });
 }
 
 extern "C" int mt_chn_composite_bwd(const float *nn_out, const float *v_t, int64_t vt_sb,
                                     const float *g_yhat, int64_t gy_sb, int64_t gy_sc, int64_t gy_sf,
                                     const float *g_comp, int64_t gc_sb, int64_t gc_sc, int64_t gc_sf,
                                     float *g_nn, int B, int F, int64_t P, mt_stream_t stream) {
-    MT_REQUIRE(nn_out && v_t && g_nn, "mt_chn_composite_bwd: NULL argument");
-    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_bwd: bad shape");
-    CompArgs a{};
-    a.nn_out = nn_out; a.v_t = v_t; a.vt_sb = vt_sb; a.g_yhat = g_yhat; a.gy_sb = gy_sb;
-    a.gy_sc = gy_sc; a.gy_sf = gy_sf; a.g_comp = g_comp; a.gc_sb = gc_sb; a.gc_sc = gc_sc;
-    a.gc_sf = gc_sf; a.g_nn = g_nn; a.F = F; a.P = P;
-    bool v4 = mult4(P) && aligned16(nn_out) && aligned16(v_t) && aligned16(g_yhat) && aligned16(g_comp) &&
-              aligned16(g_nn) && mult4(vt_sb) && mult4(gy_sb) && mult4(gy_sc) && mult4(gy_sf) &&
-              mult4(gc_sb) && mult4(gc_sc) && mult4(gc_sf);
-    const int vec = v4 ? 4 : 1;
-    dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
-    if (v4) launch(chn_composite_bwd_kernel<4>, grid, 256, 0, (cudaStream_t)stream, a);
-    else launch(chn_composite_bwd_kernel<1>, grid, 256, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_chn_composite_bwd");
+    return mt_chn_composite_bwd_dt(MT_DT_F32, nn_out, v_t, vt_sb, g_yhat, gy_sb, gy_sc, gy_sf, g_comp, gc_sb, gc_sc,
+                                   gc_sf, g_nn, B, F, P, stream);
 }
 
 extern "C" int mt_hole_update(const float *m_t, int64_t mt_sb, const float *v_map0, int64_t vm_sb,
@@ -650,18 +673,19 @@ extern "C" int mt_trivial_copy(const float *x_t, int64_t xt_sb, int64_t xt_sc, c
     return launch_status("mt_trivial_copy");
 }
 
-static int fill_l1(L1Args &a, const float *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
-                   const float *y, int64_t b_sb, int64_t b_sc, int64_t b_sf, const float *mask,
+template <typename TA, typename TB, typename TM>
+static int fill_l1(L1Args<TA, TB, TM> &a, const void *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
+                   const void *y, int64_t b_sb, int64_t b_sc, int64_t b_sf, const void *mask,
                    int64_t m_sb, int64_t m_sc, int64_t m_sf, const uint8_t *batch_mask, int B, int C,
                    int F, int64_t P, int mask_c, int reduction, float weight, const char *who) {
     MT_REQUIRE(y_hat && y, "%s: NULL input", who);  // mask == NULL: all ones (torch.ones_like(y_hat), model_dfpn.py:259-267)
     MT_REQUIRE(B > 0 && C > 0 && F > 0 && P > 0, "%s: empty shape", who);
     MT_REQUIRE(mask_c == 1 || mask_c == C, "%s: mask_c must be 1 or C", who);
     MT_REQUIRE(reduction == MT_REDUCE_MEAN || reduction == MT_REDUCE_SUM, "%s: bad reduction", who);
-    a = L1Args{};
-    a.a = y_hat; a.a_sb = a_sb; a.a_sc = a_sc; a.a_sf = a_sf;
-    a.b = y; a.b_sb = b_sb; a.b_sc = b_sc; a.b_sf = b_sf;
-    a.m = mask; a.m_sb = m_sb; a.m_sc = m_sc; a.m_sf = m_sf;
+    a = L1Args<TA, TB, TM>{};
+    a.a = static_cast<const TA *>(y_hat); a.a_sb = a_sb; a.a_sc = a_sc; a.a_sf = a_sf;
+    a.b = static_cast<const TB *>(y); a.b_sb = b_sb; a.b_sc = b_sc; a.b_sf = b_sf;
+    a.m = static_cast<const TM *>(mask); a.m_sb = m_sb; a.m_sc = m_sc; a.m_sf = m_sf;
     a.bm = batch_mask; a.B = B; a.C = C; a.F = F; a.P = P; a.mask_c = mask_c;
     a.reduction = reduction; a.weight = weight;
     // Collapse axes that are back to back in memory into the plane: the flow losses arrive as (B, F, H, W, 2) =
@@ -677,10 +701,55 @@ static int fill_l1(L1Args &a, const float *y_hat, int64_t a_sb, int64_t a_sc, in
     return MT_OK;
 }
 
-static bool l1_vec4(const L1Args &a) {
-    return mult4(a.P) && aligned16(a.a) && aligned16(a.b) && (!a.m || aligned16(a.m)) && mult4(a.a_sb) &&
-           mult4(a.a_sc) && mult4(a.a_sf) && mult4(a.b_sb) && mult4(a.b_sc) && mult4(a.b_sf) &&
+template <typename TA, typename TB, typename TM>
+static bool l1_vec4(const L1Args<TA, TB, TM> &a) {
+    return mult4(a.P) && aligned_vec4<TA>(a.a) && aligned_vec4<TB>(a.b) && (!a.m || aligned_vec4<TM>(a.m)) &&
+           mult4(a.a_sb) && mult4(a.a_sc) && mult4(a.a_sf) && mult4(a.b_sb) && mult4(a.b_sc) && mult4(a.b_sf) &&
            mult4(a.m_sb) && mult4(a.m_sc) && mult4(a.m_sf);
+}
+
+// f(TA{}, TB{}, TM{}) for the dtype codes of y_hat, y and the mask; the mask is fp32 or in the dtype of y_hat
+// (a {0,1} mask made alongside a half network output), anything else is an error
+template <typename Fn>
+static int with_l1_dtypes(int a_dtype, int b_dtype, int m_dtype, const char *who, Fn &&f) {
+    MT_REQUIRE(m_dtype == MT_DT_F32 || m_dtype == a_dtype, "%s: the mask must be fp32 or in the dtype of y_hat", who);
+    return with_dtype(a_dtype, who, [&](auto ta) {
+        return with_dtype(b_dtype, who, [&](auto tb) {
+            if (m_dtype == MT_DT_F32) return f(ta, tb, float{});
+            return f(ta, tb, ta);
+        });
+    });
+}
+
+extern "C" int mt_masked_l1_fwd_dt(int a_dtype, const void *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
+                                   int b_dtype, const void *y, int64_t b_sb, int64_t b_sc, int64_t b_sf,
+                                   int m_dtype, const void *mask, int64_t m_sb, int64_t m_sc, int64_t m_sf,
+                                   const uint8_t *batch_mask, float *out3, void *workspace, int B,
+                                   int C, int F, int64_t P, int mask_c, int64_t mask_repeat, int reduction,
+                                   float weight, mt_stream_t stream) {
+    return with_l1_dtypes(a_dtype, b_dtype, m_dtype, "mt_masked_l1_fwd", [&](auto ta, auto tb, auto tm) {
+        using TA = decltype(ta);
+        using TB = decltype(tb);
+        using TM = decltype(tm);
+        L1Args<TA, TB, TM> a;
+        int rc = fill_l1(a, y_hat, a_sb, a_sc, a_sf, y, b_sb, b_sc, b_sf, mask, m_sb, m_sc, m_sf,
+                         batch_mask, B, C, F, P, mask_c, reduction, weight, "mt_masked_l1_fwd");
+        if (rc) return rc;
+        MT_REQUIRE(out3 && workspace, "mt_masked_l1_fwd: NULL out3 / workspace");
+        MT_REQUIRE(mask_repeat >= 1, "mt_masked_l1_fwd: mask_repeat must be >= 1");
+        a.out3 = out3; a.ws = workspace; a.mask_repeat = (double)mask_repeat;
+        const bool v4 = l1_vec4(a);
+        const int vec = v4 ? 4 : 1;
+        a.chunks = (int)((a.P + 256 * vec - 1) / (256 * vec));
+        a.total_chunks = (int64_t)a.B * a.F * a.chunks;
+        int64_t want = (a.total_chunks + kL1Unroll - 1) / kL1Unroll;
+        if (want > (int64_t)sm_count() * kL1CtasPerSm) want = (int64_t)sm_count() * kL1CtasPerSm;
+        const int nblk = (int)want;
+        MT_REQUIRE(a.total_chunks + (int64_t)nblk * kL1Unroll < (1ll << 32), "mt_masked_l1_fwd: too many chunks");
+        if (v4) launch(masked_l1_fwd_kernel<TA, TB, TM, 4>, nblk, 256, 0, (cudaStream_t)stream, a);
+        else launch(masked_l1_fwd_kernel<TA, TB, TM, 1>, nblk, 256, 0, (cudaStream_t)stream, a);
+        return launch_status("mt_masked_l1_fwd");
+    });
 }
 
 extern "C" int mt_masked_l1_fwd(const float *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
@@ -689,24 +758,35 @@ extern "C" int mt_masked_l1_fwd(const float *y_hat, int64_t a_sb, int64_t a_sc, 
                                 const uint8_t *batch_mask, float *out3, void *workspace, int B,
                                 int C, int F, int64_t P, int mask_c, int64_t mask_repeat, int reduction,
                                 float weight, mt_stream_t stream) {
-    L1Args a;
-    int rc = fill_l1(a, y_hat, a_sb, a_sc, a_sf, y, b_sb, b_sc, b_sf, mask, m_sb, m_sc, m_sf,
-                     batch_mask, B, C, F, P, mask_c, reduction, weight, "mt_masked_l1_fwd");
-    if (rc) return rc;
-    MT_REQUIRE(out3 && workspace, "mt_masked_l1_fwd: NULL out3 / workspace");
-    MT_REQUIRE(mask_repeat >= 1, "mt_masked_l1_fwd: mask_repeat must be >= 1");
-    a.out3 = out3; a.ws = workspace; a.mask_repeat = (double)mask_repeat;
-    const bool v4 = l1_vec4(a);
-    const int vec = v4 ? 4 : 1;
-    a.chunks = (int)((a.P + 256 * vec - 1) / (256 * vec));
-    a.total_chunks = (int64_t)a.B * a.F * a.chunks;
-    int64_t want = (a.total_chunks + kL1Unroll - 1) / kL1Unroll;
-    if (want > (int64_t)sm_count() * kL1CtasPerSm) want = (int64_t)sm_count() * kL1CtasPerSm;
-    const int nblk = (int)want;
-    MT_REQUIRE(a.total_chunks + (int64_t)nblk * kL1Unroll < (1ll << 32), "mt_masked_l1_fwd: too many chunks");
-    if (v4) launch(masked_l1_fwd_kernel<4>, nblk, 256, 0, (cudaStream_t)stream, a);
-    else launch(masked_l1_fwd_kernel<1>, nblk, 256, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_masked_l1_fwd");
+    return mt_masked_l1_fwd_dt(MT_DT_F32, y_hat, a_sb, a_sc, a_sf, MT_DT_F32, y, b_sb, b_sc, b_sf, MT_DT_F32, mask,
+                               m_sb, m_sc, m_sf, batch_mask, out3, workspace, B, C, F, P, mask_c, mask_repeat,
+                               reduction, weight, stream);
+}
+
+extern "C" int mt_masked_l1_bwd_dt(int a_dtype, const void *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
+                                   int b_dtype, const void *y, int64_t b_sb, int64_t b_sc, int64_t b_sf,
+                                   int m_dtype, const void *mask, int64_t m_sb, int64_t m_sc, int64_t m_sf,
+                                   const uint8_t *batch_mask, const float *out3, const float *grad_out,
+                                   void *grad_y_hat, void *grad_y, int B, int C, int F, int64_t P,
+                                   int mask_c, int reduction, float weight, mt_stream_t stream) {
+    return with_l1_dtypes(a_dtype, b_dtype, m_dtype, "mt_masked_l1_bwd", [&](auto ta, auto tb, auto tm) {
+        using TA = decltype(ta);
+        using TB = decltype(tb);
+        using TM = decltype(tm);
+        L1Args<TA, TB, TM> a;
+        int rc = fill_l1(a, y_hat, a_sb, a_sc, a_sf, y, b_sb, b_sc, b_sf, mask, m_sb, m_sc, m_sf,
+                         batch_mask, B, C, F, P, mask_c, reduction, weight, "mt_masked_l1_bwd");
+        if (rc) return rc;
+        MT_REQUIRE(out3 && grad_out && (grad_y_hat || grad_y), "mt_masked_l1_bwd: NULL argument");
+        MT_REQUIRE((int64_t)a.B * a.F <= 65535, "mt_masked_l1_bwd: B*F > 65535");
+        a.out3_in = out3; a.grad_out = grad_out; a.ga = static_cast<TA *>(grad_y_hat); a.gb = static_cast<TB *>(grad_y);
+        const bool v4 = l1_vec4(a) && aligned_vec4<TA>(grad_y_hat) && aligned_vec4<TB>(grad_y);
+        const int vec = v4 ? 4 : 1;
+        dim3 grid((unsigned)((a.P + 256 * vec - 1) / (256 * vec)), a.B * a.F);
+        if (v4) launch(masked_l1_bwd_kernel<TA, TB, TM, 4>, grid, 256, 0, (cudaStream_t)stream, a);
+        else launch(masked_l1_bwd_kernel<TA, TB, TM, 1>, grid, 256, 0, (cudaStream_t)stream, a);
+        return launch_status("mt_masked_l1_bwd");
+    });
 }
 
 extern "C" int mt_masked_l1_bwd(const float *y_hat, int64_t a_sb, int64_t a_sc, int64_t a_sf,
@@ -715,19 +795,9 @@ extern "C" int mt_masked_l1_bwd(const float *y_hat, int64_t a_sb, int64_t a_sc, 
                                 const uint8_t *batch_mask, const float *out3, const float *grad_out,
                                 float *grad_y_hat, float *grad_y, int B, int C, int F, int64_t P,
                                 int mask_c, int reduction, float weight, mt_stream_t stream) {
-    L1Args a;
-    int rc = fill_l1(a, y_hat, a_sb, a_sc, a_sf, y, b_sb, b_sc, b_sf, mask, m_sb, m_sc, m_sf,
-                     batch_mask, B, C, F, P, mask_c, reduction, weight, "mt_masked_l1_bwd");
-    if (rc) return rc;
-    MT_REQUIRE(out3 && grad_out && (grad_y_hat || grad_y), "mt_masked_l1_bwd: NULL argument");
-    MT_REQUIRE((int64_t)a.B * a.F <= 65535, "mt_masked_l1_bwd: B*F > 65535");
-    a.out3_in = out3; a.grad_out = grad_out; a.ga = grad_y_hat; a.gb = grad_y;
-    const bool v4 = l1_vec4(a) && aligned16(grad_y_hat) && aligned16(grad_y);
-    const int vec = v4 ? 4 : 1;
-    dim3 grid((unsigned)((a.P + 256 * vec - 1) / (256 * vec)), a.B * a.F);
-    if (v4) launch(masked_l1_bwd_kernel<4>, grid, 256, 0, (cudaStream_t)stream, a);
-    else launch(masked_l1_bwd_kernel<1>, grid, 256, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_masked_l1_bwd");
+    return mt_masked_l1_bwd_dt(MT_DT_F32, y_hat, a_sb, a_sc, a_sf, MT_DT_F32, y, b_sb, b_sc, b_sf, MT_DT_F32, mask,
+                               m_sb, m_sc, m_sf, batch_mask, out3, grad_out, grad_y_hat, grad_y, B, C, F, P, mask_c,
+                               reduction, weight, stream);
 }
 
 static int fill_l1x3(L1x3Args &a, const float *y_hat, int64_t yh_sb, int64_t yh_sc, int64_t yh_sf,
@@ -800,7 +870,7 @@ extern "C" int mt_chn_l1x3_bwd(const float *y_hat, int64_t yh_sb, int64_t yh_sc,
     return launch_status("mt_chn_l1x3_bwd");
 }
 
-static int chn_fill_impl(const float *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
+static int chn_fill_impl(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
                          const float *v_t, int64_t vt_sb, const float *m_t, int64_t mt_sb,
                          const float *v_map0, int64_t vm_sb, const float *y_prev, const float *gate_per,
                          float gate_e, float *y_comp0, float *m_new, float *x_new, float *inp_per,
@@ -810,18 +880,30 @@ static int chn_fill_impl(const float *nn_out, const float *x_t, int64_t xt_sb, i
     MT_REQUIRE(B > 0 && P > 0, "mt_chn_fill_step: bad shape");
     MT_REQUIRE(!gate_per || y_prev, "mt_chn_fill_step_gated: a gate needs the previous step's y_comp0");
     MT_REQUIRE(inp_per != gate_per && y_prev != y_comp0, "mt_chn_fill_step_gated: outputs must not alias the gate inputs");
-    FillArgs a{nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, y_comp0, m_new, x_new, inp_per,
-               workspace, B, P, 0, 0, gate_per, y_prev, gate_e};
-    bool v4 = mult4(P) && aligned16(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(m_t) &&
-              aligned16(v_map0) && aligned16(y_comp0) && aligned16(m_new) && aligned16(x_new) && mult4(xt_sb) &&
-              mult4(xt_sc) && mult4(vt_sb) && mult4(mt_sb) && mult4(vm_sb) && aligned16(y_prev);
-    const int vec = v4 ? 4 : 1;
-    a.chunks = (int)((P + 256 * vec - 1) / (256 * vec));
-    a.total_chunks = (int64_t)B * a.chunks;
-    const int nblk = reduce_blocks(a.total_chunks);
-    if (v4) launch(chn_fill_kernel<4>, nblk, 256, 0, (cudaStream_t)stream, a);
-    else launch(chn_fill_kernel<1>, nblk, 256, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_chn_fill_step");
+    return with_dtype(nn_dtype, "mt_chn_fill_step", [&](auto tag) {
+        using T = decltype(tag);
+        FillArgs<T> a{static_cast<const T *>(nn_out), x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb,
+                      y_comp0, m_new, x_new, inp_per, workspace, B, P, 0, 0, gate_per, y_prev, gate_e};
+        bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(m_t) &&
+                  aligned16(v_map0) && aligned16(y_comp0) && aligned16(m_new) && aligned16(x_new) && mult4(xt_sb) &&
+                  mult4(xt_sc) && mult4(vt_sb) && mult4(mt_sb) && mult4(vm_sb) && aligned16(y_prev);
+        const int vec = v4 ? 4 : 1;
+        a.chunks = (int)((P + 256 * vec - 1) / (256 * vec));
+        a.total_chunks = (int64_t)B * a.chunks;
+        const int nblk = reduce_blocks(a.total_chunks);
+        if (v4) launch(chn_fill_kernel<T, 4>, nblk, 256, 0, (cudaStream_t)stream, a);
+        else launch(chn_fill_kernel<T, 1>, nblk, 256, 0, (cudaStream_t)stream, a);
+        return launch_status("mt_chn_fill_step");
+    });
+}
+
+extern "C" int mt_chn_fill_step_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
+                                   int64_t xt_sc, const float *v_t, int64_t vt_sb, const float *m_t, int64_t mt_sb,
+                                   const float *v_map0, int64_t vm_sb, float *y_comp0, float *m_new,
+                                   float *x_new, float *inp_per, void *workspace, int B, int64_t P,
+                                   mt_stream_t stream) {
+    return chn_fill_impl(nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, nullptr, nullptr,
+                         0.0f, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
 }
 
 extern "C" int mt_chn_fill_step(const float *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
@@ -829,8 +911,18 @@ extern "C" int mt_chn_fill_step(const float *nn_out, const float *x_t, int64_t x
                                 const float *v_map0, int64_t vm_sb, float *y_comp0, float *m_new,
                                 float *x_new, float *inp_per, void *workspace, int B, int64_t P,
                                 mt_stream_t stream) {
-    return chn_fill_impl(nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, nullptr, nullptr, 0.0f,
-                         y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
+    return mt_chn_fill_step_dt(MT_DT_F32, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, y_comp0,
+                               m_new, x_new, inp_per, workspace, B, P, stream);
+}
+
+extern "C" int mt_chn_fill_step_gated_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
+                                         int64_t xt_sc, const float *v_t, int64_t vt_sb, const float *m_t,
+                                         int64_t mt_sb, const float *v_map0, int64_t vm_sb, const float *y_prev,
+                                         const float *gate_per, float gate_e, float *y_comp0, float *m_new,
+                                         float *x_new, float *inp_per, void *workspace, int B, int64_t P,
+                                         mt_stream_t stream) {
+    return chn_fill_impl(nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, y_prev, gate_per,
+                         gate_e, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
 }
 
 extern "C" int mt_chn_fill_step_gated(const float *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
@@ -839,6 +931,7 @@ extern "C" int mt_chn_fill_step_gated(const float *nn_out, const float *x_t, int
                                       const float *gate_per, float gate_e, float *y_comp0, float *m_new,
                                       float *x_new, float *inp_per, void *workspace, int B, int64_t P,
                                       mt_stream_t stream) {
-    return chn_fill_impl(nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, y_prev, gate_per, gate_e,
-                         y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
+    return mt_chn_fill_step_gated_dt(MT_DT_F32, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb,
+                                     y_prev, gate_per, gate_e, y_comp0, m_new, x_new, inp_per, workspace, B, P,
+                                     stream);
 }

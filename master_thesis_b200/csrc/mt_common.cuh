@@ -7,6 +7,8 @@
 // library is compiled with -fmad=false so nvcc cannot contract anything else.
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -52,6 +54,25 @@ inline void launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
 }
 
 static inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+// the vector path of a kernel reads 4 consecutive elements of type T in one access (16 B of float, 8 B of half)
+template <typename T>
+static inline bool aligned_vec4(const void *p) {
+    return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(T) - 1)) == 0;
+}
+
+// Network operands (the CNN output, the inputs of the losses) may arrive in fp16 / bf16 under autocast: the element
+// type of such an operand is a dtype code MT_DT_*.  Calls f(T{}) with T = float, __half or __nv_bfloat16.
+template <typename Fn>
+inline int with_dtype(int dt, const char *who, Fn &&f) {
+    switch (dt) {
+        case MT_DT_F32: return f(float{});
+        case MT_DT_F16: return f(__half{});
+        case MT_DT_BF16: return f(__nv_bfloat16{});
+        default: break;
+    }
+    set_error("%s: unknown dtype code %d", who, dt);
+    return MT_ERR_INVALID;
+}
 
 // workspace layout used by the reducing kernels
 constexpr int kMaxReduceBlocks = 16384;
@@ -97,6 +118,18 @@ __device__ __forceinline__ void st_stream4(float *p, float4 v) {
 }
 __device__ __forceinline__ void st_stream1(float *p, float v) { __stcs(p, v); }
 
+// fp16 / bf16 operands: widened to float on load (exact), gradients narrowed on store (round to nearest even)
+__device__ __forceinline__ float widen(__half v) { return __half2float(v); }
+__device__ __forceinline__ float widen(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T>
+__device__ __forceinline__ T narrow(float v);
+template <>
+__device__ __forceinline__ __half narrow<__half>(float v) { return __float2half_rn(v); }
+template <>
+__device__ __forceinline__ __nv_bfloat16 narrow<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+
+// Vec<VEC>: VEC consecutive elements in float registers.  The float overloads are the fp32 path; the templates read
+// and write 2-byte element types (one 8-byte access for VEC = 4).
 template <int VEC>
 struct Vec;
 template <>
@@ -105,6 +138,10 @@ struct Vec<1> {
     __device__ __forceinline__ void load_stream(const float *p) { v[0] = ld_stream1(p); }
     __device__ __forceinline__ void load_cached(const float *p) { v[0] = __ldg(p); }
     __device__ __forceinline__ void store_stream(float *p) const { st_stream1(p, v[0]); }
+    template <typename T>
+    __device__ __forceinline__ void load_stream(const T *p) { v[0] = widen(__ldcs(p)); }
+    template <typename T>
+    __device__ __forceinline__ void store_stream(T *p) const { __stcs(p, narrow<T>(v[0])); }
 };
 template <>
 struct Vec<4> {
@@ -119,6 +156,23 @@ struct Vec<4> {
     }
     __device__ __forceinline__ void store_stream(float *p) const {
         st_stream4(p, make_float4(v[0], v[1], v[2], v[3]));
+    }
+    template <typename T>
+    __device__ __forceinline__ void load_stream(const T *p) {
+        static_assert(sizeof(T) == 2, "2-byte element types only");
+        const uint2 u = __ldcs(reinterpret_cast<const uint2 *>(p));
+        const T *e = reinterpret_cast<const T *>(&u);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) v[i] = widen(e[i]);
+    }
+    template <typename T>
+    __device__ __forceinline__ void store_stream(T *p) const {
+        static_assert(sizeof(T) == 2, "2-byte element types only");
+        uint2 u;
+        T *e = reinterpret_cast<T *>(&u);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) e[i] = narrow<T>(v[i]);
+        __stcs(reinterpret_cast<uint2 *>(p), u);
     }
 };
 

@@ -3,7 +3,9 @@
 PyTorch is plumbing here: it owns device memory (caching allocator), streams
 and autograd bookkeeping.  Every computation is a hand-written sm_100a kernel
 reached through ``_lib.call`` with raw device pointers.  CUDA fp32 tensors
-only; anything else raises - there is no CPU / eager fallback.
+only, except the network operands checked against ``NET_DTYPES`` (the CNN output
+of CHN, the inputs of masked_l1), which may also be fp16 / bf16 as autocast hands
+them over; anything else raises - there is no CPU / eager fallback.
 """
 import ctypes
 
@@ -16,6 +18,10 @@ VIS_BILINEAR = 2
 GRID_AFFINE = 4
 VIS_FROM_MASK = 8
 REDUCE = {"mean": 0, "sum": 1}
+# network operands: the kernels read them in these dtypes (widened to fp32 in registers); codes MT_DT_* of the C ABI
+NET_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
+_DT = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+_DT_NAMES = {torch.float32: "fp32", torch.float16: "fp16", torch.bfloat16: "bf16"}
 
 _workspaces = {}
 record = _lib.record      # with ops.record() as plan: ...   (see _lib.Plan)
@@ -43,6 +49,27 @@ def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+class _Net(object):
+    """A network operand of a ``_call_net`` launch (a tensor or None)."""
+    __slots__ = ("t",)
+
+    def __init__(self, t):
+        self.t = t
+
+
+def _call_net(name, *args):
+    """Launches entry point ``name`` whose network operands are given as ``_Net``: when all of them are fp32 (or absent)
+    the fp32 entry point itself, so an fp32 run launches and records what it always did; else its ``_dt`` form, with
+    the MT_DT_* code of each such operand before its pointer."""
+    nets = [a.t for a in args if isinstance(a, _Net)]
+    if all(t is None or t.dtype == torch.float32 for t in nets):
+        return _call(name, *[_ptr(a.t) if isinstance(a, _Net) else a for a in args])
+    flat = []
+    for a in args:
+        flat += [0 if a.t is None else _DT[a.t.dtype], _ptr(a.t)] if isinstance(a, _Net) else [a]
+    return _call(name + "_dt", *flat)
+
+
 _device = [None]     # device index of the operator call in progress (set by _need_cuda)
 
 
@@ -57,15 +84,21 @@ def _call(name, *args):
 
 
 def _need_cuda(*ts):
+    """Every argument is a tensor (or None) that must be a CUDA fp32 tensor, or a pair (tensor, allowed dtypes)
+    for an operand the kernels also read in other dtypes; all on one device."""
     first = None
     for t in ts:
+        allowed = (torch.float32,)
+        if isinstance(t, tuple):
+            t, allowed = t
         if t is None:
             continue
         if not isinstance(t, torch.Tensor) or not t.is_cuda:
             raise RuntimeError("master_thesis_b200: CUDA tensors required (the hot path has no CPU "
                                "fallback); got %s" % (t.device if isinstance(t, torch.Tensor) else type(t)))
-        if t.dtype != torch.float32:
-            raise RuntimeError("master_thesis_b200: fp32 tensors required, got %s" % t.dtype)
+        if t.dtype not in allowed:
+            raise RuntimeError("master_thesis_b200: %s tensors required, got %s"
+                               % (" / ".join(_DT_NAMES[d] for d in allowed), t.dtype))
         if first is None:
             first = t.device
         elif t.device != first:
@@ -341,27 +374,29 @@ def _bm(batch_mask, like):
 def masked_l1_fwd_raw(y_hat, y, mask, batch_mask=None, reduction="mean", weight=1.0):
     """mt_masked_l1_fwd without autograd.  Returns (out3, saved): out3 = [loss, sum|.|, den] on the
     device, ``saved`` feeds masked_l1_bwd_raw."""
-    _need_cuda(y_hat, y, mask)
+    # the mask is fp32 or, like a torch.ones_like of a half network output, in the dtype of y_hat
+    mask_dtypes = tuple(dict.fromkeys((torch.float32, getattr(y_hat, "dtype", torch.float32))))
+    _need_cuda((y_hat, NET_DTYPES), (y, NET_DTYPES), (mask, mask_dtypes))
     if y_hat.numel() == 0:
         raise RuntimeError("masked_l1: empty input")
     (a, b_, m), B, C, F, P, mask_c, repeat = _l1_layout(y_hat, y, mask)
     bm = _bm(batch_mask, y_hat)
     out3 = _empty(3, dtype=torch.float32, device=y_hat.device)
-    _call("mt_masked_l1_fwd", _ptr(a[0]), a[1], a[2], a[3], _ptr(b_[0]), b_[1], b_[2], b_[3],
-              _ptr(m[0]), m[1], m[2], m[3], _ptr(bm), _ptr(out3), _ptr(reduce_workspace(y_hat)),
+    _call_net("mt_masked_l1_fwd", _Net(a[0]), a[1], a[2], a[3], _Net(b_[0]), b_[1], b_[2], b_[3],
+              _Net(m[0]), m[1], m[2], m[3], _ptr(bm), _ptr(out3), _ptr(reduce_workspace(y_hat)),
               B, C, F, P, mask_c, repeat, REDUCE[reduction], float(weight), _stream(y_hat))
     meta = (a[1:], b_[1:], m[1:], B, C, F, P, mask_c, REDUCE[reduction], float(weight), tuple(y_hat.shape))
     return out3, (a[0], b_[0], m[0], out3, bm, meta)
 
 
 def masked_l1_bwd_raw(saved, grad_out, need_y_hat=True, need_y=False):
-    """mt_masked_l1_bwd: gradients w.r.t. y_hat and / or y (grad_y = -grad_y_hat)."""
+    """mt_masked_l1_bwd: gradients w.r.t. y_hat and / or y (grad_y = -grad_y_hat), each in its input's dtype."""
     a, b_, m, out3, bm, (sa, sb, sm, B, C, F, P, mask_c, red, weight, shape) = saved
     _device[0] = a.device.index
-    ga = _empty((B, C, F, P), dtype=torch.float32, device=a.device) if need_y_hat else None
-    gb = _empty((B, C, F, P), dtype=torch.float32, device=a.device) if need_y else None
-    _call("mt_masked_l1_bwd", _ptr(a), sa[0], sa[1], sa[2], _ptr(b_), sb[0], sb[1], sb[2],
-              _ptr(m), sm[0], sm[1], sm[2], _ptr(bm), _ptr(out3), _ptr(grad_out),
+    ga = _empty((B, C, F, P), dtype=a.dtype, device=a.device) if need_y_hat else None
+    gb = _empty((B, C, F, P), dtype=b_.dtype, device=a.device) if need_y else None
+    _call_net("mt_masked_l1_bwd", _Net(a), sa[0], sa[1], sa[2], _Net(b_), sb[0], sb[1], sb[2],
+              _Net(m), sm[0], sm[1], sm[2], _ptr(bm), _ptr(out3), _ptr(grad_out),
               _ptr(ga), _ptr(gb), B, C, F, P, mask_c, red, weight, _stream(a))
     ga = ga.view(shape) if ga is not None else None
     gb = gb.view(shape) if gb is not None else None
@@ -704,14 +739,14 @@ class ChnCompositeFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, nn_out, x_t, v_t, b, f):
-        _need_cuda(nn_out, x_t, v_t)
+        _need_cuda((nn_out, NET_DTYPES), x_t, v_t)
         h, w = nn_out.shape[-2:]
         no = _contig(nn_out)
         xt, vt = _planes(x_t), _planes(v_t)
         yh_mem, yh = _frame_major(b, 3, f, h, w, no)
         yc_mem, yc = _frame_major(b, 3, f, h, w, no)
-        _call("mt_chn_composite_fwd", _ptr(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt),
-                  vt.stride(0), _ptr(yh_mem), _ptr(yc_mem), b, f, h * w, _stream(no))
+        _call_net("mt_chn_composite_fwd", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt),
+              vt.stride(0), _ptr(yh_mem), _ptr(yc_mem), b, f, h * w, _stream(no))
         ctx.save_for_backward(no, vt)
         ctx.meta = (b, f, h, w)
         return yh, yc
@@ -726,7 +761,8 @@ class ChnCompositeFn(torch.autograd.Function):
 
 
 def chn_composite_bwd_raw(nn_out, v_t, g_yh, g_yc, b, f):
-    """mt_chn_composite_bwd: gradient w.r.t. the CNN output from the grads of both outputs."""
+    """mt_chn_composite_bwd: gradient w.r.t. the CNN output from the grads of both outputs, in the dtype of
+    ``nn_out`` (the fp32 gradient rounded to nearest even)."""
     h, w = nn_out.shape[-2:]
     _device[0] = nn_out.device.index
     no, vt = _contig(nn_out), _planes(v_t)
@@ -737,8 +773,8 @@ def chn_composite_bwd_raw(nn_out, v_t, g_yh, g_yc, b, f):
     if g_yc is not None:
         gc, *gc_s = _s5(g_yc)
     g = _empty_like(no)
-    _call("mt_chn_composite_bwd", _ptr(no), _ptr(vt), vt.stride(0), _ptr(gy), *gy_s, _ptr(gc),
-              *gc_s, _ptr(g), b, f, h * w, _stream(no))
+    _call_net("mt_chn_composite_bwd", _Net(no), _ptr(vt), vt.stride(0), _ptr(gy), *gy_s, _ptr(gc),
+          *gc_s, _ptr(g), b, f, h * w, _stream(no))
     return g
 
 
@@ -768,7 +804,7 @@ def chn_fill(nn_out, x_t, v_t, m_t, v_map0, gate=None):
 
     ``gate = (prev_inp_per (1-element device tensor), e, y_prev)``: device-side loop control - the step only
     happens while prev_inp_per > e, otherwise the state passes through unchanged (mt_chn_fill_step_gated)."""
-    _need_cuda(nn_out, x_t, v_t, m_t, v_map0)
+    _need_cuda((nn_out, NET_DTYPES), x_t, v_t, m_t, v_map0)
     _no_grad_inputs("chn_fill", nn_out, x_t, v_t, m_t, v_map0)
     b = x_t.shape[0]
     h, w = x_t.shape[-2:]
@@ -778,14 +814,14 @@ def chn_fill(nn_out, x_t, v_t, m_t, v_map0, gate=None):
     x_new = _empty((b, 3, h, w), dtype=torch.float32, device=no.device)
     per = _empty(1, dtype=torch.float32, device=no.device)
     if gate is None:
-        _call("mt_chn_fill_step", _ptr(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
+        _call_net("mt_chn_fill_step", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
               _ptr(mt), mt.stride(0), _ptr(vm), vm.stride(0), _ptr(yc), _ptr(m_new), _ptr(x_new), _ptr(per),
               _ptr(reduce_workspace(no)), b, h * w, _stream(no))
     else:
         prev_per, e, y_prev = gate
         _need_cuda(prev_per, y_prev)
         y_prev = _contig(y_prev)
-        _call("mt_chn_fill_step_gated", _ptr(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
+        _call_net("mt_chn_fill_step_gated", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
               _ptr(mt), mt.stride(0), _ptr(vm), vm.stride(0), _ptr(y_prev), _ptr(prev_per.reshape(1)), float(e),
               _ptr(yc), _ptr(m_new), _ptr(x_new), _ptr(per), _ptr(reduce_workspace(no)), b, h * w, _stream(no))
     return yc, m_new, x_new, per[0]
@@ -829,7 +865,7 @@ def chn_fill_lanes(nn_out, x_t, m_t, v_map0, slots, x_state, m_state, y_out, per
     (model_chn.py:246-248) per lane, decided on the device.  Nothing is returned; nothing synchronises."""
     lanes, n_slots = nn_out.shape[0], x_state.shape[0]
     slots = _lane_slots(slots, lanes, n_slots)
-    _need_cuda(nn_out, x_t, m_t, v_map0, x_state, m_state, y_out, per_out)
+    _need_cuda((nn_out, NET_DTYPES), x_t, m_t, v_map0, x_state, m_state, y_out, per_out)
     _no_grad_inputs("chn_fill_lanes", nn_out, x_t, m_t, v_map0)
     h, w = x_t.shape[-2:]
     want = {"nn_out": (nn_out, (lanes, 3, h, w)), "x_t": (x_t, (lanes, 3, h, w)), "m_t": (m_t, (lanes, 1, h, w)),
@@ -848,7 +884,7 @@ def chn_fill_lanes(nn_out, x_t, m_t, v_map0, slots, x_state, m_state, y_out, per
     with torch.cuda.device(no.device):      # the size depends on the SM count of the launching device
         nbytes = int(_lib.load().mt_chn_fill_lanes_workspace_bytes(lanes))
     ws = zeroed_scratch(no, "lanes", nbytes)
-    _call("mt_chn_fill_lanes", _ptr(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(mt), mt.stride(0), _ptr(vm),
+    _call_net("mt_chn_fill_lanes", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(mt), mt.stride(0), _ptr(vm),
           vm.stride(0), _ptr(sl), _ptr(yo), yo.stride(0), yo.stride(1), _ptr(ms), ms.stride(0), _ptr(xs),
           xs.stride(0), xs.stride(1), _ptr(per_out), _ptr(ws), lanes, h * w, int(finalize is not None), e,
           int(force), _stream(no))
