@@ -48,8 +48,8 @@ def needs_build():
 
 
 def build_library(force=False, verbose=False, defines=(), out=None):
-    """defines / out: developer knobs for tuning sweeps (e.g. -DMT_WARP_MINB=8 into another
-    file name, selected at run time with MT_B200_LIB); the product build uses neither."""
+    """defines / out: developer builds (e.g. -DMT_DEV_PROBES into another file name,
+    selected at run time with MT_B200_LIB); the product build uses neither."""
     if not force and not needs_build() and not defines and out is None:
         return LIB
     cmd = [find_nvcc()] + NVCC_FLAGS + ["-I", os.path.join(ROOT, "include"), "-I", CSRC]

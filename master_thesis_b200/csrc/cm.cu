@@ -745,7 +745,7 @@ int launch_cm(CmArgs a, cudaStream_t st) {
         int keep = 0;
         const int ctas = (mode == 2 && (int64_t)(2 * a.C + 1) * a.f * a.P < (1ll << 31)) ? cm_group_ctas<R>(&keep) : 0;
         // batches parked in shared memory between the passes.  Default 0 since the kernels ahead of this one stopped
-        // pinning the SMs' shared-memory split (corr_tc.cu kCorrEarlyTrigger): without dynamic shared memory the kernel
+        // pinning the SMs' shared-memory split (pdl_sync in mt_common.cuh): without dynamic shared memory the kernel
         // runs with the full L1, which holds a CTA's most recent pass-1 lines for pass 2 - 44.0 -> 38.2 us per call at
         // B = 8 (cfg2 step 61.9 -> 56.4 us); parking 2 batches in shared memory gave the same time as parking none
         // while the split was pinned

@@ -52,14 +52,13 @@ namespace {
 constexpr int kTile = 256;        // largest output tile: TM rows (one or two UMMA M = 128 halves) x TN <= 256 columns
 constexpr int kBK = 32;
 constexpr int kUmmaK = 8;         // tf32: 32 B of K per instruction
-// griddepcontrol.launch_dependents right after the wait (pdl_sync, the library's default) lets the next kernel's CTAs
-// take their SM slots while this kernel runs.  For this kernel that is harmful: it holds ~200 KB of shared memory per
-// SM, the pre-launched CTAs arrive while the SM is in its maximum-shared-memory configuration, and because from then
-// on an SM is never empty between PDL-chained kernels the configuration (a few KB of L1) sticks - the gather kernels
-// that follow run with almost no L1.  Measured (profiles/r2_experiments.md, call Z): warp_l1_fwd at 256 x 256 77 ->
-// 121 us several launches after a correlation; cfg3 step 431 -> 364 us, cfg1 20.0 -> 18.4 us, default workload
-// 100.9 -> 97.7 us with the trigger left to the kernel's exit.  MT_CORR_EARLY_TRIGGER=1 restores the old behaviour.
-constexpr int kCorrEarlyTrigger = 0;
+// The correlation kernels only wait and leave griddepcontrol.launch_dependents to their exit (see pdl_sync).  With the
+// library's default trigger right after the wait, the next kernel's CTAs would take their SM slots while this kernel
+// runs: it holds ~200 KB of shared memory per SM, the pre-launched CTAs arrive while the SM is in its
+// maximum-shared-memory configuration, and because from then on an SM is never empty between PDL-chained kernels the
+// configuration (a few KB of L1) sticks - the gather kernels that follow run with almost no L1.  Measured
+// (profiles/r2_experiments.md, call Z): warp_l1_fwd at 256 x 256 77 -> 121 us several launches after a correlation;
+// cfg3 step 431 -> 364 us, cfg1 20.0 -> 18.4 us, default workload 100.9 -> 97.7 us with the trigger left to the exit.
 constexpr bool kPairDefault = true;   // CTA-pair kernel for large batches (see the heuristic in corr4d_tc_launch_ex)
 
 // MN-major, SWIZZLE_128B_BASE32B shared-memory matrix descriptor (sm_100 "version 1").
@@ -129,9 +128,6 @@ struct CorrTcArgs {
     float *loss;
     double inv_count;                              // 1 / (B F P P)
     int C, F, P, tiles_m, tiles_n, n_tiles;
-    // griddepcontrol.launch_dependents right after the wait (the library's default, see pdl_sync) or not at all
-    // (the next kernel of the stream is then scheduled as this kernel's CTAs exit): see corr4d_tc_launch_ex
-    int early_trigger;
 };
 
 // visibility of feature pixel p of plane `base` (see CorrTcArgs)
@@ -319,7 +315,6 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const uint32_t tmem_base = *tmem_slot;
     // everything above is on-chip setup and overlaps the tail of the previous kernel (PDL)
     pdl_wait();
-    if (a.early_trigger) pdl_launch();
 
     const int tiles_per_frame = a.tiles_m * a.tiles_n;
     if (warp == 0) {
@@ -612,7 +607,6 @@ corr_tc2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
     pdl_wait();
-    if (a.early_trigger) pdl_launch();
 
     const int tiles_per_frame = a.tiles_m * a.tiles_n;
     if (warp == 0) {
@@ -907,7 +901,6 @@ int corr4d_tc_launch_ex(const float *ft, int64_t ft_sb, int64_t ft_sc, const flo
     a.ticket = l1 ? reinterpret_cast<unsigned int *>(l1->partials) : nullptr;   // workspace: ticket header, then partials
     a.partials = l1 ? l1->partials + 4 : nullptr;
     a.inv_count = 1.0 / ((double)B * F * P * P);
-    a.early_trigger = tuning("MT_CORR_EARLY_TRIGGER", kCorrEarlyTrigger);
     a.tiles_m = P / (pair ? kTile : tm); a.tiles_n = P / tn;
     const int64_t n_tiles = (int64_t)B * F * a.tiles_m * a.tiles_n;
     MT_REQUIRE(n_tiles < (1ll << 30), "mt_corr4d_fwd: too many tiles");

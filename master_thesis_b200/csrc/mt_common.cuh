@@ -88,8 +88,8 @@ constexpr int64_t kWorkspaceBytes = kWsTicketBytes + int64_t(kMaxReduceBlocks) *
 // be scheduled once every CTA of this one has started, so waiting CTAs can never occupy
 // the slots this kernel still needs.  Exception: the persistent kernels that hold ~200 KB of
 // shared memory per SM (corr_tc.cu, warp_tma.cu) only wait and leave the trigger to their
-// exit - dependents pre-launched beside them pin the SM's shared-memory / L1 split at its
-// maximum-shared-memory setting for the whole PDL chain behind them (corr_tc.cu kCorrEarlyTrigger).
+// exit - dependents pre-launched beside them would pin the SM's shared-memory / L1 split at its
+// maximum-shared-memory setting for the whole PDL chain behind them (measured in corr_tc.cu).
 __device__ __forceinline__ void pdl_sync() {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");

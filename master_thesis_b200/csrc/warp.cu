@@ -13,9 +13,9 @@
 // (H, W) planes.  Lanes of a warp own CONSECUTIVE pixels of the flattened plane,
 // so a gather instruction of a coherent flow touches 1-2 cache lines (a
 // 4-pixels-per-thread mapping was measured at 30% of HBM peak: every gather
-// spanned 4 lines, see profiles/).  Each thread processes U = 4 pixels 256 apart
-// for memory-level parallelism: all 4 * (4C + 1..4) gathers are issued before
-// the first use.  Grid loads (8 B/lane) and all stores (4 B/lane) are fully
+// spanned 4 lines, see profiles/).  Each thread processes kRows = 2 vertically
+// adjacent pixels of one column, and all their gathers are issued before the
+// first use.  Grid loads (8 B/lane) and all stores (4 B/lane) are fully
 // coalesced 128 B-per-warp streaming accesses.
 #include <math.h>
 
@@ -25,39 +25,17 @@
 namespace mt {
 namespace {
 
-constexpr int kCols = 128;     // forward kernel: threads per CTA = columns per CTA
-#ifndef MT_WARP_ROWS
-#define MT_WARP_ROWS 2
-#endif
-#ifndef MT_TAP_REUSE
-#define MT_TAP_REUSE 1
-#endif
-constexpr int kRows = MT_WARP_ROWS;  // forward kernel: rows per thread and iteration (swept on B200: 2 beats 4)
-constexpr bool kTapReuse = MT_TAP_REUSE != 0;  // vertically adjacent pixels of a thread share a source row of taps
-constexpr int kIters = 1;      // forward kernel: row groups per thread (swept: more groups per thread is slower)
+constexpr int kCols = 128;  // threads per CTA = columns per CTA
+constexpr int kRows = 2;    // rows per thread of every strip kernel (swept on B200: 2 beats 1 and 4, profiles/r2_experiments.md)
 // Minimum resident CTAs per SM given to ptxas.  This is a SCHEDULING knob, not an occupancy one:
 // with a bare __launch_bounds__(128) ptxas minimises registers (32-40) and does so by sinking the
 // gathers between the interpolation FMAs - 4 dependent batches of ~8 loads per thread instead of
 // all 32 in flight (SASS checked with cuobjdump; profiles/r1_experiments.md).  With a register
 // budget stated, all gathers of a thread are issued before the first use.
-#ifndef MT_WARP_MINB
-#define MT_WARP_MINB 8
-#endif
-#ifndef MT_WARP_MINB1
-#define MT_WARP_MINB1 10  // 1 row per thread: 13 taps in flight, more resident warps
-#endif
-#ifndef MT_WARP_MINB4
-#define MT_WARP_MINB4 4  // 4 rows per thread: 40 taps in flight need the registers
-#endif
-#ifndef MT_WARPB_MINB
-#define MT_WARPB_MINB 6
-#endif
-#ifndef MT_WARPL1F_MINB
-#define MT_WARPL1F_MINB 8  // fused-loss forward, loss only
-#endif
-#ifndef MT_WARPL1B_MINB
-#define MT_WARPL1B_MINB 8  // fused-loss backward: 64 registers, no spills, 79.4 -> 75.4 us at cfg3 (the forward spills at 8)
-#endif
+constexpr int kWarpMinB = 8;
+constexpr int kWarpBMinB = 6;
+constexpr int kWarpL1FMinB = 8;  // fused-loss forward, loss only
+constexpr int kWarpL1BMinB = 8;  // fused-loss backward: 64 registers, no spills, 79.4 -> 75.4 us at cfg3 (the forward spills at 8)
 
 // Forward-kernel arguments: every offset is a 32-bit ELEMENT offset (the launcher
 // checks the ranges), because 64-bit stride arithmetic dominated the per-thread
@@ -67,7 +45,6 @@ struct WarpFwdArgs {
     float *x_al, *v_al, *v_map;
     int x_sb, x_sc, x_sf, vis_sb, vis_sf, mt_sb, xa_sb, xa_sc, xa_sf;
     int F, P;
-    int iters;         // row groups of U rows per thread (per-thread setup is amortised over them)
     unsigned f_magic;  // ceil(2^32 / F): b = umulhi(n, f_magic) for n < 2^16; 0 when F == 1 (b = n)
     Sampler sp;
     bool from_mask;
@@ -79,11 +56,9 @@ struct WarpFwdArgs {
     // (FlowsUtils.resize_flow(mode='bilinear'), utils.py:107-126 as called at model_dfpn.py:100-101)
     int gh, gw;
     float gsy, gsx;  // gh / H, gw / W in fp32
-    int early_trigger;  // griddepcontrol.launch_dependents right after the wait (default) or only at exit
 };
-constexpr int kMaxRowsPerCta = 32;
 
-// Forward kernel.  Thread = one column x, U consecutive rows; a warp = 32
+// Forward kernel.  Thread = one column x, kRows consecutive rows; a warp = 32
 // consecutive columns of one row, so grid loads and all stores are 128 B
 // coalesced and no integer division is needed.  If every tap of every lane of
 // the warp is interior (0 <= xw <= W-2, 0 <= yn <= H-2: the common case) the
@@ -99,31 +74,30 @@ constexpr int kMaxRowsPerCta = 32;
 // needs no second pass over the aligned frame (SURVEY 8f-2).
 // LOWRES (dense flow only): the flow is given at gh x gw and bilinearly resized to H x W in the kernel - the
 // resized flow is never written or read back (SURVEY 8f-1); bit-identical to resizing first.
-template <int C, int U, int VIS, bool AFFINE, bool FULL, bool PACK = false, bool LOWRES = false>
-__global__ void __launch_bounds__(kCols, U >= 4 ? MT_WARP_MINB4 : (U == 1 ? MT_WARP_MINB1 : MT_WARP_MINB)) warp_fwd_kernel(const WarpFwdArgs a) {
+template <int C, int VIS, bool AFFINE, bool FULL, bool PACK = false, bool LOWRES = false>
+__global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFwdArgs a) {
     static_assert(!(AFFINE && LOWRES), "a theta needs no resize");
-    pdl_wait();
-    if (a.early_trigger) pdl_launch();
-    __shared__ float s_by[kMaxRowsPerCta];
-    __shared__ Lin s_ly[LOWRES ? kMaxRowsPerCta : 1];
+    constexpr int U = kRows;
+    pdl_sync();
+    __shared__ float s_by[U];
+    __shared__ Lin s_ly[LOWRES ? U : 1];
     const int W = a.sp.W, H = a.sp.H;
     // lanes past the last column stay alive (the warp vote below needs every lane)
     // on a clamped column and are masked at the stores
     const bool live = (int)(blockIdx.x * kCols + threadIdx.x) < W;
     const int x = min((int)(blockIdx.x * kCols + threadIdx.x), W - 1);
-    const int rows_cta = U * a.iters;
-    const int yb = blockIdx.y * rows_cta;
+    const int y0 = blockIdx.y * U;
     const unsigned n = blockIdx.z;
     const int b = a.f_magic ? (int)__umulhi(n, a.f_magic) : (int)n, f = (int)n - b * a.F;
     const bool ac = a.sp.ac;
-    if (AFFINE) {  // row term of the affine grid: rows_cta values per CTA
-        if ((int)threadIdx.x < rows_cta)
-            s_by[threadIdx.x] = base_coord(min(yb + (int)threadIdx.x, H - 1), H, a.sp.stepy, ac);
+    if (AFFINE) {  // row term of the affine grid: U values per CTA
+        if ((int)threadIdx.x < U)
+            s_by[threadIdx.x] = base_coord(min(y0 + (int)threadIdx.x, H - 1), H, a.sp.stepy, ac);
         __syncthreads();
     }
     Lin lx;
     if (LOWRES) {  // row terms of the flow resize once per CTA, the column term once per thread
-        if ((int)threadIdx.x < rows_cta) s_ly[threadIdx.x] = lin_index(min(yb + (int)threadIdx.x, H - 1), a.gh, H, a.gsy);
+        if ((int)threadIdx.x < U) s_ly[threadIdx.x] = lin_index(min(y0 + (int)threadIdx.x, H - 1), a.gh, H, a.gsy);
         lx = lin_index(x, a.gw, W, a.gsx);
         __syncthreads();
     }
@@ -142,185 +116,170 @@ __global__ void __launch_bounds__(kCols, U >= 4 ? MT_WARP_MINB4 : (U == 1 ? MT_W
     }
     const float wm2 = a.sp.wmax - 1.0f, hm2 = a.sp.hmax - 1.0f;
 
-    // dense flow: the grid values of the NEXT row group are requested before the gathers of the current one, so a
-    // CTA that walks several row groups (iters > 1) has one dependent DRAM round trip per group instead of two
     constexpr bool kDense = !AFFINE && !LOWRES;
-    float2 g_next[U];
+    float2 g[U];
     if (kDense) {
 #pragma unroll
         for (int k = 0; k < U; ++k)
-            g_next[k] = (yb + k < H) ? __ldcs(reinterpret_cast<const float2 *>(a.grid) + ((int)n * a.P + (yb + k) * W + x))
-                                     : make_float2(0.0f, 0.0f);
+            g[k] = (y0 + k < H) ? __ldcs(reinterpret_cast<const float2 *>(a.grid) + ((int)n * a.P + (y0 + k) * W + x))
+                                : make_float2(0.0f, 0.0f);
     }
-    // the per-thread setup above is paid once for U * iters pixels
-#pragma unroll 1
-    for (int it = 0; it < a.iters; ++it) {
-        const int y0 = yb + it * U;
-        if (y0 >= H) break;
-        const int p0 = y0 * W + x;
-        const int np0 = (int)n * a.P + p0;
-        // issue the target-mask loads first: they are only needed by the stores at the end
-        float mtv[U];
-        if (FULL || PACK || a.v_map) {  // PACK needs v_map for channel 8 of nn_in also when v_map itself is not requested
+    const int p0 = y0 * W + x;
+    const int np0 = (int)n * a.P + p0;
+    // issue the target-mask loads first: they are only needed by the stores at the end
+    float mtv[U];
+    if (FULL || PACK || a.v_map) {  // PACK needs v_map for channel 8 of nn_in also when v_map itself is not requested
 #pragma unroll
-            for (int k = 0; k < U; ++k) mtv[k] = (y0 + k < H) ? __ldcs(a.m_target + (mto + p0 + k * W)) : 0.0f;
-        }
-        float xtv[PACK ? 3 : 1][U], vtv[U];
-        if (PACK) {
-#pragma unroll
-            for (int k = 0; k < U; ++k) {
-                const bool in = y0 + k < H;
-                vtv[k] = in ? __ldg(a.v_t + (b * a.vt_sb + p0 + k * W)) : 0.0f;
-#pragma unroll
-                for (int c = 0; c < 3; ++c) xtv[c][k] = in ? __ldg(a.x_t + (b * a.xt_sb + c * a.xt_sc + p0 + k * W)) : 0.0f;
-            }
-        }
-        float ix[U], iy[U], xw[U], yn[U];
-        float wnw[U], wne[U], wsw[U], wse[U];
-        bool interior = true;
+        for (int k = 0; k < U; ++k) mtv[k] = (y0 + k < H) ? __ldcs(a.m_target + (mto + p0 + k * W)) : 0.0f;
+    }
+    float xtv[PACK ? 3 : 1][U], vtv[U];
+    if (PACK) {
 #pragma unroll
         for (int k = 0; k < U; ++k) {
-            float gx, gy;
-            if (AFFINE) {
-                const float by = s_by[it * U + k];
-                gx = __fadd_rn(__fmaf_rn(by, t1, bxt0), t2);  // fma(by, t1, bx*t0) + t2 (pinned order)
-                gy = __fadd_rn(__fmaf_rn(by, t4, bxt3), t5);
-            } else if (LOWRES) {
-                const Lin ly = s_ly[it * U + k];
-                const float2 *fl = reinterpret_cast<const float2 *>(a.grid) + (int)n * (a.gh * a.gw);
-                const float2 g = lin_flow(fl + ly.i0 * a.gw, fl + ly.i1 * a.gw, lx, ly.l0, ly.l1);
-                gx = g.x; gy = g.y;
-            } else {
-                gx = g_next[k].x; gy = g_next[k].y;  // rows past H hold (0, 0)
-            }
-            ix[k] = unnormalize(gx, a.sp.sfx, ac);
-            iy[k] = unnormalize(gy, a.sp.sfy, ac);
-            xw[k] = floorf(ix[k]);
-            yn[k] = floorf(iy[k]);
-            const float w = __fsub_rn(ix[k], xw[k]), e = __fsub_rn(1.0f, w);
-            const float nn = __fsub_rn(iy[k], yn[k]), ss = __fsub_rn(1.0f, nn);
-            wnw[k] = __fmul_rn(ss, e); wne[k] = __fmul_rn(ss, w);
-            wsw[k] = __fmul_rn(nn, e); wse[k] = __fmul_rn(nn, w);
-            // rows past the end of the frame are computed (harmlessly) and never stored
-            interior = interior && (xw[k] >= 0.0f) && (xw[k] <= wm2) && (yn[k] >= 0.0f) && (yn[k] <= hm2);
+            const bool in = y0 + k < H;
+            vtv[k] = in ? __ldg(a.v_t + (b * a.vt_sb + p0 + k * W)) : 0.0f;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) xtv[c][k] = in ? __ldg(a.x_t + (b * a.xt_sb + c * a.xt_sc + p0 + k * W)) : 0.0f;
         }
-        if (kDense && it + 1 < a.iters) {
+    }
+    float ix[U], iy[U], xw[U], yn[U];
+    float wnw[U], wne[U], wsw[U], wse[U];
+    bool interior = true;
 #pragma unroll
-            for (int k = 0; k < U; ++k)
-                g_next[k] = (y0 + U + k < H) ? __ldcs(reinterpret_cast<const float2 *>(a.grid) + (np0 + (U + k) * W))
-                                             : make_float2(0.0f, 0.0f);
-        }
-        float xa[C][U], va[U];
-        if (__all_sync(0xffffffffu, interior)) {
-            // ---------------- fast path ----------------
-            // Row reuse: a thread owns U vertically adjacent pixels, and where the flow is locally coherent the upper
-            // taps of pixel k are the lower taps of pixel k - 1 (same column, next source row).  Those lanes skip
-            // the two loads (predicated off) and take the registers of the row above.  A gather instruction costs the
-            // L1 one wavefront per 128-byte line its lanes touch, and the kernel is bound by exactly that: fewer
-            // lanes per tap instruction = fewer lines.  The values are the ones the loads would have returned.
-            float c00[C + 1][U], c01[C + 1][U], c10[C + 1][U], c11[C + 1][U];
-            int o[U];
-            bool same[U];
-#pragma unroll
-            for (int k = 0; k < U; ++k) {
-                o[k] = (int)yn[k] * W + (int)xw[k];
-                same[k] = kTapReuse && k > 0 && o[k] == o[k - 1] + W;
-            }
-#pragma unroll
-            for (int k = 0; k < U; ++k) {
-#pragma unroll
-                for (int c = 0; c < C; ++c) {
-                    const float *r0 = a.x + (xo + c * a.x_sc + o[k]);
-                    const float *r1 = a.x + (xo + c * a.x_sc + o[k] + W);
-                    c00[c][k] = 0.0f; c01[c][k] = 0.0f;
-                    if (!same[k]) { c00[c][k] = __ldg(r0); c01[c][k] = __ldg(r0 + 1); }
-                    c10[c][k] = __ldg(r1); c11[c][k] = __ldg(r1 + 1);
-                }
-                if (VIS == 2) {
-                    const float *r0 = vp + o[k];
-                    const float *r1 = vp + (o[k] + W);
-                    c00[C][k] = 0.0f; c01[C][k] = 0.0f;
-                    if (!same[k]) { c00[C][k] = __ldg(r0); c01[C][k] = __ldg(r0 + 1); }
-                    c10[C][k] = __ldg(r1); c11[C][k] = __ldg(r1 + 1);
-                } else {
-                    // nearest: rint (half-to-even) lands on one of the 4 interior taps: in bounds
-                    c00[C][k] = __ldg(vp + ((int)rintf(iy[k]) * W + (int)rintf(ix[k])));
-                }
-            }
-#pragma unroll
-            for (int k = 1; k < U; ++k) {
-#pragma unroll
-                for (int c = 0; c < (VIS == 2 ? C + 1 : C); ++c) {
-                    c00[c][k] = same[k] ? c10[c][k - 1] : c00[c][k];
-                    c01[c][k] = same[k] ? c11[c][k - 1] : c01[c][k];
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < U; ++k) {
-#pragma unroll
-                for (int c = 0; c < C; ++c)
-                    xa[c][k] = __fmaf_rn(c11[c][k], wse[k], __fmaf_rn(c10[c][k], wsw[k],
-                               __fmaf_rn(c01[c][k], wne[k], __fmul_rn(c00[c][k], wnw[k]))));
-                if (VIS == 2) {
-                    float v00 = c00[C][k], v01 = c01[C][k], v10 = c10[C][k], v11 = c11[C][k];
-                    if (a.from_mask) {
-                        v00 = __fsub_rn(1.0f, v00); v01 = __fsub_rn(1.0f, v01);
-                        v10 = __fsub_rn(1.0f, v10); v11 = __fsub_rn(1.0f, v11);
-                    }
-                    const float vs = __fmaf_rn(v11, wse[k], __fmaf_rn(v10, wsw[k],
-                                     __fmaf_rn(v01, wne[k], __fmul_rn(v00, wnw[k]))));
-                    va[k] = vs > 0.5f ? 1.0f : 0.0f;  // strict, model_cpn.py:88
-                } else {
-                    va[k] = a.from_mask ? __fsub_rn(1.0f, c00[C][k]) : c00[C][k];
-                }
-            }
+    for (int k = 0; k < U; ++k) {
+        float gx, gy;
+        if (AFFINE) {
+            const float by = s_by[k];
+            gx = __fadd_rn(__fmaf_rn(by, t1, bxt0), t2);  // fma(by, t1, bx*t0) + t2 (pinned order)
+            gy = __fadd_rn(__fmaf_rn(by, t4, bxt3), t5);
+        } else if (LOWRES) {
+            const Lin ly = s_ly[k];
+            const float2 *fl = reinterpret_cast<const float2 *>(a.grid) + (int)n * (a.gh * a.gw);
+            const float2 gl = lin_flow(fl + ly.i0 * a.gw, fl + ly.i1 * a.gw, lx, ly.l0, ly.l1);
+            gx = gl.x; gy = gl.y;
         } else {
-            // ---------------- generic path (border warps, out-of-frame flows) ----------------
+            gx = g[k].x; gy = g[k].y;  // rows past H hold (0, 0)
+        }
+        ix[k] = unnormalize(gx, a.sp.sfx, ac);
+        iy[k] = unnormalize(gy, a.sp.sfy, ac);
+        xw[k] = floorf(ix[k]);
+        yn[k] = floorf(iy[k]);
+        const float w = __fsub_rn(ix[k], xw[k]), e = __fsub_rn(1.0f, w);
+        const float nn = __fsub_rn(iy[k], yn[k]), ss = __fsub_rn(1.0f, nn);
+        wnw[k] = __fmul_rn(ss, e); wne[k] = __fmul_rn(ss, w);
+        wsw[k] = __fmul_rn(nn, e); wse[k] = __fmul_rn(nn, w);
+        // rows past the end of the frame are computed (harmlessly) and never stored
+        interior = interior && (xw[k] >= 0.0f) && (xw[k] <= wm2) && (yn[k] >= 0.0f) && (yn[k] <= hm2);
+    }
+    float xa[C][U], va[U];
+    if (__all_sync(0xffffffffu, interior)) {
+        // ---------------- fast path ----------------
+        // Row reuse: a thread owns U vertically adjacent pixels, and where the flow is locally coherent the upper
+        // taps of pixel k are the lower taps of pixel k - 1 (same column, next source row).  Those lanes skip
+        // the two loads (predicated off) and take the registers of the row above.  A gather instruction costs the
+        // L1 one wavefront per 128-byte line its lanes touch, and the kernel is bound by exactly that: fewer
+        // lanes per tap instruction = fewer lines.  The values are the ones the loads would have returned.
+        float c00[C + 1][U], c01[C + 1][U], c10[C + 1][U], c11[C + 1][U];
+        int o[U];
+        bool same[U];
 #pragma unroll
-            for (int k = 0; k < U; ++k) {
-                const Bil bl = bil_params(ix[k], iy[k], a.sp);
+        for (int k = 0; k < U; ++k) {
+            o[k] = (int)yn[k] * W + (int)xw[k];
+            same[k] = k > 0 && o[k] == o[k - 1] + W;
+        }
 #pragma unroll
-                for (int c = 0; c < C; ++c) xa[c][k] = interp(gather(a.x + (xo + c * a.x_sc), bl, W), bl);
-                if (VIS == 2) {
-                    Corners cv = gather(vp, bl, W);
-                    if (a.from_mask) {  // v = 1 - m inside the frame, 0 outside (zero padding of v)
-                        cv.nw = (bl.y0 && bl.x0) ? __fsub_rn(1.0f, cv.nw) : 0.0f;
-                        cv.ne = (bl.y0 && bl.x1) ? __fsub_rn(1.0f, cv.ne) : 0.0f;
-                        cv.sw = (bl.y1 && bl.x0) ? __fsub_rn(1.0f, cv.sw) : 0.0f;
-                        cv.se = (bl.y1 && bl.x1) ? __fsub_rn(1.0f, cv.se) : 0.0f;
-                    }
-                    va[k] = interp(cv, bl) > 0.5f ? 1.0f : 0.0f;
-                } else {
-                    va[k] = nearest(vp, ix[k], iy[k], a.sp, a.from_mask);
-                }
+        for (int k = 0; k < U; ++k) {
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const float *r0 = a.x + (xo + c * a.x_sc + o[k]);
+                const float *r1 = a.x + (xo + c * a.x_sc + o[k] + W);
+                c00[c][k] = 0.0f; c01[c][k] = 0.0f;
+                if (!same[k]) { c00[c][k] = __ldg(r0); c01[c][k] = __ldg(r0 + 1); }
+                c10[c][k] = __ldg(r1); c11[c][k] = __ldg(r1 + 1);
+            }
+            if (VIS == 2) {
+                const float *r0 = vp + o[k];
+                const float *r1 = vp + (o[k] + W);
+                c00[C][k] = 0.0f; c01[C][k] = 0.0f;
+                if (!same[k]) { c00[C][k] = __ldg(r0); c01[C][k] = __ldg(r0 + 1); }
+                c10[C][k] = __ldg(r1); c11[C][k] = __ldg(r1 + 1);
+            } else {
+                // nearest: rint (half-to-even) lands on one of the 4 interior taps: in bounds
+                c00[C][k] = __ldg(vp + ((int)rintf(iy[k]) * W + (int)rintf(ix[k])));
             }
         }
-        // ---------------- stores (coalesced, streaming) ----------------
-        if (live) {
 #pragma unroll
-            for (int k = 0; k < U; ++k) {
-                if (y0 + k >= H) break;
-                if (FULL || a.x_al) {
+        for (int k = 1; k < U; ++k) {
 #pragma unroll
-                    for (int c = 0; c < C; ++c) st_stream1(a.x_al + (xao + p0 + c * a.xa_sc + k * W), xa[c][k]);
-                }
-                if (FULL || a.v_al) st_stream1(a.v_al + (np0 + k * W), va[k]);
-                const float vmap = (FULL || PACK || a.v_map) ? clamp01(__fsub_rn(va[k], __fsub_rn(1.0f, mtv[k]))) : 0.0f;
-                if (FULL || a.v_map)  // clamp(v_al - (1 - m_t), 0, 1)
-                    st_stream1(a.v_map + (np0 + k * W), vmap);
-                if (PACK) {
-                    float *o = a.nn_in + ((int)n * 9 * a.P + p0 + k * W);
-#pragma unroll
-                    for (int c = 0; c < 3; ++c) {  // (x - mean) / std   model_chn.py:73-74
-                        const float m = chan_mean(c), sd = chan_std(c);
-                        st_stream1(o + c * a.P, __fdiv_rn(__fsub_rn(xtv[c][k], m), sd));
-                        st_stream1(o + (3 + c) * a.P, __fdiv_rn(__fsub_rn(xa[c][k], m), sd));
-                    }
-                    st_stream1(o + 6 * a.P, vtv[k]);
-                    st_stream1(o + 7 * a.P, va[k]);
-                    st_stream1(o + 8 * a.P, vmap);
-                }
+            for (int c = 0; c < (VIS == 2 ? C + 1 : C); ++c) {
+                c00[c][k] = same[k] ? c10[c][k - 1] : c00[c][k];
+                c01[c][k] = same[k] ? c11[c][k - 1] : c01[c][k];
             }
+        }
+#pragma unroll
+        for (int k = 0; k < U; ++k) {
+#pragma unroll
+            for (int c = 0; c < C; ++c)
+                xa[c][k] = __fmaf_rn(c11[c][k], wse[k], __fmaf_rn(c10[c][k], wsw[k],
+                           __fmaf_rn(c01[c][k], wne[k], __fmul_rn(c00[c][k], wnw[k]))));
+            if (VIS == 2) {
+                float v00 = c00[C][k], v01 = c01[C][k], v10 = c10[C][k], v11 = c11[C][k];
+                if (a.from_mask) {
+                    v00 = __fsub_rn(1.0f, v00); v01 = __fsub_rn(1.0f, v01);
+                    v10 = __fsub_rn(1.0f, v10); v11 = __fsub_rn(1.0f, v11);
+                }
+                const float vs = __fmaf_rn(v11, wse[k], __fmaf_rn(v10, wsw[k],
+                                 __fmaf_rn(v01, wne[k], __fmul_rn(v00, wnw[k]))));
+                va[k] = vs > 0.5f ? 1.0f : 0.0f;  // strict, model_cpn.py:88
+            } else {
+                va[k] = a.from_mask ? __fsub_rn(1.0f, c00[C][k]) : c00[C][k];
+            }
+        }
+    } else {
+        // ---------------- generic path (border warps, out-of-frame flows) ----------------
+#pragma unroll
+        for (int k = 0; k < U; ++k) {
+            const Bil bl = bil_params(ix[k], iy[k], a.sp);
+#pragma unroll
+            for (int c = 0; c < C; ++c) xa[c][k] = interp(gather(a.x + (xo + c * a.x_sc), bl, W), bl);
+            if (VIS == 2) {
+                Corners cv = gather(vp, bl, W);
+                if (a.from_mask) {  // v = 1 - m inside the frame, 0 outside (zero padding of v)
+                    cv.nw = (bl.y0 && bl.x0) ? __fsub_rn(1.0f, cv.nw) : 0.0f;
+                    cv.ne = (bl.y0 && bl.x1) ? __fsub_rn(1.0f, cv.ne) : 0.0f;
+                    cv.sw = (bl.y1 && bl.x0) ? __fsub_rn(1.0f, cv.sw) : 0.0f;
+                    cv.se = (bl.y1 && bl.x1) ? __fsub_rn(1.0f, cv.se) : 0.0f;
+                }
+                va[k] = interp(cv, bl) > 0.5f ? 1.0f : 0.0f;
+            } else {
+                va[k] = nearest(vp, ix[k], iy[k], a.sp, a.from_mask);
+            }
+        }
+    }
+    // ---------------- stores (coalesced, streaming) ----------------
+    if (!live) return;
+#pragma unroll
+    for (int k = 0; k < U; ++k) {
+        if (y0 + k >= H) break;
+        if (FULL || a.x_al) {
+#pragma unroll
+            for (int c = 0; c < C; ++c) st_stream1(a.x_al + (xao + p0 + c * a.xa_sc + k * W), xa[c][k]);
+        }
+        if (FULL || a.v_al) st_stream1(a.v_al + (np0 + k * W), va[k]);
+        const float vmap = (FULL || PACK || a.v_map) ? clamp01(__fsub_rn(va[k], __fsub_rn(1.0f, mtv[k]))) : 0.0f;
+        if (FULL || a.v_map)  // clamp(v_al - (1 - m_t), 0, 1)
+            st_stream1(a.v_map + (np0 + k * W), vmap);
+        if (PACK) {
+            float *o = a.nn_in + ((int)n * 9 * a.P + p0 + k * W);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {  // (x - mean) / std   model_chn.py:73-74
+                const float m = chan_mean(c), sd = chan_std(c);
+                st_stream1(o + c * a.P, __fdiv_rn(__fsub_rn(xtv[c][k], m), sd));
+                st_stream1(o + (3 + c) * a.P, __fdiv_rn(__fsub_rn(xa[c][k], m), sd));
+            }
+            st_stream1(o + 6 * a.P, vtv[k]);
+            st_stream1(o + 7 * a.P, va[k]);
+            st_stream1(o + 8 * a.P, vmap);
         }
     }
 }
@@ -381,7 +340,7 @@ __device__ __forceinline__ void gather_taps(const float *__restrict__ x, int xo,
 #pragma unroll
         for (int k = 0; k < U; ++k) {
             o[k] = (int)t.yn[k] * sp.W + (int)t.xw[k];
-            same[k] = kTapReuse && k > 0 && o[k] == o[k - 1] + sp.W;
+            same[k] = k > 0 && o[k] == o[k - 1] + sp.W;
         }
 #pragma unroll
         for (int k = 0; k < U; ++k) {
@@ -418,11 +377,6 @@ __device__ __forceinline__ float interp_k(const Corners &q, const Taps<U> &t, in
            __fmaf_rn(q.ne, __fmul_rn(t.s[k], t.w[k]), __fmul_rn(q.nw, __fmul_rn(t.s[k], t.e[k])))));
 }
 
-#ifndef MT_WARPB_ROWS
-#define MT_WARPB_ROWS 2
-#endif
-constexpr int kRowsB = MT_WARPB_ROWS;  // rows per thread in the dense-flow kernels
-
 // ---- backward w.r.t. the dense grid (generic upstream gradient) -------------
 struct WarpBwdArgs {
     const float *x, *grid, *gout;
@@ -434,7 +388,7 @@ struct WarpBwdArgs {
 };
 
 template <int C, int U>
-__global__ void __launch_bounds__(kCols, MT_WARPB_MINB) warp_bwd_grid_kernel(const WarpBwdArgs a) {
+__global__ void __launch_bounds__(kCols, kWarpBMinB) warp_bwd_grid_kernel(const WarpBwdArgs a) {
     pdl_sync();
     const int W = a.sp.W, H = a.sp.H;
     const bool live = (int)(blockIdx.x * kCols + threadIdx.x) < W;
@@ -491,7 +445,7 @@ __device__ __forceinline__ float mask_out_of(float gx, float gy) {
 // MAT: the aligned frames / visibilities are also written (a consumer asked for them); the loss-only instantiation
 // carries neither the stores nor the nearest-tap gather and fits the 64-register budget of 8 CTAs per SM.
 template <int U, bool MAT>
-__global__ void __launch_bounds__(kCols, MAT ? MT_WARPB_MINB : MT_WARPL1F_MINB) warp_l1_fwd_kernel(const WarpL1Args a) {
+__global__ void __launch_bounds__(kCols, MAT ? kWarpBMinB : kWarpL1FMinB) warp_l1_fwd_kernel(const WarpL1Args a) {
     pdl_sync();
     __shared__ float red[2 * 32];
     float acc[2] = {0.0f, 0.0f};  // sum |x_t*M - x_al*M| over 3 channels, sum M
@@ -559,7 +513,7 @@ __global__ void __launch_bounds__(kCols, MAT ? MT_WARPB_MINB : MT_WARPL1F_MINB) 
 // d loss / d flow in one pass: recomputes the sampling, never materialises
 // x_aligned or its gradient.
 template <int U>
-__global__ void __launch_bounds__(kCols, MT_WARPL1B_MINB) warp_l1_bwd_kernel(const WarpL1Args a) {
+__global__ void __launch_bounds__(kCols, kWarpL1BMinB) warp_l1_bwd_kernel(const WarpL1Args a) {
     pdl_sync();
     const int W = a.sp.W, H = a.sp.H;
     const bool live = (int)(blockIdx.x * kCols + threadIdx.x) < W;
@@ -673,7 +627,6 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     a.x_t = a.v_t = nullptr; a.nn_in = nullptr; a.xt_sb = a.xt_sc = a.vt_sb = 0;
     a.gh = lowres ? gh : H; a.gw = lowres ? gw : W;
     a.gsy = (float)a.gh / (float)H; a.gsx = (float)a.gw / (float)W;
-    a.early_trigger = tuning("MT_WARP_EARLY_TRIGGER", 1);
     if (pack) {
         MT_REQUIRE(C == 3 && m_target && pack->x_t && pack->v_t && pack->nn_in, "mt_warp_pack_fwd: C must be 3, no NULL input");
         MT_REQUIRE(pack->xt_sb >= 0 && pack->xt_sc >= 0 && pack->vt_sb >= 0 &&
@@ -684,36 +637,20 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     }
     const bool affine = (flags & MT_GRID_AFFINE) != 0;
     const bool vis_bil = (flags & MT_VIS_BILINEAR) != 0;
-    int rows = tuning("MT_WARP_ROWS", kRows);
-    rows = rows == 1 && !pack && !lowres ? 1 : (rows == 4 ? 4 : 2);
-    int iters = tuning("MT_WARP_ITERS", kIters);
-    if (iters < 1) iters = 1;
-    if (iters * rows > kMaxRowsPerCta) iters = kMaxRowsPerCta / rows;
-    a.iters = iters;
-    dim3 block(kCols), gridd((W + kCols - 1) / kCols, (H + rows * iters - 1) / (rows * iters), B * F);
+    dim3 block(kCols), gridd((W + kCols - 1) / kCols, (H + kRows - 1) / kRows, B * F);
     cudaStream_t st = (cudaStream_t)stream;
     const bool full = x_aligned && v_aligned && v_map;
     if (pack && lowres) {  // DFPN inference step at a frame size other than the flow's 256 x 256
-        if (rows == 2) launch(warp_fwd_kernel<3, 2, 1, false, false, true, true>, gridd, block, 0, st, a);
-        else launch(warp_fwd_kernel<3, 4, 1, false, false, true, true>, gridd, block, 0, st, a);
+        launch(warp_fwd_kernel<3, 1, false, false, true, true>, gridd, block, 0, st, a);
         return launch_status("mt_warp_pack_lowres_fwd");
     }
     if (lowres) {
-        if (rows == 2) {
-            if (full) launch(warp_fwd_kernel<3, 2, 1, false, true, false, true>, gridd, block, 0, st, a);
-            else launch(warp_fwd_kernel<3, 2, 1, false, false, false, true>, gridd, block, 0, st, a);
-        } else {
-            if (full) launch(warp_fwd_kernel<3, 4, 1, false, true, false, true>, gridd, block, 0, st, a);
-            else launch(warp_fwd_kernel<3, 4, 1, false, false, false, true>, gridd, block, 0, st, a);
-        }
+        if (full) launch(warp_fwd_kernel<3, 1, false, true, false, true>, gridd, block, 0, st, a);
+        else launch(warp_fwd_kernel<3, 1, false, false, false, true>, gridd, block, 0, st, a);
         return launch_status("mt_warp_lowres_fwd");
     }
     if (pack) {
-#define MT_WARP_PACK_GO(VV, AA)                                                                       \
-    do {                                                                                              \
-        if (rows == 2) launch(warp_fwd_kernel<3, 2, VV, AA, false, true>, gridd, block, 0, st, a);    \
-        else launch(warp_fwd_kernel<3, 4, VV, AA, false, true>, gridd, block, 0, st, a);              \
-    } while (0)
+#define MT_WARP_PACK_GO(VV, AA) launch(warp_fwd_kernel<3, VV, AA, false, true>, gridd, block, 0, st, a)
         if (vis_bil) { if (affine) MT_WARP_PACK_GO(2, true); else MT_WARP_PACK_GO(2, false); }
         else         { if (affine) MT_WARP_PACK_GO(1, true); else MT_WARP_PACK_GO(1, false); }
 #undef MT_WARP_PACK_GO
@@ -726,12 +663,7 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
         if (rc < 0) return rc;
         if (rc == 1) return launch_status("mt_warp_fwd");
     }
-#define MT_WARP_GO(CC, VV, AA, FF)                                                  \
-    do {                                                                            \
-        if (rows == 2) launch(warp_fwd_kernel<CC, 2, VV, AA, FF>, gridd, block, 0, st, a); \
-        else if (rows == 1) launch(warp_fwd_kernel<CC, 1, VV, AA, FF>, gridd, block, 0, st, a); \
-        else launch(warp_fwd_kernel<CC, 4, VV, AA, FF>, gridd, block, 0, st, a);        \
-    } while (0)
+#define MT_WARP_GO(CC, VV, AA, FF) launch(warp_fwd_kernel<CC, VV, AA, FF>, gridd, block, 0, st, a)
 #define MT_WARP_PICK(CC)                                                            \
     do {                                                                            \
         if (vis_bil) {                                                              \
@@ -800,7 +732,7 @@ extern "C" int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int6
     MT_REQUIRE(B > 0 && F > 0 && H > 0 && W > 0, "mt_warp_bwd_grid: empty shape");
     MT_REQUIRE(C == 1 || C == 3, "mt_warp_bwd_grid: C must be 1 or 3, got %d", C);
     MT_REQUIRE(!(flags & MT_GRID_AFFINE), "mt_warp_bwd_grid: dense grids only");
-    MT_REQUIRE((int64_t)B * F <= 65535 && (H + kRowsB - 1) / kRowsB <= 65535, "mt_warp_bwd_grid: too large");
+    MT_REQUIRE((int64_t)B * F <= 65535 && (H + kRows - 1) / kRows <= 65535, "mt_warp_bwd_grid: too large");
     MT_REQUIRE(aligned8(grid) && aligned8(ggrid), "mt_warp_bwd_grid: grids must be 8 B aligned");
     const int64_t P = (int64_t)H * W, lim = (1ll << 31) - 1;
     MT_REQUIRE(x_sb >= 0 && x_sc >= 0 && x_sf >= 0 && g_sb >= 0 && g_sc >= 0 && g_sf >= 0,
@@ -814,10 +746,10 @@ extern "C" int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int6
     a.g_sb = (int)g_sb; a.g_sc = (int)g_sc; a.g_sf = (int)g_sf;
     a.F = F; a.P = (int)P; a.f_magic = frame_magic(F);
     a.sp = make_sampler(H, W, (flags & MT_ALIGN_CORNERS) != 0);
-    dim3 block(kCols), gridd((W + kCols - 1) / kCols, (H + kRowsB - 1) / kRowsB, B * F);
+    dim3 block(kCols), gridd((W + kCols - 1) / kCols, (H + kRows - 1) / kRows, B * F);
     cudaStream_t st = (cudaStream_t)stream;
-    if (C == 3) launch(warp_bwd_grid_kernel<3, kRowsB>, gridd, block, 0, st, a);
-    else launch(warp_bwd_grid_kernel<1, kRowsB>, gridd, block, 0, st, a);
+    if (C == 3) launch(warp_bwd_grid_kernel<3, kRows>, gridd, block, 0, st, a);
+    else launch(warp_bwd_grid_kernel<1, kRows>, gridd, block, 0, st, a);
     return launch_status("mt_warp_bwd_grid");
 }
 
@@ -827,7 +759,7 @@ static int fill_l1_args(WarpL1Args &a, const float *x, int64_t x_sb, int64_t x_s
                         float weight, int flags, const char *who) {
     MT_REQUIRE(x && flow && x_target && v_target, "%s: NULL input", who);
     MT_REQUIRE(B > 0 && F > 0 && H > 0 && W > 0, "%s: empty shape", who);
-    MT_REQUIRE((int64_t)B * F <= 65535 && (H + kRowsB - 1) / kRowsB <= 65535, "%s: too large", who);
+    MT_REQUIRE((int64_t)B * F <= 65535 && (H + kRows - 1) / kRows <= 65535, "%s: too large", who);
     MT_REQUIRE(aligned8(flow), "%s: flow must be 8 B aligned", who);
     const int64_t P = (int64_t)H * W, lim = (1ll << 31) - 1;
     MT_REQUIRE(x_sb >= 0 && x_sc >= 0 && x_sf >= 0 && xt_sb >= 0 && xt_sc >= 0 && vt_sb >= 0,
@@ -843,7 +775,7 @@ static int fill_l1_args(WarpL1Args &a, const float *x, int64_t x_sb, int64_t x_s
     a.from_mask = (flags & MT_VIS_FROM_MASK) != 0;
     a.vis = nullptr; a.vis_sb = a.vis_sf = 0; a.x_al = a.v_al = nullptr; a.out3 = nullptr; a.ws = nullptr;
     a.out3_in = nullptr; a.grad_out = nullptr; a.gflow = nullptr;
-    a.row_blocks = (H + kRowsB - 1) / kRowsB;
+    a.row_blocks = (H + kRows - 1) / kRows;
     return MT_OK;
 }
 
@@ -872,15 +804,14 @@ extern "C" int mt_warp_l1_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_
     // about 16 CTAs per SM in total = two resident waves of the loss-only kernel (64 registers, 8 CTAs per SM); each CTA
     // walks a strip of row blocks.  Swept at cfg3 (profiles/r2_experiments.md, calls AC / AD): loss-only kernel, 6 / 8 / 16
     // per SM = 94.4 / 76.6 / 71.2 us at 256 x 256 and 17.4 / 15.3 / 16.6 us at 64 x 64
-    int64_t per_sm = tuning("MT_WARPL1_CTAS_PER_SM", 16);
-    if (per_sm < 1) per_sm = 1;
+    int64_t per_sm = 16;
     if (per_sm * sm_count() > kMaxReduceBlocks) per_sm = kMaxReduceBlocks / sm_count();
     int64_t cap = ((int64_t)sm_count() * per_sm) / ((int64_t)colb * B * F);
     if (cap < 1) cap = 1;
     if (gy > cap) gy = (int)cap;
     dim3 block(kCols), gridd(colb, gy, B * F);
-    if (a.x_al || a.v_al) launch(warp_l1_fwd_kernel<kRowsB, true>, gridd, block, 0, (cudaStream_t)stream, a);
-    else launch(warp_l1_fwd_kernel<kRowsB, false>, gridd, block, 0, (cudaStream_t)stream, a);
+    if (a.x_al || a.v_al) launch(warp_l1_fwd_kernel<kRows, true>, gridd, block, 0, (cudaStream_t)stream, a);
+    else launch(warp_l1_fwd_kernel<kRows, false>, gridd, block, 0, (cudaStream_t)stream, a);
     return launch_status("mt_warp_l1_fwd");
 }
 
@@ -897,7 +828,7 @@ extern "C" int mt_warp_l1_bwd(const float *x, int64_t x_sb, int64_t x_sc, int64_
     MT_REQUIRE(aligned8(gflow), "mt_warp_l1_bwd: gflow must be 8 B aligned");
     a.out3_in = out3; a.grad_out = grad_out; a.gflow = gflow;
     dim3 block(kCols), gridd((W + kCols - 1) / kCols, a.row_blocks, B * F);
-    launch(warp_l1_bwd_kernel<kRowsB>, gridd, block, 0, (cudaStream_t)stream, a);
+    launch(warp_l1_bwd_kernel<kRows>, gridd, block, 0, (cudaStream_t)stream, a);
     return launch_status("mt_warp_l1_bwd");
 }
 

@@ -35,12 +35,12 @@
 namespace mt {
 namespace {
 
-constexpr int kTileH = 32;          // output tile: TW x 32 pixels, TW = 32 or 64
-// TW / 2 consumer warps (16 x 4 pixels each); TW = 32: + a dedicated producer warp; TW = 64: 32 consumer
-// warps are the 1024-thread limit, the consumer warps take turns as producer (one tile each)
-constexpr bool staged_own_producer(int tw) { return tw == 32; }
-constexpr int staged_threads(int tw) { return (tw / 2 + (staged_own_producer(tw) ? 1 : 0)) * 32; }
-constexpr int kMaxTable = 1024;     // W, H <= 1024 (tables of the base grid in shared memory)
+constexpr int kTileW = 32, kTileH = 32;  // output tile
+constexpr int kBox = 48;                 // staged source box: kBox x kBox pixels per plane
+constexpr int kStages = 5;               // ring of 40 KB stages
+constexpr int kConsWarps = kTileW / 2;   // consumer warps of 16 x 4 pixels each, + one producer warp
+constexpr int kStagedThreads = (kConsWarps + 1) * 32;
+constexpr int kMaxTable = 1024;          // W, H <= 1024 (tables of the base grid in shared memory)
 
 struct TileDesc {  // written by the producer, read by the consumers after the full barrier
     int flags;     // bit 0: staged in smem; bit 1: every tap of the tile is inside the frame
@@ -52,57 +52,40 @@ struct TileDesc {  // written by the producer, read by the consumers after the f
 };
 static_assert(sizeof(TileDesc) == 64, "TileDesc is read as four 16 B words");
 
-// developer timeline probe (MT_WARP_DBG bit 3): per CTA globaltimer stamps
-// [0] kernel entry, [1] after setup + griddepcontrol.wait, [2] first TMA issued,
-// [3] first full barrier passed (consumer warp 0), [4] consumer warp 0 done, [5] tiles of this CTA
-__device__ unsigned long long g_timeline[256 * 8];
-__device__ __forceinline__ unsigned long long gtime() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-
 struct WarpStagedArgs {
     const float *x, *vis, *theta, *m_target;
     float *x_al, *v_al, *v_map;
     int x_sb, x_sc, x_sf, vis_sb, vis_sf, mt_sb, xa_sb, xa_sc, xa_sf;
     int F, P, tiles_x, tiles_per_frame, n_tiles;
-    int debug;  // MT_WARP_DBG (developer): bit 0 = never stage (every tile takes the direct path); bit 3 = timeline probe
     Sampler sp;
-    int early_trigger;  // griddepcontrol.launch_dependents right after the wait, or only at exit (see corr_tc.cu)
 };
 
-template <int TW, int BW, int BH, int STAGES>
-constexpr int staged_smem_bytes() {
-    return STAGES * (4 * BW * BH + TW * kTileH) * 4 + 2 * kMaxTable * 4 + STAGES * (int)sizeof(TileDesc) +
-           2 * STAGES * 8 + 128;
-}
+constexpr int kStagedSmem = kStages * (4 * kBox * kBox + kTileW * kTileH) * 4 + 2 * kMaxTable * 4 +
+                            kStages * (int)sizeof(TileDesc) + 2 * kStages * 8 + 128;
+static_assert(kStagedSmem <= 227 * 1024, "stage ring exceeds the shared memory of an SM");
 
 __device__ __forceinline__ float unnorm_t(float g, float sf, bool ac) { return unnormalize(g, sf, ac); }
 
 // AC: align_corners; FM: `vis` holds masks (v = 1 - m inside the frame, 0 outside)
-template <int TW, int BW, int BH, int STAGES, bool AC, bool FM>
-__global__ void __launch_bounds__(staged_threads(TW), 1)
+template <bool AC, bool FM>
+__global__ void __launch_bounds__(kStagedThreads, 1)
 warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_v,
                    const __grid_constant__ CUtensorMap map_t, const WarpStagedArgs a) {
-    static_assert(BW % 32 == 16, "a source row must start 16 banks after the previous one (see the lane mapping)");
-    constexpr int kConsWarps = TW / 2, kStagedThreads = staged_threads(TW);
-    constexpr int kPlane = BW * BH;
-    constexpr int kStageFloats = 4 * kPlane + TW * kTileH;  // RGB + mask boxes, target-mask tile
-    constexpr uint32_t kMtBytes = TW * kTileH * 4u;
+    static_assert(kBox % 32 == 16, "a source row must start 16 banks after the previous one (see the lane mapping)");
+    constexpr int kPlane = kBox * kBox;
+    constexpr int kStageFloats = 4 * kPlane + kTileW * kTileH;  // RGB + mask boxes, target-mask tile
+    constexpr uint32_t kMtBytes = kTileW * kTileH * 4u;
     // 128 B alignment (TMA destination) comes from the declaration: a manual round-up through
     // uintptr_t makes the compiler lose the shared address space (generic LD/ST instead of LDS/STS)
     extern __shared__ __align__(128) uint8_t smem_raw[];
     float *stage0 = reinterpret_cast<float *>(smem_raw);
-    float *s_bx = stage0 + STAGES * kStageFloats;
+    float *s_bx = stage0 + kStages * kStageFloats;
     float *s_by = s_bx + kMaxTable;
     TileDesc *desc = reinterpret_cast<TileDesc *>(s_by + kMaxTable);
-    uint64_t *full = reinterpret_cast<uint64_t *>(desc + STAGES), *empty = full + STAGES;
+    uint64_t *full = reinterpret_cast<uint64_t *>(desc + kStages), *empty = full + kStages;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int W = a.sp.W, H = a.sp.H;
-    const bool probe = (a.debug & 8) && blockIdx.x < 256;
-    if (probe && threadIdx.x == 0) g_timeline[blockIdx.x * 8 + 0] = gtime();
 
     // ---- on-chip setup: overlaps the tail of the previous kernel (PDL) ----
     for (int i = threadIdx.x; i < W; i += kStagedThreads) s_bx[i] = base_coord(i, W, a.sp.stepx, AC);
@@ -111,20 +94,20 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_x) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_v) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_t) : "memory");
-        for (int s = 0; s < STAGES; ++s) {
+        for (int s = 0; s < kStages; ++s) {
             mbar_init(smem_u32(full + s), 1);
             mbar_init(smem_u32(empty + s), kConsWarps);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
+    // no launch_dependents: this kernel holds ~200 KB of shared memory per SM and leaves the trigger to its exit
+    // (see pdl_sync; cfg5 step 121.8 -> 109.8 us: the streaming kernels behind it get their L1 back)
     pdl_wait();
-    if (a.early_trigger) pdl_launch();
-    if (probe && threadIdx.x == 0) g_timeline[blockIdx.x * 8 + 1] = gtime();
 
     const float wmax = a.sp.wmax, hmax = a.sp.hmax;
 
-    // ---- producer duty (one thread at a time) ----
+    // ---- producer duty (lane 0 of the producer warp) ----
     // The descriptor of a tile: theta load, two integer divisions, four corner evaluations.
     auto prepare = [&](int t) {
         TileDesc d;
@@ -133,7 +116,7 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
 #pragma unroll
         for (int j = 0; j < 6; ++j) d.th[j] = __ldg(a.theta + n * 6 + j);
         const int b = n / a.F, f = n - b * a.F;
-        const int xs[2] = {tx * TW, min(tx * TW + TW - 1, W - 1)};
+        const int xs[2] = {tx * kTileW, min(tx * kTileW + kTileW - 1, W - 1)};
         const int ys[2] = {ty * kTileH, min(ty * kTileH + kTileH - 1, H - 1)};
         float xlo = 3.0e38f, xhi = -3.0e38f, ylo = 3.0e38f, yhi = -3.0e38f;
         bool finite = true;
@@ -156,7 +139,7 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         // the box origin is xlo rounded down to a multiple of 4 pixels (two's complement: also for
         // negative coordinates)
         const int bx0 = finite ? ((int)xlo & ~3) : 0, by0 = finite ? (int)ylo : 0;
-        const bool fits = finite && ((int)xhi + 2 - bx0 <= BW) && ((int)yhi + 2 - by0 <= BH) && !(a.debug & 1);
+        const bool fits = finite && ((int)xhi + 2 - bx0 <= kBox) && ((int)yhi + 2 - by0 <= kBox);
         const bool inside = fits && xlo >= 0.0f && xhi + 1.0f <= wmax && ylo >= 0.0f && yhi + 1.0f <= hmax;
         d.flags = (fits ? 1 : 0) | (inside ? 2 : 0);
         d.bx0 = bx0; d.by0 = by0;
@@ -164,69 +147,49 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         d.pad[0] = d.pad[1] = 0;
         return d;
     };
-    // i-th tile of this CTA -> stage i % STAGES (waits until the consumers have released it)
+    // i-th tile of this CTA -> stage i % kStages (waits until the consumers have released it)
     auto issue = [&](int i, const TileDesc &d) {
-        const int s = i % STAGES;
-        const uint32_t ph = (uint32_t)(i / STAGES) & 1u;
+        const int s = i % kStages;
+        const uint32_t ph = (uint32_t)(i / kStages) & 1u;
         mbar_wait(smem_u32(empty + s), ph ^ 1u);
         desc[s] = d;
         const bool fits = (d.flags & 1) != 0;
         float *dst = stage0 + s * kStageFloats;
         mbar_expect_tx(smem_u32(full + s), fits ? 4u * kPlane * 4u + kMtBytes : kMtBytes);
         if (fits) {
-            // x as (W, H, C, F, B): box (BW, BH, 3, 1, 1); masks as (W, H, F, B): box (BW, BH, 1, 1)
+            // x as (W, H, C, F, B): box (kBox, kBox, 3, 1, 1); masks as (W, H, F, B): box (kBox, kBox, 1, 1)
             tma_load_5d(smem_u32(dst), &map_x, smem_u32(full + s), d.bx0, d.by0, 0, d.f, d.b);
             tma_load_4d(smem_u32(dst + 3 * kPlane), &map_v, smem_u32(full + s), d.bx0, d.by0, d.f, d.b);
         }
         // target mask as (W, H, B): the tile itself
-        tma_load_3d(smem_u32(dst + 4 * kPlane), &map_t, smem_u32(full + s), d.tx * TW, d.ty * kTileH, d.b);
-        if (probe && i == 0) g_timeline[blockIdx.x * 8 + 2] = gtime();
+        tma_load_3d(smem_u32(dst + 4 * kPlane), &map_t, smem_u32(full + s), d.tx * kTileW, d.ty * kTileH, d.b);
     };
 
-    if constexpr (staged_own_producer(TW)) {
-        if (warp == kConsWarps) {
-            // ===================== producer warp =====================
-            // The descriptor of the next tile is prepared while its stage is still in use: between
-            // "stage released" and "TMA issued" there is only the descriptor store (ncu: consumers
-            // polled the full barrier 2.9 times per tile while this chain sat behind the empty wait).
-            if (lane == 0) {
-                int t = blockIdx.x;
-                TileDesc d;
+    if (warp == kConsWarps) {
+        // ===================== producer warp =====================
+        // The descriptor of the next tile is prepared while its stage is still in use: between
+        // "stage released" and "TMA issued" there is only the descriptor store (ncu: consumers
+        // polled the full barrier 2.9 times per tile while this chain sat behind the empty wait).
+        if (lane == 0) {
+            int t = blockIdx.x;
+            TileDesc d;
+            if (t < a.n_tiles) d = prepare(t);
+            for (int i = 0; t < a.n_tiles; ++i) {
+                issue(i, d);
+                t += gridDim.x;
                 if (t < a.n_tiles) d = prepare(t);
-                for (int i = 0; t < a.n_tiles; ++i) {
-                    issue(i, d);
-                    t += gridDim.x;
-                    if (t < a.n_tiles) d = prepare(t);
-                }
-            }
-            return;
-        }
-    } else {
-        // no spare warp (32 consumer warps = 1024 threads): the first STAGES - 1 tiles are issued here,
-        // tile i + STAGES - 1 by consumer warp i % kConsWarps at the top of its iteration i
-        if (threadIdx.x == 0) {
-            for (int i = 0; i < STAGES - 1; ++i) {
-                const int t = blockIdx.x + i * gridDim.x;
-                if (t < a.n_tiles) issue(i, prepare(t));
             }
         }
+        return;
     }
 
     // ===================== consumers =====================
     const float wm2 = wmax - 1.0f, hm2 = hmax - 1.0f;
     int i = 0;
     for (int t = blockIdx.x; t < a.n_tiles; t += gridDim.x, ++i) {
-        if constexpr (!staged_own_producer(TW)) {
-            if (lane == 0 && warp == i % kConsWarps) {
-                const int tj = t + (STAGES - 1) * gridDim.x;
-                if (tj < a.n_tiles) issue(i + STAGES - 1, prepare(tj));
-            }
-            __syncwarp();
-        }
-        const int s = i % STAGES;
-        const uint32_t ph = (uint32_t)(i / STAGES) & 1u;
+        const int s = i % kStages;
+        const uint32_t ph = (uint32_t)(i / kStages) & 1u;
         mbar_wait(smem_u32(full + s), ph);
-        if (probe && i == 0 && threadIdx.x == 0) g_timeline[blockIdx.x * 8 + 3] = gtime();
         const int4 d0 = reinterpret_cast<const int4 *>(desc + s)[0];      // flags, bx0, by0, b
         const int4 d1 = reinterpret_cast<const int4 *>(desc + s)[1];      // f, n, tx, ty
         const float4 d2 = reinterpret_cast<const float4 *>(desc + s)[2];  // th0..3
@@ -237,16 +200,16 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         // the previous one, so the two half-warps read disjoint bank ranges and a tap instruction is
         // one shared-memory wavefront; the 32 x 1 mapping had 2-way conflicts wherever the footprint
         // of the 32 lanes stepped to the next source row (ncu: 44 % of the LDS wavefronts).
-        constexpr int kColGroups = TW / 16, kRowStep = 2;
+        constexpr int kColGroups = kTileW / 16, kRowStep = 2;
         const int tcol = (warp % kColGroups) * 16 + (lane & 15), trow = (warp / kColGroups) * 4 + (lane >> 4);
-        const int xg = d1.z * TW + tcol, y0 = d1.w * kTileH + trow;
+        const int xg = d1.z * kTileW + tcol, y0 = d1.w * kTileH + trow;
         const bool live = xg < W;
         const int x = min(xg, W - 1);
         const int p0 = y0 * W + x;
         const float *st = stage0 + s * kStageFloats;
         float mtv[2];
 #pragma unroll
-        for (int k = 0; k < 2; ++k) mtv[k] = st[4 * kPlane + (trow + k * kRowStep) * TW + tcol];
+        for (int k = 0; k < 2; ++k) mtv[k] = st[4 * kPlane + (trow + k * kRowStep) * kTileW + tcol];
         const float bx = s_bx[x];
         const float bxt0 = __fmul_rn(bx, d2.x), bxt3 = __fmul_rn(bx, d2.w);
         float ix[2], iy[2], xw[2], yn[2], wnw[2], wne[2], wsw[2], wse[2];
@@ -270,11 +233,11 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
             float q[4][2][4];
 #pragma unroll
             for (int k = 0; k < 2; ++k) {
-                const float *p = st + (((int)yn[k] - by0) * BW + ((int)xw[k] - bx0));
+                const float *p = st + (((int)yn[k] - by0) * kBox + ((int)xw[k] - bx0));
 #pragma unroll
                 for (int c = 0; c < 4; ++c) {
                     q[c][k][0] = p[c * kPlane]; q[c][k][1] = p[c * kPlane + 1];
-                    q[c][k][2] = p[c * kPlane + BW]; q[c][k][3] = p[c * kPlane + BW + 1];
+                    q[c][k][2] = p[c * kPlane + kBox]; q[c][k][3] = p[c * kPlane + kBox + 1];
                 }
             }
             __syncwarp();
@@ -337,98 +300,8 @@ warp_staged_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
             }
         }
     }
-    if (probe && threadIdx.x == 0) {
-        g_timeline[blockIdx.x * 8 + 4] = gtime();
-        g_timeline[blockIdx.x * 8 + 5] = (unsigned long long)i;
-    }
 }
 
-}  // namespace
-
-namespace {
-struct StagedHost {
-    const float *x, *vis, *theta, *m_target;
-    float *x_al, *v_al, *v_map;
-    int64_t x_sb, x_sc, x_sf, vis_sb, vis_sf, mt_sb, xa_sb, xa_sc, xa_sf;
-    int B, F, H, W;
-    bool ac, from_mask;
-    cudaStream_t st;
-    EncodeTiledFn enc;
-};
-
-template <int TW, int BW, int BH, int STAGES>
-int staged_go(const StagedHost &h) {
-    const int W = h.W, H = h.H;
-    const int tiles_x = (W + TW - 1) / TW, tiles_y = (H + kTileH - 1) / kTileH;
-    const int64_t n_tiles = (int64_t)h.B * h.F * tiles_x * tiles_y;
-    // tiny problems cannot fill a persistent grid of one CTA per SM: keep the strip kernel
-    if (n_tiles < 2 * (int64_t)sm_count() || n_tiles > (1ll << 30)) return 0;
-    CUtensorMap map_x, map_v, map_t;
-    {
-        cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)h.B};
-        cuuint64_t strides[2] = {(cuuint64_t)W * 4, h.mt_sb ? (cuuint64_t)h.mt_sb * 4 : 16};
-        cuuint32_t bx[3] = {(cuuint32_t)TW, (cuuint32_t)kTileH, 1};
-        cuuint32_t estr[3] = {1, 1, 1};
-        CUresult r = h.enc(&map_t, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float *>(h.m_target), dims, strides,
-                           bx, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return 0;
-    }
-    {
-        cuuint64_t dims[5] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)h.F, (cuuint64_t)h.B};
-        cuuint64_t strides[4] = {(cuuint64_t)W * 4, (cuuint64_t)h.x_sc * 4, (cuuint64_t)h.x_sf * 4,
-                                 (cuuint64_t)h.x_sb * 4};
-        // a stride of 0 bytes (B or F of extent 1 sliced out of a view) is not encodable: any multiple of 16 is fine there
-        for (int i = 1; i < 4; ++i) if (strides[i] == 0) strides[i] = 16;
-        cuuint32_t bx[5] = {(cuuint32_t)BW, (cuuint32_t)BH, 3, 1, 1};
-        cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-        CUresult r = h.enc(&map_x, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<float *>(h.x), dims, strides, bx, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return 0;  // e.g. strides beyond the encodable range: direct kernel
-    }
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)h.F, (cuuint64_t)h.B};
-        cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)h.vis_sf * 4, (cuuint64_t)h.vis_sb * 4};
-        for (int i = 1; i < 3; ++i) if (strides[i] == 0) strides[i] = 16;
-        cuuint32_t bx[4] = {(cuuint32_t)BW, (cuuint32_t)BH, 1, 1};
-        cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = h.enc(&map_v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float *>(h.vis), dims, strides, bx,
-                           estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return 0;
-    }
-    WarpStagedArgs a;
-    a.x = h.x; a.vis = h.vis; a.theta = h.theta; a.m_target = h.m_target;
-    a.x_al = h.x_al; a.v_al = h.v_al; a.v_map = h.v_map;
-    a.x_sb = (int)h.x_sb; a.x_sc = (int)h.x_sc; a.x_sf = (int)h.x_sf;
-    a.vis_sb = (int)h.vis_sb; a.vis_sf = (int)h.vis_sf; a.mt_sb = (int)h.mt_sb;
-    a.xa_sb = (int)h.xa_sb; a.xa_sc = (int)h.xa_sc; a.xa_sf = (int)h.xa_sf;
-    a.F = h.F; a.P = H * W; a.tiles_x = tiles_x; a.tiles_per_frame = tiles_x * tiles_y; a.n_tiles = (int)n_tiles;
-    a.sp = make_sampler(H, W, h.ac);
-    a.debug = tuning("MT_WARP_DBG", 0);
-    // no early launch_dependents: this kernel holds ~200 KB of shared memory per SM, see kCorrEarlyTrigger in
-    // corr_tc.cu (cfg5 step 121.8 -> 109.8 us: the streaming kernels behind it get their L1 back)
-    a.early_trigger = tuning("MT_STAGED_EARLY_TRIGGER", 0);
-    int ctas = sm_count();
-    if (ctas > n_tiles) ctas = (int)n_tiles;
-    constexpr int smem = staged_smem_bytes<TW, BW, BH, STAGES>();
-    static_assert(smem <= 227 * 1024, "stage ring exceeds the shared memory of an SM");
-#define MT_STAGED_GO(ACV, FMV)                                                                       \
-    do {                                                                                             \
-        auto kern = warp_staged_kernel<TW, BW, BH, STAGES, ACV, FMV>;                                \
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); \
-        if (e != cudaSuccess) {                                                                      \
-            set_error("mt_warp_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));               \
-            return MT_ERR_CUDA;                                                                      \
-        }                                                                                            \
-        launch(kern, dim3(ctas), dim3(staged_threads(TW)), (size_t)smem, h.st, map_x, map_v, map_t, a); \
-    } while (0)
-    if (h.ac) { if (h.from_mask) MT_STAGED_GO(true, true); else MT_STAGED_GO(true, false); }
-    else      { if (h.from_mask) MT_STAGED_GO(false, true); else MT_STAGED_GO(false, false); }
-#undef MT_STAGED_GO
-    return 1;
-}
 }  // namespace
 
 // 1 = launched, 0 = not applicable (caller uses the direct-gather kernel), < 0 = error.
@@ -449,26 +322,63 @@ int warp_staged_launch(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
         return 0;
     EncodeTiledFn enc = encode_fn();
     if (!enc) return 0;
-    StagedHost h;
-    h.x = x; h.vis = vis; h.theta = theta; h.m_target = m_target;
-    h.x_al = x_aligned; h.v_al = v_aligned; h.v_map = v_map;
-    h.x_sb = x_sb; h.x_sc = x_sc; h.x_sf = x_sf; h.vis_sb = vis_sb; h.vis_sf = vis_sf; h.mt_sb = mt_sb;
-    h.xa_sb = xa_sb; h.xa_sc = xa_sc; h.xa_sf = xa_sf;
-    h.B = B; h.F = F; h.H = H; h.W = W; h.ac = ac; h.from_mask = from_mask; h.st = st; h.enc = enc;
-    // tile 64 x 32 (32 consumer warps, box 80 x 48, 3 stages of 68 KB) or 32 x 32 (16 warps, box 48 x 48,
-    // 5 stages of 40 KB)
-    if (tuning("MT_WARP_TILE_W", 32) == 64 && W >= 64) return staged_go<64, 80, 48, 3>(h);
-    return staged_go<32, 48, 48, 5>(h);
+    const int tiles_x = (W + kTileW - 1) / kTileW, tiles_y = (H + kTileH - 1) / kTileH;
+    const int64_t n_tiles = (int64_t)B * F * tiles_x * tiles_y;
+    // tiny problems cannot fill a persistent grid of one CTA per SM: keep the strip kernel
+    if (n_tiles < 2 * (int64_t)sm_count() || n_tiles > (1ll << 30)) return 0;
+    CUtensorMap map_x, map_v, map_t;
+    {
+        cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
+        cuuint64_t strides[2] = {(cuuint64_t)W * 4, mt_sb ? (cuuint64_t)mt_sb * 4 : 16};
+        cuuint32_t bx[3] = {(cuuint32_t)kTileW, (cuuint32_t)kTileH, 1};
+        cuuint32_t estr[3] = {1, 1, 1};
+        CUresult r = enc(&map_t, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float *>(m_target), dims, strides,
+                         bx, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return 0;
+    }
+    {
+        cuuint64_t dims[5] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)F, (cuuint64_t)B};
+        cuuint64_t strides[4] = {(cuuint64_t)W * 4, (cuuint64_t)x_sc * 4, (cuuint64_t)x_sf * 4, (cuuint64_t)x_sb * 4};
+        // a stride of 0 bytes (B or F of extent 1 sliced out of a view) is not encodable: any multiple of 16 is fine there
+        for (int i = 1; i < 4; ++i) if (strides[i] == 0) strides[i] = 16;
+        cuuint32_t bx[5] = {(cuuint32_t)kBox, (cuuint32_t)kBox, 3, 1, 1};
+        cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+        CUresult r = enc(&map_x, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<float *>(x), dims, strides, bx, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return 0;  // e.g. strides beyond the encodable range: direct kernel
+    }
+    {
+        cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)F, (cuuint64_t)B};
+        cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)vis_sf * 4, (cuuint64_t)vis_sb * 4};
+        for (int i = 1; i < 3; ++i) if (strides[i] == 0) strides[i] = 16;
+        cuuint32_t bx[4] = {(cuuint32_t)kBox, (cuuint32_t)kBox, 1, 1};
+        cuuint32_t estr[4] = {1, 1, 1, 1};
+        CUresult r = enc(&map_v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float *>(vis), dims, strides, bx,
+                         estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return 0;
+    }
+    WarpStagedArgs a;
+    a.x = x; a.vis = vis; a.theta = theta; a.m_target = m_target;
+    a.x_al = x_aligned; a.v_al = v_aligned; a.v_map = v_map;
+    a.x_sb = (int)x_sb; a.x_sc = (int)x_sc; a.x_sf = (int)x_sf;
+    a.vis_sb = (int)vis_sb; a.vis_sf = (int)vis_sf; a.mt_sb = (int)mt_sb;
+    a.xa_sb = (int)xa_sb; a.xa_sc = (int)xa_sc; a.xa_sf = (int)xa_sf;
+    a.F = F; a.P = H * W; a.tiles_x = tiles_x; a.tiles_per_frame = tiles_x * tiles_y; a.n_tiles = (int)n_tiles;
+    a.sp = make_sampler(H, W, ac);
+    int ctas = sm_count();
+    if (ctas > n_tiles) ctas = (int)n_tiles;
+    auto kern = ac ? (from_mask ? warp_staged_kernel<true, true> : warp_staged_kernel<true, false>)
+                   : (from_mask ? warp_staged_kernel<false, true> : warp_staged_kernel<false, false>);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kStagedSmem);
+    if (e != cudaSuccess) {
+        set_error("mt_warp_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+        return MT_ERR_CUDA;
+    }
+    launch(kern, dim3(ctas), dim3(kStagedThreads), (size_t)kStagedSmem, st, map_x, map_v, map_t, a);
+    return 1;
 }
 
 }  // namespace mt
-
-// developer probe (not part of include/mt_b200.h; only in builds with -DMT_DEV_PROBES, see
-// tools/dbg_timeline.py): copies the timeline stamps to the host
-#ifdef MT_DEV_PROBES
-extern "C" __attribute__((visibility("default"))) int mt_debug_warp_timeline(unsigned long long *dst, int n) {
-    cudaDeviceSynchronize();
-    return cudaMemcpyFromSymbol(dst, mt::g_timeline, sizeof(unsigned long long) * (n < 2048 ? n : 2048)) == cudaSuccess
-               ? 0 : -2;
-}
-#endif

@@ -112,30 +112,24 @@ STAGED_CASES = {
 }
 
 
-DEFAULT_TILE_W = 32
-
-
 def _set_tuning(name, value):
     from master_thesis_b200 import _lib
     _lib.call("mt_set_tuning", name.encode(), value)
 
 
-@pytest.mark.parametrize("tile_w", [32, 64])
 @pytest.mark.parametrize("name", sorted(STAGED_CASES))
-def test_cpn_align_tail_staged(mtb, name, tile_w):
-    """Both tile shapes of the staged kernel against the oracle and the direct kernel."""
+def test_cpn_align_tail_staged(mtb, name):
+    """The staged kernel against the oracle and the direct kernel."""
     spec = STAGED_CASES[name]
     x, m, m_t, theta = cases.cpn_inputs(spec)
     oxa, ova, ovm = oracle.cpn_align_tail(x, m, m_t, theta=theta)
     try:
-        _set_tuning("MT_WARP_TILE_W", tile_w)
         _set_tuning("MT_WARP_STAGED", 1)
         xa, va, vm = mtb.cpn_align_tail(dev(x), dev(m), dev(m_t), dev(theta))
         _set_tuning("MT_WARP_STAGED", 0)
         xd, vd, vmd = mtb.cpn_align_tail(dev(x), dev(m), dev(m_t), dev(theta))
     finally:
         _set_tuning("MT_WARP_STAGED", 1)
-        _set_tuning("MT_WARP_TILE_W", DEFAULT_TILE_W)
     for got, direct, orc in ((xa, xd, oxa), (va, vd, ova), (vm, vmd, ovm)):
         assert np.array_equal(host(got), orc)           # staged kernel == oracle, bit for bit
         assert np.array_equal(host(direct), orc)        # direct-gather kernel == oracle
@@ -724,14 +718,9 @@ def test_no_out_of_bounds_writes(mtb):
 
     r = cases.synth.rng(123)
     with guards():
-        # staged CPN warp with partial tiles (both tile shapes), direct-gather warp with W % 4 != 0
+        # staged CPN warp with partial tiles, direct-gather warp with W % 4 != 0
         x, m, m_t, theta = cases.cpn_inputs(STAGED_CASES["rand"])
-        for tw in (32, 64):
-            try:
-                _set_tuning("MT_WARP_TILE_W", tw)
-                mtb.cpn_align_tail(dev(x), dev(m), dev(m_t), dev(theta))
-            finally:
-                _set_tuning("MT_WARP_TILE_W", DEFAULT_TILE_W)
+        mtb.cpn_align_tail(dev(x), dev(m), dev(m_t), dev(theta))
         xw, mw, mtw, flow = cases.warp_inputs(cases.WARP_CASES["f1_odd"])
         mtb.dfpn_align_tail(dev(xw), dev(mw), dev(mtw), dev(flow))
         # warp + pack, composite + hole update (odd sizes)
@@ -1143,24 +1132,6 @@ def test_flow_estimator_input_pack_full_size(mtb):
     want = oracle.flow_pack(x[:, :, t], m[:, :, t], x[:, :, r_list], m[:, :, r_list], flow)
     assert np.array_equal(host(got), want)
     assert torch.equal(xd, dev(x)) and torch.equal(md, dev(m))
-
-
-@pytest.mark.parametrize("rows,iters", [(1, 1), (1, 3), (2, 1), (4, 1), (2, 4), (4, 2)])
-@pytest.mark.parametrize("name", sorted(cases.WARP_CASES))
-def test_dfpn_align_tail_rows_per_thread(mtb, name, rows, iters):
-    """The direct-gather kernel with 1 / 2 / 4 vertically adjacent pixels per thread (taps of a shared source row are
-    loaded once and reused) and several row groups per CTA: bit-identical to the reference's golden vectors."""
-    x, m, m_t, flow = cases.warp_inputs(cases.WARP_CASES[name])
-    g = load_golden("warp_" + name)
-    try:
-        _set_tuning("MT_WARP_ROWS", rows)
-        _set_tuning("MT_WARP_ITERS", iters)
-        xa, va, vm = mtb.dfpn_align_tail(dev(x), dev(m), dev(m_t), dev(flow))
-    finally:
-        _set_tuning("MT_WARP_ROWS", 2)
-        _set_tuning("MT_WARP_ITERS", 1)
-    assert np.array_equal(host(xa), g["x_aligned"])
-    assert np.array_equal(host(va), g["v_aligned"]) and np.array_equal(host(vm), g["v_map"])
 
 
 # ---------------------------------------------------------------- 8f-3: F.l1_loss(corr, corr_y) in the epilogue

@@ -11,5 +11,4 @@ $CMD > $O/plain.log 2>&1 &&
 ncu --metrics gpu__time_duration.sum --clock-control none -s 40 -c 50 --csv --log-file $O/launches_cfg2.csv $CMD > $O/ncu_l.log 2>&1
 $CMD > $O/plain.log 2>&1 &&
 ncu --set full --clock-control none --import-source on -k regex:"warp_staged|cm_" -s 25 -c 5 -f -o $O/prof_cfg2 $CMD > $O/ncu_f.log 2>&1
-python tools/dbg_timeline.py 8 2>&1 | tail -2
 bash profiles/r1_sweep_cm2.sh
