@@ -132,6 +132,41 @@ MT_API int mt_warp_pack_lowres_fwd(const float *x, int64_t x_sb, int64_t x_sc, i
                             float *v_aligned, float *v_map,
                             int B, int F, int H, int W, int flags, mt_stream_t stream);
 
+/* The four warps above with the element type of a DENSE flow as a dtype code (MT_DT_*) before its pointer
+ * (DFPN.align, model_dfpn.py:100-101 and 128-133 under autocast).  The DFPN's flow estimators return fp16 / bf16
+ * flows there; grid_sample is on autocast's promote list (utils.py:93-103: fp32 frames, half flow -> fp32 sampling of
+ * the exactly widened flow) and the bilinear flow resize runs in fp32 too (see mt_resize_flow_dt).  The kernels widen
+ * the flow on load: every output equals the fp32 entry point's given the widened flow.  A half flow needs nearest
+ * visibility (the DFPN flavour); a theta is fp32 only.  A half flow must be 4 B aligned, an fp32 one 8 B. */
+MT_API int mt_warp_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                   const float *vis, int64_t vis_sb, int64_t vis_sf,
+                   int g_dtype, const void *grid, const float *m_target, int64_t mt_sb,
+                   float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                   float *v_aligned, float *v_map,
+                   int B, int C, int F, int H, int W, int flags, mt_stream_t stream);
+MT_API int mt_warp_pack_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                        const float *vis, int64_t vis_sb, int64_t vis_sf,
+                        int g_dtype, const void *grid, const float *m_target, int64_t mt_sb,
+                        const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                        float *nn_in,
+                        float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                        float *v_aligned, float *v_map,
+                        int B, int F, int H, int W, int flags, mt_stream_t stream);
+MT_API int mt_warp_lowres_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                          const float *vis, int64_t vis_sb, int64_t vis_sf,
+                          int g_dtype, const void *flow, int gh, int gw, const float *m_target, int64_t mt_sb,
+                          float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                          float *v_aligned, float *v_map,
+                          int B, int F, int H, int W, int flags, mt_stream_t stream);
+MT_API int mt_warp_pack_lowres_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                               const float *vis, int64_t vis_sb, int64_t vis_sf,
+                               int g_dtype, const void *flow, int gh, int gw, const float *m_target, int64_t mt_sb,
+                               const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                               float *nn_in,
+                               float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                               float *v_aligned, float *v_map,
+                               int B, int F, int H, int W, int flags, mt_stream_t stream);
+
 /* ---- K1b  backward of the bilinear warp w.r.t. the dense grid ------------
  * replaces autograd of F.grid_sample in align_set (utils.py:93-97)       (a6)
  * gout (B,C,F,H,W) strided (plane contiguous) -> ggrid (B,F,H,W,2) contiguous.
@@ -339,6 +374,18 @@ MT_API int mt_corr4d_vgg_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_sc,
                       const float *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
                       const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW,
                       float *out, int B, int C, int F, int h, int w, mt_stream_t stream);
+/* mt_corr4d_vgg_fwd with the feature dtype f_dtype (MT_DT_*): the VGG's pool-4 features under autocast
+ * (model_dfpn.py:534-565: `ft * vt` with fp32 masks and the norm run in fp32, torch.matmul rounds the normalised
+ * operands to the autocast dtype and returns a half volume).  fp16 / bf16 features run on tcgen05 kind::f16: the exact
+ * half features are multiplied with fp32 accumulation, the fp32 norm scales applied in the epilogue, and the volume
+ * `out` is stored in f_dtype, rounded once to nearest even.  Not bit-identical to the eager path (which rounds the
+ * normalised operands), at least as accurate.  Masks stay fp32.  Half features need C % 64 == 0 and feature strides
+ * that are multiples of 16 B; the L1 mode stays fp32. */
+MT_API int mt_corr4d_vgg_fwd_dt(int f_dtype, const void *feats_t, int64_t ft_sb, int64_t ft_sc,
+                         const float *m_target, int64_t mt_sb,
+                         const void *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
+                         const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW,
+                         void *out, int B, int C, int F, int h, int w, mt_stream_t stream);
 
 /* mt_corr4d_vgg_l1_fwd: the correlation above with F.l1_loss(corr, corr_y) (model_dfpn.py:254-257, SURVEY 8f-3)
  * folded into its epilogue: the volume of the ground-truth features is never written.  pred (B,F,P,P)
@@ -460,6 +507,13 @@ MT_API int mt_resize_set(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
 MT_API int mt_resize_flow(const float *flow, int64_t sb, int64_t sf, int64_t sy, int64_t sx, int64_t sc,
                    float *out, int64_t o_sb, int64_t o_sf, int64_t o_sy, int64_t o_sx, int64_t o_sc,
                    int B, int F, int h, int w, int H, int W, int mode, mt_stream_t stream);
+/* mt_resize_flow with the input flow's dtype (MT_DT_*) before its pointer: under autocast the DFPN's flow estimators
+ * return fp16 / bf16 flows, and upsample_bilinear2d / upsample_nearest2d run in fp32 (autocast's fp32 policy), so
+ * FlowsUtils.resize_flow (utils.py:107-126) returns an fp32 flow computed on the exactly widened input.  out is fp32
+ * and equals mt_resize_flow on the widened flow. */
+MT_API int mt_resize_flow_dt(int flow_dtype, const void *flow, int64_t sb, int64_t sf, int64_t sy, int64_t sx,
+                      int64_t sc, float *out, int64_t o_sb, int64_t o_sf, int64_t o_sy, int64_t o_sx, int64_t o_sc,
+                      int B, int F, int h, int w, int H, int W, int mode, mt_stream_t stream);
 MT_API int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
                        int64_t g_sc, float *g_flow, int B, int F, int h, int w, int H, int W,
                        mt_stream_t stream);

@@ -29,10 +29,10 @@ int corr4d_tc_supported(int C, int P);
 int corr4d_tc_launch(const float *ft, const float *vt, const float *fr, const float *vr, float *out,
                      void *ws, int64_t ws_bytes, int B, int C, int F, int P, cudaStream_t st);
 int64_t corr4d_tc_workspace_bytes(int B, int C, int F, int P);
-int corr4d_tc_launch_ex(const float *ft, int64_t ft_sb, int64_t ft_sc, const float *fr, int64_t fr_sb, int64_t fr_sc,
+int corr4d_tc_launch_ex(const void *ft, int64_t ft_sb, int64_t ft_sc, const void *fr, int64_t fr_sb, int64_t fr_sc,
                         int64_t fr_sf, const float *vt, int64_t vt_sb, const float *vr, int64_t vr_sb, int64_t vr_sf,
-                        int mask_mode, int MH, int MW, int fh, int fw, float *out, int B, int C, int F, int P,
-                        cudaStream_t st, const CorrL1 *l1);
+                        int mask_mode, int MH, int MW, int fh, int fw, void *out, int B, int C, int F, int P,
+                        cudaStream_t st, const CorrL1 *l1, int dtype);
 int64_t corr4d_l1_workspace_bytes();
 int corr4d_l1_bwd_launch(const signed char *sign, const float *grad_loss, float *g_pred, int64_t n, cudaStream_t st);
 
@@ -153,10 +153,16 @@ extern "C" int mt_corr4d_fwd(const float *feats_t, const float *v_t, const float
     return launch_status("mt_corr4d_fwd");
 }
 
-extern "C" int mt_corr4d_vgg_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_sc, const float *m_target,
-                                 int64_t mt_sb, const float *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
-                                 const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW, float *out,
-                                 int B, int C, int F, int h, int w, mt_stream_t stream) {
+// f_dtype (MT_DT_*): element type of feats_t, feats_r and out.  Under autocast the VGG hands over fp16 / bf16
+// features; CorrelationVGG.correlation_masked_4d (model_dfpn.py:534-565) then multiplies them by the fp32 masks (fp32),
+// normalises in fp32 (norm is on autocast's fp32 list) and its torch.matmul rounds the normalised operands to the
+// autocast dtype and returns a half volume.  The kernel multiplies the exact half features on the tensor cores
+// (kind::f16, fp32 accumulation), applies the fp32 scales in the epilogue and rounds once when it stores the volume
+// in f_dtype: not bit-identical to the eager path, at least as accurate (DESIGN.md §2).
+extern "C" int mt_corr4d_vgg_fwd_dt(int f_dtype, const void *feats_t, int64_t ft_sb, int64_t ft_sc,
+                                    const float *m_target, int64_t mt_sb, const void *feats_r, int64_t fr_sb,
+                                    int64_t fr_sc, int64_t fr_sf, const float *m_refs, int64_t mr_sb, int64_t mr_sf,
+                                    int MH, int MW, void *out, int B, int C, int F, int h, int w, mt_stream_t stream) {
     MT_REQUIRE(feats_t && feats_r && out, "mt_corr4d_vgg_fwd: NULL argument");
     MT_REQUIRE(B > 0 && C > 0 && F > 0 && h > 0 && w > 0, "mt_corr4d_vgg_fwd: empty shape");
     MT_REQUIRE((m_target == nullptr) == (m_refs == nullptr), "mt_corr4d_vgg_fwd: both masks or none");
@@ -166,7 +172,16 @@ extern "C" int mt_corr4d_vgg_fwd(const float *feats_t, int64_t ft_sb, int64_t ft
                "mt_corr4d_vgg_fwd: only shapes served by the tensor-core kernel (h*w %% 256 == 0, C %% 32 == 0); use "
                "mt_corr4d_fwd on contiguous, pre-masked inputs otherwise");
     return corr4d_tc_launch_ex(feats_t, ft_sb, ft_sc, feats_r, fr_sb, fr_sc, fr_sf, m_target, mt_sb, m_refs, mr_sb,
-                               mr_sf, m_target ? 1 : 0, MH, MW, h, w, out, B, C, F, h * w, (cudaStream_t)stream, nullptr);
+                               mr_sf, m_target ? 1 : 0, MH, MW, h, w, out, B, C, F, h * w, (cudaStream_t)stream, nullptr,
+                               f_dtype);
+}
+
+extern "C" int mt_corr4d_vgg_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_sc, const float *m_target,
+                                 int64_t mt_sb, const float *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
+                                 const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW, float *out,
+                                 int B, int C, int F, int h, int w, mt_stream_t stream) {
+    return mt_corr4d_vgg_fwd_dt(MT_DT_F32, feats_t, ft_sb, ft_sc, m_target, mt_sb, feats_r, fr_sb, fr_sc, fr_sf, m_refs,
+                                mr_sb, mr_sf, MH, MW, out, B, C, F, h, w, stream);
 }
 
 extern "C" int64_t mt_corr4d_l1_workspace_bytes(void) { return corr4d_l1_workspace_bytes(); }
@@ -186,7 +201,8 @@ extern "C" int mt_corr4d_vgg_l1_fwd(const float *feats_t, int64_t ft_sb, int64_t
                "mt_corr4d_vgg_l1_fwd: only shapes served by the tensor-core kernel (h*w %% 256 == 0, C %% 32 == 0)");
     CorrL1 l1{pred, loss, reinterpret_cast<signed char *>(sign), reinterpret_cast<float *>(workspace)};
     return corr4d_tc_launch_ex(feats_t, ft_sb, ft_sc, feats_r, fr_sb, fr_sc, fr_sf, m_target, mt_sb, m_refs, mr_sb,
-                               mr_sf, m_target ? 1 : 0, MH, MW, h, w, nullptr, B, C, F, h * w, (cudaStream_t)stream, &l1);
+                               mr_sf, m_target ? 1 : 0, MH, MW, h, w, nullptr, B, C, F, h * w, (cudaStream_t)stream, &l1,
+                               MT_DT_F32);
 }
 
 extern "C" int mt_corr4d_l1_bwd(const void *sign, const float *grad_loss, float *g_pred, int64_t n, mt_stream_t stream) {

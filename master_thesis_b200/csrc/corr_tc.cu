@@ -32,6 +32,16 @@
 // exactly in that canonical layout:
 //   4 channel rows x 128 B = one 512 B swizzle atom; SBO = 512 B between 4-channel groups;
 //   LBO = BK * 128 B between 32-pixel groups; one MMA (K = 8) spans two atoms.
+//
+// fp16 / bf16 features (the VGG's output under autocast) run the same single-CTA kernel as kind::f16, through the
+// operand traits CorrOp<T>: the exact half values are multiplied with fp32 accumulation, the two norm scales applied
+// in the fp32 epilogue and the volume rounded once, on store, to the features' dtype.  For 16-bit MN-major operands
+// the canonical layout is the ordinary 128 B swizzle (UMMA layout type 2, Swizzle<3,4,3>: the eight 16 B chunks of
+// a 128 B row are permuted by the row index mod 8), NOT the tf32 "32 B base" one.  TMA boxes of {64 pixels = 128 B,
+// 64 channels, pixel groups} with CU_TENSOR_MAP_SWIZZLE_128B land in it:
+//   8 channel rows x 128 B = one 1024 B atom; SBO = 1024 B between 8-channel groups;
+//   LBO = BK * 128 B between 64-pixel groups; one MMA (K = 16) spans two atoms.
+// A stage holds 128 B per pixel in both cases (32 fp32 or 64 half channels), so the rings and tile shapes are shared.
 #include <cuda.h>
 
 #include "mt_common.cuh"
@@ -109,6 +119,60 @@ __device__ __forceinline__ uint32_t staged_offset(int p, int k) {
     return (uint32_t)(g * (kBK * 128) + k * 128 + ((((px >> 3) ^ (k & 3)) << 5) | ((px & 7) << 2)));
 }
 
+// Operand traits of corr_tc_kernel: how features of element type T are staged, normalised and multiplied.
+template <typename T>
+struct CorrOp;
+template <>
+struct CorrOp<float> {  // kind::tf32 on the fp32 words
+    static constexpr int kBK = 32, kUmmaK = 8, kPhase = 4, kAtomBytes = 512, kGroupPx = 32;
+    static constexpr CUtensorMapDataType kTmaType = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    static constexpr CUtensorMapSwizzle kTmaSwizzle = CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
+    static constexpr uint32_t instr(int M, int N) { return instr_desc(M, N); }
+    __device__ static uint64_t desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) { return umma_desc(saddr, lbo, sbo); }
+    __device__ static void mma(uint32_t d, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t acc) {
+        umma_tf32(d, ad, bd, idesc, acc);
+    }
+    __device__ static uint32_t offset(int p, int k) { return staged_offset(p, k); }
+    __device__ static float load(const uint8_t *p) { return *reinterpret_cast<const float *>(p); }
+};
+template <typename T, uint32_t kFmt, CUtensorMapDataType kTma>
+struct CorrOpHalf {  // kind::f16; kFmt: a / b format of the instruction descriptor (F16 = 0, BF16 = 1)
+    static constexpr int kBK = 64, kUmmaK = 16, kPhase = 8, kAtomBytes = 1024, kGroupPx = 64;
+    static constexpr CUtensorMapDataType kTmaType = kTma;
+    static constexpr CUtensorMapSwizzle kTmaSwizzle = CU_TENSOR_MAP_SWIZZLE_128B;
+    // fp32 accumulate, A and B MN-major, M x N
+    static constexpr uint32_t instr(int M, int N) {
+        return (1u << 4) | (kFmt << 7) | (kFmt << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) |
+               ((uint32_t)(M >> 4) << 24);
+    }
+    // MN-major SWIZZLE_128B descriptor (sm_100 "version 1", layout type 2)
+    __device__ static uint64_t desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
+        uint64_t d = 0;
+        d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
+        d |= (uint64_t)((lbo >> 4) & 0x3FFFu) << 16;
+        d |= (uint64_t)((sbo >> 4) & 0x3FFFu) << 32;
+        d |= (uint64_t)1 << 46;
+        d |= (uint64_t)2 << 61;
+        return d;
+    }
+    __device__ static void mma(uint32_t d, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t acc) {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+            ::"r"(d), "l"(ad), "l"(bd), "r"(idesc), "r"(acc) : "memory");
+    }
+    // [pixel groups of 64][64 channels][128 B], 16 B chunks XOR-ed with (k mod 8)  (Swizzle<3,4,3>)
+    __device__ static uint32_t offset(int p, int k) {
+        const int g = p >> 6, px = p & 63;
+        return (uint32_t)(g * (kBK * 128) + k * 128 + ((((px >> 3) ^ (k & 7)) << 4) | ((px & 7) << 1)));
+    }
+    __device__ static float load(const uint8_t *p) { return widen(*reinterpret_cast<const T *>(p)); }
+};
+template <>
+struct CorrOp<__half> : CorrOpHalf<__half, 0u, CU_TENSOR_MAP_DATA_TYPE_FLOAT16> {};
+template <>
+struct CorrOp<__nv_bfloat16> : CorrOpHalf<__nv_bfloat16, 1u, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16> {};
+
 struct CorrTcArgs {
     // visibilities at feature resolution (mask_mode 0; NULL = all ones), or full-resolution masks m
     // (mask_mode 1): v = 1 - m[nearest source pixel], CorrelationVGG.forward model_dfpn.py:521-526
@@ -116,7 +180,7 @@ struct CorrTcArgs {
     const float *vr; int64_t vr_sb, vr_sf;         // (B, F, P) | (B, F, MH, MW)
     int mask_mode, MH, MW, fw;
     float msy, msx;                                // MH / fh, MW / fw in fp32 (ATen nearest: floor(dst * scale))
-    float *out;                                    // (B, F, P, P); unused in L1 mode
+    void *out;                                     // (B, F, P, P) in the features' dtype; unused in L1 mode
     // L1 mode (pred != NULL): the volume is not written; the epilogue compares it with `pred` (B, F, P, P) instead and
     // accumulates sum |pred - corr| (F.l1_loss(corr, corr_y), model_dfpn.py:254-257, SURVEY 8f-3).  sign (optional):
     // sign(pred - corr) as int8, all the backward pass needs.  partials: one float per (CTA, epilogue warp); the last
@@ -149,7 +213,8 @@ __device__ __forceinline__ signed char sign_i8(float d) { return d > 0.0f ? 1 : 
 // coalesced streaming stores of the volume, or (L1) the same rows of `pred` loaded instead (requested before the
 // TMEM read so that their latency hides under it) and |pred - corr| accumulated into `acc`.
 // `off0`: element offset of (first row of the block, first column of the tile) in the (B, F, P, P) volume.
-template <int TN, bool L1>
+// OT: element type of the volume (float, or the half features' type: each value rounded once, to nearest even).
+template <int TN, bool L1, typename OT = float>
 __device__ __forceinline__ void corr_epi_block(const CorrTcArgs &a, uint32_t taddr, float sa, const float *sbv, float *st,
                                                int64_t off0, int lane, float &acc) {
     const int rr = lane >> 3, c4 = (lane & 7) * 4;  // read-back: 4 rows x 8 float4 per instruction
@@ -196,8 +261,13 @@ __device__ __forceinline__ void corr_epi_block(const CorrTcArgs &a, uint32_t tad
                     sg.x = sign_i8(dx); sg.y = sign_i8(dy); sg.z = sign_i8(dz); sg.w = sign_i8(dw);
                     *reinterpret_cast<char4 *>(a.sign + off) = sg;
                 }
+            } else if constexpr (sizeof(OT) == 4) {
+                __stcs(reinterpret_cast<float4 *>(static_cast<float *>(a.out) + off), o);
             } else {
-                __stcs(reinterpret_cast<float4 *>(a.out + off), o);
+                uint2 u;
+                OT *e = reinterpret_cast<OT *>(&u);
+                e[0] = narrow<OT>(o.x); e[1] = narrow<OT>(o.y); e[2] = narrow<OT>(o.z); e[3] = narrow<OT>(o.w);
+                __stcs(reinterpret_cast<uint2 *>(static_cast<OT *>(a.out) + off), u);
             }
         }
         __syncwarp();
@@ -264,12 +334,15 @@ constexpr int smem_bytes_p() {
 //               instruction, which made the epilogue as long as the main loop)
 // Barriers: full/empty per smem stage (empty = MMA commit + one arrival per norm warp), tmem_full / tmem_empty and
 // scales_ready per accumulator buffer.
-template <int TM, int TN, int kStages>
+// T: element type of the features (CorrOp<T>); the volume is written in it.
+template <typename T, int TM, int TN, int kStages>
 __global__ void __launch_bounds__(kThreadsP, 1)
 corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                const CorrTcArgs a) {
+    using Op = CorrOp<T>;
+    static_assert(Op::kBK * sizeof(T) == kBK * 4, "a stage holds 128 B per pixel for every operand type");
     constexpr int kHalves = TM / 128;                 // UMMA M = 128 accumulators per tile
-    constexpr int kStageBytesA = TM * kBK * 4, kStageBytesB = TN * kBK * 4;
+    constexpr int kStageBytesA = TM * Op::kBK * (int)sizeof(T), kStageBytesB = TN * Op::kBK * (int)sizeof(T);
     constexpr int kBufCols = kHalves * TN;            // TMEM columns per accumulator buffer
     constexpr int kBufs = 2 * kBufCols <= 512 ? 2 : 1;  // accumulator buffers
     extern __shared__ uint8_t smem_raw[];
@@ -288,7 +361,7 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(scales_ready + 2);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int num_k = a.C / kBK;
+    const int num_k = a.C / Op::kBK;
 
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a) : "memory");
@@ -330,19 +403,19 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     const uint32_t ph = (it / kStages) & 1;
                     mbar_wait(smem_u32(empty + s), ph ^ 1);
                     mbar_expect_tx(smem_u32(full + s), kStageBytesA + kStageBytesB);
-                    // A: (pixel-in-group 32, channel C, pixel group P/32, batch B)
-                    tma_load_4d(smem_u32(smem_a + s * kStageBytesA), &map_a, smem_u32(full + s), 0, kb * kBK,
-                                m_tile * (TM / 32), b);
-                    // B: (pixel-in-group 32, channel C, pixel group P/32, frame F, batch B)
-                    tma_load_5d(smem_u32(smem_b + s * kStageBytesB), &map_b, smem_u32(full + s), 0, kb * kBK,
-                                n_tile * (TN / 32), f, b);
+                    // A: (pixel-in-group G, channel C, pixel group P/G, batch B), G = Op::kGroupPx
+                    tma_load_4d(smem_u32(smem_a + s * kStageBytesA), &map_a, smem_u32(full + s), 0, kb * Op::kBK,
+                                m_tile * (TM / Op::kGroupPx), b);
+                    // B: (pixel-in-group G, channel C, pixel group P/G, frame F, batch B)
+                    tma_load_5d(smem_u32(smem_b + s * kStageBytesB), &map_b, smem_u32(full + s), 0, kb * Op::kBK,
+                                n_tile * (TN / Op::kGroupPx), f, b);
                 }
             }
         }
     } else if (warp == 1) {
         // ===== MMA issuer (one elected lane) =====
         if (lane == 0) {
-            constexpr uint32_t idesc = instr_desc(128, TN);
+            constexpr uint32_t idesc = Op::instr(128, TN);
             uint32_t it = 0;
             int ti = 0;
             for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x, ++ti) {
@@ -357,14 +430,17 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     mbar_wait(smem_u32(full + s), ph);
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     const uint32_t a0 = smem_u32(smem_a + s * kStageBytesA), b0 = smem_u32(smem_b + s * kStageBytesB);
+                    // K advance inside the stage: next kUmmaK channels = two atoms (tf32 +1024 B, f16 +2048 B);
+                    // M halves: the A stage's pixel groups of the first and the second 128 pixels
+                    constexpr int kKStep = (Op::kUmmaK / Op::kPhase) * Op::kAtomBytes;
+                    constexpr int kHalfStep = (128 / Op::kGroupPx) * Op::kBK * 128;
 #pragma unroll
-                    for (int j = 0; j < kBK / kUmmaK; ++j) {
-                        // K advance inside the stage: next 8 channels = two 512 B atoms = +1024 B
-                        const uint64_t bd = umma_desc(b0 + j * 1024, kBK * 128, 512);
+                    for (int j = 0; j < Op::kBK / Op::kUmmaK; ++j) {
+                        const uint64_t bd = Op::desc(b0 + j * kKStep, Op::kBK * 128, Op::kAtomBytes);
 #pragma unroll
-                        for (int h = 0; h < kHalves; ++h) {  // M halves: pixel groups 0..3 and 4..7 of the A stage
-                            const uint64_t ad = umma_desc(a0 + h * (4 * kBK * 128) + j * 1024, kBK * 128, 512);
-                            umma_tf32(acc + h * TN, ad, bd, idesc, (kb | j) != 0 ? 1u : 0u);
+                        for (int h = 0; h < kHalves; ++h) {
+                            const uint64_t ad = Op::desc(a0 + h * kHalfStep + j * kKStep, Op::kBK * 128, Op::kAtomBytes);
+                            Op::mma(acc + h * TN, ad, bd, idesc, (kb | j) != 0 ? 1u : 0u);
                         }
                     }
                     umma_commit(smem_u32(empty + s));  // frees the smem slot when these MMAs retire
@@ -380,11 +456,12 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         constexpr bool kSplit = TM + TN <= 256;
         const bool has_a = t < TM, has_b = kSplit ? (t >= TM && t < TM + TN) : (t < TN);
         const int ta = has_a ? t : 0, tb = has_b ? (kSplit ? t - TM : t) : 0;
-        // the swizzle phase repeats every 4 channels: channel k = 4 j + r lives at base[r] + 512 j,
-        // so the loop below is 32 LDS with immediate offsets + 32 FFMA per operand, no address math
-        uint32_t base_a[4], base_b[4];
+        // the swizzle phase repeats every kPhase channels: channel k = kPhase j + r lives at base[r] + atom * j,
+        // so the loop below is kBK LDS with immediate offsets + kBK FFMA per operand, no address math (half values
+        // are widened before they are squared)
+        uint32_t base_a[Op::kPhase], base_b[Op::kPhase];
 #pragma unroll
-        for (int r = 0; r < 4; ++r) { base_a[r] = staged_offset(ta, r); base_b[r] = staged_offset(tb, r); }
+        for (int r = 0; r < Op::kPhase; ++r) { base_a[r] = Op::offset(ta, r); base_b[r] = Op::offset(tb, r); }
         uint32_t it = 0;
         int ti = 0;
         for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x, ++ti) {
@@ -403,21 +480,21 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 const uint8_t *pa = smem_a + s * kStageBytesA, *pb = smem_b + s * kStageBytesB;
                 if (has_a) {
 #pragma unroll
-                    for (int r = 0; r < 4; ++r) {
+                    for (int r = 0; r < Op::kPhase; ++r) {
 #pragma unroll
-                        for (int j = 0; j < kBK / 4; ++j) {
-                            const float va = *reinterpret_cast<const float *>(pa + base_a[r] + j * 512);
-                            qa[r] = __fmaf_rn(va, va, qa[r]);
+                        for (int j = 0; j < Op::kBK / Op::kPhase; ++j) {
+                            const float va = Op::load(pa + base_a[r] + j * Op::kAtomBytes);
+                            qa[r & 3] = __fmaf_rn(va, va, qa[r & 3]);
                         }
                     }
                 }
                 if (has_b) {
 #pragma unroll
-                    for (int r = 0; r < 4; ++r) {
+                    for (int r = 0; r < Op::kPhase; ++r) {
 #pragma unroll
-                        for (int j = 0; j < kBK / 4; ++j) {
-                            const float vb = *reinterpret_cast<const float *>(pb + base_b[r] + j * 512);
-                            qb[r] = __fmaf_rn(vb, vb, qb[r]);
+                        for (int j = 0; j < Op::kBK / Op::kPhase; ++j) {
+                            const float vb = Op::load(pb + base_b[r] + j * Op::kAtomBytes);
+                            qb[r & 3] = __fmaf_rn(vb, vb, qb[r & 3]);
                         }
                     }
                 }
@@ -463,7 +540,7 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 const int64_t off0 = ((int64_t)frame * a.P + m_tile * TM + row0) * a.P + n_tile * TN;
                 const uint32_t taddr = tmem_base + ((uint32_t)(lq * 32) << 16) + (uint32_t)(buf * kBufCols + h * TN);
                 if (a.pred) corr_epi_block<TN, true>(a, taddr, sa, sbv, st, off0, lane, l1_acc);
-                else corr_epi_block<TN, false>(a, taddr, sa, sbv, st, off0, lane, l1_acc);
+                else corr_epi_block<TN, false, T>(a, taddr, sa, sbv, st, off0, lane, l1_acc);
             }
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncwarp();
@@ -811,18 +888,71 @@ int64_t corr4d_tc_workspace_bytes(int B, int C, int F, int P) {
     return 0;  // norms are fused into the GEMM: no scratch
 }
 
+// The single-CTA launch of corr_tc_kernel<T> for the tile shape tm x tn
+template <typename T>
+static int corr_tc_single_go(const CUtensorMap &map_a, const CUtensorMap &map_b, const CorrTcArgs &a, int tm, int tn,
+                             cudaStream_t st) {
+    int ctas = sm_count();
+    if (ctas > a.n_tiles) ctas = a.n_tiles;
+    dim3 grid(ctas);
+#define MT_CORR_GO(TMV, TNV, STG)                                                                    \
+    do {                                                                                             \
+        static_assert(smem_bytes_p<TMV, TNV, STG>() <= 227 * 1024, "stage ring exceeds the shared memory of an SM"); \
+        cudaError_t e = cudaFuncSetAttribute(corr_tc_kernel<T, TMV, TNV, STG>,                       \
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes_p<TMV, TNV, STG>()); \
+        if (e != cudaSuccess) {                                                                      \
+            set_error("mt_corr4d_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));             \
+            return MT_ERR_CUDA;                                                                      \
+        }                                                                                            \
+        launch(corr_tc_kernel<T, TMV, TNV, STG>, grid, dim3(kThreadsP), (size_t)smem_bytes_p<TMV, TNV, STG>(), st, map_a, map_b, a); \
+    } while (0)
+    if (tm == 256) {
+        if (tn == 256) MT_CORR_GO(256, 256, 3);       // 3 x 64 KB
+        else if (tn == 128) MT_CORR_GO(256, 128, 4);  // 4 x 48 KB
+        else MT_CORR_GO(256, 64, 5);                  // 5 x 40 KB
+    } else {
+        if (tn == 256) MT_CORR_GO(128, 256, 4);       // 4 x 48 KB
+        else if (tn == 128) MT_CORR_GO(128, 128, 6);  // 6 x 32 KB
+        else MT_CORR_GO(128, 64, 8);                  // 8 x 24 KB
+    }
+#undef MT_CORR_GO
+    return launch_status("mt_corr4d_fwd");
+}
+
+// tensor-map parameters of the operand traits CorrOp<T>
+struct CorrMapSpec {
+    CUtensorMapDataType type;
+    CUtensorMapSwizzle swizzle;
+    int esize, group_px, bk;
+};
+template <typename T>
+static CorrMapSpec corr_map_spec() {
+    return {CorrOp<T>::kTmaType, CorrOp<T>::kTmaSwizzle, (int)sizeof(T), CorrOp<T>::kGroupPx, CorrOp<T>::kBK};
+}
+
 // Strided form.  ft (B, C, P): strides ft_sb, ft_sc; fr (B, C, F, P): fr_sb, fr_sc, fr_sf (elements; the pixel index
-// is contiguous).  Masks: see CorrTcArgs.
-int corr4d_tc_launch_ex(const float *ft, int64_t ft_sb, int64_t ft_sc, const float *fr, int64_t fr_sb, int64_t fr_sc,
+// is contiguous).  Masks: see CorrTcArgs.  dtype (MT_DT_*): element type of ft / fr and of the volume `out`; fp16 /
+// bf16 features run the single-CTA kind::f16 kernel in store mode (no L1 mode, no CTA pairs).
+int corr4d_tc_launch_ex(const void *ft, int64_t ft_sb, int64_t ft_sc, const void *fr, int64_t fr_sb, int64_t fr_sc,
                         int64_t fr_sf, const float *vt, int64_t vt_sb, const float *vr, int64_t vr_sb, int64_t vr_sf,
-                        int mask_mode, int MH, int MW, int fh, int fw, float *out, int B, int C, int F, int P,
-                        cudaStream_t st, const CorrL1 *l1) {
+                        int mask_mode, int MH, int MW, int fh, int fw, void *out, int B, int C, int F, int P,
+                        cudaStream_t st, const CorrL1 *l1, int dtype) {
+    CorrMapSpec ms{};
+    const int drc = with_dtype(dtype, "mt_corr4d_fwd", [&](auto t) {
+        ms = corr_map_spec<decltype(t)>();
+        return MT_OK;
+    });
+    if (drc) return drc;
+    const bool half = dtype != MT_DT_F32;
+    MT_REQUIRE(!half || !l1, "mt_corr4d_vgg_l1_fwd: fp32 features only");
+    MT_REQUIRE(C % ms.bk == 0, "mt_corr4d_fwd: C = %d is not a multiple of %d channels", C, ms.bk);
     MT_REQUIRE(aligned16(ft) && aligned16(fr) && (l1 || aligned16(out)), "mt_corr4d_fwd: pointers must be 16 B aligned");
     MT_REQUIRE(!l1 || (l1->pred && l1->loss && l1->partials && aligned16(l1->pred) && aligned16(l1->sign)),
                "mt_corr4d_vgg_l1_fwd: pred, loss and workspace are required, pred / sign 16 B aligned");
-    MT_REQUIRE(!((ft_sb | ft_sc | fr_sb | fr_sc | fr_sf) & 3) && ft_sc > 0 && fr_sc > 0 && (B == 1 || (ft_sb > 0 && fr_sb > 0)) &&
+    const int64_t smask = 16 / ms.esize - 1;  // tensor-map strides are multiples of 16 B
+    MT_REQUIRE(!((ft_sb | ft_sc | fr_sb | fr_sc | fr_sf) & smask) && ft_sc > 0 && fr_sc > 0 && (B == 1 || (ft_sb > 0 && fr_sb > 0)) &&
                (F == 1 || fr_sf > 0) && ft_sb >= 0 && fr_sb >= 0 && fr_sf >= 0,
-               "mt_corr4d_fwd: feature strides must be positive multiples of 4 elements");
+               "mt_corr4d_fwd: feature strides must be positive multiples of 16 B (%d elements)", (int)smask + 1);
     EncodeTiledFn enc = encode_fn();
     if (!enc) {
         set_error("mt_corr4d_fwd: cuTensorMapEncodeTiled is not available from the driver");
@@ -852,24 +982,27 @@ int corr4d_tc_launch_ex(const float *ft, int64_t ft_sb, int64_t ft_sc, const flo
     }
     if (P % tn) tn = 64;
     // CTA pairs (cta_group::2): whole-frame tiles on two SMs.  MT_CORR_2CTA = 1 forces, 0 disables; default: when the
-    // batch fills the pairs (see profiles/r2_experiments.md)
+    // batch fills the pairs (see profiles/r2_experiments.md).  fp32 features only: half features always take the
+    // single-CTA kernel
     // ncu (profiles/r2_experiments.md): 128 frames 29.8 vs 28.5 us, 256 frames 49.3 vs 51.4 us, 512 frames 84.4 vs 98.6 us
     // (pairs vs single CTAs); graph-replayed cfg3 step at 256 / 512 frames: +1.2 % / -1.2 %.  The pairs win once every
     // pair has ~5 whole-frame tiles; at 512 frames they run at 85 % of the HBM roofline (5.6 TB/s), where the op -
     // bandwidth-bound from cold DRAM at 73 flop/B - cannot go much faster
     int pair = tuning("MT_CORR_2CTA", -1);
     if (pair < 0) pair = kPairDefault && !tm_given && !tn_given && frames * 2 >= sm_count() * 5 ? 1 : 0;
+    if (half) pair = 0;
     if (pair && !tn_given) tn = 256;
     if (pair && tn == 64) tn = 128;
     CUtensorMap map_a, map_b;
     {
-        // ft (B, C, P) viewed as (32, C, P/32, B): strides in bytes for dims 1..3
-        cuuint64_t dims[4] = {32, (cuuint64_t)C, (cuuint64_t)(P / 32), (cuuint64_t)B};
-        cuuint64_t strides[3] = {(cuuint64_t)ft_sc * 4, 128, (cuuint64_t)(B > 1 ? ft_sb : (int64_t)C * P) * 4};
-        cuuint32_t box[4] = {32, (cuuint32_t)kBK, (cuuint32_t)((pair ? 128 : tm) / 32), 1};
+        // ft (B, C, P) viewed as (G, C, P/G, B), G = pixels per 128 B (32 fp32, 64 half): strides in bytes for dims 1..3
+        const int G = ms.group_px, es = ms.esize;
+        cuuint64_t dims[4] = {(cuuint64_t)G, (cuuint64_t)C, (cuuint64_t)(P / G), (cuuint64_t)B};
+        cuuint64_t strides[3] = {(cuuint64_t)ft_sc * es, 128, (cuuint64_t)(B > 1 ? ft_sb : (int64_t)C * P) * es};
+        cuuint32_t box[4] = {(cuuint32_t)G, (cuuint32_t)ms.bk, (cuuint32_t)((pair ? 128 : tm) / G), 1};
         cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = enc(&map_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float *>(ft), dims, strides, box,
-                         estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
+        CUresult r = enc(&map_a, ms.type, 4, const_cast<void *>(ft), dims, strides, box,
+                         estr, CU_TENSOR_MAP_INTERLEAVE_NONE, ms.swizzle,
                          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) {
             set_error("mt_corr4d_fwd: cuTensorMapEncodeTiled(A) failed with %d", (int)r);
@@ -877,14 +1010,15 @@ int corr4d_tc_launch_ex(const float *ft, int64_t ft_sb, int64_t ft_sc, const flo
         }
     }
     {
-        // fr (B, C, F, P) viewed as (32, C, P/32, F, B)
-        cuuint64_t dims[5] = {32, (cuuint64_t)C, (cuuint64_t)(P / 32), (cuuint64_t)F, (cuuint64_t)B};
-        cuuint64_t strides[4] = {(cuuint64_t)fr_sc * 4, 128, (cuuint64_t)(F > 1 ? fr_sf : (int64_t)P) * 4,
-                                 (cuuint64_t)(B > 1 ? fr_sb : (int64_t)C * F * P) * 4};
-        cuuint32_t box[5] = {32, (cuuint32_t)kBK, (cuuint32_t)((pair ? tn / 2 : tn) / 32), 1, 1};
+        // fr (B, C, F, P) viewed as (G, C, P/G, F, B)
+        const int G = ms.group_px, es = ms.esize;
+        cuuint64_t dims[5] = {(cuuint64_t)G, (cuuint64_t)C, (cuuint64_t)(P / G), (cuuint64_t)F, (cuuint64_t)B};
+        cuuint64_t strides[4] = {(cuuint64_t)fr_sc * es, 128, (cuuint64_t)(F > 1 ? fr_sf : (int64_t)P) * es,
+                                 (cuuint64_t)(B > 1 ? fr_sb : (int64_t)C * F * P) * es};
+        cuuint32_t box[5] = {(cuuint32_t)G, (cuuint32_t)ms.bk, (cuuint32_t)((pair ? tn / 2 : tn) / G), 1, 1};
         cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&map_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<float *>(fr), dims, strides, box,
-                         estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
+        CUresult r = enc(&map_b, ms.type, 5, const_cast<void *>(fr), dims, strides, box,
+                         estr, CU_TENSOR_MAP_INTERLEAVE_NONE, ms.swizzle,
                          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) {
             set_error("mt_corr4d_fwd: cuTensorMapEncodeTiled(B) failed with %d", (int)r);
@@ -935,38 +1069,16 @@ int corr4d_tc_launch_ex(const float *ft, int64_t ft_sb, int64_t ft_sc, const flo
 #undef MT_CORR_PAIR_GO
         return launch_status("mt_corr4d_fwd");
     }
-    int ctas = sm_count();
-    if (ctas > a.n_tiles) ctas = a.n_tiles;
-    dim3 grid(ctas);
-#define MT_CORR_GO(TMV, TNV, STG)                                                                    \
-    do {                                                                                             \
-        static_assert(smem_bytes_p<TMV, TNV, STG>() <= 227 * 1024, "stage ring exceeds the shared memory of an SM"); \
-        cudaError_t e = cudaFuncSetAttribute(corr_tc_kernel<TMV, TNV, STG>,                          \
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes_p<TMV, TNV, STG>()); \
-        if (e != cudaSuccess) {                                                                      \
-            set_error("mt_corr4d_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));             \
-            return MT_ERR_CUDA;                                                                      \
-        }                                                                                            \
-        launch(corr_tc_kernel<TMV, TNV, STG>, grid, dim3(kThreadsP), (size_t)smem_bytes_p<TMV, TNV, STG>(), st, map_a, map_b, a); \
-    } while (0)
-    if (tm == 256) {
-        if (tn == 256) MT_CORR_GO(256, 256, 3);       // 3 x 64 KB
-        else if (tn == 128) MT_CORR_GO(256, 128, 4);  // 4 x 48 KB
-        else MT_CORR_GO(256, 64, 5);                  // 5 x 40 KB
-    } else {
-        if (tn == 256) MT_CORR_GO(128, 256, 4);       // 4 x 48 KB
-        else if (tn == 128) MT_CORR_GO(128, 128, 6);  // 6 x 32 KB
-        else MT_CORR_GO(128, 64, 8);                  // 8 x 24 KB
-    }
-#undef MT_CORR_GO
-    return launch_status("mt_corr4d_fwd");
+    if (dtype == MT_DT_F16) return corr_tc_single_go<__half>(map_a, map_b, a, tm, tn, st);
+    if (dtype == MT_DT_BF16) return corr_tc_single_go<__nv_bfloat16>(map_a, map_b, a, tm, tn, st);
+    return corr_tc_single_go<float>(map_a, map_b, a, tm, tn, st);
 }
 
 int corr4d_tc_launch(const float *ft, const float *vt, const float *fr, const float *vr, float *out, void *ws,
                      int64_t ws_bytes, int B, int C, int F, int P, cudaStream_t st) {
     (void)ws; (void)ws_bytes;
     return corr4d_tc_launch_ex(ft, (int64_t)C * P, P, fr, (int64_t)C * F * P, (int64_t)F * P, P, vt, P, vr,
-                               (int64_t)F * P, P, 0, 0, 0, 0, 0, out, B, C, F, P, st, nullptr);
+                               (int64_t)F * P, P, 0, 0, 0, 0, 0, out, B, C, F, P, st, nullptr, MT_DT_F32);
 }
 
 }  // namespace mt

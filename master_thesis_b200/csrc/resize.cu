@@ -106,15 +106,25 @@ __global__ void __launch_bounds__(kThreads) resize_set_kernel(const ResizeSetArg
 }
 
 struct ResizeFlowArgs {
-    const float *in; int64_t sb, sf, sy, sx, sc;
+    const void *in; int64_t sb, sf, sy, sx, sc;  // element type: the kernel's T
     float *out; int64_t o_sb, o_sf, o_sy, o_sx, o_sc;
     int F, h, w, H, W, chunks;
     float scy, scx;  // h / H, w / W in fp32
     bool bilinear, chain;
 };
 
+// one flow component, widened to fp32 (exact)
+__device__ __forceinline__ float ld_comp(const float *p) { return __ldg(p); }
+__device__ __forceinline__ float ld_comp(const __half *p) {
+    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short *>(p))));
+}
+__device__ __forceinline__ float ld_comp(const __nv_bfloat16 *p) {
+    return __bfloat162float(__ushort_as_bfloat16(__ldg(reinterpret_cast<const unsigned short *>(p))));
+}
+
 // OUT: 0 = output through its strides, 1 = planar rows (o_sx = 1), 2 = interleaved (o_sx = 2, o_sc = 1)
-template <int OUT>
+// T: element type of the input flow (float, __half, __nv_bfloat16); the output is fp32
+template <int OUT, typename T = float>
 __global__ void __launch_bounds__(kThreads) resize_flow_kernel(const ResizeFlowArgs a) {
     pdl_sync();
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -122,26 +132,26 @@ __global__ void __launch_bounds__(kThreads) resize_flow_kernel(const ResizeFlowA
     if (oy >= a.H) return;
     const int ox0 = (idx - oy * a.chunks) * PIX;
     const int n = blockIdx.y, b = n / a.F, f = n - b * a.F;
-    const float *src = a.in + b * a.sb + f * a.sf;
+    const T *src = static_cast<const T *>(a.in) + b * a.sb + f * a.sf;
     float gx[PIX], gy[PIX];
     if (!a.bilinear) {
-        const float *row = src + nearest_index(oy, a.h, a.H, a.scy) * a.sy;
+        const T *row = src + nearest_index(oy, a.h, a.H, a.scy) * a.sy;
 #pragma unroll
         for (int i = 0; i < PIX; ++i) {
-            const float *q = row + nearest_index(min(ox0 + i, a.W - 1), a.w, a.W, a.scx) * a.sx;
-            gx[i] = __ldg(q);
-            gy[i] = __ldg(q + a.sc);
+            const T *q = row + nearest_index(min(ox0 + i, a.W - 1), a.w, a.W, a.scx) * a.sx;
+            gx[i] = ld_comp(q);
+            gy[i] = ld_comp(q + a.sc);
         }
     } else {
         const Lin ly = lin_index(oy, a.h, a.H, a.scy);
-        const float *r0 = src + ly.i0 * a.sy, *r1 = src + ly.i1 * a.sy;
+        const T *r0 = src + ly.i0 * a.sy, *r1 = src + ly.i1 * a.sy;
 #pragma unroll
         for (int i = 0; i < PIX; ++i) {
             const Lin lx = lin_index(min(ox0 + i, a.W - 1), a.w, a.W, a.scx);
             const int64_t c0 = lx.i0 * a.sx, c1 = lx.i1 * a.sx;
-            gx[i] = bil(__ldg(r0 + c0), __ldg(r0 + c1), __ldg(r1 + c0), __ldg(r1 + c1), ly, lx, a.chain);
-            gy[i] = bil(__ldg(r0 + c0 + a.sc), __ldg(r0 + c1 + a.sc), __ldg(r1 + c0 + a.sc), __ldg(r1 + c1 + a.sc),
-                        ly, lx, a.chain);
+            gx[i] = bil(ld_comp(r0 + c0), ld_comp(r0 + c1), ld_comp(r1 + c0), ld_comp(r1 + c1), ly, lx, a.chain);
+            gy[i] = bil(ld_comp(r0 + c0 + a.sc), ld_comp(r0 + c1 + a.sc), ld_comp(r1 + c0 + a.sc),
+                        ld_comp(r1 + c1 + a.sc), ly, lx, a.chain);
         }
     }
     float *dst = a.out + b * a.o_sb + f * a.o_sf + oy * a.o_sy;
@@ -235,9 +245,12 @@ extern "C" int mt_resize_set(const float *x, int64_t x_sb, int64_t x_sc, int64_t
     return launch_status("mt_resize_set");
 }
 
-extern "C" int mt_resize_flow(const float *flow, int64_t sb, int64_t sf, int64_t sy, int64_t sx, int64_t sc,
-                              float *out, int64_t o_sb, int64_t o_sf, int64_t o_sy, int64_t o_sx, int64_t o_sc,
-                              int B, int F, int h, int w, int H, int W, int mode, mt_stream_t stream) {
+// flow_dtype (MT_DT_*): element type of the input flow.  Under autocast the DFPN's flow estimators return fp16 / bf16
+// flows; upsample_bilinear2d / upsample_nearest2d run in fp32 there (autocast's fp32 policy), so FlowsUtils.resize_flow
+// (utils.py:107-126) returns an fp32 flow computed on the exactly widened input: out is fp32 for every flow_dtype.
+extern "C" int mt_resize_flow_dt(int flow_dtype, const void *flow, int64_t sb, int64_t sf, int64_t sy, int64_t sx,
+                                 int64_t sc, float *out, int64_t o_sb, int64_t o_sf, int64_t o_sy, int64_t o_sx,
+                                 int64_t o_sc, int B, int F, int h, int w, int H, int W, int mode, mt_stream_t stream) {
     MT_REQUIRE(flow && out, "mt_resize_flow: NULL argument");
     MT_REQUIRE(B > 0 && F > 0 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)B * F <= 65535 &&
                    (int64_t)H * W <= (1ll << 30),
@@ -247,12 +260,25 @@ extern "C" int mt_resize_flow(const float *flow, int64_t sb, int64_t sf, int64_t
                      F, h, w, H, W, (W + PIX - 1) / PIX,
                      (float)h / (float)H, (float)w / (float)W, mode == MT_RESIZE_BILINEAR, H + W <= 128};
     const bool al = aligned16(out) && mult4(o_sb) && mult4(o_sf) && mult4(o_sy);
+    const int out_kind = (al && o_sx == 1 && mult4(o_sc)) ? 1 : ((al && o_sx == 2 && o_sc == 1) ? 2 : 0);
     dim3 grid((unsigned)(((int64_t)H * a.chunks + kThreads - 1) / kThreads), B * F);
     cudaStream_t st = (cudaStream_t)stream;
-    if (al && o_sx == 1 && mult4(o_sc)) launch(resize_flow_kernel<1>, grid, kThreads, 0, st, a);
-    else if (al && o_sx == 2 && o_sc == 1) launch(resize_flow_kernel<2>, grid, kThreads, 0, st, a);
-    else launch(resize_flow_kernel<0>, grid, kThreads, 0, st, a);
+    const int rc = with_dtype(flow_dtype, "mt_resize_flow_dt", [&](auto t) {
+        using T = decltype(t);
+        if (out_kind == 1) launch(resize_flow_kernel<1, T>, grid, kThreads, 0, st, a);
+        else if (out_kind == 2) launch(resize_flow_kernel<2, T>, grid, kThreads, 0, st, a);
+        else launch(resize_flow_kernel<0, T>, grid, kThreads, 0, st, a);
+        return MT_OK;
+    });
+    if (rc) return rc;
     return launch_status("mt_resize_flow");
+}
+
+extern "C" int mt_resize_flow(const float *flow, int64_t sb, int64_t sf, int64_t sy, int64_t sx, int64_t sc,
+                              float *out, int64_t o_sb, int64_t o_sf, int64_t o_sy, int64_t o_sx, int64_t o_sc,
+                              int B, int F, int h, int w, int H, int W, int mode, mt_stream_t stream) {
+    return mt_resize_flow_dt(MT_DT_F32, flow, sb, sf, sy, sx, sc, out, o_sb, o_sf, o_sy, o_sx, o_sc, B, F, h, w, H, W,
+                             mode, stream);
 }
 
 extern "C" int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,

@@ -41,7 +41,9 @@ constexpr int kWarpL1BMinB = 8;  // fused-loss backward: 64 registers, no spills
 // checks the ranges), because 64-bit stride arithmetic dominated the per-thread
 // setup of the first versions.
 struct WarpFwdArgs {
-    const float *x, *vis, *grid, *m_target;
+    const float *x, *vis;
+    const void *grid;  // theta (fp32) or a dense flow of the kernel's flow element type
+    const float *m_target;
     float *x_al, *v_al, *v_map;
     int x_sb, x_sc, x_sf, vis_sb, vis_sf, mt_sb, xa_sb, xa_sc, xa_sf;
     int F, P;
@@ -74,9 +76,12 @@ struct WarpFwdArgs {
 // needs no second pass over the aligned frame (SURVEY 8f-2).
 // LOWRES (dense flow only): the flow is given at gh x gw and bilinearly resized to H x W in the kernel - the
 // resized flow is never written or read back (SURVEY 8f-1); bit-identical to resizing first.
-template <int C, int VIS, bool AFFINE, bool FULL, bool PACK = false, bool LOWRES = false>
+// G: element type of a dense flow (float, __half, __nv_bfloat16), widened on load: the output is the fp32 kernel's on
+// the widened flow.
+template <int C, int VIS, bool AFFINE, bool FULL, bool PACK = false, bool LOWRES = false, typename G = float>
 __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFwdArgs a) {
     static_assert(!(AFFINE && LOWRES), "a theta needs no resize");
+    static_assert(!AFFINE || sizeof(G) == 4, "a theta is fp32");
     constexpr int U = kRows;
     pdl_sync();
     __shared__ float s_by[U];
@@ -108,7 +113,7 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
 
     float t1 = 0.f, t2 = 0.f, t4 = 0.f, t5 = 0.f, bxt0 = 0.f, bxt3 = 0.f;
     if (AFFINE) {
-        const float *th = a.grid + n * 6;
+        const float *th = static_cast<const float *>(a.grid) + n * 6;
         const float bx = base_coord(x, W, a.sp.stepx, ac);
         bxt0 = __fmul_rn(bx, __ldg(th));
         bxt3 = __fmul_rn(bx, __ldg(th + 3));
@@ -121,7 +126,7 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
     if (kDense) {
 #pragma unroll
         for (int k = 0; k < U; ++k)
-            g[k] = (y0 + k < H) ? __ldcs(reinterpret_cast<const float2 *>(a.grid) + ((int)n * a.P + (y0 + k) * W + x))
+            g[k] = (y0 + k < H) ? flow_ldcs(static_cast<const Flow2<G> *>(a.grid) + ((int)n * a.P + (y0 + k) * W + x))
                                 : make_float2(0.0f, 0.0f);
     }
     const int p0 = y0 * W + x;
@@ -154,7 +159,7 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
             gy = __fadd_rn(__fmaf_rn(by, t4, bxt3), t5);
         } else if (LOWRES) {
             const Lin ly = s_ly[k];
-            const float2 *fl = reinterpret_cast<const float2 *>(a.grid) + (int)n * (a.gh * a.gw);
+            const Flow2<G> *fl = static_cast<const Flow2<G> *>(a.grid) + (int)n * (a.gh * a.gw);
             const float2 gl = lin_flow(fl + ly.i0 * a.gw, fl + ly.i1 * a.gw, lx, ly.l0, ly.l1);
             gx = gl.x; gy = gl.y;
         } else {
@@ -588,13 +593,32 @@ struct PackOut {
     float *nn_in;
 };
 
+// the launches of warp_fwd_impl for a half dense flow (element type G): the DFPN flavour, nearest visibility
+template <typename G>
+static void warp_half_flow_go(const WarpFwdArgs &a, dim3 gridd, dim3 block, cudaStream_t st, int C, bool pack,
+                              bool lowres, bool full) {
+    if (pack && lowres) launch(warp_fwd_kernel<3, 1, false, false, true, true, G>, gridd, block, 0, st, a);
+    else if (lowres && full) launch(warp_fwd_kernel<3, 1, false, true, false, true, G>, gridd, block, 0, st, a);
+    else if (lowres) launch(warp_fwd_kernel<3, 1, false, false, false, true, G>, gridd, block, 0, st, a);
+    else if (pack) launch(warp_fwd_kernel<3, 1, false, false, true, false, G>, gridd, block, 0, st, a);
+    else if (C == 3 && full) launch(warp_fwd_kernel<3, 1, false, true, false, false, G>, gridd, block, 0, st, a);
+    else if (C == 3) launch(warp_fwd_kernel<3, 1, false, false, false, false, G>, gridd, block, 0, st, a);
+    else if (full) launch(warp_fwd_kernel<1, 1, false, true, false, false, G>, gridd, block, 0, st, a);
+    else launch(warp_fwd_kernel<1, 1, false, false, false, false, G>, gridd, block, 0, st, a);
+}
+
+// g_dtype (MT_DT_*): element type of a dense flow; a theta is fp32
 static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
-                         const float *vis, int64_t vis_sb, int64_t vis_sf, const float *grid,
+                         const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype, const void *grid,
                          const float *m_target, int64_t mt_sb, float *x_aligned, int64_t xa_sb,
                          int64_t xa_sc, int64_t xa_sf, float *v_aligned, float *v_map, int B,
                          int C, int F, int H, int W, int flags, mt_stream_t stream, const PackOut *pack,
                          int gh = 0, int gw = 0) {
     MT_REQUIRE(x && vis && grid, "mt_warp_fwd: NULL input");
+    MT_REQUIRE(g_dtype == MT_DT_F32 || g_dtype == MT_DT_F16 || g_dtype == MT_DT_BF16,
+               "mt_warp_fwd: unknown flow dtype code %d", g_dtype);
+    MT_REQUIRE(g_dtype == MT_DT_F32 || !(flags & (MT_GRID_AFFINE | MT_VIS_BILINEAR)),
+               "mt_warp_fwd: a half grid must be a dense flow with nearest visibility (a theta is fp32)");
     const bool lowres = gh > 0 && gw > 0 && !(gh == H && gw == W);
     MT_REQUIRE(!lowres || (!(flags & MT_GRID_AFFINE) && !(flags & MT_VIS_BILINEAR) && C == 3 &&
                            (int64_t)B * F * gh * gw * 2 < (1ll << 31) - 1),
@@ -603,7 +627,9 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     MT_REQUIRE(C == 1 || C == 3, "mt_warp_fwd: C must be 1 or 3 (reference hard-codes 3, utils.py:97), got %d", C);
     MT_REQUIRE((int64_t)B * F <= 65535, "mt_warp_fwd: B*F > 65535");
     MT_REQUIRE(!v_map || m_target, "mt_warp_fwd: v_map needs m_target");
-    MT_REQUIRE((flags & MT_GRID_AFFINE) || aligned8(grid), "mt_warp_fwd: dense grid must be 8 B aligned");
+    const uintptr_t g_align = g_dtype == MT_DT_F32 ? 8u : 4u;  // one (gx, gy) pair per load
+    MT_REQUIRE((flags & MT_GRID_AFFINE) || (reinterpret_cast<uintptr_t>(grid) & (g_align - 1)) == 0,
+               "mt_warp_fwd: a dense flow must be aligned to one (gx, gy) pair (%d B)", (int)g_align);
     MT_REQUIRE((H + kRows - 1) / kRows <= 65535, "mt_warp_fwd: H too large");
     const int64_t P = (int64_t)H * W, lim = (1ll << 31) - 1;
     auto span = [&](int64_t sb, int64_t sc, int64_t sf, int c) {
@@ -640,6 +666,12 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     dim3 block(kCols), gridd((W + kCols - 1) / kCols, (H + kRows - 1) / kRows, B * F);
     cudaStream_t st = (cudaStream_t)stream;
     const bool full = x_aligned && v_aligned && v_map;
+    if (g_dtype != MT_DT_F32) {
+        if (g_dtype == MT_DT_F16) warp_half_flow_go<__half>(a, gridd, block, st, C, pack != nullptr, lowres, full);
+        else warp_half_flow_go<__nv_bfloat16>(a, gridd, block, st, C, pack != nullptr, lowres, full);
+        return launch_status(pack ? (lowres ? "mt_warp_pack_lowres_fwd_dt" : "mt_warp_pack_fwd_dt")
+                                  : (lowres ? "mt_warp_lowres_fwd_dt" : "mt_warp_fwd_dt"));
+    }
     if (pack && lowres) {  // DFPN inference step at a frame size other than the flow's 256 x 256
         launch(warp_fwd_kernel<3, 1, false, false, true, true>, gridd, block, 0, st, a);
         return launch_status("mt_warp_pack_lowres_fwd");
@@ -658,7 +690,7 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     }
     if (affine && vis_bil && C == 3 && full) {
         // CPN.align tail: persistent kernel with TMA-staged reference tiles (warp_tma.cu) when it applies
-        const int rc = warp_staged_launch(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, grid, m_target, mt_sb, x_aligned,
+        const int rc = warp_staged_launch(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, static_cast<const float *>(grid), m_target, mt_sb, x_aligned,
                                           xa_sb, xa_sc, xa_sf, v_aligned, v_map, B, F, H, W, a.sp.ac, a.from_mask, st);
         if (rc < 0) return rc;
         if (rc == 1) return launch_status("mt_warp_fwd");
@@ -680,13 +712,39 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     return launch_status("mt_warp_fwd");
 }
 
+// The _dt entry points take the element type of the dense flow (MT_DT_*).  Under autocast the DFPN's flow estimators
+// return fp16 / bf16 flows; grid_sample is on autocast's promote list, so DFPN.align (model_dfpn.py:128-133,
+// utils.py:93-103) samples the fp32 frames with the exactly widened flow, and the bilinear flow resize before it
+// (utils.py:107-126, model_dfpn.py:100-101) computes in fp32 on the widened flow too.  The kernels widen the flow on
+// load: the outputs are those of the fp32 entry points given flow.float().
+extern "C" int mt_warp_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                              const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype, const void *grid,
+                              const float *m_target, int64_t mt_sb, float *x_aligned, int64_t xa_sb,
+                              int64_t xa_sc, int64_t xa_sf, float *v_aligned, float *v_map, int B,
+                              int C, int F, int H, int W, int flags, mt_stream_t stream) {
+    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, grid, m_target, mt_sb, x_aligned, xa_sb,
+                         xa_sc, xa_sf, v_aligned, v_map, B, C, F, H, W, flags, stream, nullptr);
+}
+
 extern "C" int mt_warp_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
                            const float *vis, int64_t vis_sb, int64_t vis_sf, const float *grid,
                            const float *m_target, int64_t mt_sb, float *x_aligned, int64_t xa_sb,
                            int64_t xa_sc, int64_t xa_sf, float *v_aligned, float *v_map, int B,
                            int C, int F, int H, int W, int flags, mt_stream_t stream) {
-    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, grid, m_target, mt_sb, x_aligned, xa_sb, xa_sc,
-                         xa_sf, v_aligned, v_map, B, C, F, H, W, flags, stream, nullptr);
+    return mt_warp_fwd_dt(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, MT_DT_F32, grid, m_target, mt_sb, x_aligned, xa_sb,
+                          xa_sc, xa_sf, v_aligned, v_map, B, C, F, H, W, flags, stream);
+}
+
+extern "C" int mt_warp_pack_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                   const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype, const void *grid,
+                                   const float *m_target, int64_t mt_sb, const float *x_t, int64_t xt_sb,
+                                   int64_t xt_sc, const float *v_t, int64_t vt_sb, float *nn_in,
+                                   float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                                   float *v_aligned, float *v_map, int B, int F, int H, int W, int flags,
+                                   mt_stream_t stream) {
+    PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in};
+    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, grid, m_target, mt_sb, x_aligned, xa_sb,
+                         xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk);
 }
 
 extern "C" int mt_warp_pack_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
@@ -696,9 +754,19 @@ extern "C" int mt_warp_pack_fwd(const float *x, int64_t x_sb, int64_t x_sc, int6
                                 float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
                                 float *v_aligned, float *v_map, int B, int F, int H, int W, int flags,
                                 mt_stream_t stream) {
-    PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in};
-    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, grid, m_target, mt_sb, x_aligned, xa_sb, xa_sc,
-                         xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk);
+    return mt_warp_pack_fwd_dt(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, MT_DT_F32, grid, m_target, mt_sb, x_t, xt_sb,
+                               xt_sc, v_t, vt_sb, nn_in, x_aligned, xa_sb, xa_sc, xa_sf, v_aligned, v_map, B, F, H, W,
+                               flags, stream);
+}
+
+extern "C" int mt_warp_lowres_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                     const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype, const void *flow,
+                                     int gh, int gw, const float *m_target, int64_t mt_sb, float *x_aligned,
+                                     int64_t xa_sb, int64_t xa_sc, int64_t xa_sf, float *v_aligned, float *v_map,
+                                     int B, int F, int H, int W, int flags, mt_stream_t stream) {
+    MT_REQUIRE(gh > 0 && gw > 0, "mt_warp_lowres_fwd: empty flow");
+    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, flow, m_target, mt_sb, x_aligned, xa_sb,
+                         xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, nullptr, gh, gw);
 }
 
 extern "C" int mt_warp_lowres_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
@@ -706,9 +774,21 @@ extern "C" int mt_warp_lowres_fwd(const float *x, int64_t x_sb, int64_t x_sc, in
                                   int gw, const float *m_target, int64_t mt_sb, float *x_aligned, int64_t xa_sb,
                                   int64_t xa_sc, int64_t xa_sf, float *v_aligned, float *v_map, int B, int F,
                                   int H, int W, int flags, mt_stream_t stream) {
-    MT_REQUIRE(gh > 0 && gw > 0, "mt_warp_lowres_fwd: empty flow");
-    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, flow, m_target, mt_sb, x_aligned, xa_sb, xa_sc,
-                         xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, nullptr, gh, gw);
+    return mt_warp_lowres_fwd_dt(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, MT_DT_F32, flow, gh, gw, m_target, mt_sb,
+                                 x_aligned, xa_sb, xa_sc, xa_sf, v_aligned, v_map, B, F, H, W, flags, stream);
+}
+
+extern "C" int mt_warp_pack_lowres_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                          const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype,
+                                          const void *flow, int gh, int gw, const float *m_target, int64_t mt_sb,
+                                          const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t,
+                                          int64_t vt_sb, float *nn_in, float *x_aligned, int64_t xa_sb, int64_t xa_sc,
+                                          int64_t xa_sf, float *v_aligned, float *v_map, int B, int F, int H,
+                                          int W, int flags, mt_stream_t stream) {
+    MT_REQUIRE(gh > 0 && gw > 0, "mt_warp_pack_lowres_fwd: empty flow");
+    PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in};
+    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, flow, m_target, mt_sb, x_aligned, xa_sb,
+                         xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk, gh, gw);
 }
 
 extern "C" int mt_warp_pack_lowres_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
@@ -718,10 +798,9 @@ extern "C" int mt_warp_pack_lowres_fwd(const float *x, int64_t x_sb, int64_t x_s
                                        float *nn_in, float *x_aligned, int64_t xa_sb, int64_t xa_sc,
                                        int64_t xa_sf, float *v_aligned, float *v_map, int B, int F, int H,
                                        int W, int flags, mt_stream_t stream) {
-    MT_REQUIRE(gh > 0 && gw > 0, "mt_warp_pack_lowres_fwd: empty flow");
-    PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in};
-    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, flow, m_target, mt_sb, x_aligned, xa_sb, xa_sc,
-                         xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk, gh, gw);
+    return mt_warp_pack_lowres_fwd_dt(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, MT_DT_F32, flow, gh, gw, m_target,
+                                      mt_sb, x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in, x_aligned, xa_sb, xa_sc, xa_sf,
+                                      v_aligned, v_map, B, F, H, W, flags, stream);
 }
 
 extern "C" int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,

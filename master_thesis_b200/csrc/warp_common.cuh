@@ -119,11 +119,26 @@ __device__ __forceinline__ Lin lin_index(int dst, int in, int out, float scale) 
     r.l0 = __fsub_rn(1.0f, r.l1);
     return r;
 }
-// the resized flow at one output pixel: rows r0 / r1 of the low-resolution flow (float2 = (gx, gy)),
+// A dense flow is (gx, gy) pairs of element type G: fp32, or fp16 / bf16 as the DFPN's flow estimators return them
+// under autocast.  Flow2<G> is the pair type; the loads widen it to fp32 in registers (exact), so every operation
+// after them is the fp32 kernel's.
+template <typename G> struct Flow2Of { using type = float2; };
+template <> struct Flow2Of<__half> { using type = __half2; };
+template <> struct Flow2Of<__nv_bfloat16> { using type = __nv_bfloat162; };
+template <typename G> using Flow2 = typename Flow2Of<G>::type;
+__device__ __forceinline__ float2 flow_ldcs(const float2 *p) { return __ldcs(p); }
+__device__ __forceinline__ float2 flow_ldcs(const __half2 *p) { return __half22float2(__ldcs(p)); }
+__device__ __forceinline__ float2 flow_ldcs(const __nv_bfloat162 *p) { return __bfloat1622float2(__ldcs(p)); }
+__device__ __forceinline__ float2 flow_ldg(const float2 *p) { return __ldg(p); }
+__device__ __forceinline__ float2 flow_ldg(const __half2 *p) { return __half22float2(__ldg(p)); }
+__device__ __forceinline__ float2 flow_ldg(const __nv_bfloat162 *p) { return __bfloat1622float2(__ldg(p)); }
+
+// the resized flow at one output pixel: rows r0 / r1 of the low-resolution flow (a pair = (gx, gy)),
 // row(y) = fma(v[x0], lx0, v[x1] * lx1); out = fma(row(y0), ly0, row(y1) * ly1)   (the CPU build's order: DESIGN.md "bit-exactness")
-__device__ __forceinline__ float2 lin_flow(const float2 *__restrict__ r0, const float2 *__restrict__ r1, const Lin &lx,
+template <typename F2>
+__device__ __forceinline__ float2 lin_flow(const F2 *__restrict__ r0, const F2 *__restrict__ r1, const Lin &lx,
                                            float ly0, float ly1) {
-    const float2 a = __ldg(r0 + lx.i0), b = __ldg(r0 + lx.i1), c = __ldg(r1 + lx.i0), d = __ldg(r1 + lx.i1);
+    const float2 a = flow_ldg(r0 + lx.i0), b = flow_ldg(r0 + lx.i1), c = flow_ldg(r1 + lx.i0), d = flow_ldg(r1 + lx.i1);
     const float tx = __fmaf_rn(a.x, lx.l0, __fmul_rn(b.x, lx.l1)), ty = __fmaf_rn(a.y, lx.l0, __fmul_rn(b.y, lx.l1));
     const float bx = __fmaf_rn(c.x, lx.l0, __fmul_rn(d.x, lx.l1)), by = __fmaf_rn(c.y, lx.l0, __fmul_rn(d.y, lx.l1));
     return make_float2(__fmaf_rn(tx, ly0, __fmul_rn(bx, ly1)), __fmaf_rn(ty, ly0, __fmul_rn(by, ly1)));

@@ -4,8 +4,9 @@ PyTorch is plumbing here: it owns device memory (caching allocator), streams
 and autograd bookkeeping.  Every computation is a hand-written sm_100a kernel
 reached through ``_lib.call`` with raw device pointers.  CUDA fp32 tensors
 only, except the network operands checked against ``NET_DTYPES`` (the CNN output
-of CHN, the inputs of masked_l1), which may also be fp16 / bf16 as autocast hands
-them over; anything else raises - there is no CPU / eager fallback.
+of CHN, the inputs of masked_l1, the DFPN's flows and VGG features), which may
+also be fp16 / bf16 as autocast hands them over; anything else raises - there is
+no CPU / eager fallback.
 """
 import ctypes
 
@@ -179,9 +180,16 @@ def _grid_kind(grid, flags, b, f, h, w):
     resize bilinearly on the fly (SURVEY 8f-1)."""
     grid = _contig(grid)
     if flags & GRID_AFFINE:
+        if grid.dtype != torch.float32:     # CPN's theta is fp32 (model_cpn.py:74 under autocast: .float())
+            raise RuntimeError("master_thesis_b200: fp32 tensors required, got %s" % grid.dtype)
         if grid.numel() != b * f * 6:
             raise RuntimeError("theta must have shape (B*F,2,3)")
         return grid, 0, 0
+    if grid.dtype != torch.float32:
+        if flags & VIS_BILINEAR:
+            raise RuntimeError("a half flow needs the nearest-visibility (DFPN) flavour")
+        if grid.data_ptr() % (2 * grid.element_size()):    # the kernels load one (gx, gy) pair per access
+            grid = _lib.keep(grid.clone())
     if grid.dim() != 5 or grid.shape[0] != b or grid.shape[1] != f or grid.shape[4] != 2:
         raise RuntimeError("flow must have shape (B,F,H,W,2), got %s" % (tuple(grid.shape),))
     gh, gw = int(grid.shape[2]), int(grid.shape[3])
@@ -195,9 +203,12 @@ def warp_fwd(x, vis, grid, m_target=None, flags=ALIGN_CORNERS, want_x=True, want
     """x (B,C,F,H,W), vis (B,1,F,H,W), grid dense (B,F,H,W,2) or theta (B*F,2,3); a dense flow
     (B,F,gh,gw,2) of another resolution is resized to (H,W) inside the kernel (resize_flow, utils.py:107-126).
 
+    A dense flow may be fp16 / bf16 (the DFPN's flow estimators under autocast): the kernels widen it on load, so the
+    result is the fp32 op's on ``grid.float()`` (grid_sample promotes to fp32 under autocast, utils.py:93-103).
+
     Returns (x_aligned (B,C,F,H,W) view, v_aligned (B,1,F,H,W), v_map (B,1,F,H,W) | None).
     """
-    _need_cuda(x, vis, grid, m_target)
+    _need_cuda(x, vis, (grid, NET_DTYPES), m_target)
     _no_grad_inputs("warp_fwd", x, vis, grid, m_target)
     b, c, f, h, w = x.shape
     x, x_sb, x_sc, x_sf = _s5(x)
@@ -217,11 +228,11 @@ def warp_fwd(x, vis, grid, m_target=None, flags=ALIGN_CORNERS, want_x=True, want
     if gh and (gh, gw) != (h, w):
         if c != 3:
             raise RuntimeError("warp_fwd: a flow at another resolution needs C = 3")
-        _call("mt_warp_lowres_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _ptr(grid), gh, gw,
+        _call_net("mt_warp_lowres_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _Net(grid), gh, gw,
                   _ptr(m_target), mt_sb, _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm),
                   b, f, h, w, flags, _stream(x))
         return xa, va, vm
-    _call("mt_warp_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _ptr(grid),
+    _call_net("mt_warp_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _Net(grid),
               _ptr(m_target), mt_sb, _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm),
               b, c, f, h, w, flags, _stream(x))
     return xa, va, vm
@@ -230,8 +241,10 @@ def warp_fwd(x, vis, grid, m_target=None, flags=ALIGN_CORNERS, want_x=True, want
 def warp_pack_fwd(x, vis, grid, m_target, x_t, v_t, flags=ALIGN_CORNERS, want_aligned=False, want_v_map=True):
     """mt_warp_pack_fwd: the warp of mt_warp_fwd that also writes the CNN input of CHN.forward.
 
+    A dense flow may be fp16 / bf16, as in warp_fwd.
+
     Returns (nn_in (B*F,9,H,W), v_map (B,1,F,H,W) | None, x_aligned | None, v_aligned | None)."""
-    _need_cuda(x, vis, grid, m_target, x_t, v_t)
+    _need_cuda(x, vis, (grid, NET_DTYPES), m_target, x_t, v_t)
     _no_grad_inputs("warp_pack_fwd", x, vis, grid, m_target, x_t, v_t)
     b, c, f, h, w = x.shape
     if c != 3:
@@ -248,11 +261,11 @@ def warp_pack_fwd(x, vis, grid, m_target, x_t, v_t, flags=ALIGN_CORNERS, want_al
     vm = _empty((b, 1, f, h, w), dtype=torch.float32, device=x.device) if want_v_map else None
     nn_in = _empty((b * f, 9, h, w), dtype=torch.float32, device=x.device)
     if gh and (gh, gw) != (h, w):
-        _call("mt_warp_pack_lowres_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _ptr(grid), gh, gw,
+        _call_net("mt_warp_pack_lowres_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _Net(grid), gh, gw,
                   _ptr(m_target), m_target.stride(0), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
                   _ptr(nn_in), _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm), b, f, h, w, flags, _stream(x))
         return nn_in, vm, xa, va
-    _call("mt_warp_pack_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _ptr(grid),
+    _call_net("mt_warp_pack_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _Net(grid),
               _ptr(m_target), m_target.stride(0), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
               _ptr(nn_in), _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm), b, f, h, w, flags, _stream(x))
     return nn_in, vm, xa, va
@@ -289,6 +302,7 @@ class AlignSetFn(torch.autograd.Function):
 
 
 def align_set(x, v, flow):
+    _need_cuda(x, v, flow)          # DFPN training: fp32 flows only (warp_fwd alone also reads half flows)
     if x.requires_grad or v.requires_grad:
         raise RuntimeError("align_set: gradients w.r.t. x / v are not provided (the reference "
                            "never requests them); only the flow is differentiable")
@@ -601,15 +615,22 @@ def corr4d_vgg(feats_t, m_target, feats_r, m_refs):
     """The correlation of CorrelationVGG.forward with its neighbours (model_dfpn.py:516-528, SURVEY 8f-3):
     feats_t (B,C,h,w), feats_r (B,C,F,h,w) with ANY b / c / f strides (the transposed view of the VGG output is
     read in place), m_target (B,1,H,W) / m_refs (B,1,F,H,W) FULL-RESOLUTION masks or both None; the visibilities
-    v = F.interpolate(1 - m, (h, w), mode='nearest') are evaluated inside the kernel.  -> (B,F,h,w,h,w)."""
-    _need_cuda(feats_t, m_target, feats_r, m_refs)
-    _no_grad_inputs("corr4d_vgg", feats_t, m_target, feats_r, m_refs)
-    b, c, f, h, w = feats_r.shape
-    if not corr4d_vgg_supported(c, h * w):
-        raise RuntimeError("corr4d_vgg: (C=%d, h*w=%d) is not served by the tensor-core kernel" % (c, h * w))
+    v = F.interpolate(1 - m, (h, w), mode='nearest') are evaluated inside the kernel.  -> (B,F,h,w,h,w).
 
-    def ok(t, lead):       # strides the tensor map can encode: positive multiples of 4 elements, plane contiguous
-        return all(t.size(d) == 1 or (t.stride(d) > 0 and t.stride(d) % 4 == 0) for d in range(lead)) and \
+    The features may be fp16 / bf16 (the VGG under autocast), both of one dtype: the kind::f16 kernel multiplies the
+    exact half features with fp32 accumulation and returns the volume in their dtype, rounded once (DESIGN §2)."""
+    _need_cuda((feats_t, NET_DTYPES), m_target, (feats_r, NET_DTYPES), m_refs)
+    _no_grad_inputs("corr4d_vgg", feats_t, m_target, feats_r, m_refs)
+    if feats_t.dtype != feats_r.dtype:
+        raise RuntimeError("corr4d_vgg: feats_t and feats_r must have one dtype, got %s and %s"
+                           % (feats_t.dtype, feats_r.dtype))
+    b, c, f, h, w = feats_r.shape
+    if not corr4d_vgg_supported(c, h * w) or (feats_r.dtype != torch.float32 and c % 64):
+        raise RuntimeError("corr4d_vgg: (C=%d, h*w=%d) is not served by the tensor-core kernel" % (c, h * w))
+    es = feats_r.element_size()
+
+    def ok(t, lead):       # strides the tensor map can encode: positive multiples of 16 B, plane contiguous
+        return all(t.size(d) == 1 or (t.stride(d) > 0 and t.stride(d) * es % 16 == 0) for d in range(lead)) and \
             t.stride(-1) == 1 and t.stride(-2) == w and t.data_ptr() % 16 == 0
     ft = feats_t if ok(feats_t, 2) else _contig(feats_t)
     fr = feats_r if ok(feats_r, 3) else _contig(feats_r)
@@ -620,9 +641,14 @@ def corr4d_vgg(feats_t, m_target, feats_r, m_refs):
         mt, mr = _planes(m_target), _planes(m_refs)
         MH, MW = mt.shape[-2:]
         mt_sb, mr_sb, mr_sf = mt.stride(0), mr.stride(0), mr.stride(2)
-    out = _empty((b, f, h, w, h, w), dtype=torch.float32, device=fr.device)
-    _call("mt_corr4d_vgg_fwd", _ptr(ft), ft.stride(0), ft.stride(1), _ptr(mt), mt_sb, _ptr(fr), fr.stride(0),
-          fr.stride(1), fr.stride(2), _ptr(mr), mr_sb, mr_sf, MH, MW, _ptr(out), b, c, f, h, w, _stream(fr))
+    out = _empty((b, f, h, w, h, w), dtype=fr.dtype, device=fr.device)
+    if fr.dtype == torch.float32:
+        _call("mt_corr4d_vgg_fwd", _ptr(ft), ft.stride(0), ft.stride(1), _ptr(mt), mt_sb, _ptr(fr), fr.stride(0),
+              fr.stride(1), fr.stride(2), _ptr(mr), mr_sb, mr_sf, MH, MW, _ptr(out), b, c, f, h, w, _stream(fr))
+    else:
+        _call("mt_corr4d_vgg_fwd_dt", _DT[fr.dtype], _ptr(ft), ft.stride(0), ft.stride(1), _ptr(mt), mt_sb, _ptr(fr),
+              fr.stride(0), fr.stride(1), fr.stride(2), _ptr(mr), mr_sb, mr_sf, MH, MW, _ptr(out), b, c, f, h, w,
+              _stream(fr))
     return out
 
 
@@ -984,8 +1010,10 @@ def resize_flow_raw(flow, size, mode):
     """mt_resize_flow without autograd: flow (B,F,h,w,2), read through its five strides, -> (B,F,H,W,2) in the
     memory layout the reference returns: its ``flow.reshape(b * f, h, w, 2).permute(0, 3, 1, 2)`` is channels-last
     for an interleaved flow and after the copy ``reshape`` makes when (B, F) do not merge, and F.interpolate keeps
-    that layout (interleaved (B,F,H,W,2) memory); otherwise the result is planar (B,F,2,H,W) memory."""
-    _need_cuda(flow)
+    that layout (interleaved (B,F,H,W,2) memory); otherwise the result is planar (B,F,2,H,W) memory.  A half flow
+    (the DFPN's flow estimators under autocast) is widened in the kernel and the result is fp32, as F.interpolate's
+    under autocast."""
+    _need_cuda((flow, NET_DTYPES))
     if flow.dim() != 5 or flow.shape[4] != 2:
         raise ValueError("resize_flow: flow (B,F,h,w,2) expected, got %s" % (tuple(flow.shape),))
     b, f, h, w, _ = flow.shape
@@ -996,8 +1024,8 @@ def resize_flow_raw(flow, size, mode):
         out = _empty((b, f, H, W, 2), dtype=torch.float32, device=flow.device)
     else:
         out = _empty((b, f, 2, H, W), dtype=torch.float32, device=flow.device).permute(0, 1, 3, 4, 2)
-    _call("mt_resize_flow", _ptr(_lib.keep(flow)), *fs, _ptr(out), *out.stride(), b, f, h, w, H, W,
-          RESIZE_MODES[mode], _stream(flow))
+    _call_net("mt_resize_flow", _Net(_lib.keep(flow)), *fs, _ptr(out), *out.stride(), b, f, h, w, H, W,
+              RESIZE_MODES[mode], _stream(flow))
     return out
 
 
@@ -1016,6 +1044,7 @@ class ResizeFlowFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, flow, size):
+        _need_cuda(flow)        # the gradient path (DFPN training) is fp32
         ctx.hw = flow.shape[2:4]
         return resize_flow_raw(flow.detach(), size, "bilinear")
 
@@ -1028,7 +1057,8 @@ class ResizeFlowFn(torch.autograd.Function):
 
 def resize_flow(flow, size, mode="nearest"):
     """FlowsUtils.resize_flow (utils.py:107-126): (B,F,h,w,2) -> (B,F,H,W,2), mode 'nearest' or 'bilinear'
-    (align_corners=False); differentiable w.r.t. ``flow`` in the bilinear mode."""
+    (align_corners=False); differentiable w.r.t. ``flow`` in the bilinear mode.  Without a gradient the flow may be
+    fp16 / bf16; the result is fp32."""
     if mode not in RESIZE_MODES:
         raise ValueError("resize_flow: mode must be one of %s, got %r" % (sorted(RESIZE_MODES), mode))
     if torch.is_grad_enabled() and flow.requires_grad:

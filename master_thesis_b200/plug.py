@@ -21,6 +21,13 @@ def _cuda_fp32(*ts):
     return all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 for t in ts)
 
 
+def _cuda_autocast_half(t):
+    """True if autocast is enabled on CUDA and ``t`` is a CUDA tensor in its dtype: a network output of the
+    reference's ``--precision 16|bf16`` runs (__main__.py:69), which the kernels read natively."""
+    return isinstance(t, torch.Tensor) and t.is_cuda and torch.is_autocast_enabled("cuda") and \
+        t.dtype == torch.get_autocast_dtype("cuda") and t.dtype != torch.float32
+
+
 def _reference_original(cls, attr):
     """The reference's own ``cls.attr``, saved by ``patch()``: the resampling mirrors hand it every call their
     kernels do not serve (the reference's dataset code calls the same helpers on host tensors)."""
@@ -46,9 +53,12 @@ class FlowsUtils:
         """utils.py:107-126.  flow (B,F,h,w,2) -> (B,F,H,W,2), F.interpolate 'nearest' or 'bilinear'
         (align_corners=False), bit-identical; differentiable w.r.t. flow in the bilinear mode.  CUDA fp32 flows in
         those two modes (and nearest without a gradient) run on the kernel, anything else on the reference's own
-        function."""
+        function.  Under autocast a half flow without a gradient (the frozen DFPN aligner's) runs on the kernel
+        too and becomes fp32, as F.interpolate's fp32 autocast policy makes it."""
         grad = torch.is_grad_enabled() and isinstance(flow, torch.Tensor) and flow.requires_grad
         if _cuda_fp32(flow) and (mode == 'bilinear' or (mode == 'nearest' and not grad)):
+            return ops.resize_flow(flow, size, mode)
+        if _cuda_autocast_half(flow) and mode in ('bilinear', 'nearest') and not grad:
             return ops.resize_flow(flow, size, mode)
         return _reference_original("FlowsUtils", "resize_flow")(flow, size, mode)
 
@@ -104,11 +114,16 @@ def corr_vgg_forward(self, x_target, m_target, x_refs, m_refs):
     (cuDNN) are the module's own; what lies between them (:516-528) is ONE kernel: the transposed view of the
     reference features is read in place (no permute copy), the nearest down-sample of the two visibility
     maps (:521-526) is evaluated inside the correlation kernel from the full-resolution masks, and the
-    masking / normalisation / contraction (:534-565) run on tcgen05 (SURVEY 8f-3)."""
+    masking / normalisation / contraction (:534-565) run on tcgen05 (SURVEY 8f-3).  Under autocast the VGG returns
+    half features; they run on the kind::f16 kernel and the volume keeps their dtype, as the reference's matmul
+    returns it (DESIGN §2)."""
     b, c, ref_n, h, w = x_refs.size()
     with torch.no_grad():
         x_target_feats = self.model_vgg(x_target, normalize_input=False)[3]
         x_ref_feats = self.model_vgg(x_refs.transpose(1, 2).reshape(b * ref_n, c, h, w), normalize_input=False)[3]
+    for t in (x_target_feats, x_ref_feats):
+        if t.dtype != torch.float32 and not _cuda_autocast_half(t):     # no reference path makes them elsewhere
+            raise RuntimeError("master_thesis_b200: fp32 tensors required, got %s" % t.dtype)
     x_ref_feats = x_ref_feats.reshape(b, ref_n, -1, 16, 16).transpose(1, 2)
     fc, fh, fw = x_ref_feats.shape[1], x_ref_feats.shape[3], x_ref_feats.shape[4]
     if ops.corr4d_vgg_supported(fc, fh * fw):
