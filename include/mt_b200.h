@@ -176,6 +176,16 @@ MT_API int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int64_t 
                      const float *gout, int64_t g_sb, int64_t g_sc, int64_t g_sf,
                      float *ggrid, int B, int C, int F, int H, int W, int flags,
                      mt_stream_t stream);
+/* mt_warp_bwd_grid with the dtype code (MT_DT_*) of the flow before its pointer: align_set's backward in DFPN's own
+ * training step under autocast (utils.py:93-97, model_dfpn.py:377-385), where the flow estimators return fp16 / bf16
+ * flows.  grid_sample promotes to fp32, so the gradient w.r.t. the widened flow is the fp32 entry point's; ggrid is
+ * written in g_dtype, that gradient rounded to nearest even (the backward of autocast's cast).  A half grid / ggrid
+ * must be 4 B aligned, an fp32 one 8 B. */
+MT_API int mt_warp_bwd_grid_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                        int g_dtype, const void *grid,
+                        const float *gout, int64_t g_sb, int64_t g_sc, int64_t g_sf,
+                        void *ggrid, int B, int C, int F, int H, int W, int flags,
+                        mt_stream_t stream);
 
 /* ---- K1c  fused warp + mask_out + masked-L1 ('sum') forward --------------
  * replaces align_set (utils.py:78-104) + mask_out (model_dfpn.py:269-272) +
@@ -201,10 +211,31 @@ MT_API int mt_warp_l1_bwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_
                    const float *v_target, int64_t vt_sb,
                    const float *out3, const float *grad_out, float *gflow,
                    int B, int F, int H, int W, float weight, int flags, mt_stream_t stream);
+/* K1c forward / backward with the dtype code (MT_DT_*) of the flow before its pointer: DFPN.compute_loss under
+ * autocast (model_dfpn.py:269-287), where the flow estimators and the mixer return fp16 / bf16 flows.  grid_sample
+ * samples the fp32 frames with the exactly widened flow (utils.py:93-103), mask_out compares the half values (the same
+ * result on the widened ones) and l1_loss runs in fp32: out3 and x_aligned / v_aligned are those of the fp32 entry
+ * point on the widened flow; gflow is written in f_dtype, the fp32 gradient rounded to nearest even. */
+MT_API int mt_warp_l1_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                      const float *vis, int64_t vis_sb, int64_t vis_sf,
+                      int f_dtype, const void *flow,
+                      const float *x_target, int64_t xt_sb, int64_t xt_sc,
+                      const float *v_target, int64_t vt_sb,
+                      float *x_aligned, float *v_aligned, float *out3, void *workspace,
+                      int B, int F, int H, int W, float weight, int flags, mt_stream_t stream);
+MT_API int mt_warp_l1_bwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                      int f_dtype, const void *flow,
+                      const float *x_target, int64_t xt_sb, int64_t xt_sc,
+                      const float *v_target, int64_t vt_sb,
+                      const float *out3, const float *grad_out, void *gflow,
+                      int B, int F, int H, int W, float weight, int flags, mt_stream_t stream);
 
 /* ---- mask_out  (model_dfpn.py:269-272)                               (a4)
  * flow (n,2) -> out (n) = clamp((gx<-1)+(gx>1)+(gy<-1)+(gy>1), 0, 1) */
 MT_API int mt_mask_out(const float *flow, int64_t n, float *out, mt_stream_t stream);
+/* mt_mask_out of a flow in the dtype f_dtype (MT_DT_*): model_dfpn.py:269-272 on the half flows of DFPN training under
+ * autocast.  The comparisons of the widened values give those of the half ones; out is fp32. */
+MT_API int mt_mask_out_dt(int f_dtype, const void *flow, int64_t n, float *out, mt_stream_t stream);
 
 /* ---- masked L1  (LossesUtils.masked_l1, utils.py:139-169)            (a5)
  * y_hat, y: (B,C,F,P) strided (P contiguous); mask: (B,mask_c,F,P), mask_c in
@@ -380,7 +411,7 @@ MT_API int mt_corr4d_vgg_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_sc,
  * half features are multiplied with fp32 accumulation, the fp32 norm scales applied in the epilogue, and the volume
  * `out` is stored in f_dtype, rounded once to nearest even.  Not bit-identical to the eager path (which rounds the
  * normalised operands), at least as accurate.  Masks stay fp32.  Half features need C % 64 == 0 and feature strides
- * that are multiples of 16 B; the L1 mode stays fp32. */
+ * that are multiples of 16 B. */
 MT_API int mt_corr4d_vgg_fwd_dt(int f_dtype, const void *feats_t, int64_t ft_sb, int64_t ft_sc,
                          const float *m_target, int64_t mt_sb,
                          const void *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
@@ -403,6 +434,20 @@ MT_API int mt_corr4d_vgg_l1_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_
                          int B, int C, int F, int h, int w, mt_stream_t stream);
 MT_API int64_t mt_corr4d_l1_workspace_bytes(void);
 MT_API int mt_corr4d_l1_bwd(const void *sign, const float *grad_loss, float *g_pred, int64_t n, mt_stream_t stream);
+/* mt_corr4d_vgg_l1_fwd / mt_corr4d_l1_bwd with dtype codes (MT_DT_*) before feats_t, feats_r and pred (one dtype for
+ * all three) and before g_pred: DFPN.compute_loss under autocast (model_dfpn.py:254-257).  There the VGG returns half
+ * features, the 4-D convolution a half `corr`, corr_y is the half volume of mt_corr4d_vgg_fwd_dt and F.l1_loss (on
+ * autocast's fp32 list) compares the two widened.  The kernel rounds each volume value to the dtype as the store mode
+ * writes it, widens it again and accumulates |pred - v| in fp32; loss is fp32 and sign = sign(pred - v).  g_pred is
+ * written in g_dtype: sign * grad_loss[0] / n rounded to nearest even.  Half features take the single-CTA kernel. */
+MT_API int mt_corr4d_vgg_l1_fwd_dt(int ft_dtype, const void *feats_t, int64_t ft_sb, int64_t ft_sc,
+                            const float *m_target, int64_t mt_sb,
+                            int fr_dtype, const void *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
+                            const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW,
+                            int p_dtype, const void *pred, float *loss, void *sign, void *workspace,
+                            int64_t workspace_bytes, int B, int C, int F, int h, int w, mt_stream_t stream);
+MT_API int mt_corr4d_l1_bwd_dt(const void *sign, const float *grad_loss, int g_dtype, void *g_pred, int64_t n,
+                        mt_stream_t stream);
 
 /* ---- K3  CPN context matching --------------------------------------------
  * replaces CM_Module.forward + masked_softmax   model_cpn.py:206-254    (a8)
@@ -517,6 +562,12 @@ MT_API int mt_resize_flow_dt(int flow_dtype, const void *flow, int64_t sb, int64
 MT_API int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
                        int64_t g_sc, float *g_flow, int B, int F, int h, int w, int H, int W,
                        mt_stream_t stream);
+/* mt_resize_flow_bwd with g_flow in the dtype g_dtype (MT_DT_*) of the input flow: the bilinear resize of a half flow
+ * that needs a gradient (DFPN.forward under autocast, model_dfpn.py:86, 93) runs in fp32 (see mt_resize_flow_dt), so
+ * g_flow is the fp32 gradient of the same gather rounded to nearest even.  g_out stays fp32. */
+MT_API int mt_resize_flow_bwd_dt(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
+                          int64_t g_sc, int g_dtype, void *g_flow, int B, int F, int h, int w, int H, int W,
+                          mt_stream_t stream);
 
 /* ---- host-buffer entry points (end-to-end: H2D + kernels + D2H inside) ----
  * The reference-facing calls with HOST memory, used for the e2e metric.

@@ -20,7 +20,7 @@ namespace mt {
 
 // L1 mode of the tensor-core launcher (corr_tc.cu): prediction, loss scalar, optional int8 signs, partial sums
 struct CorrL1 {
-    const float *pred;
+    const void *pred;
     float *loss;
     signed char *sign;
     float *partials;
@@ -34,7 +34,8 @@ int corr4d_tc_launch_ex(const void *ft, int64_t ft_sb, int64_t ft_sc, const void
                         int mask_mode, int MH, int MW, int fh, int fw, void *out, int B, int C, int F, int P,
                         cudaStream_t st, const CorrL1 *l1, int dtype);
 int64_t corr4d_l1_workspace_bytes();
-int corr4d_l1_bwd_launch(const signed char *sign, const float *grad_loss, float *g_pred, int64_t n, cudaStream_t st);
+int corr4d_l1_bwd_launch(const signed char *sign, const float *grad_loss, void *g_pred, int64_t n, cudaStream_t st,
+                         int dtype);
 
 namespace {
 
@@ -186,12 +187,22 @@ extern "C" int mt_corr4d_vgg_fwd(const float *feats_t, int64_t ft_sb, int64_t ft
 
 extern "C" int64_t mt_corr4d_l1_workspace_bytes(void) { return corr4d_l1_workspace_bytes(); }
 
-extern "C" int mt_corr4d_vgg_l1_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_sc, const float *m_target,
-                                    int64_t mt_sb, const float *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
-                                    const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW,
-                                    const float *pred, float *loss, void *sign, void *workspace,
-                                    int64_t workspace_bytes, int B, int C, int F, int h, int w, mt_stream_t stream) {
+// ft_dtype / fr_dtype / p_dtype (MT_DT_*): element types of feats_t, feats_r and pred, all one.  Under autocast the
+// VGG hands over half features and the 4-D convolution a half volume `corr`; the reference's corr_y is the half volume
+// of correlation_masked_4d (mt_corr4d_vgg_fwd_dt computes it: exact half operands, fp32 accumulation and scales, one
+// rounding to the features' dtype) and F.l1_loss, on autocast's fp32 list, compares the two widened
+// (model_dfpn.py:254-257).  The kernel rounds each volume value as the store mode does, widens it again and compares
+// it with the widened pred; the loss is fp32 and the signs those of pred - corr_y.
+extern "C" int mt_corr4d_vgg_l1_fwd_dt(int ft_dtype, const void *feats_t, int64_t ft_sb, int64_t ft_sc,
+                                       const float *m_target, int64_t mt_sb, int fr_dtype, const void *feats_r,
+                                       int64_t fr_sb, int64_t fr_sc, int64_t fr_sf, const float *m_refs, int64_t mr_sb,
+                                       int64_t mr_sf, int MH, int MW, int p_dtype, const void *pred, float *loss,
+                                       void *sign, void *workspace, int64_t workspace_bytes, int B, int C, int F, int h,
+                                       int w, mt_stream_t stream) {
     MT_REQUIRE(feats_t && feats_r && pred && loss && workspace, "mt_corr4d_vgg_l1_fwd: NULL argument");
+    MT_REQUIRE(ft_dtype == fr_dtype && fr_dtype == p_dtype,
+               "mt_corr4d_vgg_l1_fwd_dt: feats_t, feats_r and pred need one dtype, got codes %d, %d and %d", ft_dtype,
+               fr_dtype, p_dtype);
     MT_REQUIRE(B > 0 && C > 0 && F > 0 && h > 0 && w > 0, "mt_corr4d_vgg_l1_fwd: empty shape");
     MT_REQUIRE((m_target == nullptr) == (m_refs == nullptr), "mt_corr4d_vgg_l1_fwd: both masks or none");
     MT_REQUIRE(!m_target || (MH > 0 && MW > 0 && mt_sb >= 0 && mr_sb >= 0 && mr_sf >= 0), "mt_corr4d_vgg_l1_fwd: bad mask shape");
@@ -202,10 +213,28 @@ extern "C" int mt_corr4d_vgg_l1_fwd(const float *feats_t, int64_t ft_sb, int64_t
     CorrL1 l1{pred, loss, reinterpret_cast<signed char *>(sign), reinterpret_cast<float *>(workspace)};
     return corr4d_tc_launch_ex(feats_t, ft_sb, ft_sc, feats_r, fr_sb, fr_sc, fr_sf, m_target, mt_sb, m_refs, mr_sb,
                                mr_sf, m_target ? 1 : 0, MH, MW, h, w, nullptr, B, C, F, h * w, (cudaStream_t)stream, &l1,
-                               MT_DT_F32);
+                               p_dtype);
+}
+
+extern "C" int mt_corr4d_vgg_l1_fwd(const float *feats_t, int64_t ft_sb, int64_t ft_sc, const float *m_target,
+                                    int64_t mt_sb, const float *feats_r, int64_t fr_sb, int64_t fr_sc, int64_t fr_sf,
+                                    const float *m_refs, int64_t mr_sb, int64_t mr_sf, int MH, int MW,
+                                    const float *pred, float *loss, void *sign, void *workspace,
+                                    int64_t workspace_bytes, int B, int C, int F, int h, int w, mt_stream_t stream) {
+    return mt_corr4d_vgg_l1_fwd_dt(MT_DT_F32, feats_t, ft_sb, ft_sc, m_target, mt_sb, MT_DT_F32, feats_r, fr_sb, fr_sc,
+                                   fr_sf, m_refs, mr_sb, mr_sf, MH, MW, MT_DT_F32, pred, loss, sign, workspace,
+                                   workspace_bytes, B, C, F, h, w, stream);
+}
+
+// g_dtype (MT_DT_*): element type of g_pred, the dtype of pred.  l1_loss's gradient w.r.t. a half `corr` is the fp32
+// gradient sign * g / n rounded to that dtype (the backward of autocast's cast, model_dfpn.py:254-257).
+extern "C" int mt_corr4d_l1_bwd_dt(const void *sign, const float *grad_loss, int g_dtype, void *g_pred, int64_t n,
+                                   mt_stream_t stream) {
+    MT_REQUIRE(sign && grad_loss && g_pred, "mt_corr4d_l1_bwd: NULL argument");
+    return corr4d_l1_bwd_launch(reinterpret_cast<const signed char *>(sign), grad_loss, g_pred, n, (cudaStream_t)stream,
+                                g_dtype);
 }
 
 extern "C" int mt_corr4d_l1_bwd(const void *sign, const float *grad_loss, float *g_pred, int64_t n, mt_stream_t stream) {
-    MT_REQUIRE(sign && grad_loss && g_pred, "mt_corr4d_l1_bwd: NULL argument");
-    return corr4d_l1_bwd_launch(reinterpret_cast<const signed char *>(sign), grad_loss, g_pred, n, (cudaStream_t)stream);
+    return mt_corr4d_l1_bwd_dt(sign, grad_loss, MT_DT_F32, g_pred, n, stream);
 }

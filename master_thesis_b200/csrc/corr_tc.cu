@@ -44,6 +44,8 @@
 // A stage holds 128 B per pixel in both cases (32 fp32 or 64 half channels), so the rings and tile shapes are shared.
 #include <cuda.h>
 
+#include <type_traits>
+
 #include "mt_common.cuh"
 #include "mt_tma.cuh"
 
@@ -51,7 +53,7 @@ namespace mt {
 
 // L1 mode of the launchers (see CorrTcArgs): prediction to compare with, loss scalar, optional int8 signs, partial sums
 struct CorrL1 {
-    const float *pred;
+    const void *pred;   // in the features' element type
     float *loss;
     signed char *sign;
     float *partials;
@@ -185,7 +187,7 @@ struct CorrTcArgs {
     // accumulates sum |pred - corr| (F.l1_loss(corr, corr_y), model_dfpn.py:254-257, SURVEY 8f-3).  sign (optional):
     // sign(pred - corr) as int8, all the backward pass needs.  partials: one float per (CTA, epilogue warp); the last
     // epilogue warp of the grid to finish (ticket) folds them in a fixed order and writes the mean to loss[0].
-    const float *pred;
+    const void *pred;                              // in the features' element type T
     signed char *sign;
     float *partials;
     unsigned int *ticket;                          // zero between launches: counts the epilogue warps that are done
@@ -213,20 +215,29 @@ __device__ __forceinline__ signed char sign_i8(float d) { return d > 0.0f ? 1 : 
 // coalesced streaming stores of the volume, or (L1) the same rows of `pred` loaded instead (requested before the
 // TMEM read so that their latency hides under it) and |pred - corr| accumulated into `acc`.
 // `off0`: element offset of (first row of the block, first column of the tile) in the (B, F, P, P) volume.
-// OT: element type of the volume (float, or the half features' type: each value rounded once, to nearest even).
+// OT: element type of the volume and of `pred` (float, or the half features' type: each value of the volume rounded
+// once, to nearest even; in L1 mode that rounded value, widened again, is compared with the widened `pred` - the
+// eager l1_loss of two half volumes runs in fp32 under autocast).
+template <typename OT> __device__ __forceinline__ float4 widen4(const float4 &v) { return v; }
+template <typename OT> __device__ __forceinline__ float4 widen4(const uint2 &u) {
+    const OT *e = reinterpret_cast<const OT *>(&u);
+    return make_float4(widen(e[0]), widen(e[1]), widen(e[2]), widen(e[3]));
+}
 template <int TN, bool L1, typename OT = float>
 __device__ __forceinline__ void corr_epi_block(const CorrTcArgs &a, uint32_t taddr, float sa, const float *sbv, float *st,
                                                int64_t off0, int lane, float &acc) {
     const int rr = lane >> 3, c4 = (lane & 7) * 4;  // read-back: 4 rows x 8 float4 per instruction
+    using Pred4 = std::conditional_t<sizeof(OT) == 4, float4, uint2>;  // 4 elements of pred: 16 B of fp32, 8 B of half
+    const OT *pred = static_cast<const OT *>(a.pred);
 #pragma unroll 1
     for (int c0 = 0; c0 < TN; c0 += 32) {
         // pred rows: the first half is requested before the TMEM read, the second once the accumulator registers
         // are free again (the lines were brought into L2 while the main loop ran, see corr_epi_prefetch)
-        float4 p[2][4];
+        Pred4 p[2][4];
         if (L1) {
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                p[0][j] = __ldcs(reinterpret_cast<const float4 *>(a.pred + off0 + (int64_t)(j * 4 + rr) * a.P + c0 + c4));
+                p[0][j] = __ldcs(reinterpret_cast<const Pred4 *>(pred + off0 + (int64_t)(j * 4 + rr) * a.P + c0 + c4));
         }
         {
             float v[32];
@@ -244,7 +255,7 @@ __device__ __forceinline__ void corr_epi_block(const CorrTcArgs &a, uint32_t tad
         if (L1) {
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                p[1][j] = __ldcs(reinterpret_cast<const float4 *>(a.pred + off0 + (int64_t)((4 + j) * 4 + rr) * a.P + c0 + c4));
+                p[1][j] = __ldcs(reinterpret_cast<const Pred4 *>(pred + off0 + (int64_t)((4 + j) * 4 + rr) * a.P + c0 + c4));
         }
         __syncwarp();
 #pragma unroll
@@ -253,8 +264,12 @@ __device__ __forceinline__ void corr_epi_block(const CorrTcArgs &a, uint32_t tad
             const float4 o = *reinterpret_cast<const float4 *>(st + row * kEpiPitch + c4);
             const int64_t off = off0 + (int64_t)row * a.P + c0 + c4;
             if (L1) {
-                const float4 pj = p[j >> 2][j & 3];
-                const float dx = pj.x - o.x, dy = pj.y - o.y, dz = pj.z - o.z, dw = pj.w - o.w;
+                const float4 pj = widen4<OT>(p[j >> 2][j & 3]);
+                float4 v = o;
+                if constexpr (sizeof(OT) == 2)  // the value the store mode writes, widened again
+                    v = make_float4(widen(narrow<OT>(o.x)), widen(narrow<OT>(o.y)), widen(narrow<OT>(o.z)),
+                                    widen(narrow<OT>(o.w)));
+                const float dx = pj.x - v.x, dy = pj.y - v.y, dz = pj.z - v.z, dw = pj.w - v.w;
                 acc += (fabsf(dx) + fabsf(dy)) + (fabsf(dz) + fabsf(dw));
                 if (a.sign) {
                     char4 sg;
@@ -274,13 +289,14 @@ __device__ __forceinline__ void corr_epi_block(const CorrTcArgs &a, uint32_t tad
     }
 }
 
-// L1 mode: lane = row of a 32-row block; asks the L2 for the TN columns of that row of `pred`.  Issued by the epilogue
-// warps before they wait for the accumulators, so the lines arrive while the main loop of the tile runs.
-template <int TN>
+// L1 mode: lane = row of a 32-row block; asks the L2 for the TN columns of that row of `pred` (elements of OT), one
+// prefetch per 128 B line.  Issued by the epilogue warps before they wait for the accumulators, so the lines arrive
+// while the main loop of the tile runs.
+template <int TN, typename OT = float>
 __device__ __forceinline__ void corr_epi_prefetch(const CorrTcArgs &a, int64_t off0, int lane) {
-    const float *row = a.pred + off0 + (int64_t)lane * a.P;
+    const OT *row = static_cast<const OT *>(a.pred) + off0 + (int64_t)lane * a.P;
 #pragma unroll
-    for (int c = 0; c < TN; c += 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + c));
+    for (int c = 0; c < TN; c += 128 / (int)sizeof(OT)) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + c));
 }
 
 // L1 mode, end of an epilogue warp's tile loop: publish the warp's partial sum; the last warp of the grid to arrive
@@ -527,7 +543,7 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             if (a.pred) {
 #pragma unroll
                 for (int h = 0; h < kHalves; ++h)
-                    corr_epi_prefetch<TN>(a, ((int64_t)frame * a.P + m_tile * TM + h * 128 + lq * 32) * a.P + n_tile * TN, lane);
+                    corr_epi_prefetch<TN, T>(a, ((int64_t)frame * a.P + m_tile * TM + h * 128 + lq * 32) * a.P + n_tile * TN, lane);
             }
             mbar_wait(smem_u32(scales_ready + buf), use & 1);
             mbar_wait(smem_u32(tmem_full + buf), use & 1);
@@ -539,7 +555,7 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 const float sa = s_sa[buf * kTile + row0 + lane];
                 const int64_t off0 = ((int64_t)frame * a.P + m_tile * TM + row0) * a.P + n_tile * TN;
                 const uint32_t taddr = tmem_base + ((uint32_t)(lq * 32) << 16) + (uint32_t)(buf * kBufCols + h * TN);
-                if (a.pred) corr_epi_block<TN, true>(a, taddr, sa, sbv, st, off0, lane, l1_acc);
+                if (a.pred) corr_epi_block<TN, true, T>(a, taddr, sa, sbv, st, off0, lane, l1_acc);
                 else corr_epi_block<TN, false, T>(a, taddr, sa, sbv, st, off0, lane, l1_acc);
             }
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -840,9 +856,11 @@ corr_tc2_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 
 // backward of mean |pred - corr| w.r.t. pred: sign * grad / count.  Thread = 4 consecutive elements (one 4-byte load,
 // one coalesced 16-byte store), 4 such groups a block stride apart per thread for loads in flight.
+// T: element type of pred and g_pred; a half gradient is the fp32 one rounded to nearest even (one 8-byte store)
+template <typename T = float>
 __global__ void __launch_bounds__(256) corr_l1_bwd_kernel(const signed char *__restrict__ sign,
                                                           const float *__restrict__ grad_loss, float inv_count,
-                                                          float *__restrict__ g_pred, int64_t n4) {
+                                                          void *__restrict__ g_pred, int64_t n4) {
     pdl_sync();
     const float g = __fmul_rn(__ldg(grad_loss), inv_count);
     const int64_t i0 = (int64_t)blockIdx.x * (4 * 256) + threadIdx.x;
@@ -861,7 +879,14 @@ __global__ void __launch_bounds__(256) corr_l1_bwd_kernel(const signed char *__r
         r.y = (float)(signed char)((w[k] >> 8) & 0xff) * g;
         r.z = (float)(signed char)((w[k] >> 16) & 0xff) * g;
         r.w = (float)(signed char)((w[k] >> 24) & 0xff) * g;
-        __stcs(reinterpret_cast<float4 *>(g_pred) + i, r);
+        if constexpr (sizeof(T) == 4) {
+            __stcs(reinterpret_cast<float4 *>(static_cast<T *>(g_pred)) + i, r);
+        } else {
+            uint2 u;
+            T *e = reinterpret_cast<T *>(&u);
+            e[0] = narrow<T>(r.x); e[1] = narrow<T>(r.y); e[2] = narrow<T>(r.z); e[3] = narrow<T>(r.w);
+            __stcs(reinterpret_cast<uint2 *>(static_cast<T *>(g_pred)) + i, u);
+        }
     }
 }
 
@@ -870,12 +895,17 @@ __global__ void __launch_bounds__(256) corr_l1_bwd_kernel(const signed char *__r
 // ticket (16 bytes, zero between launches) + one partial per (CTA, epilogue warp) of up to 2 x 148 CTAs, with slack
 int64_t corr4d_l1_workspace_bytes() { return 16 + 2 * 148 * kEpiWarps * 4 * 2; }
 
-int corr4d_l1_bwd_launch(const signed char *sign, const float *grad_loss, float *g_pred, int64_t n, cudaStream_t st) {
-    MT_REQUIRE(n > 0 && n % 4 == 0 && aligned16(sign) && aligned16(g_pred), "mt_corr4d_l1_bwd: n must be a multiple of 4, pointers 16 B aligned");
-    const int64_t n4 = n / 4;
-    launch(corr_l1_bwd_kernel, dim3((unsigned)((n4 + 1023) / 1024)), dim3(256), 0, st, sign, grad_loss,
-           (float)(1.0 / (double)n), g_pred, n4);
-    return launch_status("mt_corr4d_l1_bwd");
+int corr4d_l1_bwd_launch(const signed char *sign, const float *grad_loss, void *g_pred, int64_t n, cudaStream_t st,
+                         int dtype) {
+    return with_dtype(dtype, "mt_corr4d_l1_bwd_dt", [&](auto t) {
+        using T = decltype(t);
+        MT_REQUIRE(n > 0 && n % 4 == 0 && aligned16(sign) && aligned_vec4<T>(g_pred),
+                   "mt_corr4d_l1_bwd: n must be a multiple of 4, sign 16 B and g_pred %d B aligned", 4 * (int)sizeof(T));
+        const int64_t n4 = n / 4;
+        launch(corr_l1_bwd_kernel<T>, dim3((unsigned)((n4 + 1023) / 1024)), dim3(256), 0, st, sign, grad_loss,
+               (float)(1.0 / (double)n), g_pred, n4);
+        return launch_status("mt_corr4d_l1_bwd");
+    });
 }
 
 int corr4d_tc_supported(int C, int P) {
@@ -931,8 +961,8 @@ static CorrMapSpec corr_map_spec() {
 }
 
 // Strided form.  ft (B, C, P): strides ft_sb, ft_sc; fr (B, C, F, P): fr_sb, fr_sc, fr_sf (elements; the pixel index
-// is contiguous).  Masks: see CorrTcArgs.  dtype (MT_DT_*): element type of ft / fr and of the volume `out`; fp16 /
-// bf16 features run the single-CTA kind::f16 kernel in store mode (no L1 mode, no CTA pairs).
+// is contiguous).  Masks: see CorrTcArgs.  dtype (MT_DT_*): element type of ft / fr and of the volume `out` (or of
+// `pred` in L1 mode); fp16 / bf16 features run the single-CTA kind::f16 kernel (no CTA pairs).
 int corr4d_tc_launch_ex(const void *ft, int64_t ft_sb, int64_t ft_sc, const void *fr, int64_t fr_sb, int64_t fr_sc,
                         int64_t fr_sf, const float *vt, int64_t vt_sb, const float *vr, int64_t vr_sb, int64_t vr_sf,
                         int mask_mode, int MH, int MW, int fh, int fw, void *out, int B, int C, int F, int P,
@@ -944,7 +974,6 @@ int corr4d_tc_launch_ex(const void *ft, int64_t ft_sb, int64_t ft_sc, const void
     });
     if (drc) return drc;
     const bool half = dtype != MT_DT_F32;
-    MT_REQUIRE(!half || !l1, "mt_corr4d_vgg_l1_fwd: fp32 features only");
     MT_REQUIRE(C % ms.bk == 0, "mt_corr4d_fwd: C = %d is not a multiple of %d channels", C, ms.bk);
     MT_REQUIRE(aligned16(ft) && aligned16(fr) && (l1 || aligned16(out)), "mt_corr4d_fwd: pointers must be 16 B aligned");
     MT_REQUIRE(!l1 || (l1->pred && l1->loss && l1->partials && aligned16(l1->pred) && aligned16(l1->sign)),

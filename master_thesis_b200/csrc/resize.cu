@@ -174,7 +174,7 @@ __global__ void __launch_bounds__(kThreads) resize_flow_kernel(const ResizeFlowA
 
 struct ResizeFlowBwdArgs {
     const float *g; int64_t sb, sf, sy, sx, sc;  // gradient of the (B,F,H,W,2) output
-    float *gin;                                   // (B,F,2,h,w) contiguous
+    void *gin;                                    // (B,F,2,h,w) contiguous, element type: the kernel's T
     int F, h, w, H, W;
     float scy, scx;    // h / H, w / W (the forward's scales)
     float invy, invx;  // H / h, W / w: only to bound the candidate output range
@@ -191,6 +191,9 @@ __device__ __forceinline__ void tap_range(int i, int out, float inv, int &lo, in
     hi = min(out - 1, (int)ceilf(__fmaf_rn((float)i + 1.5f, inv, -0.5f)) + 1);
 }
 
+// T: element type of the input flow and of its gradient (a half flow of DFPN training under autocast: the fp32
+// gradient rounded to nearest even, the backward of autocast's cast)
+template <typename T = float>
 __global__ void __launch_bounds__(kThreads) resize_flow_bwd_kernel(const ResizeFlowBwdArgs a) {
     pdl_sync();
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -214,9 +217,14 @@ __global__ void __launch_bounds__(kThreads) resize_flow_bwd_kernel(const ResizeF
             ay = __fmaf_rn(__ldg(row + ox * a.sx + a.sc), wt, ay);
         }
     }
-    float *o = a.gin + (int64_t)n * 2 * a.h * a.w + p;
-    o[0] = ax;
-    o[(int64_t)a.h * a.w] = ay;
+    T *o = static_cast<T *>(a.gin) + (int64_t)n * 2 * a.h * a.w + p;
+    if constexpr (sizeof(T) == 4) {
+        o[0] = ax;
+        o[(int64_t)a.h * a.w] = ay;
+    } else {
+        o[0] = narrow<T>(ax);
+        o[(int64_t)a.h * a.w] = narrow<T>(ay);
+    }
 }
 
 bool mult4(int64_t v) { return (v & 3) == 0; }
@@ -281,9 +289,11 @@ extern "C" int mt_resize_flow(const float *flow, int64_t sb, int64_t sf, int64_t
                              mode, stream);
 }
 
-extern "C" int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
-                                  int64_t g_sc, float *g_flow, int B, int F, int h, int w, int H, int W,
-                                  mt_stream_t stream) {
+// g_dtype (MT_DT_*): element type of g_flow, the dtype of the input flow.  Under autocast the bilinear resize of a
+// half flow runs in fp32 (see mt_resize_flow_dt), so its gradient is the fp32 gradient rounded to that dtype.
+extern "C" int mt_resize_flow_bwd_dt(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
+                                     int64_t g_sc, int g_dtype, void *g_flow, int B, int F, int h, int w, int H, int W,
+                                     mt_stream_t stream) {
     MT_REQUIRE(g_out && g_flow, "mt_resize_flow_bwd: NULL argument");
     MT_REQUIRE(B > 0 && F > 0 && h > 0 && w > 0 && H > 0 && W > 0 && (int64_t)B * F <= 65535 &&
                    (int64_t)h * w <= (1ll << 30),
@@ -291,6 +301,16 @@ extern "C" int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf
     ResizeFlowBwdArgs a{g_out, g_sb, g_sf, g_sy, g_sx, g_sc, g_flow, F, h, w, H, W,
                         (float)h / (float)H, (float)w / (float)W, (float)H / (float)h, (float)W / (float)w};
     dim3 grid((unsigned)(((int64_t)h * w + kThreads - 1) / kThreads), B * F);
-    launch(resize_flow_bwd_kernel, grid, kThreads, 0, (cudaStream_t)stream, a);
+    const int rc = with_dtype(g_dtype, "mt_resize_flow_bwd_dt", [&](auto t) {
+        launch(resize_flow_bwd_kernel<decltype(t)>, grid, kThreads, 0, (cudaStream_t)stream, a);
+        return MT_OK;
+    });
+    if (rc) return rc;
     return launch_status("mt_resize_flow_bwd");
+}
+
+extern "C" int mt_resize_flow_bwd(const float *g_out, int64_t g_sb, int64_t g_sf, int64_t g_sy, int64_t g_sx,
+                                  int64_t g_sc, float *g_flow, int B, int F, int h, int w, int H, int W,
+                                  mt_stream_t stream) {
+    return mt_resize_flow_bwd_dt(g_out, g_sb, g_sf, g_sy, g_sx, g_sc, MT_DT_F32, g_flow, B, F, h, w, H, W, stream);
 }

@@ -300,22 +300,27 @@ struct Taps {
     bool interior;
 };
 
-// flow of pixel (y0 + k, x) of frame n for k < U; rows past H get a centred dummy
-template <int U>
-__device__ __forceinline__ void dense_flow_load(const float *__restrict__ flow, int np0, int y0, const Sampler &sp,
-                                                float2 (&g)[U]) {
+// the (0, 0) pair of G (make_float2 for fp32: the fp32 kernels compile to the code they had before the flow type)
+template <typename G> __device__ __forceinline__ Flow2<G> make_flow2() { return Flow2<G>{}; }
+template <> __device__ __forceinline__ float2 make_flow2<float>() { return make_float2(0.0f, 0.0f); }
+// flow of pixel (y0 + k, x) of frame n for k < U as stored (pairs of G: a half pair stays one register while the load
+// is in flight); rows past H get a centred dummy
+template <int U, typename G = float>
+__device__ __forceinline__ void dense_flow_load(const void *__restrict__ flow, int np0, int y0, const Sampler &sp,
+                                                Flow2<G> (&g)[U]) {
 #pragma unroll
     for (int k = 0; k < U; ++k)
-        g[k] = (y0 + k < sp.H) ? __ldcs(reinterpret_cast<const float2 *>(flow) + (np0 + k * sp.W)) : make_float2(0.0f, 0.0f);
+        g[k] = (y0 + k < sp.H) ? __ldcs(static_cast<const Flow2<G> *>(flow) + (np0 + k * sp.W)) : make_flow2<G>();
 }
 
-template <int U>
-__device__ __forceinline__ void dense_taps_from(const float2 (&g)[U], const Sampler &sp, Taps<U> &t) {
+// the taps of the (widened) flow pairs g
+template <int U, typename F2>
+__device__ __forceinline__ void dense_taps_from(const F2 (&g)[U], const Sampler &sp, Taps<U> &t) {
     const float wm2 = sp.wmax - 1.0f, hm2 = sp.hmax - 1.0f;
     t.interior = true;
 #pragma unroll
     for (int k = 0; k < U; ++k) {
-        t.gx[k] = g[k].x; t.gy[k] = g[k].y;
+        t.gx[k] = flow_widen(g[k]).x; t.gy[k] = flow_widen(g[k]).y;
         t.ix[k] = unnormalize(t.gx[k], sp.sfx, sp.ac);
         t.iy[k] = unnormalize(t.gy[k], sp.sfy, sp.ac);
         t.xw[k] = floorf(t.ix[k]);
@@ -326,11 +331,11 @@ __device__ __forceinline__ void dense_taps_from(const float2 (&g)[U], const Samp
     }
 }
 
-template <int U>
-__device__ __forceinline__ void dense_taps(const float *__restrict__ flow, int np0, int y0, const Sampler &sp,
+template <int U, typename G = float>
+__device__ __forceinline__ void dense_taps(const void *__restrict__ flow, int np0, int y0, const Sampler &sp,
                                            Taps<U> &t) {
-    float2 g[U];
-    dense_flow_load<U>(flow, np0, y0, sp, g);
+    Flow2<G> g[U];
+    dense_flow_load<U, G>(flow, np0, y0, sp, g);
     dense_taps_from<U>(g, sp, t);
 }
 
@@ -384,15 +389,19 @@ __device__ __forceinline__ float interp_k(const Corners &q, const Taps<U> &t, in
 
 // ---- backward w.r.t. the dense grid (generic upstream gradient) -------------
 struct WarpBwdArgs {
-    const float *x, *grid, *gout;
-    float *ggrid;
+    const float *x;
+    const void *grid;  // dense flow, pairs of the kernel's G
+    const float *gout;
+    void *ggrid;       // gradient w.r.t. the flow, pairs of G
     int x_sb, x_sc, x_sf, g_sb, g_sc, g_sf;
     int F, P;
     unsigned f_magic;
     Sampler sp;
 };
 
-template <int C, int U>
+// G: element type of the flow and of its gradient (float, or the half flow of a DFPN training step under autocast:
+// widened on load, the fp32 gradient rounded to G on store)
+template <int C, int U, typename G = float>
 __global__ void __launch_bounds__(kCols, kWarpBMinB) warp_bwd_grid_kernel(const WarpBwdArgs a) {
     pdl_sync();
     const int W = a.sp.W, H = a.sp.H;
@@ -409,7 +418,7 @@ __global__ void __launch_bounds__(kCols, kWarpBMinB) warp_bwd_grid_kernel(const 
 #pragma unroll
         for (int k = 0; k < U; ++k) go[c][k] = (y0 + k < H) ? __ldcs(a.gout + (go0 + c * a.g_sc + k * W)) : 0.0f;
     Taps<U> t;
-    dense_taps<U>(a.grid, np0, y0, a.sp, t);
+    dense_taps<U, G>(a.grid, np0, y0, a.sp, t);
     Corners q[C][U];
     gather_taps<C, U>(a.x, b * a.x_sb + f * a.x_sf, a.x_sc, a.sp, t, q);
     if (!live) return;
@@ -422,16 +431,18 @@ __global__ void __launch_bounds__(kCols, kWarpBMinB) warp_bwd_grid_kernel(const 
             ax += ((q[c][k].ne - q[c][k].nw) * t.s[k] + (q[c][k].se - q[c][k].sw) * t.n[k]) * go[c][k];
             ay += ((q[c][k].sw - q[c][k].nw) * t.e[k] + (q[c][k].se - q[c][k].ne) * t.w[k]) * go[c][k];
         }
-        __stcs(reinterpret_cast<float2 *>(a.ggrid) + (np0 + k * W), make_float2(ax * a.sp.sfx, ay * a.sp.sfy));
+        flow_stcs(static_cast<Flow2<G> *>(a.ggrid) + (np0 + k * W), make_float2(ax * a.sp.sfx, ay * a.sp.sfy));
     }
 }
 
 // ---- fused warp + mask_out + masked L1 ('sum') ------------------------------
 struct WarpL1Args {
-    const float *x, *vis, *flow, *xt, *vt;
+    const float *x, *vis;
+    const void *flow;  // dense flow, pairs of the kernel's G
+    const float *xt, *vt;
     float *x_al, *v_al;  // frame-major, may be NULL
     float *out3; void *ws;
-    const float *out3_in, *grad_out; float *gflow;  // backward only
+    const float *out3_in, *grad_out; void *gflow;  // backward only; gflow: pairs of G
     int x_sb, x_sc, x_sf, vis_sb, vis_sf, xt_sb, xt_sc, vt_sb;
     int F, P, row_blocks;
     unsigned f_magic;
@@ -449,7 +460,8 @@ __device__ __forceinline__ float mask_out_of(float gx, float gy) {
 // number of partials stays within the reduction workspace
 // MAT: the aligned frames / visibilities are also written (a consumer asked for them); the loss-only instantiation
 // carries neither the stores nor the nearest-tap gather and fits the 64-register budget of 8 CTAs per SM.
-template <int U, bool MAT>
+// G: element type of the flow, widened on load (a half flow: the loss of the fp32 kernel on the widened flow).
+template <int U, bool MAT, typename G = float>
 __global__ void __launch_bounds__(kCols, MAT ? kWarpBMinB : kWarpL1FMinB) warp_l1_fwd_kernel(const WarpL1Args a) {
     pdl_sync();
     __shared__ float red[2 * 32];
@@ -467,9 +479,9 @@ __global__ void __launch_bounds__(kCols, MAT ? kWarpBMinB : kWarpL1FMinB) warp_l
     // L2 -> L1 sector traffic for 201 MB of DRAM reads: CTAs on one SM were 100+ rows apart)
     const int per = (a.row_blocks + (int)gridDim.y - 1) / (int)gridDim.y;
     const int rb0 = (int)blockIdx.y * per, rb1 = min(rb0 + per, a.row_blocks);
-    float2 g_next[U];
+    Flow2<G> g_next[U];
     if (rb0 < rb1)
-        dense_flow_load<U>(a.flow, (int)n * a.P + rb0 * U * W + x, rb0 * U, a.sp, g_next);
+        dense_flow_load<U, G>(a.flow, (int)n * a.P + rb0 * U * W + x, rb0 * U, a.sp, g_next);
     for (int rb = rb0; rb < rb1; ++rb) {
         const int y0 = rb * U;
         const int p0 = y0 * W + x, np0 = (int)n * a.P + p0;
@@ -485,7 +497,7 @@ __global__ void __launch_bounds__(kCols, MAT ? kWarpBMinB : kWarpL1FMinB) warp_l
         dense_taps_from<U>(g_next, a.sp, t);
         {
             const int rn = rb + 1;
-            if (rn < rb1) dense_flow_load<U>(a.flow, (int)n * a.P + rn * U * W + x, rn * U, a.sp, g_next);
+            if (rn < rb1) dense_flow_load<U, G>(a.flow, (int)n * a.P + rn * U * W + x, rn * U, a.sp, g_next);
         }
         Corners q[3][U];
         gather_taps<3, U>(a.x, xo, a.x_sc, a.sp, t, q);
@@ -516,8 +528,8 @@ __global__ void __launch_bounds__(kCols, MAT ? kWarpBMinB : kWarpL1FMinB) warp_l
 }
 
 // d loss / d flow in one pass: recomputes the sampling, never materialises
-// x_aligned or its gradient.
-template <int U>
+// x_aligned or its gradient.  G: element type of the flow and of d loss / d flow (rounded to G on store).
+template <int U, typename G = float>
 __global__ void __launch_bounds__(kCols, kWarpL1BMinB) warp_l1_bwd_kernel(const WarpL1Args a) {
     pdl_sync();
     const int W = a.sp.W, H = a.sp.H;
@@ -537,7 +549,7 @@ __global__ void __launch_bounds__(kCols, kWarpL1BMinB) warp_l1_bwd_kernel(const 
         for (int c = 0; c < 3; ++c) xt[c][k] = in ? __ldg(a.xt + (b * a.xt_sb + c * a.xt_sc + p0 + k * W)) : 0.0f;
     }
     Taps<U> t;
-    dense_taps<U>(a.flow, np0, y0, a.sp, t);
+    dense_taps<U, G>(a.flow, np0, y0, a.sp, t);
     Corners q[3][U];
     gather_taps<3, U>(a.x, b * a.x_sb + f * a.x_sf, a.x_sc, a.sp, t, q);
     if (!live) return;
@@ -554,21 +566,27 @@ __global__ void __launch_bounds__(kCols, kWarpL1BMinB) warp_l1_bwd_kernel(const 
             ax += ((q[c][k].ne - q[c][k].nw) * t.s[k] + (q[c][k].se - q[c][k].sw) * t.n[k]) * go;
             ay += ((q[c][k].sw - q[c][k].nw) * t.e[k] + (q[c][k].se - q[c][k].ne) * t.w[k]) * go;
         }
-        __stcs(reinterpret_cast<float2 *>(a.gflow) + (np0 + k * W), make_float2(ax * a.sp.sfx, ay * a.sp.sfy));
+        flow_stcs(static_cast<Flow2<G> *>(a.gflow) + (np0 + k * W), make_float2(ax * a.sp.sfx, ay * a.sp.sfy));
     }
 }
 
-__global__ void __launch_bounds__(256) mask_out_kernel(const float *__restrict__ flow, int64_t n,
+// G: element type of the flow; a comparison of the widened value gives that of the half one
+template <typename G = float>
+__global__ void __launch_bounds__(256) mask_out_kernel(const void *__restrict__ flow, int64_t n,
                                                        float *__restrict__ out) {
     pdl_sync();
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
          i += (int64_t)gridDim.x * blockDim.x) {
-        const float2 g = __ldcs(reinterpret_cast<const float2 *>(flow) + i);
+        const float2 g = flow_ldcs(static_cast<const Flow2<G> *>(flow) + i);
         st_stream1(out + i, mask_out_of(g.x, g.y));
     }
 }
 
 bool aligned8(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
+// a dense flow (or its gradient) of dtype code dt is read / written one (gx, gy) pair per access
+bool flow_aligned(const void *p, int dt) {
+    return (reinterpret_cast<uintptr_t>(p) & (dt == MT_DT_F32 ? 7u : 3u)) == 0;
+}
 
 }  // namespace
 }  // namespace mt
@@ -803,16 +821,23 @@ extern "C" int mt_warp_pack_lowres_fwd(const float *x, int64_t x_sb, int64_t x_s
                                       v_aligned, v_map, B, F, H, W, flags, stream);
 }
 
-extern "C" int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
-                                const float *grid, const float *gout, int64_t g_sb, int64_t g_sc,
-                                int64_t g_sf, float *ggrid, int B, int C, int F, int H, int W,
-                                int flags, mt_stream_t stream) {
+// The _dt entry points of the DFPN training step take the dtype code (MT_DT_*) of the dense flow; the gradient w.r.t.
+// the flow is written in that dtype.  Under autocast the flow estimators return fp16 / bf16 flows, grid_sample promotes
+// them to fp32 (utils.py:93-103), the mask compares the half values (model_dfpn.py:269-272) and l1_loss runs in fp32
+// (utils.py:166-169): every loss and output is the fp32 entry point's on flow.float(), and d loss / d flow is its
+// gradient rounded to nearest even (the backward of autocast's cast).
+extern "C" int mt_warp_bwd_grid_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf, int g_dtype,
+                                   const void *grid, const float *gout, int64_t g_sb, int64_t g_sc, int64_t g_sf,
+                                   void *ggrid, int B, int C, int F, int H, int W, int flags, mt_stream_t stream) {
     MT_REQUIRE(x && grid && gout && ggrid, "mt_warp_bwd_grid: NULL argument");
     MT_REQUIRE(B > 0 && F > 0 && H > 0 && W > 0, "mt_warp_bwd_grid: empty shape");
     MT_REQUIRE(C == 1 || C == 3, "mt_warp_bwd_grid: C must be 1 or 3, got %d", C);
     MT_REQUIRE(!(flags & MT_GRID_AFFINE), "mt_warp_bwd_grid: dense grids only");
     MT_REQUIRE((int64_t)B * F <= 65535 && (H + kRows - 1) / kRows <= 65535, "mt_warp_bwd_grid: too large");
-    MT_REQUIRE(aligned8(grid) && aligned8(ggrid), "mt_warp_bwd_grid: grids must be 8 B aligned");
+    MT_REQUIRE(g_dtype == MT_DT_F32 || g_dtype == MT_DT_F16 || g_dtype == MT_DT_BF16,
+               "mt_warp_bwd_grid_dt: unknown dtype code %d", g_dtype);
+    MT_REQUIRE(flow_aligned(grid, g_dtype) && flow_aligned(ggrid, g_dtype),
+               "mt_warp_bwd_grid: grids must be aligned to one (gx, gy) pair (%d B)", g_dtype == MT_DT_F32 ? 8 : 4);
     const int64_t P = (int64_t)H * W, lim = (1ll << 31) - 1;
     MT_REQUIRE(x_sb >= 0 && x_sc >= 0 && x_sf >= 0 && g_sb >= 0 && g_sc >= 0 && g_sf >= 0,
                "mt_warp_bwd_grid: negative strides are not supported");
@@ -827,19 +852,35 @@ extern "C" int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int6
     a.sp = make_sampler(H, W, (flags & MT_ALIGN_CORNERS) != 0);
     dim3 block(kCols), gridd((W + kCols - 1) / kCols, (H + kRows - 1) / kRows, B * F);
     cudaStream_t st = (cudaStream_t)stream;
-    if (C == 3) launch(warp_bwd_grid_kernel<3, kRows>, gridd, block, 0, st, a);
-    else launch(warp_bwd_grid_kernel<1, kRows>, gridd, block, 0, st, a);
+    const int rc = with_dtype(g_dtype, "mt_warp_bwd_grid_dt", [&](auto t) {
+        using G = decltype(t);
+        if (C == 3) launch(warp_bwd_grid_kernel<3, kRows, G>, gridd, block, 0, st, a);
+        else launch(warp_bwd_grid_kernel<1, kRows, G>, gridd, block, 0, st, a);
+        return MT_OK;
+    });
+    if (rc) return rc;
     return launch_status("mt_warp_bwd_grid");
 }
 
+extern "C" int mt_warp_bwd_grid(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                const float *grid, const float *gout, int64_t g_sb, int64_t g_sc,
+                                int64_t g_sf, float *ggrid, int B, int C, int F, int H, int W,
+                                int flags, mt_stream_t stream) {
+    return mt_warp_bwd_grid_dt(x, x_sb, x_sc, x_sf, MT_DT_F32, grid, gout, g_sb, g_sc, g_sf, ggrid, B, C, F, H, W, flags,
+                               stream);
+}
+
 static int fill_l1_args(WarpL1Args &a, const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
-                        const float *flow, const float *x_target, int64_t xt_sb, int64_t xt_sc,
+                        int f_dtype, const void *flow, const float *x_target, int64_t xt_sb, int64_t xt_sc,
                         const float *v_target, int64_t vt_sb, int B, int F, int H, int W,
                         float weight, int flags, const char *who) {
     MT_REQUIRE(x && flow && x_target && v_target, "%s: NULL input", who);
+    MT_REQUIRE(f_dtype == MT_DT_F32 || f_dtype == MT_DT_F16 || f_dtype == MT_DT_BF16, "%s_dt: unknown dtype code %d",
+               who, f_dtype);
     MT_REQUIRE(B > 0 && F > 0 && H > 0 && W > 0, "%s: empty shape", who);
     MT_REQUIRE((int64_t)B * F <= 65535 && (H + kRows - 1) / kRows <= 65535, "%s: too large", who);
-    MT_REQUIRE(aligned8(flow), "%s: flow must be 8 B aligned", who);
+    MT_REQUIRE(flow_aligned(flow, f_dtype), "%s: flow must be aligned to one (gx, gy) pair (%d B)", who,
+               f_dtype == MT_DT_F32 ? 8 : 4);
     const int64_t P = (int64_t)H * W, lim = (1ll << 31) - 1;
     MT_REQUIRE(x_sb >= 0 && x_sc >= 0 && x_sf >= 0 && xt_sb >= 0 && xt_sc >= 0 && vt_sb >= 0,
                "%s: negative strides are not supported", who);
@@ -858,14 +899,14 @@ static int fill_l1_args(WarpL1Args &a, const float *x, int64_t x_sb, int64_t x_s
     return MT_OK;
 }
 
-extern "C" int mt_warp_l1_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
-                              const float *vis, int64_t vis_sb, int64_t vis_sf, const float *flow,
-                              const float *x_target, int64_t xt_sb, int64_t xt_sc,
-                              const float *v_target, int64_t vt_sb, float *x_aligned,
-                              float *v_aligned, float *out3, void *workspace, int B, int F, int H,
-                              int W, float weight, int flags, mt_stream_t stream) {
+extern "C" int mt_warp_l1_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                 const float *vis, int64_t vis_sb, int64_t vis_sf, int f_dtype, const void *flow,
+                                 const float *x_target, int64_t xt_sb, int64_t xt_sc,
+                                 const float *v_target, int64_t vt_sb, float *x_aligned,
+                                 float *v_aligned, float *out3, void *workspace, int B, int F, int H,
+                                 int W, float weight, int flags, mt_stream_t stream) {
     WarpL1Args a;
-    int rc = fill_l1_args(a, x, x_sb, x_sc, x_sf, flow, x_target, xt_sb, xt_sc, v_target, vt_sb, B,
+    int rc = fill_l1_args(a, x, x_sb, x_sc, x_sf, f_dtype, flow, x_target, xt_sb, xt_sc, v_target, vt_sb, B,
                           F, H, W, weight, flags, "mt_warp_l1_fwd");
     if (rc) return rc;
     MT_REQUIRE(out3 && workspace, "mt_warp_l1_fwd: NULL out3 / workspace");
@@ -889,9 +930,47 @@ extern "C" int mt_warp_l1_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_
     if (cap < 1) cap = 1;
     if (gy > cap) gy = (int)cap;
     dim3 block(kCols), gridd(colb, gy, B * F);
-    if (a.x_al || a.v_al) launch(warp_l1_fwd_kernel<kRows, true>, gridd, block, 0, (cudaStream_t)stream, a);
-    else launch(warp_l1_fwd_kernel<kRows, false>, gridd, block, 0, (cudaStream_t)stream, a);
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = with_dtype(f_dtype, "mt_warp_l1_fwd_dt", [&](auto t) {
+        using G = decltype(t);
+        if (a.x_al || a.v_al) launch(warp_l1_fwd_kernel<kRows, true, G>, gridd, block, 0, st, a);
+        else launch(warp_l1_fwd_kernel<kRows, false, G>, gridd, block, 0, st, a);
+        return MT_OK;
+    });
+    if (rc) return rc;
     return launch_status("mt_warp_l1_fwd");
+}
+
+extern "C" int mt_warp_l1_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                              const float *vis, int64_t vis_sb, int64_t vis_sf, const float *flow,
+                              const float *x_target, int64_t xt_sb, int64_t xt_sc,
+                              const float *v_target, int64_t vt_sb, float *x_aligned,
+                              float *v_aligned, float *out3, void *workspace, int B, int F, int H,
+                              int W, float weight, int flags, mt_stream_t stream) {
+    return mt_warp_l1_fwd_dt(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, MT_DT_F32, flow, x_target, xt_sb, xt_sc, v_target,
+                             vt_sb, x_aligned, v_aligned, out3, workspace, B, F, H, W, weight, flags, stream);
+}
+
+extern "C" int mt_warp_l1_bwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                 int f_dtype, const void *flow, const float *x_target, int64_t xt_sb,
+                                 int64_t xt_sc, const float *v_target, int64_t vt_sb,
+                                 const float *out3, const float *grad_out, void *gflow, int B, int F,
+                                 int H, int W, float weight, int flags, mt_stream_t stream) {
+    WarpL1Args a;
+    int rc = fill_l1_args(a, x, x_sb, x_sc, x_sf, f_dtype, flow, x_target, xt_sb, xt_sc, v_target, vt_sb, B,
+                          F, H, W, weight, flags, "mt_warp_l1_bwd");
+    if (rc) return rc;
+    MT_REQUIRE(out3 && grad_out && gflow, "mt_warp_l1_bwd: NULL out3 / grad_out / gflow");
+    MT_REQUIRE(flow_aligned(gflow, f_dtype), "mt_warp_l1_bwd: gflow must be aligned to one (gx, gy) pair");
+    a.out3_in = out3; a.grad_out = grad_out; a.gflow = gflow;
+    dim3 block(kCols), gridd((W + kCols - 1) / kCols, a.row_blocks, B * F);
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = with_dtype(f_dtype, "mt_warp_l1_bwd_dt", [&](auto t) {
+        launch(warp_l1_bwd_kernel<kRows, decltype(t)>, gridd, block, 0, st, a);
+        return MT_OK;
+    });
+    if (rc) return rc;
+    return launch_status("mt_warp_l1_bwd");
 }
 
 extern "C" int mt_warp_l1_bwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
@@ -899,22 +978,25 @@ extern "C" int mt_warp_l1_bwd(const float *x, int64_t x_sb, int64_t x_sc, int64_
                               int64_t xt_sc, const float *v_target, int64_t vt_sb,
                               const float *out3, const float *grad_out, float *gflow, int B, int F,
                               int H, int W, float weight, int flags, mt_stream_t stream) {
-    WarpL1Args a;
-    int rc = fill_l1_args(a, x, x_sb, x_sc, x_sf, flow, x_target, xt_sb, xt_sc, v_target, vt_sb, B,
-                          F, H, W, weight, flags, "mt_warp_l1_bwd");
+    return mt_warp_l1_bwd_dt(x, x_sb, x_sc, x_sf, MT_DT_F32, flow, x_target, xt_sb, xt_sc, v_target, vt_sb, out3,
+                             grad_out, gflow, B, F, H, W, weight, flags, stream);
+}
+
+extern "C" int mt_mask_out_dt(int f_dtype, const void *flow, int64_t n, float *out, mt_stream_t stream) {
+    MT_REQUIRE(flow && out && n > 0, "mt_mask_out: bad argument");
+    MT_REQUIRE(f_dtype == MT_DT_F32 || f_dtype == MT_DT_F16 || f_dtype == MT_DT_BF16,
+               "mt_mask_out_dt: unknown dtype code %d", f_dtype);
+    MT_REQUIRE(flow_aligned(flow, f_dtype), "mt_mask_out: flow must be aligned to one (gx, gy) pair");
+    int64_t nb = (n + 255) / 256, cap = (int64_t)sm_count() * 16;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = with_dtype(f_dtype, "mt_mask_out_dt", [&](auto t) {
+        launch(mask_out_kernel<decltype(t)>, (int)(nb < cap ? nb : cap), 256, 0, st, flow, n, out);
+        return MT_OK;
+    });
     if (rc) return rc;
-    MT_REQUIRE(out3 && grad_out && gflow, "mt_warp_l1_bwd: NULL out3 / grad_out / gflow");
-    MT_REQUIRE(aligned8(gflow), "mt_warp_l1_bwd: gflow must be 8 B aligned");
-    a.out3_in = out3; a.grad_out = grad_out; a.gflow = gflow;
-    dim3 block(kCols), gridd((W + kCols - 1) / kCols, a.row_blocks, B * F);
-    launch(warp_l1_bwd_kernel<kRows>, gridd, block, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_warp_l1_bwd");
+    return launch_status("mt_mask_out");
 }
 
 extern "C" int mt_mask_out(const float *flow, int64_t n, float *out, mt_stream_t stream) {
-    MT_REQUIRE(flow && out && n > 0, "mt_mask_out: bad argument");
-    MT_REQUIRE((reinterpret_cast<uintptr_t>(flow) & 7u) == 0, "mt_mask_out: flow must be 8 B aligned");
-    int64_t nb = (n + 255) / 256, cap = (int64_t)sm_count() * 16;
-    launch(mask_out_kernel, (int)(nb < cap ? nb : cap), 256, 0, (cudaStream_t)stream, flow, n, out);
-    return launch_status("mt_mask_out");
+    return mt_mask_out_dt(MT_DT_F32, flow, n, out, stream);
 }

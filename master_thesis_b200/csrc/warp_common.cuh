@@ -126,12 +126,20 @@ template <typename G> struct Flow2Of { using type = float2; };
 template <> struct Flow2Of<__half> { using type = __half2; };
 template <> struct Flow2Of<__nv_bfloat16> { using type = __nv_bfloat162; };
 template <typename G> using Flow2 = typename Flow2Of<G>::type;
+__device__ __forceinline__ const float2 &flow_widen(const float2 &v) { return v; }
+__device__ __forceinline__ float2 flow_widen(__half2 v) { return __half22float2(v); }
+__device__ __forceinline__ float2 flow_widen(__nv_bfloat162 v) { return __bfloat1622float2(v); }
 __device__ __forceinline__ float2 flow_ldcs(const float2 *p) { return __ldcs(p); }
 __device__ __forceinline__ float2 flow_ldcs(const __half2 *p) { return __half22float2(__ldcs(p)); }
 __device__ __forceinline__ float2 flow_ldcs(const __nv_bfloat162 *p) { return __bfloat1622float2(__ldcs(p)); }
 __device__ __forceinline__ float2 flow_ldg(const float2 *p) { return __ldg(p); }
 __device__ __forceinline__ float2 flow_ldg(const __half2 *p) { return __half22float2(__ldg(p)); }
 __device__ __forceinline__ float2 flow_ldg(const __nv_bfloat162 *p) { return __bfloat1622float2(__ldg(p)); }
+// a flow gradient stored as a pair of G: a half flow's gradient is the fp32 one rounded to nearest even (the backward
+// of autocast's cast)
+__device__ __forceinline__ void flow_stcs(float2 *p, float2 v) { __stcs(p, v); }
+__device__ __forceinline__ void flow_stcs(__half2 *p, float2 v) { __stcs(p, __float22half2_rn(v)); }
+__device__ __forceinline__ void flow_stcs(__nv_bfloat162 *p, float2 v) { __stcs(p, __float22bfloat162_rn(v)); }
 
 // the resized flow at one output pixel: rows r0 / r1 of the low-resolution flow (a pair = (gx, gy)),
 // row(y) = fma(v[x0], lx0, v[x1] * lx1); out = fma(row(y0), ly0, row(y1) * ly1)   (the CPU build's order: DESIGN.md "bit-exactness")

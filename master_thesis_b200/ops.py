@@ -5,8 +5,9 @@ and autograd bookkeeping.  Every computation is a hand-written sm_100a kernel
 reached through ``_lib.call`` with raw device pointers.  CUDA fp32 tensors
 only, except the network operands checked against ``NET_DTYPES`` (the CNN output
 of CHN, the inputs of masked_l1, the DFPN's flows and VGG features), which may
-also be fp16 / bf16 as autocast hands them over; anything else raises - there is
-no CPU / eager fallback.
+also be fp16 / bf16 as autocast hands them over; the operands of DFPN's own
+training step (``_train_dtypes``) only while autocast is on.  Anything else
+raises - there is no CPU / eager fallback.
 """
 import ctypes
 
@@ -106,6 +107,27 @@ def _need_cuda(*ts):
             raise RuntimeError("master_thesis_b200: tensors on different devices (%s, %s)" % (first, t.device))
     if first is not None:
         _device[0] = first.index
+
+
+def _train_dtypes():
+    """The dtypes an operand of DFPN's training step (a flow, the volume ``corr``, the VGG features of the loss) may
+    have: fp32, and while autocast is enabled on CUDA also autocast's dtype - the only situation in which the
+    reference's training step (``--precision 16|bf16``) produces half flows and volumes.  Checked in forward only:
+    autograd runs the backward outside the autocast region."""
+    if torch.is_autocast_enabled("cuda"):
+        dt = torch.get_autocast_dtype("cuda")
+        if dt in NET_DTYPES and dt != torch.float32:
+            return (torch.float32, dt)
+    return (torch.float32,)
+
+
+def _flow_pairs(flow):
+    """``flow`` contiguous, with its (gx, gy) pairs aligned for one load each: a half flow that starts at an odd
+    element (a view into a larger buffer) is copied."""
+    flow = _contig(flow)
+    if flow.data_ptr() % (2 * flow.element_size()):
+        flow = _lib.keep(flow.clone())
+    return flow
 
 
 def _no_grad_inputs(who, *ts):
@@ -272,13 +294,20 @@ def warp_pack_fwd(x, vis, grid, m_target, x_t, v_t, flags=ALIGN_CORNERS, want_al
 
 
 def warp_bwd_grid(x, grid, gout, flags=ALIGN_CORNERS):
-    _need_cuda(x, grid, gout)
+    """d loss / d grid of the dense-flow warp (autograd of grid_sample, utils.py:93-97), in the dtype of ``grid``: a
+    half flow (under autocast only) gets the fp32 gradient on the widened flow rounded to its dtype."""
+    _need_cuda(x, (grid, _train_dtypes()), gout)
+    return _warp_bwd_grid(x, grid, gout, flags)
+
+
+def _warp_bwd_grid(x, grid, gout, flags):
+    _need_cuda(x, (grid, NET_DTYPES), gout)
     b, c, f, h, w = x.shape
     x, x_sb, x_sc, x_sf = _s5(x)
     gout, g_sb, g_sc, g_sf = _s5(gout)
-    grid = _contig(grid)
+    grid = _flow_pairs(grid)
     gg = _empty_like(grid)
-    _call("mt_warp_bwd_grid", _ptr(x), x_sb, x_sc, x_sf, _ptr(grid), _ptr(gout), g_sb, g_sc,
+    _call_net("mt_warp_bwd_grid", _ptr(x), x_sb, x_sc, x_sf, _Net(grid), _ptr(gout), g_sb, g_sc,
               g_sf, _ptr(gg), b, c, f, h, w, flags, _stream(x))
     return gg
 
@@ -298,11 +327,13 @@ class AlignSetFn(torch.autograd.Function):
         if not ctx.needs_input_grad[2] or g_xa is None:
             return None, None, None
         # the nearest sampler has zero gradient w.r.t. the grid: g_va is ignored
-        return None, None, warp_bwd_grid(x, flow, g_xa, ALIGN_CORNERS)
+        return None, None, _warp_bwd_grid(x, flow, g_xa, ALIGN_CORNERS)
 
 
 def align_set(x, v, flow):
-    _need_cuda(x, v, flow)          # DFPN training: fp32 flows only (warp_fwd alone also reads half flows)
+    """FlowsUtils.align_set (utils.py:78-104), differentiable w.r.t. ``flow``.  Under autocast the flow may be in its
+    dtype: the outputs are the fp32 op's on ``flow.float()`` and the gradient is the fp32 one rounded to that dtype."""
+    _need_cuda(x, v, (flow, _train_dtypes()))
     if x.requires_grad or v.requires_grad:
         raise RuntimeError("align_set: gradients w.r.t. x / v are not provided (the reference "
                            "never requests them); only the flow is differentiable")
@@ -310,12 +341,12 @@ def align_set(x, v, flow):
 
 
 def mask_out(flow):
-    """model_dfpn.py:269-272: flow (B,F,H,W,2) -> (B,1,F,H,W)."""
-    _need_cuda(flow)
-    flow = _contig(flow.detach())
+    """model_dfpn.py:269-272: flow (B,F,H,W,2) -> (B,1,F,H,W) fp32; under autocast the flow may be in its dtype."""
+    _need_cuda((flow, _train_dtypes()))
+    flow = _flow_pairs(flow.detach())
     b, f, h, w, _ = flow.shape
     out = _empty((b, 1, f, h, w), dtype=torch.float32, device=flow.device)
-    _call("mt_mask_out", _ptr(flow), flow.numel() // 2, _ptr(out), _stream(flow))
+    _call_net("mt_mask_out", _Net(flow), flow.numel() // 2, _ptr(out), _stream(flow))
     return out
 
 
@@ -518,13 +549,14 @@ def chn_l1_terms(y_target, v_target, y_hat, y_hat_comp, v_map, weights=(0.5, 2.0
 def warp_l1_fwd_raw(x_refs, vis, flow, x_target, v_target, weight=1.0, materialize=False,
                     flags=ALIGN_CORNERS):
     """mt_warp_l1_fwd without autograd.  Returns (out3, x_aligned | None, v_aligned | None, saved)
-    where out3 = [loss, sum|.|, sum(mask)] on the device and ``saved`` feeds warp_l1_bwd_raw."""
-    _need_cuda(x_refs, vis if materialize else None, flow, x_target, v_target)
+    where out3 = [loss, sum|.|, sum(mask)] on the device and ``saved`` feeds warp_l1_bwd_raw.  Under autocast the
+    flow may be in its dtype: every output is the fp32 op's on ``flow.float()``."""
+    _need_cuda(x_refs, vis if materialize else None, (flow, _train_dtypes()), x_target, v_target)
     b, c, f, h, w = x_refs.shape
     if c != 3:
         raise RuntimeError("warp_masked_l1: C must be 3")
     x, x_sb, x_sc, x_sf = _s5(x_refs)
-    flow_c = _contig(flow.detach())
+    flow_c = _flow_pairs(flow.detach())
     xt = _planes(x_target)
     vt = _planes(v_target)
     out3 = _empty(3, dtype=torch.float32, device=x.device)
@@ -534,7 +566,7 @@ def warp_l1_fwd_raw(x_refs, vis, flow, x_target, v_target, weight=1.0, materiali
         xa_mem, xa = _frame_major(b, 3, f, h, w, x)
         va = _empty((b, 1, f, h, w), dtype=torch.float32, device=x.device)
         vis_t, v_sb, _, v_sf = _s5(vis)
-    _call("mt_warp_l1_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis_t), v_sb, v_sf, _ptr(flow_c),
+    _call_net("mt_warp_l1_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis_t), v_sb, v_sf, _Net(flow_c),
               _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0), _ptr(xa_mem),
               _ptr(va), _ptr(out3), _ptr(reduce_workspace(x)), b, f, h, w, float(weight),
               flags, _stream(x))
@@ -543,11 +575,11 @@ def warp_l1_fwd_raw(x_refs, vis, flow, x_target, v_target, weight=1.0, materiali
 
 
 def warp_l1_bwd_raw(saved, grad_out):
-    """mt_warp_l1_bwd: d loss / d flow (B,F,H,W,2); grad_out is a 1-element device tensor."""
+    """mt_warp_l1_bwd: d loss / d flow (B,F,H,W,2) in the flow's dtype; grad_out is a 1-element device tensor."""
     x, flow, xt, vt, out3, (x_sb, x_sc, x_sf, b, f, h, w, weight, flags) = saved
     _device[0] = x.device.index
     gflow = _empty_like(flow)
-    _call("mt_warp_l1_bwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(flow), _ptr(xt), xt.stride(0),
+    _call_net("mt_warp_l1_bwd", _ptr(x), x_sb, x_sc, x_sf, _Net(flow), _ptr(xt), xt.stride(0),
               xt.stride(1), _ptr(vt), vt.stride(0), _ptr(out3), _ptr(grad_out), _ptr(gflow), b, f, h, w,
               weight, flags, _stream(x))
     return gflow
@@ -654,14 +686,24 @@ def corr4d_vgg(feats_t, m_target, feats_r, m_refs):
 
 def corr4d_l1_fwd_raw(pred, feats_t, feats_r, m_target=None, m_refs=None, want_sign=True):
     """mean |pred - corr4d_vgg(feats_t, m_target, feats_r, m_refs)| with the volume kept on chip
-    (model_dfpn.py:254-257).  -> (loss 0-d tensor, sign int8 (B,F,h,w,h,w) or None)."""
-    _need_cuda(feats_t, m_target, feats_r, m_refs, pred)
+    (model_dfpn.py:254-257).  -> (loss 0-d tensor, sign int8 (B,F,h,w,h,w) or None).
+
+    Under autocast pred and the features may be in its dtype, all three in one: the volume is rounded to that dtype as
+    corr4d_vgg returns it, and compared with pred in fp32 (l1_loss is on autocast's fp32 list); the loss is fp32."""
+    td = _train_dtypes()
+    _need_cuda((feats_t, td), m_target, (feats_r, td), m_refs, (pred, td))
+    if not feats_t.dtype == feats_r.dtype == pred.dtype:
+        raise RuntimeError("corr4d_l1: pred, feats_t and feats_r must have one dtype, got %s, %s and %s"
+                           % (pred.dtype, feats_t.dtype, feats_r.dtype))
     b, c, f, h, w = feats_r.shape
     if tuple(pred.shape) != (b, f, h, w, h, w):
         raise ValueError("corr4d_l1: pred must be (B,F,h,w,h,w) = %s, got %s" % ((b, f, h, w, h, w), tuple(pred.shape)))
+    if feats_r.dtype != torch.float32 and c % 64:
+        raise RuntimeError("corr4d_l1: (C=%d, h*w=%d) is not served by the tensor-core kernel" % (c, h * w))
+    es = feats_r.element_size()
 
-    def ok(t, lead):
-        return all(t.size(d) == 1 or (t.stride(d) > 0 and t.stride(d) % 4 == 0) for d in range(lead)) and \
+    def ok(t, lead):       # strides the tensor map can encode: positive multiples of 16 B, plane contiguous
+        return all(t.size(d) == 1 or (t.stride(d) > 0 and t.stride(d) * es % 16 == 0) for d in range(lead)) and \
             t.stride(-1) == 1 and t.stride(-2) == w and t.data_ptr() % 16 == 0
     ft = feats_t if ok(feats_t, 2) else _contig(feats_t)
     fr = feats_r if ok(feats_r, 3) else _contig(feats_r)
@@ -676,19 +718,20 @@ def corr4d_l1_fwd_raw(pred, feats_t, feats_r, m_target=None, m_refs=None, want_s
     loss = _empty((), dtype=torch.float32, device=fr.device)
     sign = _empty(pr.shape, dtype=torch.int8, device=fr.device) if want_sign else None
     ws = zeroed_scratch(fr, "corr_l1", int(_lib.load().mt_corr4d_l1_workspace_bytes()))
-    _call("mt_corr4d_vgg_l1_fwd", _ptr(ft), ft.stride(0), ft.stride(1), _ptr(mt), mt_sb, _ptr(fr), fr.stride(0),
-          fr.stride(1), fr.stride(2), _ptr(mr), mr_sb, mr_sf, MH, MW, _ptr(pr), _ptr(loss), _ptr(sign), _ptr(ws),
-          ws.numel(), b, c, f, h, w, _stream(fr))
+    _call_net("mt_corr4d_vgg_l1_fwd", _Net(ft), ft.stride(0), ft.stride(1), _ptr(mt), mt_sb, _Net(fr), fr.stride(0),
+              fr.stride(1), fr.stride(2), _ptr(mr), mr_sb, mr_sf, MH, MW, _Net(pr), _ptr(loss), _ptr(sign), _ptr(ws),
+              ws.numel(), b, c, f, h, w, _stream(fr))
     return loss, sign
 
 
 class Corr4dL1Fn(torch.autograd.Function):
-    """F.l1_loss(pred, correlation of the ground-truth features) with autograd w.r.t. ``pred``."""
+    """F.l1_loss(pred, correlation of the ground-truth features) with autograd w.r.t. ``pred`` (the gradient in the
+    dtype of ``pred``)."""
 
     @staticmethod
     def forward(ctx, pred, feats_t, feats_r):
         loss, sign = corr4d_l1_fwd_raw(pred.detach(), feats_t, feats_r, want_sign=ctx.needs_input_grad[0])
-        ctx.sign = sign
+        ctx.sign, ctx.dtype = sign, pred.dtype
         return loss
 
     @staticmethod
@@ -696,11 +739,11 @@ class Corr4dL1Fn(torch.autograd.Function):
         sign = ctx.sign
         if sign is None:
             return None, None, None
-        gp = _empty(sign.shape, dtype=torch.float32, device=sign.device)
+        gp = _empty(sign.shape, dtype=ctx.dtype, device=sign.device)
         gg = _contig(g.to(torch.float32))
         _need_cuda(gg)
         _lib.keep(gg)
-        _call("mt_corr4d_l1_bwd", _ptr(sign), _ptr(gg), _ptr(gp), sign.numel(), _stream(sign))
+        _call_net("mt_corr4d_l1_bwd", _ptr(sign), _ptr(gg), _Net(gp), sign.numel(), _stream(sign))
         return gp, None, None
 
 
@@ -1029,13 +1072,14 @@ def resize_flow_raw(flow, size, mode):
     return out
 
 
-def resize_flow_bwd_raw(g_out, h, w):
-    """mt_resize_flow_bwd: d loss / d flow (B,F,h,w,2) of the bilinear resize, as a view of planar memory."""
+def resize_flow_bwd_raw(g_out, h, w, dtype=torch.float32):
+    """mt_resize_flow_bwd: d loss / d flow (B,F,h,w,2) of the bilinear resize, as a view of planar memory, in ``dtype``
+    (the input flow's: a half flow's gradient is the fp32 one rounded to its dtype)."""
     _need_cuda(g_out)
     b, f, H, W, _ = g_out.shape
-    g_flow = _empty((b, f, 2, h, w), dtype=torch.float32, device=g_out.device)
-    _call("mt_resize_flow_bwd", _ptr(_lib.keep(g_out)), *g_out.stride(), _ptr(g_flow), b, f, h, w, H, W,
-          _stream(g_out))
+    g_flow = _empty((b, f, 2, h, w), dtype=dtype, device=g_out.device)
+    _call_net("mt_resize_flow_bwd", _ptr(_lib.keep(g_out)), *g_out.stride(), _Net(g_flow), b, f, h, w, H, W,
+              _stream(g_out))
     return g_flow.permute(0, 1, 3, 4, 2)
 
 
@@ -1044,21 +1088,21 @@ class ResizeFlowFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, flow, size):
-        _need_cuda(flow)        # the gradient path (DFPN training) is fp32
-        ctx.hw = flow.shape[2:4]
+        _need_cuda((flow, _train_dtypes()))     # DFPN training: a half flow under autocast only
+        ctx.hw, ctx.dtype = flow.shape[2:4], flow.dtype
         return resize_flow_raw(flow.detach(), size, "bilinear")
 
     @staticmethod
     def backward(ctx, g):
         if not ctx.needs_input_grad[0]:
             return None, None
-        return resize_flow_bwd_raw(g.to(torch.float32), *ctx.hw), None
+        return resize_flow_bwd_raw(g.to(torch.float32), *ctx.hw, ctx.dtype), None
 
 
 def resize_flow(flow, size, mode="nearest"):
     """FlowsUtils.resize_flow (utils.py:107-126): (B,F,h,w,2) -> (B,F,H,W,2), mode 'nearest' or 'bilinear'
     (align_corners=False); differentiable w.r.t. ``flow`` in the bilinear mode.  Without a gradient the flow may be
-    fp16 / bf16; the result is fp32."""
+    fp16 / bf16, with one under autocast only (its gradient then has the flow's dtype); the result is fp32."""
     if mode not in RESIZE_MODES:
         raise ValueError("resize_flow: mode must be one of %s, got %r" % (sorted(RESIZE_MODES), mode))
     if torch.is_grad_enabled() and flow.requires_grad:

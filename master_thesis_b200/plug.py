@@ -53,12 +53,11 @@ class FlowsUtils:
         """utils.py:107-126.  flow (B,F,h,w,2) -> (B,F,H,W,2), F.interpolate 'nearest' or 'bilinear'
         (align_corners=False), bit-identical; differentiable w.r.t. flow in the bilinear mode.  CUDA fp32 flows in
         those two modes (and nearest without a gradient) run on the kernel, anything else on the reference's own
-        function.  Under autocast a half flow without a gradient (the frozen DFPN aligner's) runs on the kernel
-        too and becomes fp32, as F.interpolate's fp32 autocast policy makes it."""
+        function.  Under autocast a half flow in its dtype (the frozen DFPN aligner's, or the mixer's and flow
+        estimators' in DFPN training, model_dfpn.py:86, 93) runs on the kernel the same way and becomes fp32, as
+        F.interpolate's fp32 autocast policy makes it; its gradient has the flow's dtype."""
         grad = torch.is_grad_enabled() and isinstance(flow, torch.Tensor) and flow.requires_grad
-        if _cuda_fp32(flow) and (mode == 'bilinear' or (mode == 'nearest' and not grad)):
-            return ops.resize_flow(flow, size, mode)
-        if _cuda_autocast_half(flow) and mode in ('bilinear', 'nearest') and not grad:
+        if (_cuda_fp32(flow) or _cuda_autocast_half(flow)) and (mode == 'bilinear' or (mode == 'nearest' and not grad)):
             return ops.resize_flow(flow, size, mode)
         return _reference_original("FlowsUtils", "resize_flow")(flow, size, mode)
 
@@ -217,16 +216,21 @@ class DeferredAlign(object):
     ``FlowsUtils.align_set(x_refs, v_refs, flow)`` (model_dfpn.py:377-385) whose result has not been computed.
     The patched ``DFPN.compute_loss`` feeds them to the fused warp + mask_out + masked-L1 kernel, so the
     aligned frames of the training step are never written to HBM.  Anything else that touches the object
-    (attribute access, torch functions) gets the materialised ``x_aligned`` tensor."""
+    (attribute access, torch functions) gets the materialised ``x_aligned`` tensor.  The reference runs
+    ``align_set`` inside ``_train_val_wrapper``, under the autocast state of the step (``--precision 16|bf16``: a
+    half flow); the handle records that state and materialises under it, wherever it is touched."""
 
     def __init__(self, x_refs, v_refs, flow):
         self.x_refs, self.v_refs, self.flow = x_refs, v_refs, flow
+        self._autocast = (torch.is_autocast_enabled("cuda"), torch.get_autocast_dtype("cuda"))
         self._done = None
 
     def materialize(self):
         """(x_aligned, v_aligned) = FlowsUtils.align_set(x_refs, v_refs, flow), differentiable w.r.t. flow."""
         if self._done is None:
-            self._done = ops.align_set(self.x_refs, self.v_refs, self.flow)
+            enabled, dtype = self._autocast
+            with torch.autocast("cuda", dtype=dtype, enabled=enabled):
+                self._done = ops.align_set(self.x_refs, self.v_refs, self.flow)
         return self._done
 
     def __getattr__(self, name):          # only reached for names that are not set in __init__
