@@ -64,6 +64,17 @@ typedef void *mt_stream_t; /* cudaStream_t */
 #define MT_DT_F16 1
 #define MT_DT_BF16 2
 
+/* memory layout of a network operand in the *_layout entry points (the CNN input the packs write, the CNN output the
+ * composite / fill kernels read and the gradient written for it), shape (N, C, H, W) in both:
+ *   MT_LAYOUT_NCHW  planar: channel stride H*W, pixel stride 1 (the reference's default)
+ *   MT_LAYOUT_NHWC  channels-last: channel stride 1, pixel stride C (torch.channels_last), the layout cuDNN's half
+ *                   convolutions work in.  A network converted with model.to(memory_format=torch.channels_last)
+ *                   takes and returns it; handing it over as is saves a layout copy on each side.
+ * Values are the same in both: only where each element is stored differs.  Any other code is rejected with
+ * MT_ERR_INVALID. */
+#define MT_LAYOUT_NCHW 0
+#define MT_LAYOUT_NHWC 1
+
 MT_API int mt_version(void);
 MT_API const char *mt_last_error(void);
 /* developer knob (tests, sweeps): overrides one of the MT_* tuning variables the library
@@ -470,7 +481,7 @@ MT_API const float *mt_cm_workspace_gs(const void *workspace, int B, int C, int 
 /* ---- K4  CHN pack / composite / hole update ------------------------------
  * mt_chn_pack         replaces CHN.forward model_chn.py:68-80           (a9)
  *   x_t (B,3,H,W), v_t (B,1,H,W), x_al (B,3,F,H,W) strided, v_al, v_map
- *   (B,1,F,H,W) strided -> nn_in (B*F,9,H,W) contiguous NCHW for cuDNN.
+ *   (B,1,F,H,W) strided -> nn_in (B*F,9,H,W) contiguous NCHW for cuDNN (NHWC: mt_chn_pack_layout).
  * mt_chn_composite_fwd replaces model_chn.py:80-85                      (a10)
  *   nn_out (B*F,3,H,W) -> y_hat, y_comp as frame-major (B,F,3,H,W).
  * mt_chn_composite_bwd: g_nn (B*F,3,H,W) from grads of both outputs
@@ -515,7 +526,8 @@ MT_API int mt_trivial_copy(const float *x_t, int64_t xt_sb, int64_t xt_sc,
  * mt_flow_pack        replaces FlowEstimator.forward model_dfpn.py:733-741   (SURVEY 8f-4)
  *   x_refs (B,3,F,H,W) strided, x_t (B,3,H,W) strided, m_refs (B,1,F,H,W) strided, m_t (B,1,H,W),
  *   flow (B,F,H,W,2) with ALL five strides (element units; FlowsUtils.resize_flow hands over a
- *   permuted view of a (B,F,2,H,W) tensor) -> nn_in (B*F,10,H,W) contiguous NCHW for cuDNN:
+ *   permuted view of a (B,F,2,H,W) tensor) -> nn_in (B*F,10,H,W) contiguous NCHW for cuDNN (NHWC:
+ *   mt_flow_pack_layout):
  *   channels [x_refs 0-2, x_t 3-5, m_refs 6, m_t 7, flow x 8, flow y 9].  Planes of x / m must be
  *   contiguous (stride W, 1).  Pure data movement; the gradient of flow is the view
  *   g_nn_in[:, 8:10] -> (B,F,H,W,2) (no kernel needed).
@@ -583,6 +595,70 @@ MT_API int mt_cpn_align_host(const float *x_refs, const float *m_refs, const flo
 MT_API int mt_dfpn_align_host(const float *x_refs, const float *m_refs, const float *m_target,
                        const float *flow, float *x_aligned, float *v_aligned, float *v_maps,
                        int B, int F, int H, int W);
+
+/* ---- channels-last networks ---------------------------------------------------
+ * The general forms of the entry points that hand a tensor to a network or take one from it: the layout code
+ * nn_layout (MT_LAYOUT_*) of that operand comes first, then the arguments of the entry point named (its _dt form where
+ * there is one).  Every other operand keeps its layout.  The planar entry points are these with MT_LAYOUT_NCHW.
+ * A channels-last nn_in / nn_out / g_nn is the contiguous (N, H, W, C) memory of the (N, C, H, W) tensor. */
+/* mt_chn_pack: nn_in (B*F, 9, H, W) in nn_layout                                      CHN.forward model_chn.py:68-80 */
+MT_API int mt_chn_pack_layout(int nn_layout, const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t,
+                       int64_t vt_sb, const float *x_al, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                       const float *v_al, int64_t va_sb, int64_t va_sf,
+                       const float *v_map, int64_t vm_sb, int64_t vm_sf,
+                       float *nn_in, int B, int F, int64_t P, mt_stream_t stream);
+/* mt_warp_pack_fwd_dt / mt_warp_pack_lowres_fwd_dt: nn_in (B*F, 9, H, W) in nn_layout
+ *                                              model_chn.py:68-80 after model_dfpn.py:100-101, 128-133 / model_cpn.py:75-89 */
+MT_API int mt_warp_pack_fwd_layout(int nn_layout, const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                            const float *vis, int64_t vis_sb, int64_t vis_sf,
+                            int g_dtype, const void *grid, const float *m_target, int64_t mt_sb,
+                            const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                            float *nn_in,
+                            float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                            float *v_aligned, float *v_map,
+                            int B, int F, int H, int W, int flags, mt_stream_t stream);
+MT_API int mt_warp_pack_lowres_fwd_layout(int nn_layout, const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                   const float *vis, int64_t vis_sb, int64_t vis_sf,
+                                   int g_dtype, const void *flow, int gh, int gw, const float *m_target,
+                                   int64_t mt_sb, const float *x_t, int64_t xt_sb, int64_t xt_sc,
+                                   const float *v_t, int64_t vt_sb, float *nn_in,
+                                   float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                                   float *v_aligned, float *v_map,
+                                   int B, int F, int H, int W, int flags, mt_stream_t stream);
+/* mt_flow_pack: nn_in (B*F, 10, H, W) in nn_layout                      FlowEstimator.forward model_dfpn.py:733-741 */
+MT_API int mt_flow_pack_layout(int nn_layout, const float *x_refs, int64_t xr_sb, int64_t xr_sc, int64_t xr_sf,
+                        const float *x_t, int64_t xt_sb, int64_t xt_sc,
+                        const float *m_refs, int64_t mr_sb, int64_t mr_sf, const float *m_t, int64_t mt_sb,
+                        const float *flow, int64_t fl_sb, int64_t fl_sf, int64_t fl_sy, int64_t fl_sx,
+                        int64_t fl_sc, float *nn_in, int B, int F, int H, int W, mt_stream_t stream);
+/* mt_chn_composite_fwd_dt / _bwd_dt: nn_out (B*F, 3, H, W) and g_nn in nn_layout          model_chn.py:80-85 */
+MT_API int mt_chn_composite_fwd_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                                int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                                float *y_hat, float *y_comp, int B, int F, int64_t P, mt_stream_t stream);
+MT_API int mt_chn_composite_bwd_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *v_t,
+                                int64_t vt_sb, const float *g_yhat, int64_t gy_sb, int64_t gy_sc, int64_t gy_sf,
+                                const float *g_comp, int64_t gc_sb, int64_t gc_sc, int64_t gc_sf,
+                                void *g_nn, int B, int F, int64_t P, mt_stream_t stream);
+/* mt_chn_fill_step_dt / mt_chn_fill_step_gated_dt: nn_out (B, 3, H, W) in nn_layout
+ *                                                                   model_chn.py:80-85, 112, 128-131 */
+MT_API int mt_chn_fill_step_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                            int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                            const float *m_t, int64_t mt_sb, const float *v_map0, int64_t vm_sb,
+                            float *y_comp0, float *m_new, float *x_new, float *inp_per, void *workspace,
+                            int B, int64_t P, mt_stream_t stream);
+MT_API int mt_chn_fill_step_gated_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                                  int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                                  const float *m_t, int64_t mt_sb, const float *v_map0, int64_t vm_sb,
+                                  const float *y_prev, const float *gate_per, float gate_e,
+                                  float *y_comp0, float *m_new, float *x_new, float *inp_per,
+                                  void *workspace, int B, int64_t P, mt_stream_t stream);
+/* mt_chn_fill_lanes_dt: nn_out (L, 3, H, W) in nn_layout                      model_chn.py:83-84, 128-131, 242-248 */
+MT_API int mt_chn_fill_lanes_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                             int64_t xt_sl, int64_t xt_sc, const float *m_t, int64_t mt_sl,
+                             const float *v_map0, int64_t vm_sl, const int *slots, float *y_out,
+                             int64_t yo_ss, int64_t yo_sc, float *m_state, int64_t ms_ss, float *x_state,
+                             int64_t xs_ss, int64_t xs_sc, float *per_out, void *workspace, int L,
+                             int64_t P, int finalize, double e, int force, mt_stream_t stream);
 
 #ifdef __cplusplus
 }

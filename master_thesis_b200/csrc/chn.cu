@@ -30,13 +30,17 @@ struct PackArgs {
     int F; int64_t P;
 };
 
-template <int VEC>
+// NHWC: nn_in is channels-last (pixel stride 9, channel stride 1), written through the CTA's shared-memory stage; the
+// threads past the end of the frame recompute its last pixels into stage slots that are not written out, so that
+// every thread reaches the CTA barrier
+template <int VEC, bool NHWC = false>
 __global__ void __launch_bounds__(256, 4) chn_pack_kernel(const PackArgs a) {
     pdl_sync();
-    const int64_t p0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
-    if (p0 >= a.P) return;
+    const int64_t q0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
+    if (!NHWC && q0 >= a.P) return;
+    const int64_t p0 = NHWC ? min(q0, a.P - VEC) : q0;
     const int n = blockIdx.y, b = n / a.F, f = n - b * a.F;
-    float *o = a.nn_in + (int64_t)n * 9 * a.P + p0;
+    float *o = a.nn_in + (int64_t)n * 9 * a.P + p0;  // planar only
     Vec<VEC> t[3], r[3], vt, va, vm;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
@@ -54,12 +58,23 @@ __global__ void __launch_bounds__(256, 4) chn_pack_kernel(const PackArgs a) {
             t[c].v[i] = __fdiv_rn(__fsub_rn(t[c].v[i], m), s);
             r[c].v[i] = __fdiv_rn(__fsub_rn(r[c].v[i], m), s);
         }
-        t[c].store_stream(o + c * a.P);
-        r[c].store_stream(o + (3 + c) * a.P);
+        if constexpr (!NHWC) {
+            t[c].store_stream(o + c * a.P);
+            r[c].store_stream(o + (3 + c) * a.P);
+        }
     }
-    vt.store_stream(o + 6 * a.P);
-    va.store_stream(o + 7 * a.P);
-    vm.store_stream(o + 8 * a.P);
+    if constexpr (NHWC) {
+        float *stage = nhwc_stage<float, 256 * VEC * 9>();
+        const Vec<VEC> ch[9] = {t[0], t[1], t[2], r[0], r[1], r[2], vt, va, vm};
+        stage_nhwc(stage, ch);
+        __syncthreads();
+        const int64_t pb = (int64_t)blockIdx.x * blockDim.x * VEC;
+        stage_out(a.nn_in + ((int64_t)n * a.P + pb) * 9, stage, (int)(min((int64_t)blockDim.x * VEC, a.P - pb) * 9));
+    } else {
+        vt.store_stream(o + 6 * a.P);
+        va.store_stream(o + 7 * a.P);
+        vm.store_stream(o + 8 * a.P);
+    }
 }
 
 // ---- a10 composite ------------------------------------------------------------
@@ -75,7 +90,8 @@ struct CompArgs {
     int F; int64_t P;
 };
 
-template <typename T, int VEC>
+// NHWC: nn_out (and g_nn) channels-last, (B*F, 3, H, W) with pixel stride 3 and channel stride 1
+template <typename T, int VEC, bool NHWC = false>
 __global__ void __launch_bounds__(256, 4) chn_composite_fwd_kernel(const CompArgs<T> a) {
     pdl_sync();
     const int64_t p0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
@@ -86,9 +102,10 @@ __global__ void __launch_bounds__(256, 4) chn_composite_fwd_kernel(const CompArg
     // all operands of the three channels are requested before the first store (the stores may alias the loads as far
     // as the compiler knows: channel by channel it emitted three dependent round trips)
     Vec<VEC> oo[3], xx[3];
+    if constexpr (NHWC) load_nhwc(oo, a.nn_out + ((int64_t)n * a.P + p0) * 3);
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        oo[c].load_stream(a.nn_out + ((int64_t)n * 3 + c) * a.P + p0);
+        if constexpr (!NHWC) oo[c].load_stream(a.nn_out + ((int64_t)n * 3 + c) * a.P + p0);
         xx[c].load_cached(a.x_t + b * a.xt_sb + c * a.xt_sc + p0);
     }
 #pragma unroll
@@ -107,24 +124,28 @@ __global__ void __launch_bounds__(256, 4) chn_composite_fwd_kernel(const CompArg
     }
 }
 
-template <typename T, int VEC>
+// NHWC: g_nn goes through the CTA's stage; threads past the end of the frame recompute its last pixels into slots that
+// are not written out (every thread reaches the barrier)
+template <typename T, int VEC, bool NHWC = false>
 __global__ void __launch_bounds__(256, 4) chn_composite_bwd_kernel(const CompArgs<T> a) {
     pdl_sync();
-    const int64_t p0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
-    if (p0 >= a.P) return;
+    const int64_t q0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
+    if (!NHWC && q0 >= a.P) return;
+    const int64_t p0 = NHWC ? min(q0, a.P - VEC) : q0;
     const int n = blockIdx.y, b = n / a.F, f = n - b * a.F;
     Vec<VEC> vt;
     vt.load_cached(a.v_t + b * a.vt_sb + p0);
     Vec<VEC> oo[3], gyy[3], gcc[3];  // every load before the first store, as in the forward kernel
+    if constexpr (NHWC) load_nhwc(oo, a.nn_out + ((int64_t)n * a.P + p0) * 3);
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        oo[c].load_stream(a.nn_out + ((int64_t)n * 3 + c) * a.P + p0);
+        if constexpr (!NHWC) oo[c].load_stream(a.nn_out + ((int64_t)n * 3 + c) * a.P + p0);
         if (a.g_yhat) gyy[c].load_stream(a.g_yhat + b * a.gy_sb + c * a.gy_sc + f * a.gy_sf + p0);
         if (a.g_comp) gcc[c].load_stream(a.g_comp + b * a.gc_sb + c * a.gc_sc + f * a.gc_sf + p0);
     }
+    Vec<VEC> g[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        Vec<VEC> g;
         const Vec<VEC> &o = oo[c], &gy = gyy[c], &gc = gcc[c];
         const float m = chan_mean(c), s = chan_std(c);
 #pragma unroll
@@ -133,9 +154,16 @@ __global__ void __launch_bounds__(256, 4) chn_composite_bwd_kernel(const CompArg
             float gg = 0.0f;
             if (a.g_yhat) gg = gy.v[i];
             if (a.g_comp) gg = __fadd_rn(gg, __fmul_rn(__fsub_rn(1.0f, vt.v[i]), gc.v[i]));
-            g.v[i] = (pre >= 0.0f && pre <= 1.0f) ? __fmul_rn(gg, s) : 0.0f;  // clamp passes grad on [0,1]
+            g[c].v[i] = (pre >= 0.0f && pre <= 1.0f) ? __fmul_rn(gg, s) : 0.0f;  // clamp passes grad on [0,1]
         }
-        g.store_stream(a.g_nn + ((int64_t)n * 3 + c) * a.P + p0);
+        if constexpr (!NHWC) g[c].store_stream(a.g_nn + ((int64_t)n * 3 + c) * a.P + p0);
+    }
+    if constexpr (NHWC) {
+        T *stage = nhwc_stage<T, 256 * VEC * 3>();
+        stage_nhwc(stage, g);
+        __syncthreads();
+        const int64_t pb = (int64_t)blockIdx.x * blockDim.x * VEC;
+        stage_out(a.g_nn + ((int64_t)n * a.P + pb) * 3, stage, (int)(min((int64_t)blockDim.x * VEC, a.P - pb) * 3));
     }
 }
 
@@ -201,7 +229,7 @@ struct FillArgs {
     const float *gate_per, *y_prev; float gate_e;
 };
 
-template <typename T, int VEC>
+template <typename T, int VEC, bool NHWC = false>  // NHWC: nn_out channels-last
 __global__ void __launch_bounds__(256) chn_fill_kernel(const FillArgs<T> a) {
     pdl_sync();
     __shared__ float red[32];
@@ -234,9 +262,10 @@ __global__ void __launch_bounds__(256) chn_fill_kernel(const FillArgs<T> a) {
         vt.load_stream(a.v_t + b * a.vt_sb + p0);
         m.load_stream(a.m_t + b * a.mt_sb + p0);
         vm.load_stream(a.v_map0 + b * a.vm_sb + p0);
+        if constexpr (NHWC) load_nhwc(o, a.nn_out + ((int64_t)b * a.P + p0) * 3);
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            o[c].load_stream(a.nn_out + ((int64_t)b * 3 + c) * a.P + p0);
+            if constexpr (!NHWC) o[c].load_stream(a.nn_out + ((int64_t)b * 3 + c) * a.P + p0);
             xt[c].load_stream(a.x_t + b * a.xt_sb + c * a.xt_sc + p0);
         }
 #pragma unroll
@@ -560,44 +589,67 @@ int reduce_blocks(int64_t total) {
 
 using namespace mt;
 
+extern "C" int mt_chn_pack_layout(int nn_layout, const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t,
+                                  int64_t vt_sb, const float *x_al, int64_t xa_sb, int64_t xa_sc,
+                                  int64_t xa_sf, const float *v_al, int64_t va_sb, int64_t va_sf,
+                                  const float *v_map, int64_t vm_sb, int64_t vm_sf, float *nn_in, int B,
+                                  int F, int64_t P, mt_stream_t stream) {
+    MT_REQUIRE(x_t && v_t && x_al && v_al && v_map && nn_in, "mt_chn_pack: NULL argument");
+    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_pack: bad shape");
+    return with_layout(nn_layout, "mt_chn_pack", [&](auto nhwc) {
+        constexpr bool L = decltype(nhwc)::value;
+        PackArgs a{x_t, xt_sb, xt_sc, v_t, vt_sb, x_al, xa_sb, xa_sc, xa_sf, v_al, va_sb, va_sf,
+                   v_map, vm_sb, vm_sf, nn_in, F, P};
+        bool v4 = mult4(P) && aligned16(x_t) && aligned16(v_t) && aligned16(x_al) && aligned16(v_al) &&
+                  aligned16(v_map) && aligned16(nn_in) && mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb) &&
+                  mult4(xa_sb) && mult4(xa_sc) && mult4(xa_sf) && mult4(va_sb) && mult4(va_sf) &&
+                  mult4(vm_sb) && mult4(vm_sf);
+        const int vec = v4 ? 4 : 1;
+        dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
+        if (v4) launch(chn_pack_kernel<4, L>, grid, 256, 0, (cudaStream_t)stream, a);
+        else launch(chn_pack_kernel<1, L>, grid, 256, 0, (cudaStream_t)stream, a);
+        return launch_status("mt_chn_pack");
+    });
+}
+
 extern "C" int mt_chn_pack(const float *x_t, int64_t xt_sb, int64_t xt_sc, const float *v_t,
                            int64_t vt_sb, const float *x_al, int64_t xa_sb, int64_t xa_sc,
                            int64_t xa_sf, const float *v_al, int64_t va_sb, int64_t va_sf,
                            const float *v_map, int64_t vm_sb, int64_t vm_sf, float *nn_in, int B,
                            int F, int64_t P, mt_stream_t stream) {
-    MT_REQUIRE(x_t && v_t && x_al && v_al && v_map && nn_in, "mt_chn_pack: NULL argument");
-    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_pack: bad shape");
-    PackArgs a{x_t, xt_sb, xt_sc, v_t, vt_sb, x_al, xa_sb, xa_sc, xa_sf, v_al, va_sb, va_sf,
-               v_map, vm_sb, vm_sf, nn_in, F, P};
-    bool v4 = mult4(P) && aligned16(x_t) && aligned16(v_t) && aligned16(x_al) && aligned16(v_al) &&
-              aligned16(v_map) && aligned16(nn_in) && mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb) &&
-              mult4(xa_sb) && mult4(xa_sc) && mult4(xa_sf) && mult4(va_sb) && mult4(va_sf) &&
-              mult4(vm_sb) && mult4(vm_sf);
-    const int vec = v4 ? 4 : 1;
-    dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
-    if (v4) launch(chn_pack_kernel<4>, grid, 256, 0, (cudaStream_t)stream, a);
-    else launch(chn_pack_kernel<1>, grid, 256, 0, (cudaStream_t)stream, a);
-    return launch_status("mt_chn_pack");
+    return mt_chn_pack_layout(MT_LAYOUT_NCHW, x_t, xt_sb, xt_sc, v_t, vt_sb, x_al, xa_sb, xa_sc, xa_sf, v_al, va_sb,
+                              va_sf, v_map, vm_sb, vm_sf, nn_in, B, F, P, stream);
+}
+
+extern "C" int mt_chn_composite_fwd_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                                           int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                                           float *y_hat, float *y_comp, int B, int F, int64_t P,
+                                           mt_stream_t stream) {
+    MT_REQUIRE(nn_out && x_t && v_t && y_hat && y_comp, "mt_chn_composite_fwd: NULL argument");
+    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_fwd: bad shape");
+    return with_layout(nn_layout, "mt_chn_composite_fwd", [&](auto nhwc) {
+        constexpr bool L = decltype(nhwc)::value;
+        return with_dtype(nn_dtype, "mt_chn_composite_fwd", [&](auto tag) {
+            using T = decltype(tag);
+            CompArgs<T> a{};
+            a.nn_out = static_cast<const T *>(nn_out); a.x_t = x_t; a.xt_sb = xt_sb; a.xt_sc = xt_sc; a.v_t = v_t;
+            a.vt_sb = vt_sb; a.y_hat = y_hat; a.y_comp = y_comp; a.F = F; a.P = P;
+            bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(y_hat) &&
+                      aligned16(y_comp) && mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb);
+            const int vec = v4 ? 4 : 1;
+            dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
+            if (v4) launch(chn_composite_fwd_kernel<T, 4, L>, grid, 256, 0, (cudaStream_t)stream, a);
+            else launch(chn_composite_fwd_kernel<T, 1, L>, grid, 256, 0, (cudaStream_t)stream, a);
+            return launch_status("mt_chn_composite_fwd");
+        });
+    });
 }
 
 extern "C" int mt_chn_composite_fwd_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
                                        int64_t xt_sc, const float *v_t, int64_t vt_sb, float *y_hat,
                                        float *y_comp, int B, int F, int64_t P, mt_stream_t stream) {
-    MT_REQUIRE(nn_out && x_t && v_t && y_hat && y_comp, "mt_chn_composite_fwd: NULL argument");
-    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_fwd: bad shape");
-    return with_dtype(nn_dtype, "mt_chn_composite_fwd", [&](auto tag) {
-        using T = decltype(tag);
-        CompArgs<T> a{};
-        a.nn_out = static_cast<const T *>(nn_out); a.x_t = x_t; a.xt_sb = xt_sb; a.xt_sc = xt_sc; a.v_t = v_t;
-        a.vt_sb = vt_sb; a.y_hat = y_hat; a.y_comp = y_comp; a.F = F; a.P = P;
-        bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(y_hat) &&
-                  aligned16(y_comp) && mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb);
-        const int vec = v4 ? 4 : 1;
-        dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
-        if (v4) launch(chn_composite_fwd_kernel<T, 4>, grid, 256, 0, (cudaStream_t)stream, a);
-        else launch(chn_composite_fwd_kernel<T, 1>, grid, 256, 0, (cudaStream_t)stream, a);
-        return launch_status("mt_chn_composite_fwd");
-    });
+    return mt_chn_composite_fwd_layout(MT_LAYOUT_NCHW, nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, y_hat, y_comp,
+                                       B, F, P, stream);
 }
 
 extern "C" int mt_chn_composite_fwd(const float *nn_out, const float *x_t, int64_t xt_sb,
@@ -606,27 +658,38 @@ extern "C" int mt_chn_composite_fwd(const float *nn_out, const float *x_t, int64
     return mt_chn_composite_fwd_dt(MT_DT_F32, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, y_hat, y_comp, B, F, P, stream);
 }
 
+extern "C" int mt_chn_composite_bwd_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *v_t,
+                                           int64_t vt_sb, const float *g_yhat, int64_t gy_sb, int64_t gy_sc,
+                                           int64_t gy_sf, const float *g_comp, int64_t gc_sb, int64_t gc_sc,
+                                           int64_t gc_sf, void *g_nn, int B, int F, int64_t P, mt_stream_t stream) {
+    MT_REQUIRE(nn_out && v_t && g_nn, "mt_chn_composite_bwd: NULL argument");
+    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_bwd: bad shape");
+    return with_layout(nn_layout, "mt_chn_composite_bwd", [&](auto nhwc) {
+        constexpr bool L = decltype(nhwc)::value;
+        return with_dtype(nn_dtype, "mt_chn_composite_bwd", [&](auto tag) {
+            using T = decltype(tag);
+            CompArgs<T> a{};
+            a.nn_out = static_cast<const T *>(nn_out); a.v_t = v_t; a.vt_sb = vt_sb; a.g_yhat = g_yhat;
+            a.gy_sb = gy_sb; a.gy_sc = gy_sc; a.gy_sf = gy_sf; a.g_comp = g_comp; a.gc_sb = gc_sb; a.gc_sc = gc_sc;
+            a.gc_sf = gc_sf; a.g_nn = static_cast<T *>(g_nn); a.F = F; a.P = P;
+            bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(v_t) && aligned16(g_yhat) &&
+                      aligned16(g_comp) && aligned_vec4<T>(g_nn) && mult4(vt_sb) && mult4(gy_sb) && mult4(gy_sc) &&
+                      mult4(gy_sf) && mult4(gc_sb) && mult4(gc_sc) && mult4(gc_sf);
+            const int vec = v4 ? 4 : 1;
+            dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
+            if (v4) launch(chn_composite_bwd_kernel<T, 4, L>, grid, 256, 0, (cudaStream_t)stream, a);
+            else launch(chn_composite_bwd_kernel<T, 1, L>, grid, 256, 0, (cudaStream_t)stream, a);
+            return launch_status("mt_chn_composite_bwd");
+        });
+    });
+}
+
 extern "C" int mt_chn_composite_bwd_dt(int nn_dtype, const void *nn_out, const float *v_t, int64_t vt_sb,
                                        const float *g_yhat, int64_t gy_sb, int64_t gy_sc, int64_t gy_sf,
                                        const float *g_comp, int64_t gc_sb, int64_t gc_sc, int64_t gc_sf,
                                        void *g_nn, int B, int F, int64_t P, mt_stream_t stream) {
-    MT_REQUIRE(nn_out && v_t && g_nn, "mt_chn_composite_bwd: NULL argument");
-    MT_REQUIRE(B > 0 && F > 0 && P > 0 && (int64_t)B * F <= 65535, "mt_chn_composite_bwd: bad shape");
-    return with_dtype(nn_dtype, "mt_chn_composite_bwd", [&](auto tag) {
-        using T = decltype(tag);
-        CompArgs<T> a{};
-        a.nn_out = static_cast<const T *>(nn_out); a.v_t = v_t; a.vt_sb = vt_sb; a.g_yhat = g_yhat; a.gy_sb = gy_sb;
-        a.gy_sc = gy_sc; a.gy_sf = gy_sf; a.g_comp = g_comp; a.gc_sb = gc_sb; a.gc_sc = gc_sc;
-        a.gc_sf = gc_sf; a.g_nn = static_cast<T *>(g_nn); a.F = F; a.P = P;
-        bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(v_t) && aligned16(g_yhat) && aligned16(g_comp) &&
-                  aligned_vec4<T>(g_nn) && mult4(vt_sb) && mult4(gy_sb) && mult4(gy_sc) && mult4(gy_sf) &&
-                  mult4(gc_sb) && mult4(gc_sc) && mult4(gc_sf);
-        const int vec = v4 ? 4 : 1;
-        dim3 grid((unsigned)((P + 256 * vec - 1) / (256 * vec)), B * F);
-        if (v4) launch(chn_composite_bwd_kernel<T, 4>, grid, 256, 0, (cudaStream_t)stream, a);
-        else launch(chn_composite_bwd_kernel<T, 1>, grid, 256, 0, (cudaStream_t)stream, a);
-        return launch_status("mt_chn_composite_bwd");
-    });
+    return mt_chn_composite_bwd_layout(MT_LAYOUT_NCHW, nn_dtype, nn_out, v_t, vt_sb, g_yhat, gy_sb, gy_sc, gy_sf,
+                                       g_comp, gc_sb, gc_sc, gc_sf, g_nn, B, F, P, stream);
 }
 
 extern "C" int mt_chn_composite_bwd(const float *nn_out, const float *v_t, int64_t vt_sb,
@@ -870,8 +933,8 @@ extern "C" int mt_chn_l1x3_bwd(const float *y_hat, int64_t yh_sb, int64_t yh_sc,
     return launch_status("mt_chn_l1x3_bwd");
 }
 
-static int chn_fill_impl(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
-                         const float *v_t, int64_t vt_sb, const float *m_t, int64_t mt_sb,
+static int chn_fill_impl(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
+                         int64_t xt_sc, const float *v_t, int64_t vt_sb, const float *m_t, int64_t mt_sb,
                          const float *v_map0, int64_t vm_sb, const float *y_prev, const float *gate_per,
                          float gate_e, float *y_comp0, float *m_new, float *x_new, float *inp_per,
                          void *workspace, int B, int64_t P, mt_stream_t stream) {
@@ -880,21 +943,34 @@ static int chn_fill_impl(int nn_dtype, const void *nn_out, const float *x_t, int
     MT_REQUIRE(B > 0 && P > 0, "mt_chn_fill_step: bad shape");
     MT_REQUIRE(!gate_per || y_prev, "mt_chn_fill_step_gated: a gate needs the previous step's y_comp0");
     MT_REQUIRE(inp_per != gate_per && y_prev != y_comp0, "mt_chn_fill_step_gated: outputs must not alias the gate inputs");
-    return with_dtype(nn_dtype, "mt_chn_fill_step", [&](auto tag) {
-        using T = decltype(tag);
-        FillArgs<T> a{static_cast<const T *>(nn_out), x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb,
-                      y_comp0, m_new, x_new, inp_per, workspace, B, P, 0, 0, gate_per, y_prev, gate_e};
-        bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(m_t) &&
-                  aligned16(v_map0) && aligned16(y_comp0) && aligned16(m_new) && aligned16(x_new) && mult4(xt_sb) &&
-                  mult4(xt_sc) && mult4(vt_sb) && mult4(mt_sb) && mult4(vm_sb) && aligned16(y_prev);
-        const int vec = v4 ? 4 : 1;
-        a.chunks = (int)((P + 256 * vec - 1) / (256 * vec));
-        a.total_chunks = (int64_t)B * a.chunks;
-        const int nblk = reduce_blocks(a.total_chunks);
-        if (v4) launch(chn_fill_kernel<T, 4>, nblk, 256, 0, (cudaStream_t)stream, a);
-        else launch(chn_fill_kernel<T, 1>, nblk, 256, 0, (cudaStream_t)stream, a);
-        return launch_status("mt_chn_fill_step");
+    return with_layout(nn_layout, "mt_chn_fill_step", [&](auto nhwc) {
+        constexpr bool L = decltype(nhwc)::value;
+        return with_dtype(nn_dtype, "mt_chn_fill_step", [&](auto tag) {
+            using T = decltype(tag);
+            FillArgs<T> a{static_cast<const T *>(nn_out), x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb,
+                          y_comp0, m_new, x_new, inp_per, workspace, B, P, 0, 0, gate_per, y_prev, gate_e};
+            bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(v_t) && aligned16(m_t) &&
+                      aligned16(v_map0) && aligned16(y_comp0) && aligned16(m_new) && aligned16(x_new) &&
+                      mult4(xt_sb) && mult4(xt_sc) && mult4(vt_sb) && mult4(mt_sb) && mult4(vm_sb) &&
+                      aligned16(y_prev);
+            const int vec = v4 ? 4 : 1;
+            a.chunks = (int)((P + 256 * vec - 1) / (256 * vec));
+            a.total_chunks = (int64_t)B * a.chunks;
+            const int nblk = reduce_blocks(a.total_chunks);
+            if (v4) launch(chn_fill_kernel<T, 4, L>, nblk, 256, 0, (cudaStream_t)stream, a);
+            else launch(chn_fill_kernel<T, 1, L>, nblk, 256, 0, (cudaStream_t)stream, a);
+            return launch_status("mt_chn_fill_step");
+        });
     });
+}
+
+extern "C" int mt_chn_fill_step_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                                       int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                                       const float *m_t, int64_t mt_sb, const float *v_map0, int64_t vm_sb,
+                                       float *y_comp0, float *m_new, float *x_new, float *inp_per, void *workspace,
+                                       int B, int64_t P, mt_stream_t stream) {
+    return chn_fill_impl(nn_layout, nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb,
+                         nullptr, nullptr, 0.0f, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
 }
 
 extern "C" int mt_chn_fill_step_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
@@ -902,8 +978,8 @@ extern "C" int mt_chn_fill_step_dt(int nn_dtype, const void *nn_out, const float
                                    const float *v_map0, int64_t vm_sb, float *y_comp0, float *m_new,
                                    float *x_new, float *inp_per, void *workspace, int B, int64_t P,
                                    mt_stream_t stream) {
-    return chn_fill_impl(nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, nullptr, nullptr,
-                         0.0f, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
+    return mt_chn_fill_step_layout(MT_LAYOUT_NCHW, nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb,
+                                   v_map0, vm_sb, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
 }
 
 extern "C" int mt_chn_fill_step(const float *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,
@@ -915,14 +991,25 @@ extern "C" int mt_chn_fill_step(const float *nn_out, const float *x_t, int64_t x
                                m_new, x_new, inp_per, workspace, B, P, stream);
 }
 
+extern "C" int mt_chn_fill_step_gated_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                                             int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb,
+                                             const float *m_t, int64_t mt_sb, const float *v_map0, int64_t vm_sb,
+                                             const float *y_prev, const float *gate_per, float gate_e,
+                                             float *y_comp0, float *m_new, float *x_new, float *inp_per,
+                                             void *workspace, int B, int64_t P, mt_stream_t stream) {
+    return chn_fill_impl(nn_layout, nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, y_prev,
+                         gate_per, gate_e, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
+}
+
 extern "C" int mt_chn_fill_step_gated_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sb,
                                          int64_t xt_sc, const float *v_t, int64_t vt_sb, const float *m_t,
                                          int64_t mt_sb, const float *v_map0, int64_t vm_sb, const float *y_prev,
                                          const float *gate_per, float gate_e, float *y_comp0, float *m_new,
                                          float *x_new, float *inp_per, void *workspace, int B, int64_t P,
                                          mt_stream_t stream) {
-    return chn_fill_impl(nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb, v_map0, vm_sb, y_prev, gate_per,
-                         gate_e, y_comp0, m_new, x_new, inp_per, workspace, B, P, stream);
+    return mt_chn_fill_step_gated_layout(MT_LAYOUT_NCHW, nn_dtype, nn_out, x_t, xt_sb, xt_sc, v_t, vt_sb, m_t, mt_sb,
+                                         v_map0, vm_sb, y_prev, gate_per, gate_e, y_comp0, m_new, x_new, inp_per,
+                                         workspace, B, P, stream);
 }
 
 extern "C" int mt_chn_fill_step_gated(const float *nn_out, const float *x_t, int64_t xt_sb, int64_t xt_sc,

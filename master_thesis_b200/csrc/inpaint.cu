@@ -23,7 +23,7 @@ namespace {
 bool mult4(int64_t v) { return (v & 3) == 0; }
 
 struct LanesArgs {
-    const void *nn_out;                     // (L,3,P) contiguous, element type T of chn_fill_lanes_kernel
+    const void *nn_out;                     // (L,3,P) planar or (L,P,3) channels-last, element type T
     const float *x_t; int64_t xt_sl, xt_sc;
     const float *m_t; int64_t mt_sl;
     const float *v_map0; int64_t vm_sl;
@@ -48,7 +48,7 @@ int lane_block_cap(int L) {
     return n < 1 ? 1 : n;
 }
 
-template <typename T, int VEC>
+template <typename T, int VEC, bool NHWC = false>  // NHWC: nn_out channels-last
 __global__ void __launch_bounds__(256) chn_fill_lanes_kernel(const LanesArgs a) {
     pdl_sync();
     const T *nn_out = static_cast<const T *>(a.nn_out);
@@ -63,9 +63,10 @@ __global__ void __launch_bounds__(256) chn_fill_lanes_kernel(const LanesArgs a) 
         Vec<VEC> m, vm, vt, o[3], xt[3];
         m.load_stream(a.m_t + lane * a.mt_sl + p0);
         vm.load_stream(a.v_map0 + lane * a.vm_sl + p0);
+        if constexpr (NHWC) load_nhwc(o, nn_out + ((int64_t)lane * a.P + p0) * 3);
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            o[c].load_stream(nn_out + ((int64_t)lane * 3 + c) * a.P + p0);
+            if constexpr (!NHWC) o[c].load_stream(nn_out + ((int64_t)lane * 3 + c) * a.P + p0);
             xt[c].load_stream(a.x_t + lane * a.xt_sl + c * a.xt_sc + p0);
         }
 #pragma unroll
@@ -156,40 +157,54 @@ extern "C" int64_t mt_chn_fill_lanes_workspace_bytes(int L) {
     return kLaneTicketBytes + (int64_t)L * lane_block_cap(L) * 4;
 }
 
+extern "C" int mt_chn_fill_lanes_layout(int nn_layout, int nn_dtype, const void *nn_out, const float *x_t,
+                                        int64_t xt_sl, int64_t xt_sc, const float *m_t, int64_t mt_sl,
+                                        const float *v_map0, int64_t vm_sl, const int *slots, float *y_out,
+                                        int64_t yo_ss, int64_t yo_sc, float *m_state, int64_t ms_ss, float *x_state,
+                                        int64_t xs_ss, int64_t xs_sc, float *per_out, void *workspace, int L,
+                                        int64_t P, int finalize, double e, int force, mt_stream_t stream) {
+    MT_REQUIRE(nn_out && x_t && m_t && v_map0 && slots && y_out && m_state && x_state && per_out && workspace,
+               "mt_chn_fill_lanes: NULL argument");
+    MT_REQUIRE(L >= 1 && L <= kMaxLanes && P > 0, "mt_chn_fill_lanes: bad shape (L = %d, P = %lld)", L, (long long)P);
+    MT_REQUIRE(y_out != nn_out && m_state != nn_out && x_state != nn_out && per_out != nn_out,
+               "mt_chn_fill_lanes: an output aliases nn_out");
+    return with_layout(nn_layout, "mt_chn_fill_lanes", [&](auto nhwc) {
+        constexpr bool NL = decltype(nhwc)::value;
+        return with_dtype(nn_dtype, "mt_chn_fill_lanes", [&](auto tag) {
+            using T = decltype(tag);
+            LanesArgs a{nn_out, x_t, xt_sl, xt_sc, m_t, mt_sl, v_map0, vm_sl, slots, y_out, yo_ss, yo_sc,
+                        m_state, ms_ss, x_state, xs_ss, xs_sc, per_out, workspace, P, 0, force ? 1 : 0, e};
+            const bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(m_t) &&
+                            aligned16(v_map0) && aligned16(y_out) && aligned16(m_state) && aligned16(x_state) &&
+                            mult4(xt_sl) && mult4(xt_sc) && mult4(mt_sl) && mult4(vm_sl) && mult4(yo_ss) &&
+                            mult4(yo_sc) && mult4(ms_ss) && mult4(xs_ss) && mult4(xs_sc);
+            const int vec = v4 ? 4 : 1;
+            const int64_t chunks = (P + 256 * vec - 1) / (256 * vec);
+            MT_REQUIRE(chunks < (1ll << 31), "mt_chn_fill_lanes: plane too large");
+            a.chunks = (int)chunks;
+            const int cap = lane_block_cap(L);
+            const dim3 grid((unsigned)(chunks < cap ? chunks : cap), (unsigned)L);
+            const cudaStream_t st = (cudaStream_t)stream;
+            if (v4) launch(chn_fill_lanes_kernel<T, 4, NL>, grid, 256, 0, st, a);
+            else launch(chn_fill_lanes_kernel<T, 1, NL>, grid, 256, 0, st, a);
+            int rc = launch_status("mt_chn_fill_lanes");
+            if (rc || !finalize || force) return rc;
+            if (v4) launch(chn_finalize_lanes_kernel<4>, grid, 256, 0, st, a);
+            else launch(chn_finalize_lanes_kernel<1>, grid, 256, 0, st, a);
+            return launch_status("mt_chn_fill_lanes (finalize)");
+        });
+    });
+}
+
 extern "C" int mt_chn_fill_lanes_dt(int nn_dtype, const void *nn_out, const float *x_t, int64_t xt_sl,
                                     int64_t xt_sc, const float *m_t, int64_t mt_sl, const float *v_map0,
                                     int64_t vm_sl, const int *slots, float *y_out, int64_t yo_ss, int64_t yo_sc,
                                     float *m_state, int64_t ms_ss, float *x_state, int64_t xs_ss, int64_t xs_sc,
                                     float *per_out, void *workspace, int L, int64_t P, int finalize, double e,
                                     int force, mt_stream_t stream) {
-    MT_REQUIRE(nn_out && x_t && m_t && v_map0 && slots && y_out && m_state && x_state && per_out && workspace,
-               "mt_chn_fill_lanes: NULL argument");
-    MT_REQUIRE(L >= 1 && L <= kMaxLanes && P > 0, "mt_chn_fill_lanes: bad shape (L = %d, P = %lld)", L, (long long)P);
-    MT_REQUIRE(y_out != nn_out && m_state != nn_out && x_state != nn_out && per_out != nn_out,
-               "mt_chn_fill_lanes: an output aliases nn_out");
-    return with_dtype(nn_dtype, "mt_chn_fill_lanes", [&](auto tag) {
-        using T = decltype(tag);
-        LanesArgs a{nn_out, x_t, xt_sl, xt_sc, m_t, mt_sl, v_map0, vm_sl, slots, y_out, yo_ss, yo_sc,
-                    m_state, ms_ss, x_state, xs_ss, xs_sc, per_out, workspace, P, 0, force ? 1 : 0, e};
-        const bool v4 = mult4(P) && aligned_vec4<T>(nn_out) && aligned16(x_t) && aligned16(m_t) &&
-                        aligned16(v_map0) && aligned16(y_out) && aligned16(m_state) && aligned16(x_state) &&
-                        mult4(xt_sl) && mult4(xt_sc) && mult4(mt_sl) && mult4(vm_sl) && mult4(yo_ss) &&
-                        mult4(yo_sc) && mult4(ms_ss) && mult4(xs_ss) && mult4(xs_sc);
-        const int vec = v4 ? 4 : 1;
-        const int64_t chunks = (P + 256 * vec - 1) / (256 * vec);
-        MT_REQUIRE(chunks < (1ll << 31), "mt_chn_fill_lanes: plane too large");
-        a.chunks = (int)chunks;
-        const int cap = lane_block_cap(L);
-        const dim3 grid((unsigned)(chunks < cap ? chunks : cap), (unsigned)L);
-        const cudaStream_t st = (cudaStream_t)stream;
-        if (v4) launch(chn_fill_lanes_kernel<T, 4>, grid, 256, 0, st, a);
-        else launch(chn_fill_lanes_kernel<T, 1>, grid, 256, 0, st, a);
-        int rc = launch_status("mt_chn_fill_lanes");
-        if (rc || !finalize || force) return rc;
-        if (v4) launch(chn_finalize_lanes_kernel<4>, grid, 256, 0, st, a);
-        else launch(chn_finalize_lanes_kernel<1>, grid, 256, 0, st, a);
-        return launch_status("mt_chn_fill_lanes (finalize)");
-    });
+    return mt_chn_fill_lanes_layout(MT_LAYOUT_NCHW, nn_dtype, nn_out, x_t, xt_sl, xt_sc, m_t, mt_sl, v_map0, vm_sl,
+                                    slots, y_out, yo_ss, yo_sc, m_state, ms_ss, x_state, xs_ss, xs_sc, per_out,
+                                    workspace, L, P, finalize, e, force, stream);
 }
 
 extern "C" int mt_chn_fill_lanes(const float *nn_out, const float *x_t, int64_t xt_sl, int64_t xt_sc,

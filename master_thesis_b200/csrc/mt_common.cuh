@@ -12,6 +12,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "mt_b200.h"
 
 namespace mt {
@@ -71,6 +73,16 @@ inline int with_dtype(int dt, const char *who, Fn &&f) {
         default: break;
     }
     set_error("%s: unknown dtype code %d", who, dt);
+    return MT_ERR_INVALID;
+}
+
+// The memory layout of a network operand (the CNN input the packs write, the CNN output the composite / fill kernels
+// read) is a layout code MT_LAYOUT_*.  Calls f(std::bool_constant<NHWC>{}); any other code is an error.
+template <typename Fn>
+inline int with_layout(int layout, const char *who, Fn &&f) {
+    if (layout == MT_LAYOUT_NCHW) return f(std::false_type{});
+    if (layout == MT_LAYOUT_NHWC) return f(std::true_type{});
+    set_error("%s: unknown layout code %d", who, layout);
     return MT_ERR_INVALID;
 }
 
@@ -142,6 +154,12 @@ struct Vec<1> {
     __device__ __forceinline__ void load_stream(const T *p) { v[0] = widen(__ldcs(p)); }
     template <typename T>
     __device__ __forceinline__ void store_stream(T *p) const { __stcs(p, narrow<T>(v[0])); }
+    // plain store (any state space: the shared-memory stage of an NHWC tile)
+    template <typename T>
+    __device__ __forceinline__ void store_plain(T *p) const {
+        if constexpr (sizeof(T) == 4) *p = v[0];
+        else *p = narrow<T>(v[0]);
+    }
 };
 template <>
 struct Vec<4> {
@@ -174,7 +192,67 @@ struct Vec<4> {
         for (int i = 0; i < 4; ++i) e[i] = narrow<T>(v[i]);
         __stcs(reinterpret_cast<uint2 *>(p), u);
     }
+    template <typename T>
+    __device__ __forceinline__ void store_plain(T *p) const {
+        if constexpr (sizeof(T) == 4) {
+            *reinterpret_cast<float4 *>(p) = make_float4(v[0], v[1], v[2], v[3]);
+        } else {
+            uint2 u;
+            T *e = reinterpret_cast<T *>(&u);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) e[i] = narrow<T>(v[i]);
+            *reinterpret_cast<uint2 *>(p) = u;
+        }
+    }
 };
+
+// ---- channels-last (NHWC) network operands ----------------------------------------------------------------------
+// In NHWC the C channels of a pixel are adjacent, so the VEC consecutive pixels of a thread are VEC * C consecutive
+// elements.  Reads take them as C vectors and de-interleave in registers.  Writes go through a shared-memory stage
+// in output order (each thread's run at threadIdx.x * VEC * C), which the CTA then writes out as one contiguous,
+// coalesced run: VEC * C * 4 B per thread (36, 40, 12 B per pixel) does not map onto 16-byte vector stores.
+template <int VEC, int C, typename T>
+__device__ __forceinline__ void load_nhwc(Vec<VEC> (&o)[C], const T *p) {
+    Vec<VEC> r[C];
+#pragma unroll
+    for (int j = 0; j < C; ++j) r[j].load_stream(p + j * VEC);
+#pragma unroll
+    for (int i = 0; i < VEC; ++i)
+#pragma unroll
+        for (int c = 0; c < C; ++c) o[c].v[i] = r[(i * C + c) / VEC].v[(i * C + c) % VEC];
+}
+
+template <int VEC, int C, typename T>
+__device__ __forceinline__ void stage_nhwc(T *stage, const Vec<VEC> (&o)[C]) {
+    Vec<VEC> r[C];
+#pragma unroll
+    for (int i = 0; i < VEC; ++i)
+#pragma unroll
+        for (int c = 0; c < C; ++c) r[(i * C + c) / VEC].v[(i * C + c) % VEC] = o[c].v[i];
+    T *s = stage + threadIdx.x * (VEC * C);
+#pragma unroll
+    for (int j = 0; j < C; ++j) r[j].store_plain(s + j * VEC);
+}
+
+// n staged elements to dst (after a __syncthreads): 16-byte streaming stores when dst is 16-byte aligned and n fills
+// them, else one element per thread and instruction (still one contiguous run per warp)
+template <typename T>
+__device__ __forceinline__ void stage_out(T *dst, const T *stage, int n) {
+    constexpr int E = 16 / sizeof(T);
+    if ((reinterpret_cast<uintptr_t>(dst) & 15u) == 0 && n % E == 0) {
+        for (int i = threadIdx.x; i < n / E; i += blockDim.x)
+            __stcs(reinterpret_cast<uint4 *>(dst) + i, reinterpret_cast<const uint4 *>(stage)[i]);
+    } else {
+        for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = stage[i];
+    }
+}
+
+// the shared-memory stage of an NHWC tile of N elements of T (one array per kernel instantiation that asks for it)
+template <typename T, int N>
+__device__ __forceinline__ T *nhwc_stage() {
+    __shared__ __align__(16) unsigned char raw[N * sizeof(T)];
+    return reinterpret_cast<T *>(raw);
+}
 
 __device__ __forceinline__ float clamp01(float a) { return fminf(fmaxf(a, 0.0f), 1.0f); }
 

@@ -78,9 +78,13 @@ struct WarpFwdArgs {
 // resized flow is never written or read back (SURVEY 8f-1); bit-identical to resizing first.
 // G: element type of a dense flow (float, __half, __nv_bfloat16), widened on load: the output is the fp32 kernel's on
 // the widened flow.
-template <int C, int VIS, bool AFFINE, bool FULL, bool PACK = false, bool LOWRES = false, typename G = float>
+// NHWC (PACK only): nn_in is channels-last (pixel stride 9).  The CTA stages its kRows runs of up to kCols pixels x 9
+// channels in shared memory and writes each run out as one contiguous stretch of memory.
+template <int C, int VIS, bool AFFINE, bool FULL, bool PACK = false, bool LOWRES = false, typename G = float,
+          bool NHWC = false>
 __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFwdArgs a) {
     static_assert(!(AFFINE && LOWRES), "a theta needs no resize");
+    static_assert(PACK || !NHWC, "only the CNN input has a channels-last form");
     static_assert(!AFFINE || sizeof(G) == 4, "a theta is fp32");
     constexpr int U = kRows;
     pdl_sync();
@@ -145,6 +149,15 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
             vtv[k] = in ? __ldg(a.v_t + (b * a.vt_sb + p0 + k * W)) : 0.0f;
 #pragma unroll
             for (int c = 0; c < 3; ++c) xtv[c][k] = in ? __ldg(a.x_t + (b * a.xt_sb + c * a.xt_sc + p0 + k * W)) : 0.0f;
+        }
+    }
+    if constexpr (NHWC) {  // x_t and v_t go to the stage now: their registers are free for the gathers
+#pragma unroll
+        for (int k = 0; k < U; ++k) {
+            float *s = nhwc_stage<float, U * kCols * 9>() + (k * kCols + threadIdx.x) * 9;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) s[c] = __fdiv_rn(__fsub_rn(xtv[c][k], chan_mean(c)), chan_std(c));
+            s[6] = vtv[k];
         }
     }
     float ix[U], iy[U], xw[U], yn[U];
@@ -262,10 +275,10 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
         }
     }
     // ---------------- stores (coalesced, streaming) ----------------
-    if (!live) return;
+    if (!NHWC && !live) return;
 #pragma unroll
     for (int k = 0; k < U; ++k) {
-        if (y0 + k >= H) break;
+        if (y0 + k >= H || (NHWC && !live)) break;  // NHWC: every thread goes on to the CTA barrier below
         if (FULL || a.x_al) {
 #pragma unroll
             for (int c = 0; c < C; ++c) st_stream1(a.x_al + (xao + p0 + c * a.xa_sc + k * W), xa[c][k]);
@@ -274,7 +287,13 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
         const float vmap = (FULL || PACK || a.v_map) ? clamp01(__fsub_rn(va[k], __fsub_rn(1.0f, mtv[k]))) : 0.0f;
         if (FULL || a.v_map)  // clamp(v_al - (1 - m_t), 0, 1)
             st_stream1(a.v_map + (np0 + k * W), vmap);
-        if (PACK) {
+        if constexpr (PACK && NHWC) {
+            float *s = nhwc_stage<float, U * kCols * 9>() + (k * kCols + threadIdx.x) * 9;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) s[3 + c] = __fdiv_rn(__fsub_rn(xa[c][k], chan_mean(c)), chan_std(c));
+            s[7] = va[k];
+            s[8] = vmap;
+        } else if (PACK) {
             float *o = a.nn_in + ((int)n * 9 * a.P + p0 + k * W);
 #pragma unroll
             for (int c = 0; c < 3; ++c) {  // (x - mean) / std   model_chn.py:73-74
@@ -285,6 +304,16 @@ __global__ void __launch_bounds__(kCols, kWarpMinB) warp_fwd_kernel(const WarpFw
             st_stream1(o + 6 * a.P, vtv[k]);
             st_stream1(o + 7 * a.P, va[k]);
             st_stream1(o + 8 * a.P, vmap);
+        }
+    }
+    if constexpr (NHWC) {
+        __syncthreads();
+        const int x0 = blockIdx.x * kCols, ncol = min(kCols, W - x0);
+#pragma unroll
+        for (int k = 0; k < U; ++k) {
+            if (y0 + k >= H) break;
+            float *o = a.nn_in + ((int)n * a.P + (y0 + k) * W + x0) * 9;
+            stage_out(o, nhwc_stage<float, U * kCols * 9>() + k * kCols * 9, ncol * 9);
         }
     }
 }
@@ -609,13 +638,16 @@ struct PackOut {
     const float *x_t; int64_t xt_sb, xt_sc;
     const float *v_t; int64_t vt_sb;
     float *nn_in;
+    bool nhwc;  // nn_in channels-last
 };
 
 // the launches of warp_fwd_impl for a half dense flow (element type G): the DFPN flavour, nearest visibility
 template <typename G>
 static void warp_half_flow_go(const WarpFwdArgs &a, dim3 gridd, dim3 block, cudaStream_t st, int C, bool pack,
-                              bool lowres, bool full) {
-    if (pack && lowres) launch(warp_fwd_kernel<3, 1, false, false, true, true, G>, gridd, block, 0, st, a);
+                              bool lowres, bool full, bool nhwc) {
+    if (pack && lowres && nhwc) launch(warp_fwd_kernel<3, 1, false, false, true, true, G, true>, gridd, block, 0, st, a);
+    else if (pack && nhwc) launch(warp_fwd_kernel<3, 1, false, false, true, false, G, true>, gridd, block, 0, st, a);
+    else if (pack && lowres) launch(warp_fwd_kernel<3, 1, false, false, true, true, G>, gridd, block, 0, st, a);
     else if (lowres && full) launch(warp_fwd_kernel<3, 1, false, true, false, true, G>, gridd, block, 0, st, a);
     else if (lowres) launch(warp_fwd_kernel<3, 1, false, false, false, true, G>, gridd, block, 0, st, a);
     else if (pack) launch(warp_fwd_kernel<3, 1, false, false, true, false, G>, gridd, block, 0, st, a);
@@ -685,19 +717,28 @@ static int warp_fwd_impl(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_s
     cudaStream_t st = (cudaStream_t)stream;
     const bool full = x_aligned && v_aligned && v_map;
     if (g_dtype != MT_DT_F32) {
-        if (g_dtype == MT_DT_F16) warp_half_flow_go<__half>(a, gridd, block, st, C, pack != nullptr, lowres, full);
-        else warp_half_flow_go<__nv_bfloat16>(a, gridd, block, st, C, pack != nullptr, lowres, full);
+        const bool nhwc = pack && pack->nhwc;
+        if (g_dtype == MT_DT_F16) warp_half_flow_go<__half>(a, gridd, block, st, C, pack != nullptr, lowres, full, nhwc);
+        else warp_half_flow_go<__nv_bfloat16>(a, gridd, block, st, C, pack != nullptr, lowres, full, nhwc);
         return launch_status(pack ? (lowres ? "mt_warp_pack_lowres_fwd_dt" : "mt_warp_pack_fwd_dt")
                                   : (lowres ? "mt_warp_lowres_fwd_dt" : "mt_warp_fwd_dt"));
     }
     if (pack && lowres) {  // DFPN inference step at a frame size other than the flow's 256 x 256
-        launch(warp_fwd_kernel<3, 1, false, false, true, true>, gridd, block, 0, st, a);
+        if (pack->nhwc) launch(warp_fwd_kernel<3, 1, false, false, true, true, float, true>, gridd, block, 0, st, a);
+        else launch(warp_fwd_kernel<3, 1, false, false, true, true>, gridd, block, 0, st, a);
         return launch_status("mt_warp_pack_lowres_fwd");
     }
     if (lowres) {
         if (full) launch(warp_fwd_kernel<3, 1, false, true, false, true>, gridd, block, 0, st, a);
         else launch(warp_fwd_kernel<3, 1, false, false, false, true>, gridd, block, 0, st, a);
         return launch_status("mt_warp_lowres_fwd");
+    }
+    if (pack && pack->nhwc) {
+#define MT_WARP_PACK_GO(VV, AA) launch(warp_fwd_kernel<3, VV, AA, false, true, false, float, true>, gridd, block, 0, st, a)
+        if (vis_bil) { if (affine) MT_WARP_PACK_GO(2, true); else MT_WARP_PACK_GO(2, false); }
+        else         { if (affine) MT_WARP_PACK_GO(1, true); else MT_WARP_PACK_GO(1, false); }
+#undef MT_WARP_PACK_GO
+        return launch_status("mt_warp_pack_fwd");
     }
     if (pack) {
 #define MT_WARP_PACK_GO(VV, AA) launch(warp_fwd_kernel<3, VV, AA, false, true>, gridd, block, 0, st, a)
@@ -753,6 +794,20 @@ extern "C" int mt_warp_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x
                           xa_sc, xa_sf, v_aligned, v_map, B, C, F, H, W, flags, stream);
 }
 
+extern "C" int mt_warp_pack_fwd_layout(int nn_layout, const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
+                                       const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype,
+                                       const void *grid, const float *m_target, int64_t mt_sb, const float *x_t,
+                                       int64_t xt_sb, int64_t xt_sc, const float *v_t, int64_t vt_sb, float *nn_in,
+                                       float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
+                                       float *v_aligned, float *v_map, int B, int F, int H, int W, int flags,
+                                       mt_stream_t stream) {
+    return with_layout(nn_layout, "mt_warp_pack_fwd", [&](auto nhwc) {
+        PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in, decltype(nhwc)::value};
+        return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, grid, m_target, mt_sb, x_aligned,
+                             xa_sb, xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk);
+    });
+}
+
 extern "C" int mt_warp_pack_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
                                    const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype, const void *grid,
                                    const float *m_target, int64_t mt_sb, const float *x_t, int64_t xt_sb,
@@ -760,9 +815,9 @@ extern "C" int mt_warp_pack_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, i
                                    float *x_aligned, int64_t xa_sb, int64_t xa_sc, int64_t xa_sf,
                                    float *v_aligned, float *v_map, int B, int F, int H, int W, int flags,
                                    mt_stream_t stream) {
-    PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in};
-    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, grid, m_target, mt_sb, x_aligned, xa_sb,
-                         xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk);
+    return mt_warp_pack_fwd_layout(MT_LAYOUT_NCHW, x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, grid, m_target,
+                                   mt_sb, x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in, x_aligned, xa_sb, xa_sc, xa_sf,
+                                   v_aligned, v_map, B, F, H, W, flags, stream);
 }
 
 extern "C" int mt_warp_pack_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
@@ -796,6 +851,22 @@ extern "C" int mt_warp_lowres_fwd(const float *x, int64_t x_sb, int64_t x_sc, in
                                  x_aligned, xa_sb, xa_sc, xa_sf, v_aligned, v_map, B, F, H, W, flags, stream);
 }
 
+extern "C" int mt_warp_pack_lowres_fwd_layout(int nn_layout, const float *x, int64_t x_sb, int64_t x_sc,
+                                              int64_t x_sf, const float *vis, int64_t vis_sb, int64_t vis_sf,
+                                              int g_dtype, const void *flow, int gh, int gw, const float *m_target,
+                                              int64_t mt_sb, const float *x_t, int64_t xt_sb, int64_t xt_sc,
+                                              const float *v_t, int64_t vt_sb, float *nn_in, float *x_aligned,
+                                              int64_t xa_sb, int64_t xa_sc, int64_t xa_sf, float *v_aligned,
+                                              float *v_map, int B, int F, int H, int W, int flags,
+                                              mt_stream_t stream) {
+    MT_REQUIRE(gh > 0 && gw > 0, "mt_warp_pack_lowres_fwd: empty flow");
+    return with_layout(nn_layout, "mt_warp_pack_lowres_fwd", [&](auto nhwc) {
+        PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in, decltype(nhwc)::value};
+        return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, flow, m_target, mt_sb, x_aligned,
+                             xa_sb, xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk, gh, gw);
+    });
+}
+
 extern "C" int mt_warp_pack_lowres_fwd_dt(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,
                                           const float *vis, int64_t vis_sb, int64_t vis_sf, int g_dtype,
                                           const void *flow, int gh, int gw, const float *m_target, int64_t mt_sb,
@@ -803,10 +874,9 @@ extern "C" int mt_warp_pack_lowres_fwd_dt(const float *x, int64_t x_sb, int64_t 
                                           int64_t vt_sb, float *nn_in, float *x_aligned, int64_t xa_sb, int64_t xa_sc,
                                           int64_t xa_sf, float *v_aligned, float *v_map, int B, int F, int H,
                                           int W, int flags, mt_stream_t stream) {
-    MT_REQUIRE(gh > 0 && gw > 0, "mt_warp_pack_lowres_fwd: empty flow");
-    PackOut pk{x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in};
-    return warp_fwd_impl(x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, flow, m_target, mt_sb, x_aligned, xa_sb,
-                         xa_sc, xa_sf, v_aligned, v_map, B, 3, F, H, W, flags, stream, &pk, gh, gw);
+    return mt_warp_pack_lowres_fwd_layout(MT_LAYOUT_NCHW, x, x_sb, x_sc, x_sf, vis, vis_sb, vis_sf, g_dtype, flow, gh,
+                                          gw, m_target, mt_sb, x_t, xt_sb, xt_sc, v_t, vt_sb, nn_in, x_aligned, xa_sb,
+                                          xa_sc, xa_sf, v_aligned, v_map, B, F, H, W, flags, stream);
 }
 
 extern "C" int mt_warp_pack_lowres_fwd(const float *x, int64_t x_sb, int64_t x_sc, int64_t x_sf,

@@ -24,6 +24,8 @@ REDUCE = {"mean": 0, "sum": 1}
 NET_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
 _DT = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
 _DT_NAMES = {torch.float32: "fp32", torch.float16: "fp16", torch.bfloat16: "bf16"}
+# memory layout of a network operand: codes MT_LAYOUT_* of the C ABI
+LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 _workspaces = {}
 record = _lib.record      # with ops.record() as plan: ...   (see _lib.Plan)
@@ -59,17 +61,39 @@ class _Net(object):
         self.t = t
 
 
-def _call_net(name, *args):
+def _call_net(name, *args, layout=0):
     """Launches entry point ``name`` whose network operands are given as ``_Net``: when all of them are fp32 (or absent)
-    the fp32 entry point itself, so an fp32 run launches and records what it always did; else its ``_dt`` form, with
-    the MT_DT_* code of each such operand before its pointer."""
+    and ``layout`` is planar, the fp32 entry point itself, so an fp32 run launches and records what it always did; else
+    its ``_dt`` form, with the MT_DT_* code of each such operand before its pointer.  A channels-last network operand
+    (``layout`` LAYOUT_NHWC) takes the ``_layout`` form: the layout code, then the arguments of the ``_dt`` form (of
+    ``name`` itself where it has none)."""
     nets = [a.t for a in args if isinstance(a, _Net)]
-    if all(t is None or t.dtype == torch.float32 for t in nets):
+    if layout == LAYOUT_NCHW and all(t is None or t.dtype == torch.float32 for t in nets):
         return _call(name, *[_ptr(a.t) if isinstance(a, _Net) else a for a in args])
     flat = []
     for a in args:
         flat += [0 if a.t is None else _DT[a.t.dtype], _ptr(a.t)] if isinstance(a, _Net) else [a]
-    return _call(name + "_dt", *flat)
+    if layout == LAYOUT_NCHW:
+        return _call(name + "_dt", *flat)
+    return _call(name + "_layout", layout, *flat)
+
+
+def _net_layout(t):
+    """(operand, LAYOUT_* code) of a network output: a planar-contiguous or channels-last-contiguous tensor is read
+    where it is, any other one is copied to planar.  A tensor that is contiguous in both formats counts as planar."""
+    if t.is_contiguous():
+        return _contig(t), LAYOUT_NCHW
+    if t.dim() == 4 and t.is_contiguous(memory_format=torch.channels_last):
+        return _lib.keep(t), LAYOUT_NHWC
+    return _contig(t), LAYOUT_NCHW
+
+
+def _net_input(shape, device, channels_last):
+    """(tensor, LAYOUT_* code): the CNN input a pack writes, planar, or with channels-last strides (same shape) for a
+    channels-last network."""
+    fmt = torch.channels_last if channels_last else torch.contiguous_format
+    return _empty(shape, dtype=torch.float32, device=device, memory_format=fmt), \
+        LAYOUT_NHWC if channels_last else LAYOUT_NCHW
 
 
 _device = [None]     # device index of the operator call in progress (set by _need_cuda)
@@ -260,10 +284,12 @@ def warp_fwd(x, vis, grid, m_target=None, flags=ALIGN_CORNERS, want_x=True, want
     return xa, va, vm
 
 
-def warp_pack_fwd(x, vis, grid, m_target, x_t, v_t, flags=ALIGN_CORNERS, want_aligned=False, want_v_map=True):
+def warp_pack_fwd(x, vis, grid, m_target, x_t, v_t, flags=ALIGN_CORNERS, want_aligned=False, want_v_map=True,
+                  channels_last=False):
     """mt_warp_pack_fwd: the warp of mt_warp_fwd that also writes the CNN input of CHN.forward.
 
-    A dense flow may be fp16 / bf16, as in warp_fwd.
+    A dense flow may be fp16 / bf16, as in warp_fwd.  ``channels_last``: nn_in has channels-last strides (the input of
+    a network converted to torch.channels_last), same shape and values.
 
     Returns (nn_in (B*F,9,H,W), v_map (B,1,F,H,W) | None, x_aligned | None, v_aligned | None)."""
     _need_cuda(x, vis, (grid, NET_DTYPES), m_target, x_t, v_t)
@@ -281,15 +307,17 @@ def warp_pack_fwd(x, vis, grid, m_target, x_t, v_t, flags=ALIGN_CORNERS, want_al
         xa_mem, xa = _frame_major(b, c, f, h, w, x)
         va = _empty((b, 1, f, h, w), dtype=torch.float32, device=x.device)
     vm = _empty((b, 1, f, h, w), dtype=torch.float32, device=x.device) if want_v_map else None
-    nn_in = _empty((b * f, 9, h, w), dtype=torch.float32, device=x.device)
+    nn_in, layout = _net_input((b * f, 9, h, w), x.device, channels_last)
     if gh and (gh, gw) != (h, w):
         _call_net("mt_warp_pack_lowres_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _Net(grid), gh, gw,
                   _ptr(m_target), m_target.stride(0), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
-                  _ptr(nn_in), _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm), b, f, h, w, flags, _stream(x))
+                  _ptr(nn_in), _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm), b, f, h, w, flags, _stream(x),
+                  layout=layout)
         return nn_in, vm, xa, va
     _call_net("mt_warp_pack_fwd", _ptr(x), x_sb, x_sc, x_sf, _ptr(vis), v_sb, v_sf, _Net(grid),
               _ptr(m_target), m_target.stride(0), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
-              _ptr(nn_in), _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm), b, f, h, w, flags, _stream(x))
+              _ptr(nn_in), _ptr(xa_mem), f * c * p, p, c * p, _ptr(va), _ptr(vm), b, f, h, w, flags, _stream(x),
+              layout=layout)
     return nn_in, vm, xa, va
 
 
@@ -787,8 +815,8 @@ def cm_match(c_feats, v_t, v_aligned, return_gs=False):
 # --------------------------------------------------------------------------
 # K4 CHN
 # --------------------------------------------------------------------------
-def chn_pack(x_t, v_t, x_al, v_al, v_map):
-    """model_chn.py:68-80 -> nn_input (B*F,9,H,W) NCHW."""
+def chn_pack(x_t, v_t, x_al, v_al, v_map, channels_last=False):
+    """model_chn.py:68-80 -> nn_input (B*F,9,H,W), NCHW or with ``channels_last`` strides (same values)."""
     _need_cuda(x_t, v_t, x_al, v_al, v_map)
     _no_grad_inputs("chn_pack", x_t, v_t, x_al, v_al, v_map)
     b, _, f, h, w = x_al.shape
@@ -796,26 +824,27 @@ def chn_pack(x_t, v_t, x_al, v_al, v_map):
     xa, xa_sb, xa_sc, xa_sf = _s5(x_al)
     va, va_sb, _, va_sf = _s5(v_al)
     vm, vm_sb, _, vm_sf = _s5(v_map)
-    out = _empty((b * f, 9, h, w), dtype=torch.float32, device=xa.device)
-    _call("mt_chn_pack", _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0), _ptr(xa),
+    out, layout = _net_input((b * f, 9, h, w), xa.device, channels_last)
+    _call_net("mt_chn_pack", _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0), _ptr(xa),
               xa_sb, xa_sc, xa_sf, _ptr(va), va_sb, va_sf, _ptr(vm), vm_sb, vm_sf, _ptr(out), b, f,
-              h * w, _stream(xa))
+              h * w, _stream(xa), layout=layout)
     return out
 
 
 class ChnCompositeFn(torch.autograd.Function):
-    """model_chn.py:80-85 with autograd w.r.t. the CNN output."""
+    """model_chn.py:80-85 with autograd w.r.t. the CNN output.  A channels-last CNN output is read where it is, and
+    its gradient is returned channels-last."""
 
     @staticmethod
     def forward(ctx, nn_out, x_t, v_t, b, f):
         _need_cuda((nn_out, NET_DTYPES), x_t, v_t)
         h, w = nn_out.shape[-2:]
-        no = _contig(nn_out)
+        no, layout = _net_layout(nn_out)
         xt, vt = _planes(x_t), _planes(v_t)
         yh_mem, yh = _frame_major(b, 3, f, h, w, no)
         yc_mem, yc = _frame_major(b, 3, f, h, w, no)
         _call_net("mt_chn_composite_fwd", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt),
-              vt.stride(0), _ptr(yh_mem), _ptr(yc_mem), b, f, h * w, _stream(no))
+              vt.stride(0), _ptr(yh_mem), _ptr(yc_mem), b, f, h * w, _stream(no), layout=layout)
         ctx.save_for_backward(no, vt)
         ctx.meta = (b, f, h, w)
         return yh, yc
@@ -831,19 +860,19 @@ class ChnCompositeFn(torch.autograd.Function):
 
 def chn_composite_bwd_raw(nn_out, v_t, g_yh, g_yc, b, f):
     """mt_chn_composite_bwd: gradient w.r.t. the CNN output from the grads of both outputs, in the dtype of
-    ``nn_out`` (the fp32 gradient rounded to nearest even)."""
+    ``nn_out`` (the fp32 gradient rounded to nearest even) and in its layout (planar or channels-last)."""
     h, w = nn_out.shape[-2:]
     _device[0] = nn_out.device.index
-    no, vt = _contig(nn_out), _planes(v_t)
+    (no, layout), vt = _net_layout(nn_out), _planes(v_t)
     gy = gc = None
     gy_s = gc_s = (0, 0, 0)
     if g_yh is not None:
         gy, *gy_s = _s5(g_yh)
     if g_yc is not None:
         gc, *gc_s = _s5(g_yc)
-    g = _empty_like(no)
+    g = _empty_like(no)         # in the layout of no
     _call_net("mt_chn_composite_bwd", _Net(no), _ptr(vt), vt.stride(0), _ptr(gy), *gy_s, _ptr(gc),
-          *gc_s, _ptr(g), b, f, h * w, _stream(no))
+          *gc_s, _ptr(g), b, f, h * w, _stream(no), layout=layout)
     return g
 
 
@@ -869,7 +898,7 @@ def hole_update(m_t, v_map0, y_comp0):
 
 def chn_fill(nn_out, x_t, v_t, m_t, v_map0, gate=None):
     """mt_chn_fill_step: composite (model_chn.py:80-85) + hole update (:128-131) of one inference step
-    with a single reference frame.  nn_out (B,3,H,W).  Returns (y_comp0 (B,3,H,W), m_new, x_new, inp_per).
+    with a single reference frame.  nn_out (B,3,H,W), planar or channels-last.  Returns (y_comp0 (B,3,H,W), m_new, x_new, inp_per).
 
     ``gate = (prev_inp_per (1-element device tensor), e, y_prev)``: device-side loop control - the step only
     happens while prev_inp_per > e, otherwise the state passes through unchanged (mt_chn_fill_step_gated)."""
@@ -877,7 +906,7 @@ def chn_fill(nn_out, x_t, v_t, m_t, v_map0, gate=None):
     _no_grad_inputs("chn_fill", nn_out, x_t, v_t, m_t, v_map0)
     b = x_t.shape[0]
     h, w = x_t.shape[-2:]
-    no, xt, vt, mt, vm = _contig(nn_out), _planes(x_t), _planes(v_t), _planes(m_t), _planes(v_map0)
+    (no, layout), xt, vt, mt, vm = _net_layout(nn_out), _planes(x_t), _planes(v_t), _planes(m_t), _planes(v_map0)
     yc = _empty((b, 3, h, w), dtype=torch.float32, device=no.device)
     m_new = _empty((b, 1, h, w), dtype=torch.float32, device=no.device)
     x_new = _empty((b, 3, h, w), dtype=torch.float32, device=no.device)
@@ -885,14 +914,15 @@ def chn_fill(nn_out, x_t, v_t, m_t, v_map0, gate=None):
     if gate is None:
         _call_net("mt_chn_fill_step", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
               _ptr(mt), mt.stride(0), _ptr(vm), vm.stride(0), _ptr(yc), _ptr(m_new), _ptr(x_new), _ptr(per),
-              _ptr(reduce_workspace(no)), b, h * w, _stream(no))
+              _ptr(reduce_workspace(no)), b, h * w, _stream(no), layout=layout)
     else:
         prev_per, e, y_prev = gate
         _need_cuda(prev_per, y_prev)
         y_prev = _contig(y_prev)
         _call_net("mt_chn_fill_step_gated", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(vt), vt.stride(0),
               _ptr(mt), mt.stride(0), _ptr(vm), vm.stride(0), _ptr(y_prev), _ptr(prev_per.reshape(1)), float(e),
-              _ptr(yc), _ptr(m_new), _ptr(x_new), _ptr(per), _ptr(reduce_workspace(no)), b, h * w, _stream(no))
+              _ptr(yc), _ptr(m_new), _ptr(x_new), _ptr(per), _ptr(reduce_workspace(no)), b, h * w, _stream(no),
+              layout=layout)
     return yc, m_new, x_new, per[0]
 
 
@@ -926,7 +956,7 @@ def _out_planes(t, who):
 
 def chn_fill_lanes(nn_out, x_t, m_t, v_map0, slots, x_state, m_state, y_out, per_out, finalize=None):
     """mt_chn_fill_lanes: composite (model_chn.py:83-84) + hole update (:128-131) of L independent F = 1 steps, one
-    target frame per lane, with a hole percentage per lane.  nn_out (L,3,H,W); x_t (L,3,H,W), m_t and v_map0
+    target frame per lane, with a hole percentage per lane.  nn_out (L,3,H,W), planar or channels-last; x_t (L,3,H,W), m_t and v_map0
     (L,1,H,W), strided with contiguous planes (v_t = 1 - m_t is formed in the kernel).  ``slots``: a host list,
     lane i writes state slot slots[i] of x_state (S,3,H,W) (x_new), m_state (S,1,H,W) (m_new), y_out (S,3,H,W)
     (y_comp) and per_out (S,) (inp_per), all in place and strided.  x_t / m_t may be views of the state slots
@@ -946,7 +976,7 @@ def chn_fill_lanes(nn_out, x_t, m_t, v_map0, slots, x_state, m_state, y_out, per
             raise ValueError("chn_fill_lanes: %s must be %s, got %s" % (name, shape, tuple(t.shape)))
     if not per_out.is_contiguous():
         raise RuntimeError("chn_fill_lanes: per_out must be contiguous")
-    no, xt, mt, vm = _contig(nn_out), _planes(x_t), _planes(m_t), _planes(v_map0)
+    (no, layout), xt, mt, vm = _net_layout(nn_out), _planes(x_t), _planes(m_t), _planes(v_map0)
     xs, ms, yo = _out_planes(x_state, "x_state"), _out_planes(m_state, "m_state"), _out_planes(y_out, "y_out")
     sl = _lib.keep(index_tensor(slots, no.device, torch.int32))
     e, force = (1.0, False) if finalize is None else (float(finalize[0]), bool(finalize[1]))
@@ -956,7 +986,7 @@ def chn_fill_lanes(nn_out, x_t, m_t, v_map0, slots, x_state, m_state, y_out, per
     _call_net("mt_chn_fill_lanes", _Net(no), _ptr(xt), xt.stride(0), xt.stride(1), _ptr(mt), mt.stride(0), _ptr(vm),
           vm.stride(0), _ptr(sl), _ptr(yo), yo.stride(0), yo.stride(1), _ptr(ms), ms.stride(0), _ptr(xs),
           xs.stride(0), xs.stride(1), _ptr(per_out), _ptr(ws), lanes, h * w, int(finalize is not None), e,
-          int(force), _stream(no))
+          int(force), _stream(no), layout=layout)
 
 
 def trivial_copy(x_t, x_al, v_map):
@@ -976,8 +1006,9 @@ def trivial_copy(x_t, x_al, v_map):
 # --------------------------------------------------------------------------
 # K5 FlowEstimator input pack
 # --------------------------------------------------------------------------
-def flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre):
-    """model_dfpn.py:733-741 -> nn_input (B*F,10,H,W) NCHW; the flow is read through its own strides."""
+def flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre, channels_last=False):
+    """model_dfpn.py:733-741 -> nn_input (B*F,10,H,W), NCHW or with ``channels_last`` strides (same values); the flow
+    is read through its own strides."""
     _need_cuda(x_target, m_target, x_refs, m_refs, flow_pre)
     b, c, f, h, w = x_refs.shape
     if c != 3 or tuple(flow_pre.shape) != (b, f, h, w, 2) or tuple(m_refs.shape) != (b, 1, f, h, w):
@@ -985,35 +1016,38 @@ def flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre):
     xt, mt = _planes(x_target), _planes(m_target)
     xr, xr_sb, xr_sc, xr_sf = _s5(x_refs)
     mr, mr_sb, _, mr_sf = _s5(m_refs)
-    out = _empty((b * f, 10, h, w), dtype=torch.float32, device=xr.device)
+    out, layout = _net_input((b * f, 10, h, w), xr.device, channels_last)
     fs = flow_pre.stride()
-    _call("mt_flow_pack", _ptr(xr), xr_sb, xr_sc, xr_sf, _ptr(xt), xt.stride(0), xt.stride(1), _ptr(mr), mr_sb,
-          mr_sf, _ptr(mt), mt.stride(0), _ptr(flow_pre), fs[0], fs[1], fs[2], fs[3], fs[4], _ptr(out), b, f, h, w,
-          _stream(xr))
+    _call_net("mt_flow_pack", _ptr(xr), xr_sb, xr_sc, xr_sf, _ptr(xt), xt.stride(0), xt.stride(1), _ptr(mr), mr_sb,
+              mr_sf, _ptr(mt), mt.stride(0), _ptr(flow_pre), fs[0], fs[1], fs[2], fs[3], fs[4], _ptr(out), b, f, h,
+              w, _stream(xr), layout=layout)
     return out
 
 
 class FlowPackFn(torch.autograd.Function):
     """The pack with the only gradient the reference's `cat` carries in DFPN training: the one of ``flow_pre``
-    (frames and masks are data).  It is a view of the gradient of channels 8-9 - no kernel."""
+    (frames and masks are data).  It is a view of the gradient of channels 8-9 - no kernel.  Of a channels-last
+    gradient that view is an interleaved flow with pixel stride 10, which its consumers (the resize and warp
+    backward kernels) read through its strides."""
 
     @staticmethod
-    def forward(ctx, flow_pre, x_target, m_target, x_refs, m_refs):
+    def forward(ctx, flow_pre, x_target, m_target, x_refs, m_refs, channels_last):
         ctx.meta = x_refs.shape
-        return flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre.detach())
+        return flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre.detach(), channels_last)
 
     @staticmethod
     def backward(ctx, g):
         b, _, f, h, w = ctx.meta
-        return g[:, 8:10].reshape(b, f, 2, h, w).permute(0, 1, 3, 4, 2), None, None, None, None
+        return g[:, 8:10].reshape(b, f, 2, h, w).permute(0, 1, 3, 4, 2), None, None, None, None, None
 
 
-def flow_pack(x_target, m_target, x_refs, m_refs, flow_pre):
-    """FlowEstimator.forward's `nn_input` (model_dfpn.py:733-741); differentiable w.r.t. ``flow_pre``."""
+def flow_pack(x_target, m_target, x_refs, m_refs, flow_pre, channels_last=False):
+    """FlowEstimator.forward's `nn_input` (model_dfpn.py:733-741); differentiable w.r.t. ``flow_pre``.
+    ``channels_last``: the result has channels-last strides (the input of a channels-last estimator)."""
     _no_grad_inputs("flow_pack", x_target, m_target, x_refs, m_refs)
     if torch.is_grad_enabled() and flow_pre.requires_grad:
-        return FlowPackFn.apply(flow_pre, x_target, m_target, x_refs, m_refs)
-    return flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre)
+        return FlowPackFn.apply(flow_pre, x_target, m_target, x_refs, m_refs, channels_last)
+    return flow_pack_raw(x_target, m_target, x_refs, m_refs, flow_pre, channels_last)
 
 
 # --------------------------------------------------------------------------

@@ -28,6 +28,26 @@ def _cuda_autocast_half(t):
         t.dtype == torch.get_autocast_dtype("cuda") and t.dtype != torch.float32
 
 
+def _channels_last(net):
+    """True if ``net`` takes channels-last input: the weight of its first convolution is channels-last (the user ran
+    ``net.to(memory_format=torch.channels_last)``).  A weight contiguous in both formats (a 1 x 1 kernel) and a
+    network without convolutions (or a plain callable) count as NCHW.  The packs then write the network's input in that
+    layout, so the convolution does not copy it."""
+    if not isinstance(net, nn.Module):
+        return False
+    for m in net.modules():
+        if isinstance(m, nn.Conv2d):
+            w = m.weight
+            return w.dim() == 4 and not w.is_contiguous() and w.is_contiguous(memory_format=torch.channels_last)
+    return False
+
+
+def _layout_kw(net):
+    """The keyword that asks a pack for ``net``'s input layout: ``channels_last=True`` for a channels-last network,
+    nothing for an NCHW one (whose calls stay exactly what they were)."""
+    return {"channels_last": True} if _channels_last(net) else {}
+
+
 def _reference_original(cls, attr):
     """The reference's own ``cls.attr``, saved by ``patch()``: the resampling mirrors hand it every call their
     kernels do not serve (the reference's dataset code calls the same helpers on host tensors)."""
@@ -167,9 +187,10 @@ def flow_estimator_forward(self, x_target, m_target, x_refs, m_refs, flow_pre):
     """FlowEstimator.forward (model_dfpn.py:714-744): the 10-channel input of the estimator's conv stack is
     written by one kernel (``ops.flow_pack``: the reference builds it from two transposes, two repeats, a permute
     and a `cat`, :733-741); the conv stack (``self.nn``, cuDNN) and the closing reshape / permute (:743-744)
-    are the reference's.  The gradient reaches ``flow_pre`` as it does through the reference's `cat`."""
+    are the reference's.  The gradient reaches ``flow_pre`` as it does through the reference's `cat`.  A channels-last
+    conv stack gets its input channels-last."""
     b, _, ref_n, h, w = x_refs.size()
-    nn_input = ops.flow_pack(x_target, m_target, x_refs, m_refs, flow_pre)
+    nn_input = ops.flow_pack(x_target, m_target, x_refs, m_refs, flow_pre, **_layout_kw(self.nn))
     return self.nn(nn_input).reshape(b, ref_n, 2, h, w).permute(0, 1, 3, 4, 2)
 
 
@@ -331,9 +352,10 @@ def cpn_align_tail(x_refs, m_refs, m_target, theta):
 # ---------------------------------------------------------------------------
 def chn_forward(self, x_target, v_target, x_refs_aligned, v_refs_aligned, v_maps):
     """Replaces CHN.forward (model_chn.py:44-85): pack kernel -> self.nn (RRDBNet, cuDNN)
-    -> composite kernel.  Returns (y_hat, y_hat_comp), both (B,C,F,H,W)."""
+    -> composite kernel.  Returns (y_hat, y_hat_comp), both (B,C,F,H,W).  A channels-last RRDBNet gets its input
+    channels-last, and its channels-last output is read where it is."""
     b, c, f, h, w = x_refs_aligned.size()
-    nn_input = ops.chn_pack(x_target, v_target, x_refs_aligned, v_refs_aligned, v_maps)
+    nn_input = ops.chn_pack(x_target, v_target, x_refs_aligned, v_refs_aligned, v_maps, **_layout_kw(self.nn))
     nn_output = self.nn(nn_input)
     return ops.chn_composite(nn_output, x_target, v_target, b, f)
 
@@ -380,7 +402,7 @@ def _fill_step(chn, aligner, x_t, m_t, x_ref, m_ref, gate=None):
     if grid_fn is not None:
         grid, flags = grid_fn(aligner, x_t, m_t, x_ref, m_ref)
         v_t = 1 - m_t
-        nn_in, v_map, _, _ = ops.warp_pack_fwd(x_ref, m_ref, grid, m_t, x_t, v_t, flags)
+        nn_in, v_map, _, _ = ops.warp_pack_fwd(x_ref, m_ref, grid, m_t, x_t, v_t, flags, **_layout_kw(chn.nn))
         y_comp, m_new, x_new, per = ops.chn_fill(chn.nn(nn_in), x_t, v_t, m_t, v_map[:, :, 0], gate)
         return y_comp, m_new, x_new, per
     x_al, v_al, v_map = aligner.align(x_t, m_t, x_ref, m_ref)
@@ -439,7 +461,7 @@ def _lanes_step(chn, grid_fn, x_t, m_t, x_ref, m_ref, slots, x_state, m_state, y
     CNN-input pack and one RRDBNet call on L rows, then ops.chn_fill_lanes, which writes y_comp, the new state and
     the hole percentage of lane i into slot ``slots[i]`` of y_out / x_state / m_state / per, in place."""
     grid, flags = grid_fn(chn.model_aligner, x_t, m_t, x_ref, m_ref)
-    nn_in, v_map, _, _ = ops.warp_pack_fwd(x_ref, m_ref, grid, m_t, x_t, 1 - m_t, flags)
+    nn_in, v_map, _, _ = ops.warp_pack_fwd(x_ref, m_ref, grid, m_t, x_t, 1 - m_t, flags, **_layout_kw(chn.nn))
     ops.chn_fill_lanes(chn.nn(nn_in), x_t, m_t, v_map[:, :, 0], slots, x_state, m_state, y_out, per, finalize)
 
 
